@@ -1,10 +1,13 @@
 #!/usr/bin/env python
 """Headline benchmark of the PAMRec train step (BASELINE.json: train samples/sec; gather/Adam HBM GB/s vs peak).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload NAME] [--dump-outputs DIR]
 
 One "step" = one optimisation step (forward + losses + backward + per-tensor clip + Adam) over one batch of
 synthetic MX-TakaTak-shaped input.  Prints ONE JSON line (rank 0).  Keys: see DESIGN.md "Measurement".
+--dump-outputs DIR writes what the last of the K timed steps computed (rank 0): the losses and the logits of a training step, the
+predictions of a scoring step.  The inputs are seeded, so two builds run with the same arguments can be compared array by array.
+Every timed training step starts from the seeded initial model, so the last one computes from the same state on every run.
 """
 import argparse
 import gc
@@ -285,6 +288,26 @@ def settle_sampler(clocks, dev, world, step):
         torch.cuda.synchronize()
 
 
+DUMP_ROWS = 65536            # --dump-outputs: an array with more rows than this is written as a fixed sample of its rows
+DUMP_LIMIT = 64 << 20        # bytes of all dumped arrays together
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes name -> array as <out_dir>/<name>.npy in float32 (float64 stays float64).  An array of more than DUMP_ROWS rows is
+    cut to the same DUMP_ROWS rows on every run (seeded choice, ascending order), so that two builds compare output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, a in arrays.items():
+        a = a.detach().cpu().numpy() if torch.is_tensor(a) else np.asarray(a)
+        a = a.astype(np.float64 if a.dtype == np.float64 else np.float32, copy=False)
+        if a.ndim and a.shape[0] > DUMP_ROWS:
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], DUMP_ROWS, replace=False))]
+        total += a.nbytes
+        if total > DUMP_LIMIT:
+            raise RuntimeError(f"--dump-outputs: more than {DUMP_LIMIT >> 20} MB at {name}")
+        np.save(os.path.join(out_dir, name.replace("/", ".") + ".npy"), np.ascontiguousarray(a))
+
+
 def run_ours(args, w, rank, world):
     from pamrec_b200 import synth
     pk = peaks()
@@ -304,6 +327,15 @@ def run_ours(args, w, rank, world):
     resident = [eng.upload(f) for f in feeds]
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)          # > 126 MB L2
     K, W = args.steps, args.warmup
+    # Every timed step starts from the seeded initial model: variables, Adam slots, BN statistics and the device's Adam step, put
+    # back before each step's L2 flush.  A step sums with float atomics, and Adam turns that rounding into +-learning_rate moves of
+    # some variables (tests/test_gpu_quickstart.py: _worst_difference), so the state after a trajectory of steps differs from run to
+    # run; steps from one state compute the same from the same inputs on every run, whatever the warm-up took.
+    state = [eng.pool[k] for k in eng.pool if k != "workspace"] + [eng.ws("adam.step")]
+    initial = [t.clone() for t in state]
+
+    def restore():
+        torch._foreach_copy_(state, initial)
 
     def barrier():
         if world > 1:
@@ -329,14 +361,18 @@ def run_ours(args, w, rank, world):
     barrier()
     t_wall0 = time.perf_counter()
     for i in range(K):
+        restore()
         flush.fill_(i & 0xFF)
         a, b = evs[i]
         a.record()
-        eng.train_step(resident[i % N_POOL])
+        losses = eng.train_step(resident[i % N_POOL])
         b.record()
     barrier()
     t_wall = time.perf_counter() - t_wall0
     gc.enable()
+    # what the last timed step computed from its inputs: the losses and the logits of the heads.  Not the variables it leaves: where a
+    # gradient is zero but for rounding (a bias in front of a batch norm), Adam's first step turns that rounding into the value.
+    outputs = {"losses": losses.clone(), "logits": eng.ws("logits", B).clone()} if args.dump_outputs else None
     step_ms = [a.elapsed_time(b) for a, b in evs]
     step_sorted = sorted(step_ms)
     launches = eng.launches()
@@ -376,6 +412,7 @@ def run_ours(args, w, rank, world):
     # ---- per-launcher device time over a second pass of the same K steps (CUDA events around every launch)
     eng.profile(True)
     for i in range(K):
+        restore()
         flush.fill_(i & 0xFF)
         eng.train_step(resident[i % N_POOL])
     tab = eng.profile_table()
@@ -399,6 +436,8 @@ def run_ours(args, w, rank, world):
                            "tables replicated (small vocabularies): gradient tables all-reduced with the dense gradients") +
                        ", sync-BN through NVLink peer mailboxes inside the persistent head kernels"),
                    "l2": "flushed between timed steps (256 MiB write); per-step working set also exceeds L2",
+                   "state": "every timed step starts from the seeded initial model (variables, Adam slots and step, BN statistics), "
+                            "restored before its L2 flush",
                    "warmup_steps_run": max(W, 2 * N_POOL),
                    "launch": "the step is replayed from a CUDA graph (one per resident / staged batch, captured during warm-up)" if eng.graph and world == 1 else "kernel by kernel",
                    "batch_note": "BASELINE batch 1024 rounded to 1025: batches must be multiples of 5",
@@ -409,7 +448,7 @@ def run_ours(args, w, rank, world):
         "kernels": kernels, "wall_s_timed_region": t_wall,
         "ms_per_step_median": step_sorted[len(step_sorted) // 2], "ms_per_step_max": step_sorted[-1],
     }
-    return out, model
+    return out, model, outputs
 
 
 def rooflines(w, tab, K, ms_per_step, pk, clk, workload):
@@ -513,9 +552,10 @@ def run_score(args, w, rank, world):
         flush.fill_(i & 0xFF)
         a, b = evs[i]
         a.record()
-        eng.forward(resident[i % N_POOL], training=False)
+        pred = eng.forward(resident[i % N_POOL], training=False)
         b.record()
     barrier()
+    outputs = {"pred": pred} if args.dump_outputs else None
     launches = eng.launches()
     total_ms = sum(a.elapsed_time(b) for a, b in evs)
     if world > 1:
@@ -568,7 +608,7 @@ def run_score(args, w, rank, world):
         "e2e": e2e, "gpu_launches": int(launches) * K, "gpu_launches_per_step": int(launches), "clocks": clk, "roofline": roof,
         "roofline_step": roof_step, "kernels": kernels,
     }
-    return out, model
+    return out, model, outputs
 
 
 def sample_rows(w):
@@ -617,8 +657,12 @@ def run_reference(args, w, rank):
         step(feeds[i % 4])
     t0 = time.perf_counter()
     for i in range(args.steps):
-        step(feeds[i % 4])
+        last = step(feeds[i % 4])
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"pred": last.t["pred"].reshape(-1)} if score else
+                     {"losses": np.array([last["losses"][k] for k in ("loss", "data_loss", "regular_loss", "auxiliary_data_loss",
+                                                                      "order_loss")])})
     v = args.steps * rows / dt
     whole = rows == w["B"]
     cb = {"value": v, "unit": "samples/s", "cores": torch.get_num_threads(), "kind": "port",
@@ -643,7 +687,10 @@ def main():
     ap.add_argument("--impl", default="pamrec_b200", choices=["pamrec_b200", "reference"])
     ap.add_argument("--workload", default="takatak_b1025_t50", choices=list(WORKLOADS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
     w = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", 0))
@@ -666,8 +713,10 @@ def main():
         local = int(os.environ.get("LOCAL_RANK", rank))
         torch.cuda.set_device(local)
         torch.distributed.init_process_group("nccl", device_id=torch.device("cuda", local))
-    out, model = (run_score if w.get("kind") == "score" else run_ours)(args, w, rank, world)
+    out, model, outputs = (run_score if w.get("kind") == "score" else run_ours)(args, w, rank, world)
     if rank == 0:
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         if world == 1 and not args.no_cpu_baseline:
             out["cpu_baseline"] = cpu_baseline(w)
         print(json.dumps(out), file=real_stdout, flush=True)

@@ -9,8 +9,8 @@ Runs the reference's own ``io/sequential_iterator.py`` and the metric functions 
                         batches in full
   metrics.json          cal_metric / cal_weighted_metric outputs on seeded random labels / scores
 
-The reference cannot travel to the GPU box, so the fixtures are committed; tests/test_iterator.py also
-re-runs this live comparison whenever /root/reference is present.
+The reference is not part of this repository, so the fixtures are committed, and
+tests/test_iterator_and_metrics.py compares with them.
 
     python -m oracle.gen_golden            # regenerate tests/golden/*
 """

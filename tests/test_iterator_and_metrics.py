@@ -1,6 +1,6 @@
 """Host logic pinned against the reference: batches of pamrec_b200.SequentialIterator are BIT-EXACT with the
 reference's SequentialIterator (golden fixtures made by oracle/gen_golden.py from the unmodified reference run
-under a stub tensorflow; re-checked live whenever /root/reference is mounted), bucket ids and metrics likewise."""
+under a stub tensorflow), bucket ids and metrics likewise."""
 import json
 import os
 import tempfile
@@ -13,7 +13,6 @@ from pamrec_b200 import deeprec_utils as DU
 from pamrec_b200 import sequential_iterator as IT
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-HAVE_REF = os.path.isdir(os.path.join(G.REF, "reco_utils"))
 
 
 def _ours(case, data_dir):
@@ -47,21 +46,22 @@ def test_iterator_matches_golden(case):
         assert (a == a[:, :1]).all(), k
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference tree not mounted")
 @pytest.mark.parametrize("case", list(G.CASES))
 def test_iterator_matches_reference_live(case):
-    _, RIT = G.reference_modules()
+    """A run of one epoch, then the valid pass, against the reference's batches as oracle/gen_golden.py recorded them (a digest
+    of the name, dtype, shape and bytes of every array of every batch): the first epoch of the recorded two-epoch run is this
+    run, and the valid pass does not depend on how many epochs came before it."""
+    z = np.load(os.path.join(GOLDEN, f"iterator_{case}.npz"))
     with tempfile.TemporaryDirectory() as tmp:
         data_dir = G.synth_case(case, tmp)
         hp = G.hparams_for(case, data_dir)
-        ref = G.run_iterator(lambda: RIT.SequentialIterator(hp, G._Graph()), data_dir, epochs=1)
         got = G.run_iterator(lambda: IT.SequentialIterator(hp, None), data_dir, epochs=1)
+    first_epoch = {"wechat_small": 134, "takatak_small": 370}[case]         # of the 269 / 739 recorded train batches
+    ref = {"train": z["train_digests"].tolist()[:first_epoch], "valid": z["valid_digests"].tolist()}
     for split in ("train", "valid"):
-        assert len(ref[split]) == len(got[split])
-        for i, (a, b) in enumerate(zip(ref[split], got[split])):
-            for name in G.FEED_NAMES:
-                assert a[name].dtype == b[name].dtype, (split, i, name)
-                assert np.array_equal(a[name], b[name], equal_nan=True), (split, i, name)
+        assert len(got[split]) == len(ref[split]) > 0, split
+        for i, (b, want) in enumerate(zip(got[split], ref[split])):
+            assert G.batch_digest(b) == want, (split, i)
 
 
 def test_lisan_known_answers():

@@ -2,10 +2,10 @@
 against this repository - its imports resolve through compat/, its absl flags and prepare_hparams kwargs are accepted, and
 fit_step -> tf.train.latest_checkpoint -> load_model -> run_weighted_eval -> predict complete on synthetic wechat-shaped files.
 
-The driver file itself lives only under /root/reference (it is never copied into this repository), and /root/reference does
-not exist on the GPU box, so this test runs where the reference is mounted: on a machine with a GPU the real engine runs the
-device steps, on the CPU-only build container `StubEngine` (tests/test_host_loops.py) stands in for them - everything
-between the driver and the C ABI (hparams, iterator, host loops, checkpoints, metrics) is the product code either way.
+The driver file belongs to the reference project and is not part of this repository, so this test runs only where
+PAMREC_REFERENCE names a checkout of it: on a machine with a GPU the real engine runs the device steps, on one without
+`StubEngine` (tests/test_host_loops.py) stands in for them - everything between the driver and the C ABI (hparams, iterator,
+host loops, checkpoints, metrics) is the product code either way.
 tests/test_gpu_quickstart.py runs the same flow on the GPU through compat/'s own copy of the flag set."""
 import os
 import runpy
@@ -16,9 +16,10 @@ import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_DRIVER = "/root/reference/example/00_quick_start/sequential.py"
+REF = os.environ.get("PAMREC_REFERENCE")
+REF_DRIVER = os.path.join(REF, "example", "00_quick_start", "sequential.py") if REF else ""
 
-pytestmark = pytest.mark.skipif(not os.path.exists(REF_DRIVER), reason="reference tree not mounted")
+pytestmark = pytest.mark.skipif(not os.path.isfile(REF_DRIVER), reason="PAMREC_REFERENCE does not name a reference checkout")
 
 
 @pytest.mark.parametrize("model_flag", ["PAMREC", "MMOE_ORIGINAL", "PLE", "SHAREBOTTOM", "SASREC"])
