@@ -31,6 +31,7 @@
 extern "C" {
 #endif
 
+/* PAMRec's embedding widths (also what a sibling model runs with PamrecConfig.item_dim / cate_dim / user_dim = 0) */
 #define PAMREC_ITEM_DIM 16
 #define PAMREC_CATE_DIM 4
 #define PAMREC_USER_DIM 20
@@ -96,6 +97,10 @@ typedef struct PamrecConfig {
   int32_t loss_kind;
   int32_t softmax_group;             /* used by PAMREC_LOSS_SOFTMAX only; 0 is read as 1                */
   int32_t model_kind;                /* PAMREC_MODEL_*                                                  */
+  /* embedding widths (hparams.item_embedding_dim / cate_embedding_dim / user_embedding_dim); 0 = 16 / 4 / 20 each.  PAMREC_MODEL_PAMREC
+   * runs 16 / 4 / 20 only.  The sibling models run (item, cate) = (16, 4) or (32, 8) - the reference's config/ple.yaml,
+   * sharebottom.yaml and sasrec.yaml use 32 / 8 - with user = 16, 20 or 40; any other set is refused (pamrec_create returns -10). */
+  int32_t item_dim, cate_dim, user_dim;
 } PamrecConfig;
 
 /* One batch, device pointers (layouts of io/sequential_iterator.py:1111-1135). */
@@ -125,10 +130,10 @@ typedef struct PamrecBuffers {
   float* dense_param; float* dense_grad; float* dense_m; float* dense_v; /* [dense_numel] each      */
   float* bn_moving;                                                      /* [bn_numel] mean|var sets */
   /* tables: [rows,width] with rows = vocabulary size (PAMREC_TABLES_LOCAL / _REPLICATED) or pamrec_shard_rows (SHARDED) */
-  float* item_w; float* item_m; float* item_v;                           /* [rows(n_items),16]      */
-  float* cate_w; float* cate_m; float* cate_v;                           /* [rows(n_cates),4]       */
-  float* ulong_w; float* ulong_m; float* ulong_v;                        /* [rows(n_users),20]      */
-  float* ushort_w; float* ushort_m; float* ushort_v;                     /* [rows(n_users),20]      */
+  float* item_w; float* item_m; float* item_v;                           /* [rows(n_items),item_dim] */
+  float* cate_w; float* cate_m; float* cate_v;                           /* [rows(n_cates),cate_dim] */
+  float* ulong_w; float* ulong_m; float* ulong_v;                        /* [rows(n_users),user_dim] */
+  float* ushort_w; float* ushort_m; float* ushort_v;                     /* [rows(n_users),user_dim] */
   void* workspace; size_t workspace_bytes;                               /* >= pamrec_workspace_bytes */
 } PamrecBuffers;
 

@@ -29,6 +29,7 @@ class PamrecConfig(C.Structure):
         ("fuzhu_weight", C.c_float), ("order_weight", C.c_float), ("sparse_adam_mode", C.c_int32),
         ("world_size", C.c_int32), ("rank", C.c_int32), ("table_mode", C.c_int32),
         ("loss_kind", C.c_int32), ("softmax_group", C.c_int32), ("model_kind", C.c_int32),
+        ("item_dim", C.c_int32), ("cate_dim", C.c_int32), ("user_dim", C.c_int32),
     ]
 
 

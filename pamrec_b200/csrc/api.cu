@@ -177,9 +177,14 @@ int pamrec_create(const PamrecConfig* cfg, PamrecHandle* out) {
   if (cfg->model_kind < PAMREC_MODEL_PAMREC || cfg->model_kind > PAMREC_MODEL_SASREC) return -9;
   if (cfg->model_kind != PAMREC_MODEL_PAMREC && (world != 1 || cfg->table_mode != PAMREC_TABLES_LOCAL || cfg->loss_kind != PAMREC_LOSS_XENT))
     return -9;                                                               // sibling models: one GPU, whole tables, cross entropy
+  const int di = cfg->item_dim ? cfg->item_dim : PAMREC_ITEM_DIM, dc = cfg->cate_dim ? cfg->cate_dim : PAMREC_CATE_DIM;
+  const int du = cfg->user_dim ? cfg->user_dim : PAMREC_USER_DIM;
+  if (!((di == 16 && dc == 4) || (di == 32 && dc == 8)) || !(du == 16 || du == 20 || du == 40)) return -10;
+  if (cfg->model_kind == PAMREC_MODEL_PAMREC && (di != PAMREC_ITEM_DIM || dc != PAMREC_CATE_DIM || du != PAMREC_USER_DIM)) return -10;
   PamrecHandle h = new PamrecHandle_();
   h->cfg = *cfg;
   h->cfg.world_size = world;
+  h->cfg.item_dim = di; h->cfg.cate_dim = dc; h->cfg.user_dim = du;
   if (h->cfg.softmax_group < 1) h->cfg.softmax_group = 1;
   h->L.build(h->cfg);
   const int n_seg = (int)h->L.dense.size();
@@ -313,6 +318,8 @@ int pamrec_bind(PamrecHandle h, const PamrecBuffers* bufs, void* stream) {
     }
   }
   if (init_encoder_kernels(h->cfg.max_seq_len)) return check_cuda(h, "shared-memory opt-in of the encoder kernels");
+  if (h->cfg.model_kind == PAMREC_MODEL_SASREC && init_sas_kernels(h->cfg.max_seq_len))
+    return check_cuda(h, "shared-memory opt-in of the SASRec attention kernels");
   {
     int dev = 0;
     cudaGetDevice(&dev);

@@ -131,7 +131,9 @@ __device__ __forceinline__ void stage_rows_T2(float* __restrict__ dst, const flo
   }
 }
 
-// shared memory: As | Bs | red (kDenseFwdSmem bytes)
+// shared memory: As | Bs | red (kDenseFwdSmem bytes).  A contraction longer than kKMax (the attention MLP of the sibling models at
+// 32 / 8 widths: K = 160) runs in chunks of kKMax: As / Bs hold one chunk and the products accumulate in k order, so a layer with
+// K <= kKMax is one chunk with the weight tile staged once per CTA.
 constexpr int kDenseFwdSmem = 2 * kKMax * kTM * 4 + 2 * (kHT / 8) * kTN * 8;
 __device__ __forceinline__ void dense_fwd_item(const DenseP& p, int M, double* out_sums, int tiles_m, int bx, int gx, int by, unsigned char* smem) {
   float* As = reinterpret_cast<float*>(smem);
@@ -143,22 +145,24 @@ __device__ __forceinline__ void dense_fwd_item(const DenseP& p, int M, double* o
   const int nc = min(kTN, p.N - c0);
   const int xo = p.x_off[g], zo = p.z_off[g] + c0;
   const float* W = p.W + (int64_t)g * p.w_stride;
-  // weight tile Bs[k][n] = W[k][c0+n]
-  {
+  const bool one_chunk = p.K <= kKMax;
+  // weight tile Bs[k][n] = W[k0+k][c0+n], k < kc
+  auto stage_w = [&](int k0, int kc) {
     const bool vec = ((p.N | c0) & 3) == 0 && (nc & 3) == 0 && aligned16(W);
     if (vec) {
       const int n4 = nc >> 2;
-      for (int i = tid; i < p.K * (kTN / 4); i += kHT) {
+      for (int i = tid; i < kc * (kTN / 4); i += kHT) {
         const int k = i / (kTN / 4), q = i % (kTN / 4);
-        st4(Bs + k * kTN + 4 * q, q < n4 ? ld4(W + (int64_t)k * p.N + c0 + 4 * q) : f4_zero());
+        st4(Bs + k * kTN + 4 * q, q < n4 ? ld4(W + (int64_t)(k0 + k) * p.N + c0 + 4 * q) : f4_zero());
       }
     } else {
-      for (int i = tid; i < p.K * kTN; i += kHT) {
+      for (int i = tid; i < kc * kTN; i += kHT) {
         const int k = i / kTN, n = i % kTN;
-        Bs[i] = n < nc ? W[(int64_t)k * p.N + c0 + n] : 0.f;
+        Bs[i] = n < nc ? W[(int64_t)(k0 + k) * p.N + c0 + n] : 0.f;
       }
     }
-  }
+  };
+  if (one_chunk) stage_w(0, p.K);
   float bias[4];
 #pragma unroll
   for (int j = 0; j < 4; ++j) bias[j] = (4 * tx + j < nc) ? p.bias[(int64_t)g * p.b_stride + c0 + 4 * tx + j] : 0.f;
@@ -167,21 +171,26 @@ __device__ __forceinline__ void dense_fwd_item(const DenseP& p, int M, double* o
   for (int tm = bx; tm < tiles_m; tm += gx) {
     const int m0 = tm * kTM;
     const int rows = min(kTM, M - m0);
-    __syncthreads();                                  // previous tile's As fully consumed (and Bs written, first pass)
-    const float* X = p.X + (int64_t)m0 * p.ldx + xo;
-    if (p.in_stat) {
-      const float* st = p.in_stat; const float* ga = p.in_gamma; const float* be = p.in_beta;
-      stage_rows_T(As, X, p.ldx, rows, p.K, tid, [=](float v, int k) { return bn_relu(v, st, ga, be, xo + k); });
-    } else {
-      stage_rows_T(As, X, p.ldx, rows, p.K, tid, [](float v, int) { return v; });
-    }
-    __syncthreads();
     float acc[2][4];
 #pragma unroll
     for (int i = 0; i < 2; ++i)
 #pragma unroll
       for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
-    tile_mma(As, Bs, p.K, ty, tx, acc);
+    for (int k0 = 0; k0 < p.K; k0 += kKMax) {
+      const int kc = min(kKMax, p.K - k0);
+      __syncthreads();                                // previous chunk's / tile's As (and Bs) fully consumed; Bs written (one chunk)
+      if (!one_chunk) stage_w(k0, kc);
+      const float* X = p.X + (int64_t)m0 * p.ldx + xo + k0;
+      if (p.in_stat) {
+        const float* st = p.in_stat; const float* ga = p.in_gamma; const float* be = p.in_beta;
+        const int xk = xo + k0;
+        stage_rows_T(As, X, p.ldx, rows, kc, tid, [=](float v, int k) { return bn_relu(v, st, ga, be, xk + k); });
+      } else {
+        stage_rows_T(As, X, p.ldx, rows, kc, tid, [](float v, int) { return v; });
+      }
+      __syncthreads();
+      tile_mma(As, Bs, kc, ty, tx, acc);
+    }
     // the bias joins the finished product (as tf.matmul + bias does): ONE rounding at the bias's magnitude instead of K of them.
     // It matters where a batch norm follows: a bias of 0.1 in front of a signal of std 5e-4 (the attention MLPs of the sibling
     // models at init) puts every partial sum on a 1.5e-8 grid, and the normalisation then amplifies that by 1 / sqrt(eps) = 100.

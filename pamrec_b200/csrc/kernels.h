@@ -90,7 +90,7 @@ void launch_sigmoid_col0(const float* logits, float* pred, int B, cudaStream_t s
 
 // ---- kernels_optim.cu
 struct SparseTable {
-  int width;                  // floats per row (16 / 4 / 20)
+  int width;                  // floats per row: 4, 8, 16, 20, 32 or 40 (the sparse kernels refuse any other width)
   int64_t n_rows;
   float* w; float* m; float* v;
   int* keys; int* idx; int* skeys; int* sidx; int* uidx; int* ukeys; int* slot;
@@ -111,12 +111,13 @@ int launch_sparse_reduce(const SparseTable& t, const int* hist_ids, const int* t
 int launch_sparse_plan(const SparseTable& t, const int* hist_ids, const int* tgt_ids, int64_t n_hist, int64_t n_tgt,
                        int world, int64_t rps, int64_t key_range, bool fill_slot, void* cub_temp, size_t cub_bytes,
                        cudaStream_t st);
-void launch_sparse_segreduce(const SparseTable& t, int64_t n, int64_t n_hist, const float* hist_grad, int hist_ld, int hist_col,
-                             const float* tgt_grad, int tgt_ld, int tgt_col, double* normsq, cudaStream_t st);
+// launch_sparse_segreduce / _l2norm / _adam return -1 (nothing launched) for a table width they have no instantiation for
+int launch_sparse_segreduce(const SparseTable& t, int64_t n, int64_t n_hist, const float* hist_grad, int hist_ld, int hist_col,
+                            const float* tgt_grad, int tgt_ld, int tgt_col, double* normsq, cudaStream_t st);
 void launch_slot_reset(const SparseTable& t, int64_t n_keys, cudaStream_t st);
 // L2 rows of the unique ids: adds their squared norm to normsq and 0.5*l2*|w|^2 to reg_acc
-void launch_sparse_l2norm(const SparseTable& t, int64_t n_keys, float l2, double* reg_acc, cudaStream_t st);
-void launch_sparse_adam(const SparseTable& t, int64_t n_keys, int mode, float l2, float lr_t, float b1, float b2, float eps,
+int launch_sparse_l2norm(const SparseTable& t, int64_t n_keys, float l2, double* reg_acc, cudaStream_t st);
+int launch_sparse_adam(const SparseTable& t, int64_t n_keys, int mode, float l2, float lr_t, float b1, float b2, float eps,
                         float clip, int is_clip, cudaStream_t st);
 void launch_dense_norm(const float* P, const float* G, const int* seg_tab, int n_seg, float layer_l2, double* seg_normsq,
                        const double* pos_normsq, double* reg_acc, cudaStream_t st);
@@ -161,45 +162,46 @@ void launch_sp2_lazy_finish(const Sp2& s, const AdamP& a, cudaStream_t st);
 void launch_sp2_adam_sweep(const Sp2& s, const AdamP& a, int lazy, cudaStream_t st);
 void launch_sp2_rep_l2(const Sp2& s, cudaStream_t st);
 
-// ---- kernels_sibling.cu (MMoE_original / PLE / ShareBottom: DIN attention pooling, mixing, loss)
+// ---- kernels_sibling.cu (MMoE_original / PLE / ShareBottom: DIN attention pooling, mixing, loss); item_dim = 16 or 32 (cate = item / 4)
 void launch_sib_gather(const int* sat_item, const int* sat_cate, const int* hist_item, const int* hist_cate, const int* items,
                        const int* cates, const float* item_w, const float* cate_w, float* h, float* tgt, int* ids_item,
-                       int* ids_cate, int B, int T, cudaStream_t st);
+                       int* ids_cate, int B, int T, int item_dim, cudaStream_t st);
 void launch_sib_has0(const int* hist_item, const int* hist_cate, const int* items, const int* cates, int B, int T, int* has0,
                      cudaStream_t st);
-void launch_sib_feat_fwd(float* feat, const float* tgt, int B, int T, cudaStream_t st);
-void launch_sib_feat_bwd(const float* d_feat, const float* feat, const float* tgt, float* d_att, float* dq, int B, int T,
+void launch_sib_feat_fwd(float* feat, const float* tgt, int B, int T, int item_dim, cudaStream_t st);
+void launch_sib_feat_bwd(const float* d_feat, const float* feat, const float* tgt, float* d_att, float* dq, int B, int T, int item_dim,
                          cudaStream_t st);
 void launch_sib_pool_fwd(const float* h, const float* score, const int* sat_mask, const int* mask, const float* tgt, float* aw,
-                         float* x, int B, int T, cudaStream_t st);
+                         float* x, int B, int T, int item_dim, cudaStream_t st);
 void launch_sib_pool_bwd(const float* h, const float* aw, const int* sat_mask, const int* mask, const float* d_x, float* d_score,
-                         float* dh, int B, int T, cudaStream_t st);
-void launch_sib_tgt_total(const float* d_tgt, const float* d_x, const float* dq, float* out, int B, cudaStream_t st);
+                         float* dh, int B, int T, int item_dim, cudaStream_t st);
+void launch_sib_tgt_total(const float* d_tgt, const float* d_x, const float* dq, float* out, int B, int item_dim, cudaStream_t st);
 void launch_sib_mix_fwd(const float* ZE1, const float* ZG1, const BnSet& e1, const BnSet& g1, const float* tgt, float* U, int n_expert,
-                        const int sel[2][5], int B, cudaStream_t st);
+                        const int sel[2][5], int B, int item_dim, cudaStream_t st);
 void launch_sib_mix_bwd(const float* ZE1, const float* ZG1, const BnSet& e1, const BnSet& g1, const float* dU, float* dE1, float* dG1,
-                        float* dTgt, int n_expert, const int sel[2][5], int B, cudaStream_t st);
+                        float* dTgt, int n_expert, const int sel[2][5], int B, int item_dim, cudaStream_t st);
 // heads = 2: logits [B,2] (satisfied label, play label x aux_w); heads = 1: logits [B,1], data loss only (SASRec)
 void launch_sib_loss(const float* logits, const float* y_sat, const float* y_play, float* d_logits, double* loss_acc, int B, float aux_w,
                      int heads, cudaStream_t st);
 void launch_sib_pred(const float* logits, float* pred, int B, int heads, cudaStream_t st);
 
-// ---- kernels_sasrec.cu (SASRecModel: two 20-wide self-attention blocks with dense Q / K / V)
-void launch_sas_embed(const float* h, const float* pos, float* x0, int B, int T, cudaStream_t st);
+// ---- kernels_sasrec.cu (SASRecModel: two S-wide self-attention blocks with dense Q / K / V; S = item + cate width, 20 or 40)
+int init_sas_kernels(int max_T);       // opt-in to > 48 KB dynamic shared memory of the S = 40 attention kernels (called by pamrec_bind)
+void launch_sas_embed(const float* h, const float* pos, float* x0, int B, int T, int S, cudaStream_t st);
 void launch_sas_proj_fwd(const float* X, const float* W, const float* bias, const float* ln_beta, const float* ln_gamma, float* XQ,
-                         float* QKV, int64_t N, cudaStream_t st);
+                         float* QKV, int64_t N, int S, cudaStream_t st);
 void launch_sas_proj_bwd(const float* XQ, const float* dQKV, const float* dY, const float* W, const float* ln_gamma, float* dX,
-                         float* g_gamma, float* g_beta, int64_t N, cudaStream_t st);
-void launch_sas_attn_fwd(const float* QKV, const float* XQ, const int* mask, float* Y, float* ML, int B, int T, cudaStream_t st);
+                         float* g_gamma, float* g_beta, int64_t N, int S, cudaStream_t st);
+void launch_sas_attn_fwd(const float* QKV, const float* XQ, const int* mask, float* Y, float* ML, int B, int T, int S, cudaStream_t st);
 void launch_sas_attn_bwd(const float* QKV, const float* XQ, const float* Y, const float* dY, const float* ML, const int* mask, float* dQKV,
-                         float* Dq, int B, int T, cudaStream_t st);
+                         float* Dq, int B, int T, int S, cudaStream_t st);
 void launch_sas_ffn_fwd(const float* Y, const float* W1, const float* b1, const float* W2, const float* b2, const float* ln_beta,
-                        const float* ln_gamma, float* F, float* HPRE, float* OUT, int64_t N, cudaStream_t st);
+                        const float* ln_gamma, float* F, float* HPRE, float* OUT, int64_t N, int S, cudaStream_t st);
 void launch_sas_ffn_bwd(const float* Y, const float* HPRE, const float* dOUT, const float* W1, const float* W2, const float* ln_gamma,
-                        float* HID, float* DHPRE, float* dY, float* g_gamma, float* g_beta, int64_t N, cudaStream_t st);
-void launch_sas_final_fwd(const float* SEQ, const int* mask, const float* tgt, float* U, int B, int T, cudaStream_t st);
-void launch_sas_final_bwd(const float* dU, const int* mask, float* dSEQ, float* dTgt, int B, int T, cudaStream_t st);
-void launch_sas_pos_bwd(const float* dX0, float* dPos, double* normsq, int B, int T, cudaStream_t st);
+                        float* HID, float* DHPRE, float* dY, float* g_gamma, float* g_beta, int64_t N, int S, cudaStream_t st);
+void launch_sas_final_fwd(const float* SEQ, const int* mask, const float* tgt, float* U, int B, int T, int S, cudaStream_t st);
+void launch_sas_final_bwd(const float* dU, const int* mask, float* dSEQ, float* dTgt, int B, int T, int S, cudaStream_t st);
+void launch_sas_pos_bwd(const float* dX0, float* dPos, double* normsq, int B, int T, int S, cudaStream_t st);
 
 // ---- kernels_p2p.cu (small all-reduces through NVLink peer mailboxes)
 constexpr int kP2PMaxDoubles = 2048;     // payload capacity of one mailbox slot (expert + gate layer-0 sums: 1256)

@@ -205,22 +205,28 @@ int launch_sparse_plan(const SparseTable& t, const int* hist_ids, const int* tgt
 }
 
 // duplicate rows summed into accum[unique index]; normsq += sum of squares of every (un-deduplicated) row
-void launch_sparse_segreduce(const SparseTable& t, int64_t n, int64_t n_hist, const float* hist_grad, int hist_ld, int hist_col,
-                             const float* tgt_grad, int tgt_ld, int tgt_col, double* normsq, cudaStream_t st) {
+int launch_sparse_segreduce(const SparseTable& t, int64_t n, int64_t n_hist, const float* hist_grad, int hist_ld, int hist_col,
+                            const float* tgt_grad, int tgt_ld, int tgt_col, double* normsq, cudaStream_t st) {
   PAMREC_PROF("sparse_segreduce", 1, st);
-  if (n == 0) return;
+  if (t.width != 4 && t.width != 8 && t.width != 16 && t.width != 32) return -1;
+  if (n == 0) return 0;
   cudaMemsetAsync(t.accum, 0, (size_t)n * t.width * sizeof(float), st);
   // blocks of 32 positions per warp walk: 1 while the grid would not fill the GPU otherwise, up to 16 for large batches
   int64_t iters = n / (148 * 8 * 8 * 32);
   iters = iters < 1 ? 1 : (iters > 16 ? 16 : iters);
   const int64_t per_cta = 8 * 32 * iters;                        // 8 warps per CTA
   const unsigned gw = (unsigned)((n + per_cta - 1) / per_cta);
-  if (t.width == 16)
-    k_seg_reduce<16><<<gw, 256, 0, st>>>(t.skeys, t.sidx, t.uidx, n, n_hist, hist_grad, hist_ld, hist_col, tgt_grad, tgt_ld,
-                                         tgt_col, t.accum, normsq, (int)iters);
-  else
-    k_seg_reduce<4><<<gw, 256, 0, st>>>(t.skeys, t.sidx, t.uidx, n, n_hist, hist_grad, hist_ld, hist_col, tgt_grad, tgt_ld,
-                                        tgt_col, t.accum, normsq, (int)iters);
+#define PAMREC_SEG_REDUCE(W)                                                                                                   \
+  k_seg_reduce<W><<<gw, 256, 0, st>>>(t.skeys, t.sidx, t.uidx, n, n_hist, hist_grad, hist_ld, hist_col, tgt_grad, tgt_ld, tgt_col, \
+                                      t.accum, normsq, (int)iters)
+  switch (t.width) {
+    case 16: PAMREC_SEG_REDUCE(16); break;
+    case 4: PAMREC_SEG_REDUCE(4); break;
+    case 32: PAMREC_SEG_REDUCE(32); break;
+    default: PAMREC_SEG_REDUCE(8); break;
+  }
+#undef PAMREC_SEG_REDUCE
+  return 0;
 }
 
 int launch_sparse_reduce(const SparseTable& t, const int* hist_ids, const int* tgt_ids, int64_t n_hist, int64_t n_tgt,
@@ -228,7 +234,7 @@ int launch_sparse_reduce(const SparseTable& t, const int* hist_ids, const int* t
                          void* cub_temp, size_t cub_bytes, cudaStream_t st) {
   if (launch_sparse_plan(t, hist_ids, tgt_ids, n_hist, n_tgt, 1, 0, t.n_rows, true, cub_temp, cub_bytes, st)) return -1;
   if (t.accum != nullptr && hist_grad != nullptr)
-    launch_sparse_segreduce(t, n_hist + n_tgt, n_hist, hist_grad, hist_ld, hist_col, tgt_grad, tgt_ld, tgt_col, t.normsq, st);
+    return launch_sparse_segreduce(t, n_hist + n_tgt, n_hist, hist_grad, hist_ld, hist_col, tgt_grad, tgt_ld, tgt_col, t.normsq, st);
   return 0;
 }
 
@@ -260,13 +266,25 @@ k_sparse_l2norm(const int* __restrict__ ukeys, const int* __restrict__ nuniq, co
     }
   }
 }
-void launch_sparse_l2norm(const SparseTable& t, int64_t n_keys, float l2, double* reg_acc, cudaStream_t st) { PAMREC_PROF("sparse_l2norm", 1, st);
+int launch_sparse_l2norm(const SparseTable& t, int64_t n_keys, float l2, double* reg_acc, cudaStream_t st) { PAMREC_PROF("sparse_l2norm", 1, st);
   int64_t total = n_keys * (t.width / 4);
-  if (total == 0) return;
   unsigned g = (unsigned)((total + 255) / 256);
-  if (t.width == 16) k_sparse_l2norm<16><<<g, 256, 0, st>>>(t.ukeys, t.nuniq, t.w, l2, t.normsq, reg_acc, t.l2_has0);
-  else if (t.width == 4) k_sparse_l2norm<4><<<g, 256, 0, st>>>(t.ukeys, t.nuniq, t.w, l2, t.normsq, reg_acc, t.l2_has0);
-  else k_sparse_l2norm<20><<<g, 256, 0, st>>>(t.ukeys, t.nuniq, t.w, l2, t.normsq, reg_acc, t.l2_has0);
+#define PAMREC_L2NORM(W) k_sparse_l2norm<W><<<g, 256, 0, st>>>(t.ukeys, t.nuniq, t.w, l2, t.normsq, reg_acc, t.l2_has0)
+  switch (t.width) {
+    case 4: case 8: case 16: case 20: case 32: case 40: break;
+    default: return -1;
+  }
+  if (total == 0) return 0;
+  switch (t.width) {
+    case 16: PAMREC_L2NORM(16); break;
+    case 4: PAMREC_L2NORM(4); break;
+    case 20: PAMREC_L2NORM(20); break;
+    case 32: PAMREC_L2NORM(32); break;
+    case 8: PAMREC_L2NORM(8); break;
+    default: PAMREC_L2NORM(40); break;
+  }
+#undef PAMREC_L2NORM
+  return 0;
 }
 
 __device__ __forceinline__ void adam_row4(float4& w, float4& m, float4& v, const float4& g, float lr, float b1, float b2,
@@ -352,11 +370,18 @@ static void sparse_adam_w(const SparseTable& t, int64_t n_keys, int mode, float 
                                                                         lr, b1, b2, eps, clip, is_clip, t.l2_has0);
   }
 }
-void launch_sparse_adam(const SparseTable& t, int64_t n_keys, int mode, float l2, float lr_t, float b1, float b2, float eps,
-                        float clip, int is_clip, cudaStream_t st) { PAMREC_PROF("sparse_adam", 1, st);
-  if (t.width == 16) sparse_adam_w<16>(t, n_keys, mode, l2, lr_t, b1, b2, eps, clip, is_clip, st);
-  else if (t.width == 4) sparse_adam_w<4>(t, n_keys, mode, l2, lr_t, b1, b2, eps, clip, is_clip, st);
-  else sparse_adam_w<20>(t, n_keys, mode, l2, lr_t, b1, b2, eps, clip, is_clip, st);
+int launch_sparse_adam(const SparseTable& t, int64_t n_keys, int mode, float l2, float lr_t, float b1, float b2, float eps,
+                       float clip, int is_clip, cudaStream_t st) { PAMREC_PROF("sparse_adam", 1, st);
+  switch (t.width) {
+    case 16: sparse_adam_w<16>(t, n_keys, mode, l2, lr_t, b1, b2, eps, clip, is_clip, st); break;
+    case 4: sparse_adam_w<4>(t, n_keys, mode, l2, lr_t, b1, b2, eps, clip, is_clip, st); break;
+    case 20: sparse_adam_w<20>(t, n_keys, mode, l2, lr_t, b1, b2, eps, clip, is_clip, st); break;
+    case 32: sparse_adam_w<32>(t, n_keys, mode, l2, lr_t, b1, b2, eps, clip, is_clip, st); break;
+    case 8: sparse_adam_w<8>(t, n_keys, mode, l2, lr_t, b1, b2, eps, clip, is_clip, st); break;
+    case 40: sparse_adam_w<40>(t, n_keys, mode, l2, lr_t, b1, b2, eps, clip, is_clip, st); break;
+    default: return -1;
+  }
+  return 0;
 }
 void launch_slot_reset(const SparseTable& t, int64_t n_keys, cudaStream_t st) { PAMREC_PROF("slot_reset", 1, st);
   if (n_keys == 0) return;

@@ -51,9 +51,11 @@ struct Layout {
   int model_kind = PAMREC_MODEL_PAMREC;
   int n_expert = 0;                             // 5 (MMoE), 7 (PLE: 3 shared, 2 main, 2 sub), 0 (share-bottom)
   int gate_sel[2][5] = {{0, 1, 2, 3, 4}, {0, 1, 2, 3, 4}};   // experts mixed by gate_main / gate_sub (ple.py:51-58)
-  int tower_in = 0;                             // 84 = 64 + 20 (mixing output | target) or 60 (share-bottom: x itself)
+  int tower_in = 0;                             // 64 + E (mixing output | target) or 3 E (share-bottom: x itself)
   MlpOff att;                                   // att_fcn of long_term, short_term (group-strided)
-  int64_t att_mat = 0;                          // attention_mat of long_term; short_term follows at + 400
+  int64_t att_mat = 0;                          // attention_mat of long_term; short_term follows at + emb_dim^2
+  // embedding widths (pamrec_create has validated them): item | cate = one history token of emb_dim floats; PAMRec: 16 / 4 / 20
+  int item_dim = kI, cate_dim = kC, user_dim = PAMREC_USER_DIM, emb_dim = kE;
 
   int64_t add_dense(const std::string& name, std::initializer_list<int64_t> shape, int flags) {
     TensorDesc t;
@@ -153,13 +155,14 @@ struct Layout {
   void build_sibling(const PamrecConfig& c) {
     const int L2 = PAMREC_SEG_L2;
     const int64_t B = Bcap, N = (int64_t)Bcap * T;
+    const int E = emb_dim;
     const std::string clsr = "sequential/clsr/";
     // ---- dense pool
-    att_mat = add_dense(clsr + "long_term/attention_fcn/attention_mat", {kE, kE}, L2);          // mmoe.py:315-319
-    add_dense(clsr + "short_term/attention_fcn/attention_mat", {kE, kE}, L2);
-    att = add_mlp({clsr + "long_term/attention_fcn/att_fcn", clsr + "short_term/attention_fcn/att_fcn"}, {L2, L2}, 4 * kE, 80, 40, true,
+    att_mat = add_dense(clsr + "long_term/attention_fcn/attention_mat", {E, E}, L2);          // mmoe.py:315-319
+    add_dense(clsr + "short_term/attention_fcn/attention_mat", {E, E}, L2);
+    att = add_mlp({clsr + "long_term/attention_fcn/att_fcn", clsr + "short_term/attention_fcn/att_fcn"}, {L2, L2}, 4 * E, 80, 40, true,
                   &bnoff[BN_S0], &bnoff[BN_S1]);                                                 // mmoe.py:327-329
-    const int x_dim = 3 * kE;
+    const int x_dim = 3 * E;
     std::vector<std::string> ex;
     if (model_kind == PAMREC_MODEL_MMOE) {
       for (int j = 0; j < 5; ++j) ex.push_back(clsr + "expert_" + std::to_string(j));           // mmoe.py:38-41
@@ -174,7 +177,7 @@ struct Layout {
     if (n_expert) {
       expert = add_mlp(ex, std::vector<int>(ex.size(), L2), x_dim, 100, 64, false, &bnoff[BN_E0], &bnoff[BN_E1]);
       gate = add_mlp({clsr + "gate_main", clsr + "gate_sub"}, {L2, L2}, x_dim, 64, 5, false, &bnoff[BN_G0], &bnoff[BN_G1]);
-      tower_in = 64 + kE;
+      tower_in = 64 + E;
     } else {
       bnoff[BN_E0] = bnoff[BN_E1] = bnoff[BN_G0] = bnoff[BN_G1] = BnOff{0, 0, 0, 0, 0};
       tower_in = x_dim;                                                                          // sharebottom.py:200-201
@@ -183,19 +186,19 @@ struct Layout {
     // ---- workspace.  Branch 0 = long_term (satisfied-only history), branch 1 = short_term (full history).
     add_ws("sib.ids_item", PAMREC_I32, {2, N});      // lookups of the item table in branch order (keys of the sparse plan)
     add_ws("sib.ids_cate", PAMREC_I32, {2, N});
-    add_ws("sib.h", PAMREC_F32, {2, N, kE});         // gathered history tokens item | cate
-    add_ws("tgt", PAMREC_F32, {B, kE});
-    add_ws("sib.feat", PAMREC_F32, {N, 160});        // per branch: a = h A | q | a - q | a * q   (mmoe.py:320-326)
+    add_ws("sib.h", PAMREC_F32, {2, N, E});         // gathered history tokens item | cate
+    add_ws("tgt", PAMREC_F32, {B, E});
+    add_ws("sib.feat", PAMREC_F32, {N, 8 * E});      // per branch: a = h A | q | a - q | a * q   (mmoe.py:320-326)
     add_ws("z1", PAMREC_F32, {N, 160});              // att_fcn layer 0 pre-activations (both branches)
     add_ws("z2", PAMREC_F32, {N, 80});               // layer 1
     add_ws("sib.score", PAMREC_F32, {N, 2});         // linear output = attention logits
     add_ws("sib.aw", PAMREC_F32, {2, N});            // softmax weights, kept for the backward pass
-    add_ws("x", PAMREC_F32, {B, 60});                // long | short | target
+    add_ws("x", PAMREC_F32, {B, x_dim});             // long | short | target
     add_ws("ze0", PAMREC_F32, {B, (int64_t)n_expert * 100});
     add_ws("zg0", PAMREC_F32, {B, n_expert ? 128 : 0});
     add_ws("ze1", PAMREC_F32, {B, (int64_t)n_expert * 64});
     add_ws("zg1", PAMREC_F32, {B, n_expert ? 10 : 0});
-    add_ws("u", PAMREC_F32, {B, 168});
+    add_ws("u", PAMREC_F32, {B, 2 * (64 + E)});   // main | target | sub | target
     add_ws("zt0", PAMREC_F32, {B, 200});
     add_ws("zt1", PAMREC_F32, {B, 128});
     add_ws("logits", PAMREC_F32, {B, 2});            // logit_fcn (satisfied label), valid_logit_fcn (play label)
@@ -204,21 +207,21 @@ struct Layout {
     add_ws("d_logits", PAMREC_F32, {B, 2});
     add_ws("d_t1", PAMREC_F32, {B, 128});
     add_ws("d_t0", PAMREC_F32, {B, 200});
-    add_ws("d_u", PAMREC_F32, {B, 168});
+    add_ws("d_u", PAMREC_F32, {B, 2 * (64 + E)});
     add_ws("d_e1", PAMREC_F32, {B, (int64_t)n_expert * 64});
     add_ws("d_g1", PAMREC_F32, {B, n_expert ? 10 : 0});
     add_ws("d_e0", PAMREC_F32, {B, (int64_t)n_expert * 100});
     add_ws("d_g0", PAMREC_F32, {B, n_expert ? 128 : 0});
-    add_ws("d_x", PAMREC_F32, {B, 60});
-    add_ws("d_tgt", PAMREC_F32, {B, kE});            // from the towers' target columns
-    add_ws("d_tgt_total", PAMREC_F32, {B, kE});
+    add_ws("d_x", PAMREC_F32, {B, x_dim});
+    add_ws("d_tgt", PAMREC_F32, {B, E});            // from the towers' target columns
+    add_ws("d_tgt_total", PAMREC_F32, {B, E});
     add_ws("sib.d_score", PAMREC_F32, {N, 2});
     add_ws("sib.d_a1", PAMREC_F32, {N, 80});
     add_ws("sib.d_a0", PAMREC_F32, {N, 160});
-    add_ws("sib.d_feat", PAMREC_F32, {N, 160});
-    add_ws("sib.d_att", PAMREC_F32, {2, N, kE});     // gradient of a = h A
-    add_ws("sib.dq", PAMREC_F32, {B, 2, kE});        // gradient of the query (target) through the feature rows, per branch
-    add_ws("sib.dh", PAMREC_F32, {2, N, kE});        // gradient of the gathered tokens = rows of the sparse gradient
+    add_ws("sib.d_feat", PAMREC_F32, {N, 8 * E});
+    add_ws("sib.d_att", PAMREC_F32, {2, N, E});     // gradient of a = h A
+    add_ws("sib.dq", PAMREC_F32, {B, 2, E});        // gradient of the query (target) through the feature rows, per branch
+    add_ws("sib.dh", PAMREC_F32, {2, N, E});        // gradient of the gathered tokens = rows of the sparse gradient
     add_ws("sib.zero", PAMREC_F32, {256});           // never written: the bias of the bias-free attention_mat product
     add_ws("sib.dummy", PAMREC_F32, {256});          // sink of that product's bias gradient
     add_ws("sib.has0", PAMREC_I32, {4});             // [0] item [1] category: id 0 occurs among the history / target ids; when it
@@ -233,7 +236,7 @@ struct Layout {
       std::string p = std::string("sp.") + t + ".";
       for (const char* n : {"keys", "idx", "skeys", "sidx", "uidx", "ukeys"}) add_ws(p + n, PAMREC_I32, {NK});
       add_ws(p + "slot", PAMREC_I32, {t[0] == 'i' ? n_items : n_cates});
-      add_ws(p + "accum", PAMREC_F32, {NK, t[0] == 'i' ? kI : kC});
+      add_ws(p + "accum", PAMREC_F32, {NK, t[0] == 'i' ? item_dim : cate_dim});
     }
     for (const char* n : {"keys", "idx", "skeys", "sidx", "uidx", "ukeys"}) add_ws(std::string("sp.user.") + n, PAMREC_I32, {B});
     add_ws("sp.user.slot", PAMREC_I32, {n_users});
@@ -250,46 +253,47 @@ struct Layout {
   void build_sasrec(const PamrecConfig& c) {
     const int L2 = PAMREC_SEG_L2;
     const int64_t B = Bcap, N = (int64_t)Bcap * T;
-    pos = add_dense("sequential/embedding/position_embedding", {T, kE}, PAMREC_SEG_POS);       // sasrec.py:29-34
+    const int E = emb_dim;
+    pos = add_dense("sequential/embedding/position_embedding", {T, E}, PAMREC_SEG_POS);       // sasrec.py:29-34
     for (int b = 0; b < 2; ++b) {
       const std::string p = "sequential/sasrec/num_blocks_" + std::to_string(b) + "/";
       SasBlock& o = sas[b];
       // Q, K, V kernels adjacent (one grouped weight-gradient GEMM), then their biases
-      o.wqkv = add_dense(p + "self_attention/dense/kernel", {kE, kE}, L2);
-      add_dense(p + "self_attention/dense_1/kernel", {kE, kE}, L2);
-      add_dense(p + "self_attention/dense_2/kernel", {kE, kE}, L2);
-      o.bqkv = add_dense(p + "self_attention/dense/bias", {kE}, L2);
-      add_dense(p + "self_attention/dense_1/bias", {kE}, L2);
-      add_dense(p + "self_attention/dense_2/bias", {kE}, L2);
-      o.ln_a_beta = add_dense(p + "ln/Variable", {kE}, L2);
-      o.ln_a_gamma = add_dense(p + "ln/Variable_1", {kE}, L2);
-      o.w1 = add_dense(p + "multihead_attention/conv1d/kernel", {1, kE, kE}, L2);
-      o.w2 = add_dense(p + "multihead_attention/conv1d_1/kernel", {1, kE, kE}, L2);
-      o.b1 = add_dense(p + "multihead_attention/conv1d/bias", {kE}, L2);
-      o.b2 = add_dense(p + "multihead_attention/conv1d_1/bias", {kE}, L2);
-      o.ln_b_beta = add_dense(p + "ln_1/Variable", {kE}, L2);
-      o.ln_b_gamma = add_dense(p + "ln_1/Variable_1", {kE}, L2);
+      o.wqkv = add_dense(p + "self_attention/dense/kernel", {E, E}, L2);
+      add_dense(p + "self_attention/dense_1/kernel", {E, E}, L2);
+      add_dense(p + "self_attention/dense_2/kernel", {E, E}, L2);
+      o.bqkv = add_dense(p + "self_attention/dense/bias", {E}, L2);
+      add_dense(p + "self_attention/dense_1/bias", {E}, L2);
+      add_dense(p + "self_attention/dense_2/bias", {E}, L2);
+      o.ln_a_beta = add_dense(p + "ln/Variable", {E}, L2);
+      o.ln_a_gamma = add_dense(p + "ln/Variable_1", {E}, L2);
+      o.w1 = add_dense(p + "multihead_attention/conv1d/kernel", {1, E, E}, L2);
+      o.w2 = add_dense(p + "multihead_attention/conv1d_1/kernel", {1, E, E}, L2);
+      o.b1 = add_dense(p + "multihead_attention/conv1d/bias", {E}, L2);
+      o.b2 = add_dense(p + "multihead_attention/conv1d_1/bias", {E}, L2);
+      o.ln_b_beta = add_dense(p + "ln_1/Variable", {E}, L2);
+      o.ln_b_gamma = add_dense(p + "ln_1/Variable_1", {E}, L2);
     }
     for (int i = 0; i < BN_COUNT; ++i) bnoff[i] = BnOff{0, 0, 0, 0, 0};
-    tower_in = 2 * kE;
+    tower_in = 2 * E;
     tower = add_mlp({"sequential/logit_fcn"}, {L2}, tower_in, 100, 64, true, &bnoff[BN_T0], &bnoff[BN_T1]);   // sequential_base_model.py:76-79
     // ---- workspace
     add_ws("sib.ids_item", PAMREC_I32, {2, N});      // satisfied-only ids (looked up), then the full-history ids (L2 rows only)
     add_ws("sib.ids_cate", PAMREC_I32, {2, N});
-    add_ws("sib.h", PAMREC_F32, {2, N, kE});
-    add_ws("tgt", PAMREC_F32, {B, kE});
-    add_ws("x0", PAMREC_F32, {N, kE});               // history token + position row
+    add_ws("sib.h", PAMREC_F32, {2, N, E});
+    add_ws("tgt", PAMREC_F32, {B, E});
+    add_ws("x0", PAMREC_F32, {N, E});               // history token + position row
     for (int b = 0; b < 2; ++b) {
       const std::string p = "blk" + std::to_string(b) + ".";
-      add_ws(p + "xq", PAMREC_F32, {N, 2 * kE});     // LN(x) | x
-      add_ws(p + "qkv", PAMREC_F32, {N, 3 * kE});
+      add_ws(p + "xq", PAMREC_F32, {N, 2 * E});     // LN(x) | x
+      add_ws(p + "qkv", PAMREC_F32, {N, 3 * E});
       add_ws(p + "ml", PAMREC_F32, {N, 2});
-      add_ws(p + "y", PAMREC_F32, {N, kE});
-      add_ws(p + "f", PAMREC_F32, {N, kE});          // LN_1(y)
-      add_ws(p + "hpre", PAMREC_F32, {N, kE});       // f W1 + b1 (the ReLU pattern of the point-wise FFN)
-      add_ws(p + "out", PAMREC_F32, {N, kE});
+      add_ws(p + "y", PAMREC_F32, {N, E});
+      add_ws(p + "f", PAMREC_F32, {N, E});          // LN_1(y)
+      add_ws(p + "hpre", PAMREC_F32, {N, E});       // f W1 + b1 (the ReLU pattern of the point-wise FFN)
+      add_ws(p + "out", PAMREC_F32, {N, E});
     }
-    add_ws("u", PAMREC_F32, {B, 2 * kE});            // final state | target
+    add_ws("u", PAMREC_F32, {B, 2 * E});            // final state | target
     add_ws("zt0", PAMREC_F32, {B, 100});
     add_ws("zt1", PAMREC_F32, {B, 64});
     add_ws("logits", PAMREC_F32, {B, 1});
@@ -298,16 +302,16 @@ struct Layout {
     add_ws("d_logits", PAMREC_F32, {B, 1});
     add_ws("d_t1", PAMREC_F32, {B, 64});
     add_ws("d_t0", PAMREC_F32, {B, 100});
-    add_ws("d_u", PAMREC_F32, {B, 2 * kE});
-    add_ws("d_tgt_total", PAMREC_F32, {B, kE});
-    add_ws("sas.g_a", PAMREC_F32, {N, kE});          // gradient of a block's output (ping)
-    add_ws("sas.g_b", PAMREC_F32, {N, kE});          // ... (pong)
-    add_ws("sas.hid", PAMREC_F32, {N, kE});
-    add_ws("sas.d_hpre", PAMREC_F32, {N, kE});
-    add_ws("sas.d_y", PAMREC_F32, {N, kE});
-    add_ws("sas.d_qkv", PAMREC_F32, {N, 3 * kE});
+    add_ws("d_u", PAMREC_F32, {B, 2 * E});
+    add_ws("d_tgt_total", PAMREC_F32, {B, E});
+    add_ws("sas.g_a", PAMREC_F32, {N, E});          // gradient of a block's output (ping)
+    add_ws("sas.g_b", PAMREC_F32, {N, E});          // ... (pong)
+    add_ws("sas.hid", PAMREC_F32, {N, E});
+    add_ws("sas.d_hpre", PAMREC_F32, {N, E});
+    add_ws("sas.d_y", PAMREC_F32, {N, E});
+    add_ws("sas.d_qkv", PAMREC_F32, {N, 3 * E});
     add_ws("sas.dq", PAMREC_F32, {N});
-    add_ws("sib.dh", PAMREC_F32, {2, N, kE});        // [0] = gradient of x0 = rows of the satisfied lookups; [1] = 0 (L2 rows only)
+    add_ws("sib.dh", PAMREC_F32, {2, N, E});        // [0] = gradient of x0 = rows of the satisfied lookups; [1] = 0 (L2 rows only)
     add_ws("sib.has0", PAMREC_I32, {4});
     add_bn_ws();
     add_optim_ws();
@@ -317,7 +321,7 @@ struct Layout {
       std::string p = std::string("sp.") + t + ".";
       for (const char* n : {"keys", "idx", "skeys", "sidx", "uidx", "ukeys"}) add_ws(p + n, PAMREC_I32, {NK});
       add_ws(p + "slot", PAMREC_I32, {t[0] == 'i' ? n_items : n_cates});
-      add_ws(p + "accum", PAMREC_F32, {NK, t[0] == 'i' ? kI : kC});
+      add_ws(p + "accum", PAMREC_F32, {NK, t[0] == 'i' ? item_dim : cate_dim});
     }
     add_ws("sp.nuniq", PAMREC_I32, {8});
     add_ws("dp.scalars", PAMREC_F64, {8});
@@ -330,6 +334,8 @@ struct Layout {
     n_users = c.n_users; n_items = c.n_items; n_cates = c.n_cates; T = c.max_seq_len; Bcap = c.max_batch;
     world = c.world_size < 1 ? 1 : c.world_size; table_mode = c.table_mode;
     model_kind = c.model_kind;
+    item_dim = c.item_dim ? c.item_dim : kI; cate_dim = c.cate_dim ? c.cate_dim : kC; user_dim = c.user_dim ? c.user_dim : PAMREC_USER_DIM;
+    emb_dim = item_dim + cate_dim;
     if (model_kind == PAMREC_MODEL_SASREC) { build_sasrec(c); return; }
     if (model_kind != PAMREC_MODEL_PAMREC) { build_sibling(c); return; }
     const int L2 = PAMREC_SEG_L2;

@@ -10,19 +10,21 @@ from . import _lib as L
 from . import dist as D
 
 EMB = "sequential/embedding/"
+# table -> (buffer prefix, index of its width in emb_dims = (item, cate, user))
 TABLES = {
-    EMB + "item_embedding": ("item", 16),
-    EMB + "cate_embedding": ("cate", 4),
-    EMB + "user_long_embedding": ("ulong", 20),
-    EMB + "user_short_embedding": ("ushort", 20),
+    EMB + "item_embedding": ("item", 0),
+    EMB + "cate_embedding": ("cate", 1),
+    EMB + "user_long_embedding": ("ulong", 2),
+    EMB + "user_short_embedding": ("ushort", 2),
 }
 # variables that exist in the reference graph but never receive a gradient (SURVEY.md A.4): kept on the
-# host so that checkpoints carry the complete variable list of base_model.py:62.
+# host so that checkpoints carry the complete variable list of base_model.py:62.  Shapes from (n_users, emb_dims).
 FROZEN = {
-    EMB + "user_embedding": lambda nu: (nu, 20),
-    EMB + "looptimes_embedding": lambda nu: (10, 4),
-    EMB + "play_lookup": lambda nu: (10, 40),
+    EMB + "user_embedding": lambda nu, d: (nu, d[2]),
+    EMB + "looptimes_embedding": lambda nu, d: (10, d[1]),
+    EMB + "play_lookup": lambda nu, d: (10, 40),
 }
+EMB_DIMS = (16, 4, 20)               # (item, cate, user) embedding widths of config/mmoe.yaml; PAMRec's only set
 _TORCH_DTYPE = {L.F32: torch.float32, L.I32: torch.int32, L.F64: torch.float64, L.U8: torch.uint8}
 _ESIZE = {L.F32: 4, L.I32: 4, L.F64: 8, L.U8: 1}
 
@@ -89,9 +91,11 @@ class PendingHost:
 
 class Engine:
     def __init__(self, n_users, n_items, n_cates, max_seq_len, max_batch, hp=None, sparse_adam="dense_exact",
-                 world_size=1, rank=0, tables=None, model="pamrec", graph=None):
+                 world_size=1, rank=0, tables=None, model="pamrec", graph=None, emb_dims=EMB_DIMS):
         """model: "pamrec" (PAMRECModel) or one of the sibling baselines "mmoe" (MMoEModel_original), "ple" (PLEModel),
         "sharebottom" (ShareBottomModel), "sasrec" (SASRecModel) - those run on one GPU with whole tables.
+        emb_dims: (item, cate, user) embedding widths.  PAMRec runs (16, 4, 20) only; the sibling models run (item, cate) = (16, 4)
+        or (32, 8) (the reference's ple.yaml / sharebottom.yaml / sasrec.yaml) with user = 16, 20 or 40.
         graph: replay the train step from a CUDA graph (one graph per resident / staged DeviceBatch, captured at its second use;
         one GPU, whole tables, PAMRec only).  None reads PAMREC_GRAPH (default on; PAMREC_GRAPH=0 launches kernel by kernel).
         tables: "local" (whole tables on this GPU, world_size 1), "replicated" (every rank holds whole tables; the merged
@@ -119,6 +123,7 @@ class Engine:
             h.update(hp)
         self.hp = h
         self.dims = (int(n_users), int(n_items), int(n_cates), int(max_seq_len), int(max_batch))
+        self.emb_dims = tuple(int(d) for d in emb_dims)
         mode = {"dense_exact": L.ADAM_DENSE_EXACT, "lazy": L.ADAM_LAZY}[sparse_adam]
         self.cfg = L.PamrecConfig(
             n_users=n_users, n_items=n_items, n_cates=n_cates, max_seq_len=max_seq_len, max_batch=max_batch,
@@ -128,12 +133,14 @@ class Engine:
             order_weight=h["discrepancy_loss_weight"], sparse_adam_mode=mode, world_size=world_size, rank=rank,
             table_mode={"local": L.TABLES_LOCAL, "sharded": L.TABLES_SHARDED, "replicated": L.TABLES_REPLICATED}[tables],
             loss_kind={"cross_entropy_loss": L.LOSS_XENT, "softmax": L.LOSS_SOFTMAX}[h["loss"]], softmax_group=int(h["softmax_group"]),
-            model_kind=MODELS[model])
+            model_kind=MODELS[model], item_dim=self.emb_dims[0], cate_dim=self.emb_dims[1], user_dim=self.emb_dims[2])
         self.handle = C.c_void_p()
         rc = self.lib.pamrec_create(C.byref(self.cfg), C.byref(self.handle))
         if rc != 0:
             raise PamrecError(f"pamrec_create failed ({rc}): check vocabulary sizes, max_seq_len <= 256, max_batch, "
-                              "world_size <= 64, rank, table mode, model (siblings: one GPU, cross_entropy_loss)")
+                              "world_size <= 64, rank, table mode, model (siblings: one GPU, cross_entropy_loss), embedding widths "
+                              f"{self.emb_dims} (item / cate / user: PAMRec 16 / 4 / 20 only; siblings 16 / 4 or 32 / 8 with user "
+                              "16, 20 or 40)")
         self.dense_numel = self.lib.pamrec_dense_numel(self.handle)
         self.bn_numel = self.lib.pamrec_bn_numel(self.handle)
         self.workspace_bytes = self.lib.pamrec_workspace_bytes(self.handle)
@@ -145,7 +152,8 @@ class Engine:
         self.graph = bool(graph)
         self._graphs, self._profiling = {}, False
         self._dev_step = None                        # value of the device-side step counter, when known to equal self.step
-        self.frozen = {n: np.zeros(f(n_users), np.float32) for n, f in FROZEN.items() if model != "sasrec" or not n.endswith("play_lookup")}
+        self.frozen = {n: np.zeros(f(n_users, self.emb_dims), np.float32) for n, f in FROZEN.items()
+                       if model != "sasrec" or not n.endswith("play_lookup")}
 
     # ------------------------------------------------------------------ inventory (host only)
     def _query(self, pool):
@@ -162,7 +170,7 @@ class Engine:
         nu, ni, nc, T, _ = self.dims
         shapes = {n: d["shape"] for n, d in self.info[L.POOL_DENSE].items()}
         rows = {"item": ni, "cate": nc, "ulong": nu, "ushort": nu}
-        shapes.update({n: (rows[pre], w) for n, (pre, w) in self.tables_by_name.items()})
+        shapes.update({n: (rows[pre], self.emb_dims[k]) for n, (pre, k) in self.tables_by_name.items()})
         shapes.update({n: a.shape for n, a in self.frozen.items()})
         shapes.update({n: d["shape"] for n, d in self.info[L.POOL_BN].items()})
         return shapes
@@ -181,7 +189,8 @@ class Engine:
         z = lambda *s: torch.zeros(*s, dtype=torch.float32, device=self.device)
         self.pool = {k: z(self.dense_numel) for k in ("dense_param", "dense_grad", "dense_m", "dense_v")}
         self.pool["bn_moving"] = z(self.bn_numel)
-        for pre, rows, w in (("item", ni, 16), ("cate", nc, 4), ("ulong", nu, 20), ("ushort", nu, 20)):
+        di, dc, du = self.emb_dims
+        for pre, rows, w in (("item", ni, di), ("cate", nc, dc), ("ulong", nu, du), ("ushort", nu, du)):
             for s in ("w", "m", "v"):
                 self.pool[f"{pre}_{s}"] = z(self.table_rows(rows), w)
         self.pool["workspace"] = torch.zeros(self.workspace_bytes, dtype=torch.uint8, device=self.device)

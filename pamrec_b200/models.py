@@ -182,8 +182,7 @@ class BaseModel:
         need(hp.loss in ("cross_entropy_loss", "softmax"), "loss must be cross_entropy_loss or softmax (BM:195-242; square_loss and "
                                                             "log_loss have no auxiliary branch that PAMRec defines consistently)")
         need(hp.optimizer == "adam", "optimizer must be adam (BM:270-271)")
-        need(hp.item_embedding_dim == 16 and hp.cate_embedding_dim == 4 and hp.user_embedding_dim == 20,
-             "embedding dims must be 16 / 4 / 20 (config/mmoe.yaml:22-24)")
+        self._check_emb_dims(hp, need)
         need(list(hp.layer_sizes) == [100, 64], "tower sizes of config/mmoe.yaml")
         self._check_mixing(hp, need)
         need(list(hp.activation)[:2] == ["relu", "relu"], "activation must be [relu, relu]")
@@ -200,6 +199,15 @@ class BaseModel:
     def _check_mixing(self, hp, need):
         need(list(hp.expert_layer_sizes) == [100, 64] and list(hp.gate_layer_sizes) == [64, 5] and hp.expert_num == 5,
              "expert / gate sizes of config/mmoe.yaml")
+
+    def _check_emb_dims(self, hp, need):
+        need(hp.item_embedding_dim == 16 and hp.cate_embedding_dim == 4 and hp.user_embedding_dim == 20,
+             "embedding dims must be 16 / 4 / 20 (config/mmoe.yaml:22-24)")
+
+    @staticmethod
+    def _emb_dims(hp):
+        """(item, cate, user) embedding widths of the engine, as _check_supported admitted them."""
+        return int(hp.item_embedding_dim), int(hp.cate_embedding_dim), int(hp.user_embedding_dim)
 
     def _build_graph(self):
         raise NotImplementedError
@@ -479,7 +487,7 @@ class PAMRECModel(SequentialBaseModel):
             cap = max(-(-(cap // 5) // world) * 5, -(-cap // world))
         tables = getattr(hp, "tables", None)
         self.engine = Engine(n_users, n_items, n_cates, hp.max_seq_length, cap, hp=engine_hp, sparse_adam=mode,
-                             world_size=world, rank=rank, tables=tables, model=self.ENGINE_MODEL)
+                             world_size=world, rank=rank, tables=tables, model=self.ENGINE_MODEL, emb_dims=self._emb_dims(hp))
         default_dev = "cuda:{}".format(int(os.environ.get("LOCAL_RANK", 0))) if world > 1 else "cuda:0"
         self.engine.allocate(getattr(hp, "device", default_dev))
         self.engine.init_comm()
@@ -546,9 +554,9 @@ class _DinMultiTask(PAMRECModel):
     """What MMoEModel_original, PLEModel and ShareBottomModel share (models/sequential/mmoe.py, ple.py, sharebottom.py): the
     input pipeline, DIN attention pooling of the satisfied-only and of the full history against the target (`_attention_fcn`),
     two towers, loss = data + regular + 0.5 * auxiliary, and the host loops - which differ from PAMRec's only in the 7-tuple
-    that train() returns (no order loss, MM:341-373).  One GPU; embedding dims 16 / 4 / 20 (config/mmoe.yaml) - the kernels'
-    table widths are compile-time constants, so config/ple.yaml and config/sharebottom.yaml are shipped with those dims instead
-    of the reference files' 32 / 8 / 40."""
+    that train() returns (no order loss, MM:341-373).  One GPU.  Embedding widths (item / cate / user): 16 / 4 (config/mmoe.yaml)
+    or 32 / 8 (the reference's ple.yaml and sharebottom.yaml, and 32 / 8 / 16 in its sasrec.yaml), each with a user width of 16,
+    20 or 40; the kernels are compiled for both item / cate pairs."""
 
     def _check_supported(self, hp):
         super()._check_supported(hp)
@@ -556,6 +564,11 @@ class _DinMultiTask(PAMRECModel):
             raise ValueError("pamrec_b200: unsupported configuration: att_fcn_layer_sizes must be [80, 40]")
         if hp.loss != "cross_entropy_loss":
             raise ValueError("pamrec_b200: unsupported configuration: the sibling models train with cross_entropy_loss")
+
+    def _check_emb_dims(self, hp, need):
+        need((hp.item_embedding_dim, hp.cate_embedding_dim) in ((16, 4), (32, 8)) and hp.user_embedding_dim in (16, 20, 40),
+             "embedding dims (item / cate / user) must be 16 / 4 or 32 / 8, with user 16, 20 or 40 "
+             "(config/mmoe.yaml: 16 / 4 / 20; the reference's ple.yaml / sharebottom.yaml: 32 / 8 / 40, sasrec.yaml: 32 / 8 / 16)")
         if torch.distributed.is_available() and torch.distributed.is_initialized() and torch.distributed.get_world_size() > 1:
             raise ValueError("pamrec_b200: the sibling models run on one GPU")
 
@@ -600,7 +613,7 @@ class _PendingStep5(_PendingStep):
 
 
 class SASRecModel(_DinMultiTask):
-    """models/sequential/sasrec.py:16: the satisfied-only history + a position table through two 20-wide self-attention blocks with
+    """models/sequential/sasrec.py:16: the satisfied-only history + a position table through two (item + cate)-wide self-attention blocks with
     dense Q / K / V, read out at the last satisfied position, one tower; loss = data + regular.  train() returns the base class's
     5-tuple (update, extra_update_ops, loss, data_loss, summary) (BM:350-372)."""
     ENGINE_MODEL = "sasrec"
