@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libpamrec_b200.so")
-SOURCES = ["api.cu", "prof.cu", "comm.cu", "kernels_encoder.cu", "kernels_attn_tc.cu", "kernels_attn_mma.cu", "kernels_head.cu", "kernels_head2.cu", "kernels_sibling.cu", "kernels_sasrec.cu", "kernels_optim.cu", "kernels_sparse2.cu", "kernels_shard.cu", "kernels_p2p.cu", "batcher.cu", "tokenizer.cu", "crc32c.cu"]
+SOURCES = ["api.cu", "prof.cu", "comm.cu", "kernels_encoder.cu", "kernels_attn_mma.cu", "kernels_head.cu", "kernels_head2.cu", "kernels_sibling.cu", "kernels_sasrec.cu", "kernels_optim.cu", "kernels_sparse2.cu", "kernels_shard.cu", "kernels_p2p.cu", "batcher.cu", "tokenizer.cu", "crc32c.cu"]
 HEADERS = sorted(f for f in os.listdir(CSRC) if f.endswith((".h", ".cuh", ".inl"))) + [os.path.join("..", "..", "include", "pamrec_b200.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

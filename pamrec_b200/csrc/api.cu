@@ -55,9 +55,8 @@ struct PamrecHandle_ {
   unsigned* head_bar = nullptr;      // 64 words of barrier state, then 2 x 32 trace stamps (forward, backward)
   bool head_trace = false;
   unsigned long long* head_trace_cta = nullptr;   // debug: arrival stamps of every CTA at every barrier (2 kernels x 16 x 256)
-  int n_sm = 148;
-  int attn_tc = 0;                  // 1: attention forward on tcgen05 (kernels_attn_tc.cu) where the sequence length allows it
-  int attn_mma = 1;                 // attention on warp-level tensor-core MMAs (kernels_attn_mma.cu); PAMREC_ATTN=ffma: the FFMA kernels
+  int attn_mma = 1;                 // PAMREC_ATTN=mma (default): attention on warp-level tensor-core MMAs (kernels_attn_mma.cu),
+                                    // the backward only up to T = 128; PAMREC_ATTN=ffma: the FFMA kernels (kernels_encoder.cu)
   uint32_t coop_epoch = 0;          // mailbox epoch of the cooperative kernels (one per launch, all ranks in lockstep)
   // row-stationary persistent head kernels (kernels_head2.cu): the default; PAMREC_HEAD_LEGACY=1 (or a device without
   // cooperative launch, or more than 8 ranks) selects the stand-alone kernels of kernels_head.cu
@@ -73,7 +72,7 @@ struct PamrecHandle_ {
   int64_t xr_dense() const { return (L.dense_numel + 63) / 64 * 64; }
   int64_t xr_floats() const { return xr_dense() + (replicated() ? sp2_rep_floats(cfg.n_items, cfg.n_cates, cfg.n_users) : 0); }
   char* xr_region(int p) const { return static_cast<char*>(mbox_peer[p]) + p2p_xr_offset(cfg.world_size); }
-  bool use_xr() const { return mbox_open && cfg.world_size > 1 && getenv("PAMREC_NCCL_GRADS") == nullptr; }
+  bool use_xr() const { return mbox_open && cfg.world_size > 1; }
   uint32_t xr_epoch = 0;
   // the replicated tables' gradient tables + touch counts: inside the exchange buffers when those exist (the run walk writes
   // the contribution in place, the Adam sweep reads the reduced copy), else a workspace tensor reduced by NCCL
@@ -97,7 +96,6 @@ struct PamrecHandle_ {
   // run fn(side) after everything enqueued on `main` so far
   template <typename F>
   void fork(cudaStream_t main, F fn) {
-    if (getenv("PAMREC_NO_SIDE_STREAM") != nullptr) { fn(main); return; }   // debugging aid: everything on one stream
     cudaEvent_t e = ev_side[ev_next];
     ev_next = (ev_next + 1) % 12;
     cudaEventRecord(e, main);
@@ -105,7 +103,6 @@ struct PamrecHandle_ {
     fn(side);
   }
   void join(cudaStream_t main) {
-    if (getenv("PAMREC_NO_SIDE_STREAM") != nullptr) return;
     cudaEventRecord(ev_join, side);
     cudaStreamWaitEvent(main, ev_join, 0);
   }
@@ -304,32 +301,15 @@ int pamrec_bind(PamrecHandle h, const PamrecBuffers* bufs, void* stream) {
     return fail(h, "null buffer");
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) { cudaGetLastError(); return fail(h, "no CUDA device: the CUDA path is the only path"); }
+  const char* attn_env = getenv("PAMREC_ATTN");
+  const std::string attn = attn_env ? attn_env : "mma";
+  if (attn != "mma" && attn != "ffma") return fail(h, "PAMREC_ATTN=%s: the attention kernels are mma (the default) or ffma", attn.c_str());
+  h->attn_mma = attn == "mma" ? 1 : 0;
   h->buf = *bufs;
-  {
-    // experiment hook: DRAM -> L2 fetch granularity (a device-wide hint, 32 / 64 / 128 bytes); unset = leave the driver's default
-    const char* fg = getenv("PAMREC_L2_FETCH");
-    if (fg != nullptr) {
-      size_t before = 0, after = 0;
-      cudaDeviceGetLimit(&before, cudaLimitMaxL2FetchGranularity);
-      cudaDeviceSetLimit(cudaLimitMaxL2FetchGranularity, (size_t)atoi(fg));
-      cudaDeviceGetLimit(&after, cudaLimitMaxL2FetchGranularity);
-      fprintf(stderr, "pamrec: L2 fetch granularity %zu -> %zu\n", before, after);
-      cudaGetLastError();
-    }
-  }
   if (init_encoder_kernels(h->cfg.max_seq_len)) return check_cuda(h, "shared-memory opt-in of the encoder kernels");
   if (h->cfg.model_kind == PAMREC_MODEL_SASREC && init_sas_kernels(h->cfg.max_seq_len))
     return check_cuda(h, "shared-memory opt-in of the SASRec attention kernels");
-  {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&h->n_sm, cudaDevAttrMultiProcessorCount, dev);
-    const char* a = getenv("PAMREC_ATTN");
-    h->attn_tc = (a != nullptr && std::string(a) == "tc") ? 1 : 0;
-    h->attn_mma = (a == nullptr || std::string(a) == "mma") ? 1 : 0;
-    if (init_attn_mma_kernels(h->cfg.max_seq_len)) return check_cuda(h, "shared-memory opt-in of the MMA attention kernels");
-    if (h->attn_tc && init_attn_tc_kernels(h->cfg.max_seq_len)) return check_cuda(h, "shared-memory opt-in of the tcgen05 attention kernel");
-  }
+  if (init_attn_mma_kernels(h->cfg.max_seq_len)) return check_cuda(h, "shared-memory opt-in of the MMA attention kernels");
   if (!h->side) {
     if (cudaStreamCreateWithFlags(&h->side, cudaStreamNonBlocking) != cudaSuccess) return fail(h, "cannot create the side stream");
     for (auto& e : h->ev_side) cudaEventCreateWithFlags(&e, cudaEventDisableTiming);
@@ -633,7 +613,7 @@ int pamrec_forward(PamrecHandle h, const PamrecBatch* b, int training, float* pr
   int* ctl = h->wi("bucket_ctl");
   // The bucket sort of the tokens depends on the play-ratio buckets of the batch only: on the side stream beside the gather
   // (whole tables; the sharded exchange synchronises with the host and keeps everything on one stream)
-  const bool bucket_aside = !h->sharded() && getenv("PAMREC_NO_SIDE_STREAM") == nullptr;
+  const bool bucket_aside = !h->sharded();
   if (bucket_aside) {
     h->fork(st, [&](cudaStream_t s2) {
       launch_bucket_plan(b->item_loop_times_history, N, h->wi("bucket"), h->wi("perm"), ctl, h->wi("tile_bucket"), h->wi("tile_begin"),
@@ -671,9 +651,6 @@ int pamrec_forward(PamrecHandle h, const PamrecBatch* b, int training, float* pr
                     h->wf(p + "K"), h->wf(p + "V"), st);
     if (h->attn_mma)
       launch_attn_fwd_mma(h->wf(p + "Q"), h->wf(p + "K"), h->wf(p + "V"), h->wf(p + "qin"), b->mask, h->wf(p + "y"), h->wf(p + "ml"), B, T, st);
-    else if (h->attn_tc && attn_tc_supported(T))
-      launch_attn_fwd_tc(h->wf(p + "Q"), h->wf(p + "K"), h->wf(p + "V"), h->wf(p + "qin"), b->mask, h->wf(p + "y"), h->wf(p + "ml"), B, T,
-                         h->n_sm, reinterpret_cast<int*>(h->head_bar + 3), st);
     else
       launch_attn_fwd(h->wf(p + "Q"), h->wf(p + "K"), h->wf(p + "V"), h->wf(p + "qin"), b->mask, h->wf(p + "y"), h->wf(p + "ml"), B, T, st);
     float* hdbg = (training && (h->debug & PAMREC_DEBUG_SAVE_FFN_HIDDEN)) ? h->wf(k == 0 ? "d_Q" : "d_K") : nullptr;
@@ -1041,7 +1018,7 @@ int pamrec_backward(PamrecHandle h, const PamrecBatch* b, void* stream) {
                    h->G(o.w1), h->G(o.b1), h->G(o.w2), h->G(o.b2), h->G(o.ln_b_beta), h->G(o.ln_b_gamma), N, st);
     // backward: the MMA kernel keeps K, V, Q and dY of a sample in shared memory (141 KB at T = 200: one CTA per SM), measured slower
     // than the FFMA kernel there (8.5 vs 6.4 ms per step on long_b4095_t200) and faster below (T = 100: 230 vs 292 us, T = 50: 152 vs 196 us)
-    if (h->attn_mma && (T <= 128 || getenv("PAMREC_ATTN_BWD_MMA") != nullptr) && getenv("PAMREC_ATTN_BWD_FFMA") == nullptr)
+    if (h->attn_mma && T <= 128)
       launch_attn_bwd_mma(h->wf(p + "Q"), h->wf(p + "K"), h->wf(p + "V"), h->wf("d_y"), h->wf(p + "y"), h->wf(p + "qin"), h->wf(p + "ml"),
                           b->mask, h->wf("d_Q"), h->wf("d_K"), h->wf("d_V"), B, T, st);
     else
@@ -1159,7 +1136,7 @@ int pamrec_apply_gradients(PamrecHandle h, const PamrecBatch* b, int64_t step, v
     }
   } else {
     // ---- whole tables on this GPU: one-sort plan (side stream, beside the forward pass) -> run walk -> Adam
-    if (c.world_size == 1 && getenv("PAMREC_NO_SIDE_STREAM") == nullptr) {
+    if (c.world_size == 1) {
       // one GPU: the dense variables' clip norms + Adam share nothing with the tables' walk + sweep: side stream, joined before the losses
       dense_aside = true;
       h->fork(st, [&](cudaStream_t s2) {

@@ -54,12 +54,6 @@ void launch_proj_bwd(const float* X, const float* dY, const float* dQ, const flo
                      const float* Wq, const float* Wk, const float* Wv, const float* ln_beta, const float* ln_gamma,
                      float* dX, float* dWq, float* dWk, float* dWv, float* dbeta, float* dgamma, cudaStream_t st);
 
-// ---- kernels_attn_tc.cu (tcgen05 / tensor-memory attention forward)
-bool attn_tc_supported(int T);
-int init_attn_tc_kernels(int max_T);
-void launch_attn_fwd_tc(const float* Q, const float* K, const float* V, const float* QIN, const int* mask, float* Y, float* ML, int B, int T,
-                        int n_sm, int* err, cudaStream_t st);
-
 // ---- kernels_attn_mma.cu (attention forward + backward on warp-level tensor-core MMAs, 3xTF32; the default)
 int init_attn_mma_kernels(int max_T);
 void launch_attn_fwd_mma(const float* Q, const float* K, const float* V, const float* QIN, const int* mask, float* Y, float* ML, int B, int T,

@@ -4,7 +4,7 @@
 //   backward: dQ = dS K,  dK = dS^T Q,  dV = P^T dY  with  dS = P o (dY V^T - D) / sqrt(40),  D_t = dY_t . (y_t - qin_t)
 //
 // Why m16n8k8 and not tcgen05 here: a sample is a 50 x 50 (T x T) problem.  A tcgen05 tile is 128 rows - two and a half samples of
-// padding per sample at T = 50 (measured: kernels_attn_tc.cu loses to the FFMA kernel, profiles/r02_attn_tc.log) - while a
+// padding per sample at T = 50 (measured: a tcgen05 forward lost to the FFMA kernel, DESIGN.md section 4) - while a
 // 16-row warp tile wastes 14 of 64 rows.  The FFMA kernels (kernels_encoder.cu) are bound by the latency of one thread's serial
 // walk over the keys at 10 % occupancy; here a warp owns 16 query rows (or 16 key rows), scores live in accumulator fragments,
 // and the probabilities feed the second product straight from registers: within a block of 8 keys the product's contraction
@@ -199,8 +199,7 @@ __host__ __device__ inline size_t bwd_smem(int T) {
   return ((size_t)2 * Tp16 * kSt + 2 * Tp8 * kSt + 3 * Tp8 + 2 * T4 + 4) * 4;
 }
 
-template <int MINB>                      // resident CTAs per SM the register allocation must allow (3: no spills; 4: 128 registers)
-__global__ void __launch_bounds__(kThreads, MINB)
+__global__ void __launch_bounds__(kThreads, 3)      // 3 resident CTAs per SM: the most the registers allow without spills
 k_attn_bwd_mma(const float* __restrict__ Q, const float* __restrict__ K, const float* __restrict__ V, const float* __restrict__ dY,
                const float* __restrict__ Y, const float* __restrict__ QIN, const float* __restrict__ ML, const int* __restrict__ mask,
                float* __restrict__ dQ, float* __restrict__ dK, float* __restrict__ dV, int T) {
@@ -382,8 +381,7 @@ int init_attn_mma_kernels(int max_T) {
   set((const void*)amma::k_attn_fwd_mma<13>, f);
   set((const void*)amma::k_attn_fwd_mma<25>, f);
   set((const void*)amma::k_attn_fwd_mma<32>, f);
-  set((const void*)amma::k_attn_bwd_mma<3>, b);
-  set((const void*)amma::k_attn_bwd_mma<4>, b);
+  set((const void*)amma::k_attn_bwd_mma, b);
   return e == cudaSuccess ? 0 : -1;
 }
 
@@ -401,10 +399,7 @@ void launch_attn_bwd_mma(const float* Q, const float* K, const float* V, const f
                          const int* mask, float* dQ, float* dK, float* dV, int B, int T, cudaStream_t st) {
   PAMREC_PROF("attn_bwd", 1, st);
   if (B == 0) return;
-  static const bool occ4 = getenv("PAMREC_ATTN_BWD_OCC4") != nullptr;      // experiment switch: 4 CTAs / SM at the price of spills
-  const dim3 grid(B, (T + 63) / 64);
-  if (occ4) amma::k_attn_bwd_mma<4><<<grid, amma::kThreads, amma::bwd_smem(T), st>>>(Q, K, V, dY, Y, QIN, ML, mask, dQ, dK, dV, T);
-  else amma::k_attn_bwd_mma<3><<<grid, amma::kThreads, amma::bwd_smem(T), st>>>(Q, K, V, dY, Y, QIN, ML, mask, dQ, dK, dV, T);
+  amma::k_attn_bwd_mma<<<dim3(B, (T + 63) / 64), amma::kThreads, amma::bwd_smem(T), st>>>(Q, K, V, dY, Y, QIN, ML, mask, dQ, dK, dV, T);
 }
 
 }  // namespace pamrec

@@ -49,10 +49,22 @@ CASES = [
 ]
 
 
-@pytest.mark.parametrize("nu,ni,nc,T,B", CASES)
-def test_train_step_stagewise(nu, ni, nc, T, B):
+def _case_id(c):
+    return "-".join(map(str, c))
+
+
+# the default head at every shape; the stand-alone head (PAMREC_HEAD_LEGACY=1, kernels_head.cu: the head beyond 8 ranks and
+# without peer mailboxes) at the four small ones
+STAGEWISE = ([pytest.param(*c, False, id=_case_id(c)) for c in CASES] +
+             [pytest.param(*c, True, id=_case_id(c) + "-legacy_head") for c in CASES[:4]])
+
+
+@pytest.mark.parametrize("nu,ni,nc,T,B,legacy_head", STAGEWISE)
+def test_train_step_stagewise(nu, ni, nc, T, B, legacy_head, monkeypatch):
     from pamrec_b200 import _lib as L
     from relu_masks import engine_relu_masks
+    if legacy_head:
+        monkeypatch.setenv("PAMREC_HEAD_LEGACY", "1")
     om, eng = _setup(nu, ni, nc, T, B, seed=11)
     om.proj = "grouped"                     # same sums as the reference's [B,T,40,40] gather without materialising it
     batch = O.make_batch(5, B, T, nu, ni, nc)
@@ -295,8 +307,8 @@ def test_lazy_fused_adam_equals_dense_exact_on_the_first_step(shape):
     lazy.close(); exact.close()
 
 
-def test_error_paths():
-    from pamrec_b200.engine import PamrecError
+def test_error_paths(monkeypatch):
+    from pamrec_b200.engine import Engine, PamrecError
     nu, ni, nc, T, B = 50, 300, 20, 12, 20
     om, eng = _setup(nu, ni, nc, T, B, seed=1)
     bad = O.make_batch(1, 10, T, nu, ni, nc)
@@ -308,6 +320,11 @@ def test_error_paths():
     with pytest.raises(PamrecError):          # larger than max_batch
         eng.forward(eng.upload(big), training=False)
     eng.close()
+    monkeypatch.setenv("PAMREC_ATTN", "tc")
+    tc = Engine(nu, ni, nc, T, B)
+    with pytest.raises(PamrecError, match="PAMREC_ATTN"):     # the attention kernels are mma or ffma
+        tc.allocate()
+    tc.close()
 
 
 @pytest.mark.parametrize("T,B", [(12, 20), (50, 130), (100, 35), (200, 10), (256, 5)])

@@ -23,10 +23,6 @@ FWD = ["F1 score layer 0 (tokens)", "F2 score layer 1 (tokens)", "F3 pooling + e
 BWD = ["K0 weight transposes + losses", "K1 dA(t1)", "K2 dz(t1) -> dA(t0)", "K3 dz(t0) -> d_u -> mixing backward", "K4 dz(e1, g1) -> dA(e0, g0)",
        "K5 dz(e0, g0) -> d_new_long -> pooling backward", "K6 dz2 -> sums of BN_S0, score layer 1 gradients",
        "K7 dz1 -> dH, score layer 0 gradients (to the end of CTA 0)"]
-if os.environ.get("PAMREC_HEAD") == "tiles":
-    FWD = ["s0 fwd (N rows)", "s1 fwd (N rows)", "pool fwd", "e0 + g0 fwd", "e1 + g1 fwd", "combine fwd", "t0 fwd", "t1 fwd", "tout fwd (to the end of CTA 0)"]
-    BWD = ["loss", "tout dx + dw", "t1 dx + dw", "t0 dx + dw", "combine bwd", "e1 / g1 dx + dw", "e0 dx, e0 / g0 dw", "g0 dx", "pool bwd",
-           "s1 dx + dw (N rows)", "s0 dx + dw (N rows, to the end of CTA 0)"]
 
 
 def main():
