@@ -189,9 +189,9 @@ int pamrec_train_step(PamrecHandle h, const PamrecBatch* b, int64_t step, float*
 int pamrec_comm_unique_id(const char* nccl_path, char id_out[PAMREC_COMM_ID_BYTES]);
 int pamrec_comm_init(PamrecHandle h, const char* nccl_path, const char id[PAMREC_COMM_ID_BYTES]);
 int pamrec_comm_destroy(PamrecHandle h);
-/* Optional peer-memory mailboxes (NVLink P2P, world_size <= 8): with them the twelve small all-reduces of a train step
- * (batch-norm column sums) run as ONE single-CTA kernel per rank that stores into its peers' mailboxes, waits on epoch flags
- * and - forward pass - finalises the batch-norm statistics in the same kernel; without them these all-reduces use NCCL.
+/* Optional peer-memory mailboxes (NVLink P2P, world_size <= 8): with them the persistent head kernels exchange the batch-norm
+ * column sums of a train step inside their grid barriers, by stores into their peers' mailboxes, and the gradients are summed
+ * through the mailboxes as well; without them NCCL does both.
  * Every rank calls _create, the host all-gathers the 64-byte handles (rank-major), every rank calls _open. */
 #define PAMREC_IPC_HANDLE_BYTES 64
 int pamrec_comm_mailbox_create(PamrecHandle h, char handle_out[PAMREC_IPC_HANDLE_BYTES]);

@@ -46,28 +46,21 @@ struct PamrecHandle_ {
   int ev_next = 0;
   const void* plan_for = nullptr;   // batch whose sparse plan is in flight / ready on the side stream (local tables)
   int plan_rows = -1;
-  // peer-memory mailboxes for the small all-reduces (kernels_p2p.cu); payload | flags | error word
+  // peer-memory mailboxes (kernels.h: p2p_mailbox_bytes): error word | persistent head exchanges | gradient exchange
   void* mbox = nullptr;
   void* mbox_peer[kP2PMaxWorld] = {};
   bool mbox_open = false;
-  uint32_t mbox_epoch[kP2PSlots] = {};
   // persistent cooperative head kernels (kernels_head2.cu): barrier words, trace stamps
   unsigned* head_bar = nullptr;      // 64 words of barrier state, then 2 x 32 trace stamps (forward, backward)
   bool head_trace = false;
   unsigned long long* head_trace_cta = nullptr;   // debug: arrival stamps of every CTA at every barrier (2 kernels x 16 x 256)
-  int attn_mma = 1;                 // PAMREC_ATTN=mma (default): attention on warp-level tensor-core MMAs (kernels_attn_mma.cu),
-                                    // the backward only up to T = 128; PAMREC_ATTN=ffma: the FFMA kernels (kernels_encoder.cu)
   uint32_t coop_epoch = 0;          // mailbox epoch of the cooperative kernels (one per launch, all ranks in lockstep)
   // row-stationary persistent head kernels (kernels_head2.cu): the default; PAMREC_HEAD_LEGACY=1 (or a device without
   // cooperative launch, or more than 8 ranks) selects the stand-alone kernels of kernels_head.cu
   Head2 head2;
   int head2_grid = 0;
   bool use_head2() const { return head2_grid > 0 && (cfg.world_size == 1 || mbox_open); }
-  double* mbox_slots(int p) const { return static_cast<double*>(mbox_peer[p]); }
-  uint32_t* mbox_flags(int p) const {
-    return reinterpret_cast<uint32_t*>(static_cast<char*>(mbox_peer[p]) + (size_t)kP2PSlots * cfg.world_size * kP2PMaxDoubles * sizeof(double));
-  }
-  uint32_t* mbox_err() const { return mbox_flags(cfg.rank) + kP2PSlots * cfg.world_size; }
+  uint32_t* mbox_err() const { return static_cast<uint32_t*>(mbox); }
   // gradient exchange through peer memory (kernels_p2p.cu:k_xr_*): dense gradients, then the replicated tables' gradient tables
   int64_t xr_dense() const { return (L.dense_numel + 63) / 64 * 64; }
   int64_t xr_floats() const { return xr_dense() + (replicated() ? sp2_rep_floats(cfg.n_items, cfg.n_cates, cfg.n_users) : 0); }
@@ -301,10 +294,6 @@ int pamrec_bind(PamrecHandle h, const PamrecBuffers* bufs, void* stream) {
     return fail(h, "null buffer");
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) { cudaGetLastError(); return fail(h, "no CUDA device: the CUDA path is the only path"); }
-  const char* attn_env = getenv("PAMREC_ATTN");
-  const std::string attn = attn_env ? attn_env : "mma";
-  if (attn != "mma" && attn != "ffma") return fail(h, "PAMREC_ATTN=%s: the attention kernels are mma (the default) or ffma", attn.c_str());
-  h->attn_mma = attn == "mma" ? 1 : 0;
   h->buf = *bufs;
   if (init_encoder_kernels(h->cfg.max_seq_len)) return check_cuda(h, "shared-memory opt-in of the encoder kernels");
   if (h->cfg.model_kind == PAMREC_MODEL_SASREC && init_sas_kernels(h->cfg.max_seq_len))
@@ -569,6 +558,7 @@ static int sib_backward(PamrecHandle h, const PamrecBatch* b, cudaStream_t st);
 static int sib_apply(PamrecHandle h, const PamrecBatch* b, int64_t step, cudaStream_t st);
 static int sas_forward(PamrecHandle h, const PamrecBatch* b, int training, float* pred_out, cudaStream_t st);
 static int sas_backward(PamrecHandle h, const PamrecBatch* b, cudaStream_t st);
+static int head_forward(PamrecHandle h, const PamrecBatch* b, bool training, float* pred_out, cudaStream_t st);
 
 int pamrec_forward(PamrecHandle h, const PamrecBatch* b, int training, float* pred_out, void* stream) {
   if (int rc = check_batch(h, b, training != 0)) return rc;
@@ -578,37 +568,6 @@ int pamrec_forward(PamrecHandle h, const PamrecBatch* b, int training, float* pr
   if (h->sibling()) return sib_forward(h, b, training, pred_out, st);
   const Layout& L = h->L;
   const int B = b->batch, T = h->cfg.max_seq_len, N = B * T;
-  const int W = h->cfg.world_size;
-  const int Bg = b->global_batch > 0 ? b->global_batch : B * W;
-  const double cntN = (double)Bg * T, cntB = (double)Bg;
-  int64_t nl = 0;
-  int crc = 0;
-  // Training: batch statistics of the listed sets -> (mean, invstd), moving averages.  Data parallel: the column sums
-  // (plus, once, the listwise-group count) are first summed over ranks - through the peer mailboxes in ONE kernel that also
-  // finalises (kernels_p2p.cu), else NCCL all-reduce + finalize launches.
-  int p2p_slot = 0;
-  auto sync_finalize = [&](std::initializer_list<int> ids, double cnt, bool with_scalars) {
-    if (!training) return;
-    if (W > 1 && h->mbox_open) {
-      P2PArgs a;
-      memset(&a, 0, sizeof a);
-      for (int id : ids) { a.buf[a.nbuf] = h->bn[id].sums; a.n[a.nbuf++] = 2 * h->bn[id].C; a.bn[a.nbn] = h->bn[id]; a.count[a.nbn++] = cnt; }
-      if (with_scalars) { a.buf[a.nbuf] = h->wd("dp.scalars"); a.n[a.nbuf++] = 8; }
-      for (int p = 0; p < W; ++p) { a.peer_slots[p] = h->mbox_slots(p); a.peer_flags[p] = h->mbox_flags(p); }
-      a.world = W; a.rank = h->cfg.rank; a.slot = p2p_slot; a.epoch = ++h->mbox_epoch[p2p_slot]; a.err = h->mbox_err();
-      ++p2p_slot;
-      launch_p2p_allreduce(a, st); nl += 1;
-      return;
-    }
-    if (W > 1 && !crc) {
-      PAMREC_PROF("allreduce_bn_fwd", 1, st);
-      crc |= h->comm.group_start();
-      for (int id : ids) crc |= h->comm.all_reduce(h->bn[id].sums, 2 * (int64_t)h->bn[id].C, COMM_F64, st);
-      if (with_scalars) crc |= h->comm.all_reduce(h->wd("dp.scalars"), 8, COMM_F64, st);
-      crc |= h->comm.group_end();
-    }
-    for (int id : ids) { launch_bn_finalize(h->bn[id], cnt, st); nl += 1; }
-  };
   float* x0 = h->wf("x0");
   int* ctl = h->wi("bucket_ctl");
   // The bucket sort of the tokens depends on the play-ratio buckets of the batch only: on the side stream beside the gather
@@ -622,7 +581,6 @@ int pamrec_forward(PamrecHandle h, const PamrecBatch* b, int training, float* pr
     });
   }
   if (int rc = embed_forward(h, b, training != 0, x0, st)) return rc;
-  nl += 1;
   if (training && !h->sharded() && B > 0) {
     // the id sort / unique pass of the sparse backward depends on the batch only: run it beside the forward pass
     int prc = 0;
@@ -633,14 +591,9 @@ int pamrec_forward(PamrecHandle h, const PamrecBatch* b, int training, float* pr
     if (prc) return fail(h, "cub sort failed");
     h->plan_for = b->item_history; h->plan_rows = B;
   }
-  if (training && W > 1 && !h->use_head2()) {             // (the row-stationary head kernel counts them itself)
-    cudaMemsetAsync(h->wd("dp.scalars"), 0, 8 * sizeof(double), st);
-    launch_count_valid_groups(b->plays, B, h->wd("dp.scalars"), st);
-  }
   if (bucket_aside) cudaStreamWaitEvent(st, h->ev_bucket, 0);
   else launch_bucket_plan(b->item_loop_times_history, N, h->wi("bucket"), h->wi("perm"), ctl, h->wi("tile_bucket"),
                           h->wi("tile_begin"), h->wi("tile_count"), st);
-  nl += 3;
   const int max_tiles = N / kTokTile + kNB + 1;
   const float* xin = x0;
   for (int k = 0; k < 2; ++k) {
@@ -649,42 +602,70 @@ int pamrec_forward(PamrecHandle h, const PamrecBatch* b, int training, float* pr
     launch_proj_fwd(xin, h->wi("perm"), ctl, h->wi("tile_bucket"), h->wi("tile_begin"), h->wi("tile_count"), max_tiles,
                     h->P(o.wq), h->P(o.wk), h->P(o.wv), h->P(o.ln_a_beta), h->P(o.ln_a_gamma), h->wf(p + "qin"), h->wf(p + "Q"),
                     h->wf(p + "K"), h->wf(p + "V"), st);
-    if (h->attn_mma)
+    // the MMA kernel up to T = 128, the FFMA kernel beyond: attn_fwd per step on a B200 (1000 W) MMA vs FFMA 0.046 vs 0.066 ms on
+    // takatak_b1025_t50, 0.078 vs 0.099 ms on wechat_b500_t100, 2.18 vs 1.45 ms on long_b4095_t200 (no T in between measured)
+    if (T <= 128)
       launch_attn_fwd_mma(h->wf(p + "Q"), h->wf(p + "K"), h->wf(p + "V"), h->wf(p + "qin"), b->mask, h->wf(p + "y"), h->wf(p + "ml"), B, T, st);
     else
       launch_attn_fwd(h->wf(p + "Q"), h->wf(p + "K"), h->wf(p + "V"), h->wf(p + "qin"), b->mask, h->wf(p + "y"), h->wf(p + "ml"), B, T, st);
     float* hdbg = (training && (h->debug & PAMREC_DEBUG_SAVE_FFN_HIDDEN)) ? h->wf(k == 0 ? "d_Q" : "d_K") : nullptr;
     launch_ffn_fwd(h->wf(p + "y"), h->P(o.w1), h->P(o.b1), h->P(o.w2), h->P(o.b2), h->P(o.ln_b_beta), h->P(o.ln_b_gamma),
                    h->wf(p + "out"), hdbg, N, st);
-    nl += 3;
     xin = h->wf(p + "out");
   }
-  const float* H = xin;
-  BnSet* bn = h->bn;
   if (h->use_head2()) {
     // the whole head as ONE persistent cooperative kernel, row-stationary (kernels_head2.cu)
     HeadDyn d = head_dyn(h, b, training != 0, 0);
     d.pred = pred_out;
     if (launch_head2_fwd(h->head2, d, h->head2_grid, training ? "head_fwd" : "head_score", st)) return check_cuda(h, "cooperative head launch");
-    return check_cuda(h, "forward");
+  } else if (int rc = head_forward(h, b, training != 0, pred_out, st)) {
+    return rc;
   }
+  return check_cuda(h, "forward");
+}
+
+// The stand-alone head (kernels_head.cu): a launch per layer.  Training: batch statistics of the listed sets -> (mean, invstd), moving
+// averages; data parallel: the column sums (plus, once, the listwise-group count) are first summed over the ranks by NCCL.
+static int head_forward(PamrecHandle h, const PamrecBatch* b, bool training, float* pred_out, cudaStream_t st) {
+  const Layout& L = h->L;
+  const int B = b->batch, T = h->cfg.max_seq_len, N = B * T;
+  const int W = h->cfg.world_size;
+  const int Bg = b->global_batch > 0 ? b->global_batch : B * W;
+  const double cntN = (double)Bg * T, cntB = (double)Bg;
+  int crc = 0;
+  auto sync_finalize = [&](std::initializer_list<int> ids, double cnt, bool with_scalars) {
+    if (!training) return;
+    if (W > 1 && !crc) {
+      PAMREC_PROF("allreduce_bn_fwd", 1, st);
+      crc |= h->comm.group_start();
+      for (int id : ids) crc |= h->comm.all_reduce(h->bn[id].sums, 2 * (int64_t)h->bn[id].C, COMM_F64, st);
+      if (with_scalars) crc |= h->comm.all_reduce(h->wd("dp.scalars"), 8, COMM_F64, st);
+      crc |= h->comm.group_end();
+    }
+    for (int id : ids) launch_bn_finalize(h->bn[id], cnt, st);
+  };
+  if (training && W > 1) {
+    cudaMemsetAsync(h->wd("dp.scalars"), 0, 8 * sizeof(double), st);
+    launch_count_valid_groups(b->plays, B, h->wd("dp.scalars"), st);
+  }
+  const float* H = h->wf("blk1.out");
+  BnSet* bn = h->bn;
   if (!training) {
     for (int i = 0; i < BN_COUNT; ++i) launch_bn_eval_stat(bn[i], st);
-    nl += BN_COUNT;
   }
   // attention pooling score MLP (pamrec.py:273)
   {
     DenseP p = dense_p(H, kD, N, 1, kD, 20, h->P(L.score.w0), 0, h->P(L.score.b0), 0, h->wf("z1"), 20);
     p.out_sums = training ? bn[BN_S0].sums : nullptr;
-    launch_dense_fwd(p, st); nl += 1;
+    launch_dense_fwd(p, st);
     sync_finalize({BN_S0}, cntN, true);
     DenseP q = dense_p(h->wf("z1"), 20, N, 1, 20, 1, h->P(L.score.w1), 0, h->P(L.score.b1), 0, h->wf("z2"), 1);
     set_in_bn(q, bn[BN_S0]);
     q.out_sums = training ? bn[BN_S1].sums : nullptr;
-    launch_dense_fwd(q, st); nl += 1;
+    launch_dense_fwd(q, st);
     sync_finalize({BN_S1}, cntN, false);
   }
-  launch_pool_fwd(H, h->wf("z2"), bn[BN_S1], b->mask, h->wf("new_long"), B, T, st); nl += 1;
+  launch_pool_fwd(H, h->wf("z2"), bn[BN_S1], b->mask, h->wf("new_long"), B, T, st);
   // MMoE (pamrec.py:26-50)
   {
     DenseP e0 = dense_p(h->wf("new_long"), kD, B, 5, kD, 100, h->P(L.expert.w0), 4000, h->P(L.expert.b0), 100, h->wf("ze0"), 500);
@@ -695,7 +676,6 @@ int pamrec_forward(PamrecHandle h, const PamrecBatch* b, int training, float* pr
     for (int g = 0; g < 2; ++g) { g0.x_off[g] = 0; g0.z_off[g] = g * 64; }
     g0.out_sums = training ? bn[BN_G0].sums : nullptr;
     launch_dense_fwd(g0, st);
-    nl += 2;
     sync_finalize({BN_E0, BN_G0}, cntB, false);
     DenseP e1 = dense_p(h->wf("ze0"), 500, B, 5, 100, 64, h->P(L.expert.w1), 6400, h->P(L.expert.b1), 64, h->wf("ze1"), 320);
     for (int g = 0; g < 5; ++g) { e1.x_off[g] = g * 100; e1.z_off[g] = g * 64; }
@@ -707,32 +687,31 @@ int pamrec_forward(PamrecHandle h, const PamrecBatch* b, int training, float* pr
     set_in_bn(g1, bn[BN_G0]);
     g1.out_sums = training ? bn[BN_G1].sums : nullptr;
     launch_dense_fwd(g1, st);
-    nl += 2;
     sync_finalize({BN_E1, BN_G1}, cntB, false);
   }
-  launch_combine_fwd(h->wf("ze1"), h->wf("zg1"), bn[BN_E1], bn[BN_G1], h->wf("tgt"), h->wf("u"), B, st); nl += 1;
+  launch_combine_fwd(h->wf("ze1"), h->wf("zg1"), bn[BN_E1], bn[BN_G1], h->wf("tgt"), h->wf("u"), B, st);
   // towers: logit_fcn(main|tgt), valid_logit_fcn(sub|tgt), xilidu_logit_fcn(main|tgt)   pamrec.py:212-215, 71
   {
     DenseP t0 = dense_p(h->wf("u"), 168, B, 3, 84, 100, h->P(L.tower.w0), 8400, h->P(L.tower.b0), 100, h->wf("zt0"), 300);
     t0.x_off[0] = 0; t0.x_off[1] = 84; t0.x_off[2] = 0;
     for (int g = 0; g < 3; ++g) t0.z_off[g] = g * 100;
     t0.out_sums = training ? bn[BN_T0].sums : nullptr;
-    launch_dense_fwd(t0, st); nl += 1;
+    launch_dense_fwd(t0, st);
     sync_finalize({BN_T0}, cntB, false);
     DenseP t1 = dense_p(h->wf("zt0"), 300, B, 3, 100, 64, h->P(L.tower.w1), 6400, h->P(L.tower.b1), 64, h->wf("zt1"), 192);
     for (int g = 0; g < 3; ++g) { t1.x_off[g] = g * 100; t1.z_off[g] = g * 64; }
     set_in_bn(t1, bn[BN_T0]);
     t1.out_sums = training ? bn[BN_T1].sums : nullptr;
-    launch_dense_fwd(t1, st); nl += 1;
+    launch_dense_fwd(t1, st);
     sync_finalize({BN_T1}, cntB, false);
     DenseP to = dense_p(h->wf("zt1"), 192, B, 3, 64, 1, h->P(L.tower.wout), 64, h->P(L.tower.bout), 1, h->wf("logits"), 3);
     for (int g = 0; g < 3; ++g) { to.x_off[g] = g * 64; to.z_off[g] = g; }
     set_in_bn(to, bn[BN_T1]);
-    launch_dense_fwd(to, st); nl += 1;
+    launch_dense_fwd(to, st);
   }
-  if (pred_out) { launch_sigmoid_col0(h->wf("logits"), pred_out, B, st); nl += 1; }
+  if (pred_out) launch_sigmoid_col0(h->wf("logits"), pred_out, B, st);
   if (crc) return fail(h, "nccl: %s", h->comm.err.c_str());
-  return check_cuda(h, "forward");
+  return 0;
 }
 
 // ------------------------------------------------------------------------------------------
@@ -771,10 +750,7 @@ static HeadDyn head_dyn(PamrecHandle h, const PamrecBatch* b, bool training, int
   d.trace = h->head_trace ? reinterpret_cast<unsigned long long*>(h->head_bar + 64) + (slot0 ? 32 : 0) : nullptr;
   d.trace_cta = (h->head_trace && h->head_trace_cta) ? h->head_trace_cta + (slot0 ? 16 * 256 : 0) : nullptr;
   if (W > 1) {
-    for (int p = 0; p < W; ++p) {
-      d.peer_slots[p] = h->mbox_slots(p); d.peer_flags[p] = h->mbox_flags(p);
-      d.peer_ll[p] = reinterpret_cast<uint4*>(static_cast<char*>(h->mbox_peer[p]) + p2p_ll_offset(W));
-    }
+    for (int p = 0; p < W; ++p) d.peer_ll[p] = reinterpret_cast<uint4*>(static_cast<char*>(h->mbox_peer[p]) + p2p_ll_offset());
     d.p2p_epoch = ++h->coop_epoch; d.p2p_slot0 = slot0; d.p2p_err = h->mbox_err();
   }
   return d;
@@ -824,12 +800,10 @@ static int build_head(PamrecHandle h, cudaStream_t st) {
   return check_cuda(h, "head2");
 }
 
-int pamrec_backward(PamrecHandle h, const PamrecBatch* b, void* stream) {
-  if (int rc = check_batch(h, b, true)) return rc;
-  ProfBind _pb(h);
-  cudaStream_t st = (cudaStream_t)stream;
-  if (h->cfg.model_kind == PAMREC_MODEL_SASREC) return sas_backward(h, b, st);
-  if (h->sibling()) return sib_backward(h, b, st);
+// The stand-alone head's backward pass (kernels_head.cu), loss through attention pooling: the gradient of blk1.out ends in g_a, the
+// weight-gradient GEMMs (no consumer before the optimiser) run on the side stream.  Data parallel: the batch-norm gradient sums are
+// summed over the ranks by NCCL.  Returns non-zero when an NCCL call failed; the caller reports it after joining the side stream.
+static int head_backward(PamrecHandle h, const PamrecBatch* b, cudaStream_t st) {
   const Layout& L = h->L;
   const int B = b->batch, T = h->cfg.max_seq_len, N = B * T;
   const int W = h->cfg.world_size;
@@ -837,43 +811,17 @@ int pamrec_backward(PamrecHandle h, const PamrecBatch* b, void* stream) {
   const double cntN = (double)Bg * T, cntB = (double)Bg;
   const float gs = 1.0f / (float)W;    // BN parameter gradients are already global: the dense all-reduce sums W copies
   BnSet* bn = h->bn;
-  int64_t nl = 0;
   int crc = 0;
   const float* Pb = h->buf.dense_param;
-  cudaMemsetAsync(h->buf.dense_grad, 0, (size_t)L.dense_numel * 4, st);
-  cudaMemsetAsync(h->wd("loss_acc"), 0, 8 * sizeof(double), st);
-  cudaMemsetAsync(h->wd("sp_normsq"), 0, 8 * sizeof(double), st);
-  const bool rows = h->use_head2();
-  const bool coop = rows;
-  if (!coop) {
   launch_loss(h->wf("logits"), b->labels_satisfied, b->labels_play, b->plays, h->wf("d_logits"), h->wd("loss_acc"), B, Bg,
               W > 1 ? h->wd("dp.scalars") : nullptr, h->cfg.fuzhu_weight, h->cfg.order_weight,
-              h->cfg.loss_kind == PAMREC_LOSS_SOFTMAX ? h->cfg.softmax_group : 0, st); nl += 1;
-  }
+              h->cfg.loss_kind == PAMREC_LOSS_SOFTMAX ? h->cfg.softmax_group : 0, st);
   // Batch-norm backward is folded into the dense kernels (common.cuh: BnGrad / BnGradOut): the kernel that produces a
   // gradient buffer also accumulates the two column sums of its layer's BN, the consumers turn dA into dz while loading.
   // Buffers produced by the mixing / pooling kernels get their sums from k_bn_bwd_stats.  Data parallel: sums over ranks.
   cudaMemsetAsync(h->wd("bn.bsums"), 0, (size_t)L.ws[L.ws_index.at("bn.bsums")].numel * sizeof(double), st);
-  if (rows) {
-    // loss + the dX chain of the head as ONE persistent cooperative kernel; the weight gradients (no consumer before the
-    // optimiser) run on the side stream beside the encoder's backward pass
-    HeadDyn d = head_dyn(h, b, true, 12);
-    if (launch_head2_bwd(h->head2, d, h->head2_grid, st)) return check_cuda(h, "cooperative head launch");
-    h->fork(st, [&](cudaStream_t s2) { launch_head2_dw(h->head2, B, s2); });
-  }
-  int p2p_slot = 6;
   auto sync_bsums = [&](std::initializer_list<int> ids) {
     if (W == 1 || crc) return;
-    if (h->mbox_open) {
-      P2PArgs a;
-      memset(&a, 0, sizeof a);
-      for (int id : ids) { a.buf[a.nbuf] = bn[id].bsums; a.n[a.nbuf++] = 2 * bn[id].C; }
-      for (int p = 0; p < W; ++p) { a.peer_slots[p] = h->mbox_slots(p); a.peer_flags[p] = h->mbox_flags(p); }
-      a.world = W; a.rank = h->cfg.rank; a.slot = p2p_slot; a.epoch = ++h->mbox_epoch[p2p_slot]; a.err = h->mbox_err();
-      ++p2p_slot;
-      launch_p2p_allreduce(a, st);
-      return;
-    }
     PAMREC_PROF("allreduce_bn_bwd", 1, st);
     crc |= h->comm.group_start();
     for (int id : ids) crc |= h->comm.all_reduce(bn[id].bsums, 2 * (int64_t)bn[id].C, COMM_F64, st);
@@ -890,7 +838,6 @@ int pamrec_backward(PamrecHandle h, const PamrecBatch* b, void* stream) {
   auto dw_bn = [&](DenseDwP& w, int id, const float* Z, double cnt) {
     w.g = grad_of(id, Z, cnt); w.g_dgamma = bn[id].dgamma; w.g_dbeta = bn[id].dbeta; w.g_C = bn[id].C; w.g_scale = gs;
   };
-  if (!coop) {
   // ---- towers
   {
     DenseDwP w = dw_p(h->wf("zt1"), 192, B, 3, 64, 1, h->wf("d_logits"), 3, h->G(L.tower.wout), 64, h->G(L.tower.bout), 1);
@@ -901,7 +848,6 @@ int pamrec_backward(PamrecHandle h, const PamrecBatch* b, void* stream) {
     for (int g = 0; g < 3; ++g) dx_add(x, g, g * 64, g, L.tower.wout + g * 64, 1);
     x.o = out_of(BN_T1, h->wf("zt1"));
     launch_dense_dx(x, st);
-    nl += 2;
     sync_bsums({BN_T1});
     DenseDwP w1 = dw_p(h->wf("zt0"), 300, B, 3, 100, 64, h->wf("d_t1"), 192, h->G(L.tower.w1), 6400, h->G(L.tower.b1), 64);
     for (int g = 0; g < 3; ++g) { w1.x_off[g] = g * 100; w1.z_off[g] = g * 64; }
@@ -913,7 +859,6 @@ int pamrec_backward(PamrecHandle h, const PamrecBatch* b, void* stream) {
     x1.g = grad_of(BN_T1, h->wf("zt1"), cntB);
     x1.o = out_of(BN_T0, h->wf("zt0"));
     launch_dense_dx(x1, st);
-    nl += 2;
     sync_bsums({BN_T0});
     DenseDwP w0 = dw_p(h->wf("u"), 168, B, 3, 84, 100, h->wf("d_t0"), 300, h->G(L.tower.w0), 8400, h->G(L.tower.b0), 100);
     w0.x_off[0] = 0; w0.x_off[1] = 84; w0.x_off[2] = 0;
@@ -926,15 +871,13 @@ int pamrec_backward(PamrecHandle h, const PamrecBatch* b, void* stream) {
     dx_add(x0, 1, 84, 100, L.tower.w0 + 8400, 100);
     x0.g = grad_of(BN_T0, h->wf("zt0"), cntB);
     launch_dense_dx(x0, st);
-    nl += 2;
   }
   launch_combine_bwd(h->wf("ze1"), h->wf("zg1"), bn[BN_E1], bn[BN_G1], h->wf("d_u"), h->wf("d_e1"), h->wf("d_g1"),
-                     h->wf("d_tgt"), B, st); nl += 1;
+                     h->wf("d_tgt"), B, st);
   // ---- MMoE
   {
     launch_bn_bwd_stats(bn[BN_E1], h->wf("d_e1"), h->wf("ze1"), B, st);
     launch_bn_bwd_stats(bn[BN_G1], h->wf("d_g1"), h->wf("zg1"), B, st);
-    nl += 2;
     sync_bsums({BN_E1, BN_G1});
     DenseDwP we = dw_p(h->wf("ze0"), 500, B, 5, 100, 64, h->wf("d_e1"), 320, h->G(L.expert.w1), 6400, h->G(L.expert.b1), 64);
     for (int g = 0; g < 5; ++g) { we.x_off[g] = g * 100; we.z_off[g] = g * 64; }
@@ -956,7 +899,6 @@ int pamrec_backward(PamrecHandle h, const PamrecBatch* b, void* stream) {
     xg.g = grad_of(BN_G1, h->wf("zg1"), cntB);
     xg.o = out_of(BN_G0, h->wf("zg0"));
     launch_dense_dx(xg, st);
-    nl += 4;
     sync_bsums({BN_E0, BN_G0});
     DenseDwP we0 = dw_p(h->wf("new_long"), kD, B, 5, kD, 100, h->wf("d_e0"), 500, h->G(L.expert.w0), 4000, h->G(L.expert.b0), 100);
     for (int g = 0; g < 5; ++g) { we0.x_off[g] = 0; we0.z_off[g] = g * 100; }
@@ -974,37 +916,57 @@ int pamrec_backward(PamrecHandle h, const PamrecBatch* b, void* stream) {
     for (int g = 0; g < 2; ++g) dx_add(xg0, 0, 0, g * 64, L.gate.w0 + (int64_t)g * 2560, 64);
     xg0.g = grad_of(BN_G0, h->wf("zg0"), cntB);
     launch_dense_dx(xg0, st);
-    nl += 4;
   }
-  }  // !coop (towers, mixing, MMoE)
   // ---- attention pooling
   const float* H = h->wf("blk1.out");
   float* g_a = h->wf("g_a");
-  float* g_b = h->wf("g_b");
-  if (!coop) {
-    launch_pool_bwd(H, h->wf("z2"), bn[BN_S1], b->mask, h->wf("d_new_long"), h->wf("d_z2"), g_a, B, T, st); nl += 1;
-    launch_bn_bwd_stats(bn[BN_S1], h->wf("d_z2"), h->wf("z2"), N, st); nl += 1;
-    sync_bsums({BN_S1});
-    DenseDwP w1 = dw_p(h->wf("z1"), 20, N, 1, 20, 1, h->wf("d_z2"), 1, h->G(L.score.w1), 0, h->G(L.score.b1), 0);
-    set_in_bn_dw(w1, bn[BN_S0]);
-    dw_bn(w1, BN_S1, h->wf("z2"), cntN);
-    h->fork(st, [&](cudaStream_t s2) { launch_dense_dw(w1, s2); });
-    DenseDxP x1 = dx_p(h->wf("d_z2"), 1, N, 20, Pb, h->wf("d_a1"), 20, 0);
-    dx_add(x1, 0, 0, 0, L.score.w1, 1);
-    x1.g = grad_of(BN_S1, h->wf("z2"), cntN);
-    x1.o = out_of(BN_S0, h->wf("z1"));
-    launch_dense_dx(x1, st);
-    nl += 2;
-    sync_bsums({BN_S0});
-    DenseDwP w0 = dw_p(H, kD, N, 1, kD, 20, h->wf("d_a1"), 20, h->G(L.score.w0), 0, h->G(L.score.b0), 0);
-    dw_bn(w0, BN_S0, h->wf("z1"), cntN);
-    h->fork(st, [&](cudaStream_t s2) { launch_dense_dw(w0, s2); });
-    DenseDxP x0 = dx_p(h->wf("d_a1"), 20, N, kD, Pb, g_a, kD, 1);
-    dx_add(x0, 0, 0, 0, L.score.w0, 20);
-    x0.g = grad_of(BN_S0, h->wf("z1"), cntN);
-    launch_dense_dx(x0, st);
-    nl += 2;
+  launch_pool_bwd(H, h->wf("z2"), bn[BN_S1], b->mask, h->wf("d_new_long"), h->wf("d_z2"), g_a, B, T, st);
+  launch_bn_bwd_stats(bn[BN_S1], h->wf("d_z2"), h->wf("z2"), N, st);
+  sync_bsums({BN_S1});
+  DenseDwP w1 = dw_p(h->wf("z1"), 20, N, 1, 20, 1, h->wf("d_z2"), 1, h->G(L.score.w1), 0, h->G(L.score.b1), 0);
+  set_in_bn_dw(w1, bn[BN_S0]);
+  dw_bn(w1, BN_S1, h->wf("z2"), cntN);
+  h->fork(st, [&](cudaStream_t s2) { launch_dense_dw(w1, s2); });
+  DenseDxP x1 = dx_p(h->wf("d_z2"), 1, N, 20, Pb, h->wf("d_a1"), 20, 0);
+  dx_add(x1, 0, 0, 0, L.score.w1, 1);
+  x1.g = grad_of(BN_S1, h->wf("z2"), cntN);
+  x1.o = out_of(BN_S0, h->wf("z1"));
+  launch_dense_dx(x1, st);
+  sync_bsums({BN_S0});
+  DenseDwP w0 = dw_p(H, kD, N, 1, kD, 20, h->wf("d_a1"), 20, h->G(L.score.w0), 0, h->G(L.score.b0), 0);
+  dw_bn(w0, BN_S0, h->wf("z1"), cntN);
+  h->fork(st, [&](cudaStream_t s2) { launch_dense_dw(w0, s2); });
+  DenseDxP x0 = dx_p(h->wf("d_a1"), 20, N, kD, Pb, g_a, kD, 1);
+  dx_add(x0, 0, 0, 0, L.score.w0, 20);
+  x0.g = grad_of(BN_S0, h->wf("z1"), cntN);
+  launch_dense_dx(x0, st);
+  return crc;
+}
+
+int pamrec_backward(PamrecHandle h, const PamrecBatch* b, void* stream) {
+  if (int rc = check_batch(h, b, true)) return rc;
+  ProfBind _pb(h);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (h->cfg.model_kind == PAMREC_MODEL_SASREC) return sas_backward(h, b, st);
+  if (h->sibling()) return sib_backward(h, b, st);
+  const Layout& L = h->L;
+  const int B = b->batch, T = h->cfg.max_seq_len, N = B * T;
+  int crc = 0;
+  cudaMemsetAsync(h->buf.dense_grad, 0, (size_t)L.dense_numel * 4, st);
+  cudaMemsetAsync(h->wd("loss_acc"), 0, 8 * sizeof(double), st);
+  cudaMemsetAsync(h->wd("sp_normsq"), 0, 8 * sizeof(double), st);
+  if (h->use_head2()) {
+    cudaMemsetAsync(h->wd("bn.bsums"), 0, (size_t)L.ws[L.ws_index.at("bn.bsums")].numel * sizeof(double), st);
+    // loss + the dX chain of the head as ONE persistent cooperative kernel; the weight gradients (no consumer before the
+    // optimiser) run on the side stream beside the encoder's backward pass
+    HeadDyn d = head_dyn(h, b, true, 12);
+    if (launch_head2_bwd(h->head2, d, h->head2_grid, st)) return check_cuda(h, "cooperative head launch");
+    h->fork(st, [&](cudaStream_t s2) { launch_head2_dw(h->head2, B, s2); });
+  } else {
+    crc = head_backward(h, b, st);
   }
+  float* g_a = h->wf("g_a");
+  float* g_b = h->wf("g_b");
   // ---- encoder blocks (grad of blk1.out is in g_a)
   const int max_tiles = N / kTokTile + kNB + 1;
   int* ctl = h->wi("bucket_ctl");
@@ -1018,7 +980,7 @@ int pamrec_backward(PamrecHandle h, const PamrecBatch* b, void* stream) {
                    h->G(o.w1), h->G(o.b1), h->G(o.w2), h->G(o.b2), h->G(o.ln_b_beta), h->G(o.ln_b_gamma), N, st);
     // backward: the MMA kernel keeps K, V, Q and dY of a sample in shared memory (141 KB at T = 200: one CTA per SM), measured slower
     // than the FFMA kernel there (8.5 vs 6.4 ms per step on long_b4095_t200) and faster below (T = 100: 230 vs 292 us, T = 50: 152 vs 196 us)
-    if (h->attn_mma && T <= 128)
+    if (T <= 128)
       launch_attn_bwd_mma(h->wf(p + "Q"), h->wf(p + "K"), h->wf(p + "V"), h->wf("d_y"), h->wf(p + "y"), h->wf(p + "qin"), h->wf(p + "ml"),
                           b->mask, h->wf("d_Q"), h->wf("d_K"), h->wf("d_V"), B, T, st);
     else
@@ -1027,11 +989,10 @@ int pamrec_backward(PamrecHandle h, const PamrecBatch* b, void* stream) {
     launch_proj_bwd(xin, h->wf("d_y"), h->wf("d_Q"), h->wf("d_K"), h->wf("d_V"), h->wi("perm"), ctl, h->wi("tile_bucket"),
                     h->wi("tile_begin"), h->wi("tile_count"), max_tiles, h->P(o.wq), h->P(o.wk), h->P(o.wv), h->P(o.ln_a_beta),
                     h->P(o.ln_a_gamma), gin, h->G(o.wq), h->G(o.wk), h->G(o.wv), h->G(o.ln_a_beta), h->G(o.ln_a_gamma), st);
-    nl += 3;
   }
   // dX0 is in g_a
   launch_embed_bwd_reduce(g_a, h->wf("d_tgt"), h->wf("d_tgt_total"), h->G(L.pos), h->wd("sp_normsq") + 4,
-                          h->sharded() ? nullptr : h->wd("sp_normsq"), B, T, st); nl += 2;
+                          h->sharded() ? nullptr : h->wd("sp_normsq"), B, T, st);
   h->join(st);                    // the head's weight-gradient GEMMs (side stream) are complete from here on
   if (crc) return fail(h, "nccl: %s", h->comm.err.c_str());
   return check_cuda(h, "backward");
@@ -1080,7 +1041,6 @@ int pamrec_apply_gradients(PamrecHandle h, const PamrecBatch* b, int64_t step, v
   double* reg = h->wd("loss_acc") + 3;
   void* tmp = h->ws<char>("cub_temp");
   size_t tmp_bytes = (size_t)L.ws[L.ws_index.at("cub_temp")].numel;
-  int64_t nl = 0;
   bool dense_aside = false;
   const float* dX0 = h->wf("g_a");
   const float* dT = h->wf("d_tgt_total");
@@ -1155,7 +1115,7 @@ int pamrec_apply_gradients(PamrecHandle h, const PamrecBatch* b, int64_t step, v
     if (planned) cudaStreamWaitEvent(st, h->ev_plan, 0);
     else if (launch_sp2_plan(s2, tmp, tmp_bytes, st)) return fail(h, "cub sort failed");
     launch_sp2_walk(s2, ap, st);
-    nl += 10;
+   
     if (h->replicated()) {
       // replicated tables: gradient tables + touch counts, dense gradients, clip norms and losses summed over the ranks
       Sp2 s3 = s2;                                           // after the all-reduce: the summed gradient tables
@@ -1178,11 +1138,11 @@ int pamrec_apply_gradients(PamrecHandle h, const PamrecBatch* b, int64_t step, v
       }
       launch_sp2_rep_l2(s3, st);
       launch_sp2_adam_sweep(s3, ap, c.sparse_adam_mode == PAMREC_ADAM_LAZY ? 1 : 0, st);
-      nl += 3;
+     
     } else if (s2.mode == SP2_FUSED) {
-      launch_sp2_lazy_finish(s2, ap, st); nl += 1;
+      launch_sp2_lazy_finish(s2, ap, st);
     } else {
-      launch_sp2_adam_sweep(s2, ap, 0, st); nl += 1;
+      launch_sp2_adam_sweep(s2, ap, 0, st);
     }
   }
   const int n_seg = (int)L.dense.size();
@@ -1196,7 +1156,7 @@ int pamrec_apply_gradients(PamrecHandle h, const PamrecBatch* b, int64_t step, v
                       c.is_clip_norm, st);
   }
   launch_finish_losses(h->wd("loss_acc"), h->wf("losses"), h->sharded() ? nullptr : h->wd("sp2.l2sq"), c.embed_l2, h->wd("sp_normsq"), st);
-  nl += 3;
+ 
   return check_cuda(h, "apply_gradients");
 }
 

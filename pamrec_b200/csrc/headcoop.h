@@ -11,7 +11,6 @@ struct HeadDyn {
   const int* mask; const float* y_sat; const float* y_play; const float* plays;
   float fuzhu_w, order_w; int sm_group;
   unsigned* bar;                                    // [0] arrivals [2] error word [32] release epoch (own 128-byte line)
-  double* peer_slots[kP2PMaxWorld]; uint32_t* peer_flags[kP2PMaxWorld];
   uint32_t p2p_epoch; int p2p_slot0; uint32_t* p2p_err;
   uint4* peer_ll[kP2PMaxWorld];                     // flag-in-data mailboxes [slot][rank][kP2PMaxDoubles] (kernels.h:p2p_ll_offset)
   unsigned long long* trace;                        // [32] %globaltimer of the kernel start ([31]) and of every barrier release; may be null

@@ -54,7 +54,7 @@ void launch_proj_bwd(const float* X, const float* dY, const float* dQ, const flo
                      const float* Wq, const float* Wk, const float* Wv, const float* ln_beta, const float* ln_gamma,
                      float* dX, float* dWq, float* dWk, float* dWv, float* dbeta, float* dgamma, cudaStream_t st);
 
-// ---- kernels_attn_mma.cu (attention forward + backward on warp-level tensor-core MMAs, 3xTF32; the default)
+// ---- kernels_attn_mma.cu (attention forward + backward on warp-level tensor-core MMAs, 3xTF32; used up to T = 128)
 int init_attn_mma_kernels(int max_T);
 void launch_attn_fwd_mma(const float* Q, const float* K, const float* V, const float* QIN, const int* mask, float* Y, float* ML, int B, int T,
                          cudaStream_t st);
@@ -197,29 +197,18 @@ void launch_sas_final_fwd(const float* SEQ, const int* mask, const float* tgt, f
 void launch_sas_final_bwd(const float* dU, const int* mask, float* dSEQ, float* dTgt, int B, int T, int S, cudaStream_t st);
 void launch_sas_pos_bwd(const float* dX0, float* dPos, double* normsq, int B, int T, int S, cudaStream_t st);
 
-// ---- kernels_p2p.cu (small all-reduces through NVLink peer mailboxes)
+// ---- kernels_p2p.cu + kernels_head2.cu (data-parallel exchanges through NVLink peer mailboxes)
 constexpr int kP2PMaxDoubles = 2048;     // payload capacity of one mailbox slot (expert + gate layer-0 sums: 1256)
 constexpr int kP2PSlots = 24;            // sync points per step (each has its own slot): 12 forward + 12 backward barriers
 constexpr int kP2PMaxWorld = 8;
-struct P2PArgs {
-  double* buf[3]; int n[3]; int nbuf;                     // buffers reduced in place (concatenated in the slot)
-  double* peer_slots[kP2PMaxWorld];                       // every rank's mailbox payload area [slot][rank][kP2PMaxDoubles]
-  uint32_t* peer_flags[kP2PMaxWorld];                     // every rank's mailbox flags [slot][rank]
-  int world, rank, slot; uint32_t epoch;
-  uint32_t* err;                                          // this rank's error word (0 = ok)
-  BnSet bn[2]; double count[2]; int nbn;                  // optional fused batch-norm finalize
-};
-void launch_p2p_allreduce(const P2PArgs& a, cudaStream_t st);
-// payload | flags | error word (k_p2p_allreduce), then the flag-in-data region of the persistent head kernels: 16 bytes per double
-// ({low word, epoch, high word, epoch}: the arrival of the data IS the signal - one NVLink trip per exchange instead of
+// A mailbox starts with a 256-byte header whose first word is the rank's error word (0 = ok; a peer that never arrived: 1 + slot from
+// the persistent head kernels, 200 + flag set from k_xr_*).  Then the flag-in-data region of the persistent head kernels: 16 bytes
+// per double ({low word, epoch, high word, epoch}: the arrival of the data IS the signal - one NVLink trip per exchange instead of
 // payload, system fence, flag)
-inline size_t p2p_ll_offset(int world) {
-  const size_t b = (size_t)kP2PSlots * world * kP2PMaxDoubles * sizeof(double) + (size_t)kP2PSlots * world * sizeof(uint32_t) + 256;
-  return (b + 255) / 256 * 256;
-}
+constexpr size_t p2p_ll_offset() { return 256; }
 // ... then the gradient exchange region of k_xr_* (kernels_p2p.cu): flags | scalars | own contribution | reduced result
 constexpr int kXrScalars = 16;           // doubles per rank travelling with the gradients (8 clip norms + 4 loss sums)
-inline size_t p2p_xr_offset(int world) { return (p2p_ll_offset(world) + (size_t)kP2PSlots * world * kP2PMaxDoubles * 16 + 255) / 256 * 256; }
+inline size_t p2p_xr_offset(int world) { return (p2p_ll_offset() + (size_t)kP2PSlots * world * kP2PMaxDoubles * 16 + 255) / 256 * 256; }
 inline int64_t p2p_xr_cap(int world, int64_t n_floats) { const int64_t q = 64 * (int64_t)world; return (n_floats + q - 1) / q * q; }
 inline size_t p2p_xr_header_bytes() { return 512 + (size_t)kP2PMaxWorld * kXrScalars * sizeof(double); }
 inline size_t p2p_mailbox_bytes(int world, int64_t xr_floats) {

@@ -6,7 +6,8 @@
 // and weight gradient - runs on the tensor cores as an error-compensated 3xTF32 mma.sync (mma.cuh); LayerNorm and
 // its backward are evaluated in the MMA fragment layout (row sums are 4-lane shuffles).  Tokens are bucket-sorted
 // first so that a CTA needs exactly one (Wq,Wk,Wv)[bucket] triple: the reference instead materialises a
-// [B,T,40,40] gather per matrix (pamrec.py:714-728).  Attention: one thread per query row, see k_attn_fwd.
+// [B,T,40,40] gather per matrix (pamrec.py:714-728).  Attention beyond T = 128 (up to there: kernels_attn_mma.cu): one thread
+// per query row, see k_attn_fwd.
 #include "kernels.h"
 #include "mma.cuh"
 

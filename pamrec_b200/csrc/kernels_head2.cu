@@ -16,7 +16,7 @@
 //     so it is the same column kernel; dW = act(x)^T dz has no consumer before the optimiser and runs as k_head2_dw on the
 //     side stream while the encoder's backward pass runs on the main stream.
 // Grid barrier with a leader section (batch-norm finalize, moving statistics, gamma / beta gradients, data parallel: all-reduce
-// of the fp64 sums through the NVLink peer mailboxes, kernels_p2p.cu protocol) as before.
+// of the fp64 sums through the NVLink peer mailboxes, leader_p2p) as before.
 #include <cstdio>
 
 #include "head2.h"

@@ -1,15 +1,5 @@
-// Small all-reduces over NVLink peer memory, fused with what follows them.
-//
-// The data-parallel step synchronises twelve tiny fp64 vectors (batch-norm column sums, <= 1000 values each).  A
-// library all-reduce costs a launch plus a protocol round trip per call; here ONE single-CTA kernel per rank does the
-// whole exchange through mailboxes that every rank maps from its peers (cudaIpc, api.cu): it stores its contribution
-// into slot [sync point][own rank] of every peer's mailbox (plain stores that travel over NVLink), publishes an epoch
-// flag after a system-scope fence, spins on the flags of its own mailbox, sums the W contributions in rank order (so
-// every rank gets bit-identical results) and - forward pass - finalises the batch-norm statistics in the same kernel.
-//
-// Re-use of a slot is safe without a second handshake: a rank reaches sync point k of step i+1 only after it has
-// passed the later sync points of step i, which need every peer's contribution, which the peer enqueues after its own
-// read of slot k (stream order).  A bounded spin turns a lost peer into an error word instead of a hang.
+// Gradient all-reduce over NVLink peer memory (k_xr_*), through the exchange region of the mailboxes that every rank maps from its
+// peers (cudaIpc, api.cu).
 #include "kernels.h"
 
 namespace pamrec {
@@ -19,58 +9,6 @@ __device__ __forceinline__ uint32_t ld_flag(const uint32_t* p) {
   uint32_t v;
   asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
   return v;
-}
-
-__global__ void __launch_bounds__(256) k_p2p_allreduce(const P2PArgs a) {
-  const int tid = threadIdx.x;
-  int total = 0;
-  for (int b = 0; b < a.nbuf; ++b) total += a.n[b];
-  // 1. push this rank's contribution into every mailbox (own one included)
-  for (int i = tid; i < total; i += blockDim.x) {
-    int b = 0, o = i;
-    while (o >= a.n[b]) { o -= a.n[b]; ++b; }
-    const double v = a.buf[b][o];
-    for (int p = 0; p < a.world; ++p) a.peer_slots[p][(size_t)(a.slot * a.world + a.rank) * kP2PMaxDoubles + i] = v;
-  }
-  __threadfence_system();
-  __syncthreads();
-  if (tid < a.world) st_flag(a.peer_flags[tid] + a.slot * a.world + a.rank, a.epoch);
-  // 2. wait for every rank's contribution to arrive in this rank's mailbox
-  if (tid < a.world) {
-    const uint32_t* f = a.peer_flags[a.rank] + a.slot * a.world + tid;
-    uint32_t spins = 0;
-    while ((int32_t)(ld_flag(f) - a.epoch) < 0) {
-      if (++spins > (1u << 27)) { *a.err = 1u + (uint32_t)a.slot; break; }
-      __nanosleep(20);
-    }
-  }
-  __syncthreads();
-  // 3. sum in rank order, bypassing L1 (the slots were written by other GPUs)
-  const double* mine = a.peer_slots[a.rank] + (size_t)a.slot * a.world * kP2PMaxDoubles;
-  for (int i = tid; i < total; i += blockDim.x) {
-    double s = 0.0;
-    for (int p = 0; p < a.world; ++p) s += __ldcg(mine + (size_t)p * kP2PMaxDoubles + i);
-    int b = 0, o = i;
-    while (o >= a.n[b]) { o -= a.n[b]; ++b; }
-    a.buf[b][o] = s;
-  }
-  if (a.nbn == 0) return;
-  __syncthreads();
-  // 4. batch-norm finalize of the sets whose sums were just reduced (same arithmetic as k_bn_finalize)
-  for (int k = 0; k < a.nbn; ++k) {
-    const BnSet& s = a.bn[k];
-    for (int c = tid; c < s.C; c += blockDim.x) {
-      const double mean = s.sums[2 * c] / a.count[k];
-      double var = s.sums[2 * c + 1] / a.count[k] - mean * mean;
-      if (var < 0.0) var = 0.0;
-      s.stat[2 * c] = (float)mean;
-      s.stat[2 * c + 1] = (float)(1.0 / sqrt(var + (double)kBnEps));
-      s.mmean[c] -= (s.mmean[c] - (float)mean) * kBnDecay;
-      s.mvar[c] -= (s.mvar[c] - (float)var) * kBnDecay;
-      s.sums[2 * c] = 0.0;
-      s.sums[2 * c + 1] = 0.0;
-    }
-  }
 }
 
 // ------------------------------------------------------------------------------------------ gradient all-reduce over peer memory
@@ -166,11 +104,6 @@ void launch_xr_allreduce(const XrArgs& a, float* dense_grad_out, cudaStream_t st
   k_xr_pack<<<g_pack, kXrThreads, 0, st>>>(a);
   k_xr_reduce<<<g_red, kXrThreads, 0, st>>>(a);
   k_xr_finish<<<g_pack, kXrThreads, 0, st>>>(a, dense_grad_out);
-}
-
-void launch_p2p_allreduce(const P2PArgs& a, cudaStream_t st) {
-  PAMREC_PROF("p2p_allreduce", 1, st);
-  k_p2p_allreduce<<<1, 256, 0, st>>>(a);
 }
 
 }  // namespace pamrec

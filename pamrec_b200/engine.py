@@ -227,7 +227,8 @@ class Engine:
         torch.cuda.set_device(self.device)
         self._check(self.lib.pamrec_comm_init(self.handle, cpath, box[0]))
         if self.world <= 8 and os.environ.get("PAMREC_NO_MAILBOX", "0") != "1":
-            # NVLink peer mailboxes for the small all-reduces (kernels_p2p.cu): exchange the cudaIpc handles
+            # NVLink peer mailboxes for the batch-norm sums and the gradients (kernels_head2.cu, kernels_p2p.cu): exchange the
+            # cudaIpc handles
             buf = C.create_string_buffer(L.IPC_HANDLE_BYTES)
             self._check(self.lib.pamrec_comm_mailbox_create(self.handle, buf))
             handles = [None] * self.world

@@ -307,8 +307,8 @@ def test_lazy_fused_adam_equals_dense_exact_on_the_first_step(shape):
     lazy.close(); exact.close()
 
 
-def test_error_paths(monkeypatch):
-    from pamrec_b200.engine import Engine, PamrecError
+def test_error_paths():
+    from pamrec_b200.engine import PamrecError
     nu, ni, nc, T, B = 50, 300, 20, 12, 20
     om, eng = _setup(nu, ni, nc, T, B, seed=1)
     bad = O.make_batch(1, 10, T, nu, ni, nc)
@@ -320,40 +320,46 @@ def test_error_paths(monkeypatch):
     with pytest.raises(PamrecError):          # larger than max_batch
         eng.forward(eng.upload(big), training=False)
     eng.close()
-    monkeypatch.setenv("PAMREC_ATTN", "tc")
-    tc = Engine(nu, ni, nc, T, B)
-    with pytest.raises(PamrecError, match="PAMREC_ATTN"):     # the attention kernels are mma or ffma
-        tc.allocate()
-    tc.close()
 
 
 @pytest.mark.parametrize("T,B", [(12, 20), (50, 130), (100, 35), (200, 10), (256, 5)])
-def test_attention_mma_and_ffma_paths_agree(T, B, monkeypatch):
-    """The default attention kernels (warp-level 3xTF32 MMAs over the live keys, kernels_attn_mma.cu) against the FFMA kernels
-    (PAMREC_ATTN=ffma, kernels_encoder.cu) on the same batch - including a sample without any live key (uniform weights) and
-    arbitrary, non-prefix masks: outputs, saved row statistics and all three gradients."""
+def test_attention_matches_oracle(T, B):
+    """The attention kernels against the fp64 oracle on arbitrary, non-prefix masks, including a listwise group without any live
+    key (uniform weights): warp-level 3xTF32 MMAs over the live keys up to T = 128 (kernels_attn_mma.cu), the FFMA kernels of
+    kernels_encoder.cu beyond - outputs, saved row statistics and all three gradients."""
+    from pamrec_b200 import _lib as L
+    from relu_masks import engine_relu_masks
     nu, ni, nc = 200, 2000, 40
+    om, eng = _setup(nu, ni, nc, T, B, seed=11)
+    om.proj = "grouped"
     batch = O.make_batch(21, B, T, nu, ni, nc)
     rng = np.random.default_rng(3)
     batch["mask"][5:10] = 0                                             # one listwise group without history
     batch["mask"][10:15] = (rng.random((1, T)) < 0.5).astype(np.int32)  # holes in the middle of a history
-    got = {}
-    for mode in ("ffma", "mma"):
-        monkeypatch.setenv("PAMREC_ATTN", mode)
-        om, eng = _setup(nu, ni, nc, T, B, seed=11)
-        db = eng.upload(batch)
-        eng.forward(db, training=True, want_pred=False)
-        eng.backward(db)
-        torch.cuda.synchronize()
-        got[mode] = {k: eng.ws(k, B).cpu().numpy().copy() for k in ("blk0.y", "blk1.y", "blk0.ml", "blk1.ml", "d_Q", "d_K", "d_V", "g_a")}
-        got[mode]["logits"] = eng.ws("logits", B).cpu().numpy().copy()
-        eng.close()
-    for k in got["mma"]:
-        a, b = got["ffma"][k].astype(np.float64), got["mma"][k].astype(np.float64)
-        if k.endswith(".ml"):
-            # row maximum and row sum: the sum is relative to the maximum, which the two kernels round differently
-            assert np.allclose(a[..., 0], b[..., 0], rtol=1e-5, atol=1e-5), k
-            assert np.allclose(a[..., 1], b[..., 1], rtol=1e-4), k
-            continue
-        scale = max(np.abs(a).max(), 1e-30)
-        assert np.abs(a - b).max() <= 1e-5 * scale, (k, float(np.abs(a - b).max() / scale))
+    db = eng.upload(batch)
+    eng.set_debug(L.DEBUG_SAVE_FFN_HIDDEN)                              # differentiate on the engine's ReLU pattern (tests/relu_masks.py)
+    eng.forward(db, training=True, want_pred=False)
+    masks = engine_relu_masks(eng, B)
+    eng.set_debug(0)
+    ref = om.train_step(batch, apply=False, keep=("blk0.Q", "blk0.K", "blk0.V", "x0"), relu_masks=masks)
+    t = ref["t"]
+    rep = []
+    for k in range(2):
+        _close(f"blk{k}.y", eng.ws(f"blk{k}.y", B).cpu().numpy(), t[f"blk{k}.y"].detach().numpy(), report=rep)
+        # row maximum and row sum of the scaled, masked scores (a sample without a live key: the padding constant and T)
+        Q, K = t[f"blk{k}.Q"].detach(), t[f"blk{k}.K"].detach()
+        S = Q @ K.transpose(1, 2) / math.sqrt(Q.shape[-1])
+        S = torch.where(torch.as_tensor(batch["mask"])[:, None, :] == 0, torch.full_like(S, O.MASK_NEG), S)
+        m = S.max(-1).values
+        want = np.stack([m.numpy(), torch.exp(S - m[..., None]).sum(-1).numpy()], -1)
+        ml = eng.ws(f"blk{k}.ml", B).cpu().numpy().astype(np.float64).reshape(want.shape)
+        assert np.allclose(ml[..., 0], want[..., 0], rtol=1e-5, atol=1e-5), f"blk{k}.ml row max"
+        assert np.allclose(ml[..., 1], want[..., 1], rtol=1e-4), f"blk{k}.ml row sum"
+    _close("logits", eng.ws("logits", B).cpu().numpy(), t["logits"].detach().numpy(), report=rep)
+    eng.backward(db)
+    torch.cuda.synchronize()
+    for nm in ("Q", "K", "V"):                                          # the workspace holds block 0's after the backward
+        _close(f"d_{nm}", eng.ws(f"d_{nm}", B).cpu().numpy(), t[f"blk0.{nm}"].grad.numpy(), rtol=1e-4, report=rep)
+    _close("d_x0", eng.ws("g_a", B).cpu().numpy(), t["x0"].grad.numpy(), rtol=1e-4, report=rep)
+    print(f"\n[T={T},B={B}] max err / max|ref|: " + ", ".join(f"{n} {e:.2e}" for n, e in rep))
+    eng.close()
