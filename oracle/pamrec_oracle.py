@@ -316,17 +316,28 @@ def gather(p, batch):
     return g, rows
 
 
+def bucket_ids(loop_times):
+    """Row of the time-aware tables for each token: tf.cast(float -> int32) truncates (PAM:716).  An id outside 0..NB-1 (lisan
+    returns NB for a play / duration ratio beyond its last border and for a zero duration) maps to the extra row NB, which
+    _timeaware reads as a zero matrix: tf.gather on the GPU returns zeros for an out-of-range index (it raises on the CPU)."""
+    lt = torch.as_tensor(loop_times).to(torch.float64)
+    ok = (lt > -1) & (lt < NB)                                                   # NaN is out of range too
+    return torch.where(ok, torch.where(ok, lt, 0.0).long(), torch.full_like(lt, NB, dtype=torch.long))
+
+
 def _timeaware(x, table, bucket, proj):
-    """x[b,t,:] @ reshape(table[bucket[b,t]], (D, D))  (PAM:714-728).  proj="gather" materialises the [B,T,D,D] gather like the
+    """x[b,t,:] @ reshape(table[bucket[b,t]], (D, D))  (PAM:714-728); bucket NB (see bucket_ids) selects a zero matrix, so such a
+    token's product is 0 and it adds nothing to the table's gradient.  proj="gather" materialises the [B,T,D,D] gather like the
     reference's graph does (the CPU baseline keeps that cost shape); proj="grouped" multiplies the tokens of one bucket by
     that bucket's matrix - the same sums, 1600 x less memory, which is what lets the fp64 check run at B = 4095, T = 200."""
     B, T, _ = x.shape
+    table = torch.cat([table, torch.zeros_like(table[:1])], 0)                  # row NB: the GPU gather's zeros
     if proj == "gather":
         return torch.einsum("bti,btij->btj", x, table[bucket].reshape(B, T, D, D))
     xf, bf = x.reshape(-1, D), bucket.reshape(-1)
     order = torch.argsort(bf, stable=True)
-    counts = torch.bincount(bf, minlength=NB).tolist()
-    W = table.reshape(NB, D, D)
+    counts = torch.bincount(bf, minlength=NB + 1).tolist()
+    W = table.reshape(NB + 1, D, D)
     parts = [seg @ W[k] for k, seg in enumerate(torch.split(xf[order], counts)) if seg.shape[0]]
     inv = torch.empty_like(order)
     inv[order] = torch.arange(order.numel())
@@ -340,7 +351,7 @@ def forward(p, bn_state, batch, training, rows=None, dtype=torch.float64, relu_m
     if rows is None:
         _, rows = gather(p, batch)
     mask = torch.as_tensor(batch["mask"]).long()
-    bucket = torch.as_tensor(batch["item_loop_times_history"]).long()   # tf.cast(float, int32) PAM:716
+    bucket = bucket_ids(batch["item_loop_times_history"])                # tf.cast(float, int32) PAM:716
     B, T = mask.shape
     t = ctx.t
 

@@ -594,7 +594,7 @@ int pamrec_forward(PamrecHandle h, const PamrecBatch* b, int training, float* pr
   if (bucket_aside) cudaStreamWaitEvent(st, h->ev_bucket, 0);
   else launch_bucket_plan(b->item_loop_times_history, N, h->wi("bucket"), h->wi("perm"), ctl, h->wi("tile_bucket"),
                           h->wi("tile_begin"), h->wi("tile_count"), st);
-  const int max_tiles = N / kTokTile + kNB + 1;
+  const int max_tiles = N / kTokTile + kNB + 1;   // at most one partial tile per bin: the 10 buckets and the zero bin
   const float* xin = x0;
   for (int k = 0; k < 2; ++k) {
     const BlockOff& o = L.blk[k];
@@ -605,9 +605,9 @@ int pamrec_forward(PamrecHandle h, const PamrecBatch* b, int training, float* pr
     // the MMA kernel up to T = 128, the FFMA kernel beyond: attn_fwd per step on a B200 (1000 W) MMA vs FFMA 0.046 vs 0.066 ms on
     // takatak_b1025_t50, 0.078 vs 0.099 ms on wechat_b500_t100, 2.18 vs 1.45 ms on long_b4095_t200 (no T in between measured)
     if (T <= 128)
-      launch_attn_fwd_mma(h->wf(p + "Q"), h->wf(p + "K"), h->wf(p + "V"), h->wf(p + "qin"), b->mask, h->wf(p + "y"), h->wf(p + "ml"), B, T, st);
+      launch_attn_fwd_mma(h->wf(p + "Q"), h->wf(p + "K"), h->wf(p + "V"), h->wf(p + "qin"), b->mask, h->wf(p + "y"), h->wf(p + "pv"), h->wf(p + "ml"), B, T, st);
     else
-      launch_attn_fwd(h->wf(p + "Q"), h->wf(p + "K"), h->wf(p + "V"), h->wf(p + "qin"), b->mask, h->wf(p + "y"), h->wf(p + "ml"), B, T, st);
+      launch_attn_fwd(h->wf(p + "Q"), h->wf(p + "K"), h->wf(p + "V"), h->wf(p + "qin"), b->mask, h->wf(p + "y"), h->wf(p + "pv"), h->wf(p + "ml"), B, T, st);
     float* hdbg = (training && (h->debug & PAMREC_DEBUG_SAVE_FFN_HIDDEN)) ? h->wf(k == 0 ? "d_Q" : "d_K") : nullptr;
     launch_ffn_fwd(h->wf(p + "y"), h->P(o.w1), h->P(o.b1), h->P(o.w2), h->P(o.b2), h->P(o.ln_b_beta), h->P(o.ln_b_gamma),
                    h->wf(p + "out"), hdbg, N, st);
@@ -981,10 +981,10 @@ int pamrec_backward(PamrecHandle h, const PamrecBatch* b, void* stream) {
     // backward: the MMA kernel keeps K, V, Q and dY of a sample in shared memory (141 KB at T = 200: one CTA per SM), measured slower
     // than the FFMA kernel there (8.5 vs 6.4 ms per step on long_b4095_t200) and faster below (T = 100: 230 vs 292 us, T = 50: 152 vs 196 us)
     if (T <= 128)
-      launch_attn_bwd_mma(h->wf(p + "Q"), h->wf(p + "K"), h->wf(p + "V"), h->wf("d_y"), h->wf(p + "y"), h->wf(p + "qin"), h->wf(p + "ml"),
+      launch_attn_bwd_mma(h->wf(p + "Q"), h->wf(p + "K"), h->wf(p + "V"), h->wf("d_y"), h->wf(p + "pv"), h->wf(p + "ml"),
                           b->mask, h->wf("d_Q"), h->wf("d_K"), h->wf("d_V"), B, T, st);
     else
-      launch_attn_bwd(h->wf(p + "Q"), h->wf(p + "K"), h->wf(p + "V"), h->wf("d_y"), h->wf(p + "y"), h->wf(p + "qin"), h->wf(p + "ml"),
+      launch_attn_bwd(h->wf(p + "Q"), h->wf(p + "K"), h->wf(p + "V"), h->wf("d_y"), h->wf(p + "pv"), h->wf(p + "ml"),
                       b->mask, h->wf("d_Q"), h->wf("d_K"), h->wf("d_V"), B, T, st);
     launch_proj_bwd(xin, h->wf("d_y"), h->wf("d_Q"), h->wf("d_K"), h->wf("d_V"), h->wi("perm"), ctl, h->wi("tile_bucket"),
                     h->wi("tile_begin"), h->wi("tile_count"), max_tiles, h->P(o.wq), h->P(o.wk), h->P(o.wv), h->P(o.ln_a_beta),

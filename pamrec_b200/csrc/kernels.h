@@ -40,15 +40,15 @@ void launch_bucket_plan(const float* lt, int n, int* bucket, int* perm, int* ctl
 void launch_proj_fwd(const float* X, const int* perm, const int* ctl, const int* tile_bucket, const int* tile_begin,
                      const int* tile_count, int max_tiles, const float* Wq, const float* Wk, const float* Wv,
                      const float* ln_beta, const float* ln_gamma, float* QIN, float* Q, float* K, float* V, cudaStream_t st);
-void launch_attn_fwd(const float* Q, const float* K, const float* V, const float* QIN, const int* mask, float* Y, float* ML,
-                     int B, int T, cudaStream_t st);
+void launch_attn_fwd(const float* Q, const float* K, const float* V, const float* QIN, const int* mask, float* Y, float* PV,
+                     float* ML, int B, int T, cudaStream_t st);
 void launch_ffn_fwd(const float* Y, const float* W1, const float* b1, const float* W2, const float* b2,
                     const float* ln_beta, const float* ln_gamma, float* OUT, float* Hdbg, int n_tok, cudaStream_t st);
 void launch_ffn_bwd(const float* Y, const float* dOUT, const float* W1, const float* b1, const float* W2,
                     const float* ln_beta, const float* ln_gamma, float* dY, float* dW1, float* db1, float* dW2,
                     float* db2, float* dbeta, float* dgamma, int n_tok, cudaStream_t st);
-void launch_attn_bwd(const float* Q, const float* K, const float* V, const float* dY, const float* Y, const float* QIN,
-                     const float* ML, const int* mask, float* dQ, float* dK, float* dV, int B, int T, cudaStream_t st);
+void launch_attn_bwd(const float* Q, const float* K, const float* V, const float* dY, const float* PV, const float* ML,
+                     const int* mask, float* dQ, float* dK, float* dV, int B, int T, cudaStream_t st);
 void launch_proj_bwd(const float* X, const float* dY, const float* dQ, const float* dK, const float* dV, const int* perm,
                      const int* ctl, const int* tile_bucket, const int* tile_begin, const int* tile_count, int max_tiles,
                      const float* Wq, const float* Wk, const float* Wv, const float* ln_beta, const float* ln_gamma,
@@ -56,9 +56,9 @@ void launch_proj_bwd(const float* X, const float* dY, const float* dQ, const flo
 
 // ---- kernels_attn_mma.cu (attention forward + backward on warp-level tensor-core MMAs, 3xTF32; used up to T = 128)
 int init_attn_mma_kernels(int max_T);
-void launch_attn_fwd_mma(const float* Q, const float* K, const float* V, const float* QIN, const int* mask, float* Y, float* ML, int B, int T,
-                         cudaStream_t st);
-void launch_attn_bwd_mma(const float* Q, const float* K, const float* V, const float* dY, const float* Y, const float* QIN, const float* ML,
+void launch_attn_fwd_mma(const float* Q, const float* K, const float* V, const float* QIN, const int* mask, float* Y, float* PV, float* ML,
+                         int B, int T, cudaStream_t st);
+void launch_attn_bwd_mma(const float* Q, const float* K, const float* V, const float* dY, const float* PV, const float* ML,
                          const int* mask, float* dQ, float* dK, float* dV, int B, int T, cudaStream_t st);
 
 // ---- kernels_head.cu

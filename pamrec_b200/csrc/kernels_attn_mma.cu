@@ -1,7 +1,7 @@
 // Attention on the tensor cores with warp-level MMAs (mma.sync.m16n8k8 TF32, error-compensated 3xTF32 split of mma.cuh):
 //
 //   S = Q K^T / sqrt(40),  P = softmax_j(mask_j ? S : -(2^32)+1),  y = P V + qin                      (pamrec.py:768-810)
-//   backward: dQ = dS K,  dK = dS^T Q,  dV = P^T dY  with  dS = P o (dY V^T - D) / sqrt(40),  D_t = dY_t . (y_t - qin_t)
+//   backward: dQ = dS K,  dK = dS^T Q,  dV = P^T dY  with  dS = P o (dY V^T - D) / sqrt(40),  D_t = dY_t . (P V)_t
 //
 // Why m16n8k8 and not tcgen05 here: a sample is a 50 x 50 (T x T) problem.  A tcgen05 tile is 128 rows - two and a half samples of
 // padding per sample at T = 50 (measured: a tcgen05 forward lost to the FFMA kernel, DESIGN.md section 4) - while a
@@ -104,7 +104,7 @@ __host__ __device__ inline size_t fwd_smem(int T) { const int Tp = (T + 7) & ~7,
 template <int NTM>
 __global__ void __launch_bounds__(kThreads)
 k_attn_fwd_mma(const float* __restrict__ Q, const float* __restrict__ K, const float* __restrict__ V, const float* __restrict__ QIN,
-               const int* __restrict__ mask, float* __restrict__ Y, float* __restrict__ ML, int T) {
+               const int* __restrict__ mask, float* __restrict__ Y, float* __restrict__ PV, float* __restrict__ ML, int T) {
   extern __shared__ __align__(16) float sm[];
   const int Tp = (T + 7) & ~7, T4 = (T + 3) & ~3;
   float* Ks = sm;
@@ -179,10 +179,12 @@ k_attn_fwd_mma(const float* __restrict__ Q, const float* __restrict__ K, const f
     if (ra < T) {
       const float2 r = *reinterpret_cast<const float2*>(QIN + (base + ra) * kD + col);
       *reinterpret_cast<float2*>(Y + (base + ra) * kD + col) = make_float2(fmaf(o[nt][0], ia, r.x), fmaf(o[nt][1], ia, r.y));
+      *reinterpret_cast<float2*>(PV + (base + ra) * kD + col) = make_float2(o[nt][0] * ia, o[nt][1] * ia);
     }
     if (rb < T) {
       const float2 r = *reinterpret_cast<const float2*>(QIN + (base + rb) * kD + col);
       *reinterpret_cast<float2*>(Y + (base + rb) * kD + col) = make_float2(fmaf(o[nt][2], ib, r.x), fmaf(o[nt][3], ib, r.y));
+      *reinterpret_cast<float2*>(PV + (base + rb) * kD + col) = make_float2(o[nt][2] * ib, o[nt][3] * ib);
     }
   }
   if (t == 0) {
@@ -201,7 +203,7 @@ __host__ __device__ inline size_t bwd_smem(int T) {
 
 __global__ void __launch_bounds__(kThreads, 3)      // 3 resident CTAs per SM: the most the registers allow without spills
 k_attn_bwd_mma(const float* __restrict__ Q, const float* __restrict__ K, const float* __restrict__ V, const float* __restrict__ dY,
-               const float* __restrict__ Y, const float* __restrict__ QIN, const float* __restrict__ ML, const int* __restrict__ mask,
+               const float* __restrict__ PV, const float* __restrict__ ML, const int* __restrict__ mask,
                float* __restrict__ dQ, float* __restrict__ dK, float* __restrict__ dV, int T) {
   extern __shared__ __align__(16) float sm[];
   const int Tp8 = (T + 7) & ~7, Tp16 = (T + 15) & ~15, T4 = (T + 3) & ~3;
@@ -218,7 +220,7 @@ k_attn_bwd_mma(const float* __restrict__ Q, const float* __restrict__ K, const f
   const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
   const int64_t base = (int64_t)b * T;
   for (int j = tid; j < T; j += kThreads) mk[j] = mask[base + j];
-  // Q, dY of every query row; D_t = dY_t . (y_t - qin_t); row statistics.  Padding rows: zeros, statistics that give p = 0.
+  // Q, dY of every query row; D_t = dY_t . (P V)_t; row statistics.  Padding rows: zeros, statistics that give p = 0.
   for (int i = tid; i < Tp8 * 10; i += kThreads) {
     const int r = i / 10, c = i % 10;
     float4 q = f4_zero(), gy = f4_zero();
@@ -232,8 +234,8 @@ k_attn_bwd_mma(const float* __restrict__ Q, const float* __restrict__ K, const f
       const int64_t tok = base + r;
 #pragma unroll
       for (int i = 0; i < 10; ++i) {
-        const float4 gy = ld4(dY + tok * kD + 4 * i), y = ld4(Y + tok * kD + 4 * i), qi = ld4(QIN + tok * kD + 4 * i);
-        d = fmaf(gy.x, y.x - qi.x, d); d = fmaf(gy.y, y.y - qi.y, d); d = fmaf(gy.z, y.z - qi.z, d); d = fmaf(gy.w, y.w - qi.w, d);
+        const float4 gy = ld4(dY + tok * kD + 4 * i), o = ld4(PV + tok * kD + 4 * i);
+        d = fmaf(gy.x, o.x, d); d = fmaf(gy.y, o.y, d); d = fmaf(gy.z, o.z, d); d = fmaf(gy.w, o.w, d);
       }
       m = ML[2 * tok]; il = 1.0f / ML[2 * tok + 1];
     }
@@ -364,9 +366,9 @@ k_attn_bwd_mma(const float* __restrict__ Q, const float* __restrict__ K, const f
 }
 
 template <int NTM>
-static void launch_fwd(const float* Q, const float* K, const float* V, const float* QIN, const int* mask, float* Y, float* ML, int B, int T,
-                       cudaStream_t st) {
-  k_attn_fwd_mma<NTM><<<dim3(B, (T + 63) / 64), kThreads, fwd_smem(T), st>>>(Q, K, V, QIN, mask, Y, ML, T);
+static void launch_fwd(const float* Q, const float* K, const float* V, const float* QIN, const int* mask, float* Y, float* PV, float* ML,
+                       int B, int T, cudaStream_t st) {
+  k_attn_fwd_mma<NTM><<<dim3(B, (T + 63) / 64), kThreads, fwd_smem(T), st>>>(Q, K, V, QIN, mask, Y, PV, ML, T);
 }
 
 }  // namespace amma
@@ -380,26 +382,24 @@ int init_attn_mma_kernels(int max_T) {
   set((const void*)amma::k_attn_fwd_mma<7>, f);
   set((const void*)amma::k_attn_fwd_mma<13>, f);
   set((const void*)amma::k_attn_fwd_mma<25>, f);
-  set((const void*)amma::k_attn_fwd_mma<32>, f);
   set((const void*)amma::k_attn_bwd_mma, b);
   return e == cudaSuccess ? 0 : -1;
 }
 
-void launch_attn_fwd_mma(const float* Q, const float* K, const float* V, const float* QIN, const int* mask, float* Y, float* ML, int B, int T,
-                         cudaStream_t st) {
+void launch_attn_fwd_mma(const float* Q, const float* K, const float* V, const float* QIN, const int* mask, float* Y, float* PV, float* ML,
+                         int B, int T, cudaStream_t st) {
   PAMREC_PROF("attn_fwd", 1, st);
   if (B == 0) return;
-  if (T <= 56) amma::launch_fwd<7>(Q, K, V, QIN, mask, Y, ML, B, T, st);
-  else if (T <= 104) amma::launch_fwd<13>(Q, K, V, QIN, mask, Y, ML, B, T, st);
-  else if (T <= 200) amma::launch_fwd<25>(Q, K, V, QIN, mask, Y, ML, B, T, st);
-  else amma::launch_fwd<32>(Q, K, V, QIN, mask, Y, ML, B, T, st);
+  if (T <= 56) amma::launch_fwd<7>(Q, K, V, QIN, mask, Y, PV, ML, B, T, st);
+  else if (T <= 104) amma::launch_fwd<13>(Q, K, V, QIN, mask, Y, PV, ML, B, T, st);
+  else amma::launch_fwd<25>(Q, K, V, QIN, mask, Y, PV, ML, B, T, st);      // up to 200 keys; the dispatch sends T <= 128 only
 }
 
-void launch_attn_bwd_mma(const float* Q, const float* K, const float* V, const float* dY, const float* Y, const float* QIN, const float* ML,
+void launch_attn_bwd_mma(const float* Q, const float* K, const float* V, const float* dY, const float* PV, const float* ML,
                          const int* mask, float* dQ, float* dK, float* dV, int B, int T, cudaStream_t st) {
   PAMREC_PROF("attn_bwd", 1, st);
   if (B == 0) return;
-  amma::k_attn_bwd_mma<<<dim3(B, (T + 63) / 64), amma::kThreads, amma::bwd_smem(T), st>>>(Q, K, V, dY, Y, QIN, ML, mask, dQ, dK, dV, T);
+  amma::k_attn_bwd_mma<<<dim3(B, (T + 63) / 64), amma::kThreads, amma::bwd_smem(T), st>>>(Q, K, V, dY, PV, ML, mask, dQ, dK, dV, T);
 }
 
 }  // namespace pamrec

@@ -83,28 +83,34 @@ void launch_embed_fwd(const int* ih, const int* ch, const int* items, const int*
 }
 
 // ------------------------------------------------------------------------------------------
-// Bucket planning: counting sort of tokens by play-ratio bucket (10 bins) and a tile table.
+// Bucket planning: counting sort of tokens by play-ratio bucket and a tile table.  Bins 0..9 are the rows of the time-aware
+// tables; bin kZeroBin holds every token whose bucket id lies outside 0..9 (lisan gives 10 for a ratio beyond its last border,
+// or for a zero duration).  The reference gathers those tokens' matrices with tf.gather on the GPU, which returns a zero row
+// for an out-of-range index: their Q, K and V are 0 and they add nothing to the tables' gradients (k_proj_fwd / k_proj_bwd).
 // ctl: [0..15] counts, [16..31] cursors, [32] number of tiles.
+constexpr int kZeroBin = kNB;
+constexpr int kBins = kNB + 1;
 __global__ void k_bucket_hist(const float* __restrict__ lt, int n, int* __restrict__ bucket, int* __restrict__ ctl) {
   __shared__ int h[16];
   if (threadIdx.x < 16) h[threadIdx.x] = 0;
   __syncthreads();
   int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) {
-    int k = (int)lt[i];                 // tf.cast(float -> int32) truncates, pamrec.py:716
-    k = min(max(k, 0), kNB - 1);
+    // tf.cast(float -> int32) truncates (pamrec.py:716): ids 0..9 are the values in (-1, 10); NaN falls out of range too
+    const float v = lt[i];
+    const int k = (v > -1.f && v < (float)kNB) ? (int)v : kZeroBin;
     bucket[i] = k;
     atomicAdd(&h[k], 1);
   }
   __syncthreads();
-  if (threadIdx.x < kNB && h[threadIdx.x]) atomicAdd(&ctl[threadIdx.x], h[threadIdx.x]);
+  if (threadIdx.x < kBins && h[threadIdx.x]) atomicAdd(&ctl[threadIdx.x], h[threadIdx.x]);
 }
 
 __global__ void k_bucket_plan(int* __restrict__ ctl, int* __restrict__ tile_bucket, int* __restrict__ tile_begin,
                               int* __restrict__ tile_count) {
   if (threadIdx.x != 0 || blockIdx.x != 0) return;
   int start = 0, nt = 0;
-  for (int k = 0; k < kNB; ++k) {
+  for (int k = 0; k < kBins; ++k) {
     int cnt = ctl[k];
     ctl[16 + k] = start;
     for (int o = 0; o < cnt; o += kTokTile) {
@@ -126,7 +132,7 @@ __global__ void k_bucket_scatter(const int* __restrict__ bucket, int n, int* __r
   int k = -1, r = 0;
   if (i < n) { k = bucket[i]; r = atomicAdd(&h[k], 1); }
   __syncthreads();
-  if (threadIdx.x < kNB) base[threadIdx.x] = h[threadIdx.x] ? atomicAdd(&ctl[16 + threadIdx.x], h[threadIdx.x]) : 0;
+  if (threadIdx.x < kBins) base[threadIdx.x] = h[threadIdx.x] ? atomicAdd(&ctl[16 + threadIdx.x], h[threadIdx.x]) : 0;
   __syncthreads();
   if (i < n) perm[base[k] + r] = i;
 }
@@ -176,9 +182,10 @@ k_proj_fwd(const float* __restrict__ X, const int* __restrict__ perm, const int*
   __shared__ int toks[kTokTile];
   const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
   const int k = tile_bucket[tile], begin = tile_begin[tile], cnt = tile_count[tile];
-  load_split_mat(Whi, Wlo, Wq + (int64_t)k * kDD, tid);
-  load_split_mat(Whi + kDD, Wlo + kDD, Wk + (int64_t)k * kDD, tid);
-  load_split_mat(Whi + 2 * kDD, Wlo + 2 * kDD, Wv + (int64_t)k * kDD, tid);
+  const bool zero = k == kZeroBin;                          // zero matrices: Q = K = V = 0, qin as for any token
+  load_split_mat(Whi, Wlo, zero ? nullptr : Wq + (int64_t)k * kDD, tid);
+  load_split_mat(Whi + kDD, Wlo + kDD, zero ? nullptr : Wk + (int64_t)k * kDD, tid);
+  load_split_mat(Whi + 2 * kDD, Wlo + 2 * kDD, zero ? nullptr : Wv + (int64_t)k * kDD, tid);
   if (tid < kD) { lnp[tid] = ln_beta[tid]; lnp[kD + tid] = ln_gamma[tid]; }
   if (tid < cnt) toks[tid] = perm[begin + tid];
   __syncthreads();
@@ -268,8 +275,8 @@ __device__ __forceinline__ float dot40(const float4 (&q)[10], const float* __res
 
 __global__ void __launch_bounds__(256)
 k_attn_fwd(const float* __restrict__ Q, const float* __restrict__ K, const float* __restrict__ V,
-           const float* __restrict__ QIN, const int* __restrict__ mask, float* __restrict__ Y, float* __restrict__ ML,
-           int B, int T) {
+           const float* __restrict__ QIN, const int* __restrict__ mask, float* __restrict__ Y, float* __restrict__ PV,
+           float* __restrict__ ML, int B, int T) {
   extern __shared__ __align__(16) float sm[];
   const int nw = attn_nw(T), spb = attn_spb(T), tps = nw * 32;
   const int per = attn_fwd_per(T);                          // floats per sample: K | V | mask
@@ -347,18 +354,19 @@ k_attn_fwd(const float* __restrict__ Q, const float* __restrict__ K, const float
   for (int i = 0; i < 10; ++i) {
     const float4 r = ld4(QIN + row + 4 * i);
     st4(Y + row + 4 * i, make_float4(fmaf(o[i].x, inv, r.x), fmaf(o[i].y, inv, r.y), fmaf(o[i].z, inv, r.z), fmaf(o[i].w, inv, r.w)));
+    st4(PV + row + 4 * i, make_float4(o[i].x * inv, o[i].y * inv, o[i].z * inv, o[i].w * inv));
   }
   ML[2 * ((int64_t)(b0 + sl) * T + t)] = m;
   ML[2 * ((int64_t)(b0 + sl) * T + t) + 1] = l;
 }
 
-void launch_attn_fwd(const float* Q, const float* K, const float* V, const float* QIN, const int* mask, float* Y, float* ML,
-                     int B, int T, cudaStream_t st) {
+void launch_attn_fwd(const float* Q, const float* K, const float* V, const float* QIN, const int* mask, float* Y, float* PV,
+                     float* ML, int B, int T, cudaStream_t st) {
   PAMREC_PROF("attn_fwd", 1, st);
   if (B == 0) return;
   const size_t smem = attn_fwd_smem(T);
   const int spb = attn_spb(T), threads = spb * attn_nw(T) * 32;
-  k_attn_fwd<<<(B + spb - 1) / spb, threads, smem, st>>>(Q, K, V, QIN, mask, Y, ML, B, T);
+  k_attn_fwd<<<(B + spb - 1) / spb, threads, smem, st>>>(Q, K, V, QIN, mask, Y, PV, ML, B, T);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -373,7 +381,7 @@ __device__ __forceinline__ void load_split_mat(uint32_t* __restrict__ hi, uint32
 #pragma unroll
   for (int it = 0; it < IT; ++it) {
     const int i = tid + it * kTokThreads;
-    if (i < kDD / 4) v[it] = ld4(W + 4 * i);
+    if (i < kDD / 4) v[it] = W != nullptr ? ld4(W + 4 * i) : f4_zero();
   }
 #pragma unroll
   for (int it = 0; it < IT; ++it) {
@@ -744,7 +752,7 @@ void launch_ffn_bwd(const float* Y, const float* dOUT, const float* W1, const fl
 
 // ------------------------------------------------------------------------------------------
 // Attention backward.  In: Q, K, V, dY (grad of y = P V + qin), the forward's y, qin and row statistics (m, l).
-// Out: dQ, dK, dV.  Same thread mapping as the forward: with D_t = dy_t . (y_t - qin_t) (= sum_j p_tj dP_tj) known
+// Out: dQ, dK, dV.  Same thread mapping as the forward: with D_t = dy_t . (P V)_t (= sum_j p_tj dP_tj) known
 // up front, pass A (thread == query row t) forms dQ_t in one sweep over the keys and pass B (thread == key j) forms
 // dK_j and dV_j in one sweep over the queries; both recompute p = exp(s - m_t) / l_t from the saved statistics, all
 // shared-memory reads are warp-wide broadcasts.
@@ -753,7 +761,7 @@ inline size_t attn_bwd_smem(int T) { return (size_t)attn_spb(T) * attn_bwd_per(T
 
 __global__ void __launch_bounds__(256)
 k_attn_bwd(const float* __restrict__ Q, const float* __restrict__ K, const float* __restrict__ V,
-           const float* __restrict__ dY, const float* __restrict__ Y, const float* __restrict__ QIN,
+           const float* __restrict__ dY, const float* __restrict__ PV,
            const float* __restrict__ ML, const int* __restrict__ mask, float* __restrict__ dQ, float* __restrict__ dK,
            float* __restrict__ dV, int B, int T) {
   extern __shared__ __align__(16) float sm[];
@@ -780,8 +788,8 @@ k_attn_bwd(const float* __restrict__ Q, const float* __restrict__ K, const float
     float d = 0.f;
 #pragma unroll
     for (int i = 0; i < 10; ++i) {
-      const float4 g = ld4(dY + tok * kD + 4 * i), y = ld4(Y + tok * kD + 4 * i), r = ld4(QIN + tok * kD + 4 * i);
-      d = fmaf(g.x, y.x - r.x, d); d = fmaf(g.y, y.y - r.y, d); d = fmaf(g.z, y.z - r.z, d); d = fmaf(g.w, y.w - r.w, d);
+      const float4 g = ld4(dY + tok * kD + 4 * i), o = ld4(PV + tok * kD + 4 * i);
+      d = fmaf(g.x, o.x, d); d = fmaf(g.y, o.y, d); d = fmaf(g.z, o.z, d); d = fmaf(g.w, o.w, d);
     }
     S[4 * TS + t] = ML[2 * tok];
     S[4 * TS + T + t] = 1.0f / ML[2 * tok + 1];
@@ -852,13 +860,12 @@ k_attn_bwd(const float* __restrict__ Q, const float* __restrict__ K, const float
   }
 }
 
-void launch_attn_bwd(const float* Q, const float* K, const float* V, const float* dY, const float* Y, const float* QIN,
-                     const float* ML, const int* mask, float* dQ, float* dK, float* dV, int B, int T, cudaStream_t st) {
+void launch_attn_bwd(const float* Q, const float* K, const float* V, const float* dY, const float* PV, const float* ML, const int* mask, float* dQ, float* dK, float* dV, int B, int T, cudaStream_t st) {
   PAMREC_PROF("attn_bwd", 1, st);
   if (B == 0) return;
   const size_t smem = attn_bwd_smem(T);
   const int spb = attn_spb(T), threads = spb * attn_nw(T) * 32;
-  k_attn_bwd<<<(B + spb - 1) / spb, threads, smem, st>>>(Q, K, V, dY, Y, QIN, ML, mask, dQ, dK, dV, B, T);
+  k_attn_bwd<<<(B + spb - 1) / spb, threads, smem, st>>>(Q, K, V, dY, PV, ML, mask, dQ, dK, dV, B, T);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -890,9 +897,11 @@ k_proj_bwd(const float* __restrict__ X, const float* __restrict__ dY, const floa
   const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
   const int g = lane >> 2, t = lane & 3;
   const int k = tile_bucket[tile], begin = tile_begin[tile], cnt = tile_count[tile];
-  load_split_mat(Whi, Wlo, Wq + (int64_t)k * kDD, tid);
-  load_split_mat(Whi + kDD, Wlo + kDD, Wk + (int64_t)k * kDD, tid);
-  load_split_mat(Whi + 2 * kDD, Wlo + 2 * kDD, Wv + (int64_t)k * kDD, tid);
+  // zero matrices (bucket id outside 0..9): dX = LN_a'(dY) only, and no table row receives a gradient
+  const bool zero = k == kZeroBin;
+  load_split_mat(Whi, Wlo, zero ? nullptr : Wq + (int64_t)k * kDD, tid);
+  load_split_mat(Whi + kDD, Wlo + kDD, zero ? nullptr : Wk + (int64_t)k * kDD, tid);
+  load_split_mat(Whi + 2 * kDD, Wlo + 2 * kDD, zero ? nullptr : Wv + (int64_t)k * kDD, tid);
   if (tid < kD) { lnp[tid] = ln_beta[tid]; lnp[kD + tid] = ln_gamma[tid]; }
   if (tid < 2 * kD) red[tid] = 0.f;
   for (int i = tid; i < kDD; i += kTokThreads) acc[i] = 0.f;
@@ -945,7 +954,7 @@ k_proj_bwd(const float* __restrict__ X, const float* __restrict__ dY, const floa
   // one global atomic per element and CTA; the accumulator is cleared for the next matrix (barriers: top of the loop below)
   auto flush_acc = [&](float* dW) {
     __syncthreads();
-    for (int i = tid; i < kDD; i += kTokThreads) { atomicAdd(dW + i, acc[i]); acc[i] = 0.f; }
+    for (int i = tid; i < kDD; i += kTokThreads) { if (!zero) atomicAdd(dW + i, acc[i]); acc[i] = 0.f; }
   };
   flush_acc(dWs[0]);
   // ---- dX = dK Wk^T + dV Wv^T (+ LN backward below)

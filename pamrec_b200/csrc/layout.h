@@ -386,7 +386,9 @@ struct Layout {
     add_ws("tgt", PAMREC_F32, {B, kE});
     for (int b = 0; b < 2; ++b) {
       std::string p = "blk" + std::to_string(b) + ".";
-      for (const char* n : {"qin", "Q", "K", "V", "y", "out"}) add_ws(p + n, PAMREC_F32, {B, T, kD});
+      // pv: the attention output before the residual, P V = y - qin, kept apart because |qin| ~ 100 |P V|: the backward's
+      // D = dY . (P V) taken from y - qin lost 8 bits (1e-4 of dQ, dK), which TF's softmax gradient does not
+      for (const char* n : {"qin", "Q", "K", "V", "y", "pv", "out"}) add_ws(p + n, PAMREC_F32, {B, T, kD});
       add_ws(p + "ml", PAMREC_F32, {B, T, 2});   // softmax row maximum and row sum, kept for the backward pass
     }
     add_ws("z1", PAMREC_F32, {B, T, 20});

@@ -59,6 +59,21 @@ def _batch(seed, B, T, nu, ni, nc, min_len=1, grouped=True):
     return S.add_satisfied_fields(O.make_batch(seed, B, T, nu, ni, nc, min_len=min_len, grouped=grouped), seed=seed + 1)
 
 
+def satisfied_edge_rows(batch):
+    """Rows 3, 4 and 6 of a batch of at least 7 rows: no satisfied item (read-out = zeros, uniform attention), a single one at the
+    last position, every position satisfied."""
+    for k in ("satisfied_mask", "satisfied_item_history", "satisfied_cate_history"):
+        batch[k][3] = 0
+        batch[k][4] = 0
+    batch["satisfied_mask"][4, -1] = 1
+    batch["satisfied_item_history"][4, -1] = max(int(batch["item_history"][4, 0]), 1)
+    batch["satisfied_cate_history"][4, -1] = max(int(batch["item_cate_history"][4, 0]), 1)
+    batch["satisfied_mask"][6] = 1
+    batch["satisfied_item_history"][6] = np.maximum(batch["item_history"][6], 1)
+    batch["satisfied_cate_history"][6] = np.maximum(batch["item_cate_history"][6], 1)
+    return batch
+
+
 def _on(z, stat, gamma, beta):
     xh = (z.astype(np.float32) - stat[:, 0].astype(np.float32)) * stat[:, 1].astype(np.float32)
     return gamma.astype(np.float64) * xh.astype(np.float64) + beta.astype(np.float64) > 0
@@ -104,6 +119,11 @@ CASES = [
     ("sharebottom", 100, 1000, 30, 200, 10, 1),    # T = 200
     ("mmoe", 50000, 30000, 50, 50, 1025, 1),       # the takatak bench shape
     ("ple", 20000, 100000, 500, 100, 500, 1),      # the quick-start shape
+    # the DIN pooling keeps 8 scores per lane (kernels_sibling.cu): T = 33 is the first with a second one, 256 the last; T = 1
+    # (shared by all three DIN models)
+    ("mmoe", 50, 300, 20, 1, 20, 1),
+    ("mmoe", 100, 1000, 30, 33, 20, 1),
+    ("mmoe", 60, 2000, 30, 256, 10, 1),
 ]
 
 
@@ -272,6 +292,11 @@ SAS_CASES = [
     (400, 5000, 60, 50, 130, 50),
     (100, 1000, 30, 200, 10, 1),
     (50000, 30000, 50, 50, 1025, 1),
+    # a thread of the attention kernels loops over query rows in steps of 128 (kernels_sasrec.cu): T = 129 is the first T where
+    # one thread owns two rows
+    (50, 300, 20, 1, 20, 1),
+    (100, 1000, 30, 128, 15, 1),
+    (100, 1000, 30, 129, 10, 1),
 ]
 
 
@@ -282,9 +307,7 @@ def test_sasrec_step_stagewise(nu, ni, nc, T, B, min_len):
     om, eng = _setup("sasrec", nu, ni, nc, T, B, seed=11)
     batch = _batch(5, B, T, nu, ni, nc, min_len=min_len)
     if B >= 10:
-        batch["satisfied_mask"][3] = 0                     # a row without any satisfied item: read-out = zeros, uniform attention
-        batch["satisfied_item_history"][3] = 0
-        batch["satisfied_cate_history"][3] = 0
+        satisfied_edge_rows(batch)
     N = B * T
     FAILS.clear()
     db = eng.upload(batch)

@@ -11,7 +11,8 @@ import torch
 
 from oracle import pamrec_oracle as O
 import siblings_oracle_dims as D
-from test_gpu_siblings import EMB, FAILS, ROOT, _batch, _branches, _close, _expect, _on, expert_scopes, sibling_relu_masks
+from test_gpu_siblings import (EMB, FAILS, ROOT, _batch, _branches, _close, _expect, _on, expert_scopes, satisfied_edge_rows,
+                               sibling_relu_masks)
 
 pytestmark = pytest.mark.gpu
 
@@ -172,6 +173,7 @@ SAS_CASES = [
     (100, 1000, 30, 200, 10, 1),
     (50000, 30000, 50, 50, 1025, 1),
     (60, 2000, 30, 256, 10, 1),                      # T = 256: 81 / 83 KB of shared memory per attention CTA (the opt-in at bind)
+    (100, 1000, 30, 129, 10, 1),                     # T = 129: a thread's second query row (kernels_sasrec.cu) at model width 40
 ]
 
 
@@ -182,9 +184,7 @@ def test_sasrec_step_stagewise_reference_dims(nu, ni, nc, T, B, min_len):
     Sw = dims[0] + dims[1]                                   # model width
     om, eng = _setup("sasrec", nu, ni, nc, T, B, 11, dims)
     batch = _batch(5, B, T, nu, ni, nc, min_len=min_len)
-    batch["satisfied_mask"][3] = 0                         # a row without any satisfied item: read-out = zeros, uniform attention
-    batch["satisfied_item_history"][3] = 0
-    batch["satisfied_cate_history"][3] = 0
+    satisfied_edge_rows(batch)                             # none, a single one at the last position, all satisfied
     N = B * T
     FAILS.clear()
     db = eng.upload(batch)

@@ -196,3 +196,50 @@ def test_forced_relu_masks_and_grouped_projection():
     w = "sequential/pamrec/expert_2/nn_part/w_nn_layer0"
     assert float((other["grads"][w] - grp["grads"][w]).abs().max()) > 0
     assert sp  # (score scopes use the same mechanism; exercised on the GPU by tests/relu_masks.py)
+
+
+def test_out_of_range_bucket_reads_a_zero_matrix():
+    """lisan gives bucket 10 - one past the [10, 1600] time-aware tables - for a play / duration ratio beyond its last border and
+    for a zero duration.  tf.gather on the GPU returns a zero row for that index: the token's Q, K and V are 0, its qin still goes
+    through the LayerNorm into the attention residual, and no table row gets a gradient from it.  Both projection forms agree."""
+    nu, ni, nc, T, B = 60, 400, 20, 14, 20
+    om = O.OracleModel(nu, ni, nc, T, seed=5)
+    O.perturb_params(om.params, om.bn_state, seed=6)
+    batch = O.make_batch(3, B, T, nu, ni, nc)
+    lt = batch["item_loop_times_history"]
+    lt[:, 3] = 10.0                                  # one position of every history
+    lt[:5, :] = 10.0                                 # one listwise group entirely out of range
+    lt[10:15, 5] = 12.5
+    lt[10:15, 6] = -1.0
+    lt[10:15, 7] = 9.99                              # truncates to 9: in range
+    lt[10:15, 8] = -0.5                              # truncates to 0: in range
+    want = np.where((lt > -1) & (lt < 10), np.trunc(np.where((lt > -1) & (lt < 10), lt, 0)), 10).astype(np.int64)
+    assert np.array_equal(O.bucket_ids(lt).numpy(), want)
+    out = (want == 10) & (batch["mask"] == 1)
+    assert out.sum() > 5 and (want == 9).any() and (want == 0).any()
+    keep = ("blk0.Q", "blk0.K", "blk0.V", "blk1.Q", "blk1.K", "blk1.V", "blk0.qin", "blk0.y")
+    base = om.train_step(batch, apply=False, keep=keep)
+    om.proj = "grouped"
+    grp = om.train_step(batch, apply=False, keep=keep)
+    assert abs(base["losses"]["loss"] - grp["losses"]["loss"]) < 1e-14
+    for n in base["grads"]:
+        assert float((base["grads"][n] - grp["grads"][n]).abs().max()) < 1e-14, n
+    z = torch.as_tensor(want == 10)
+    t = grp["t"]
+    for k in keep[:6]:
+        assert float(t[k].detach()[z].abs().max()) == 0.0, k      # padded positions included: they take the same path
+    # tokens in range: qin (Q) or x0 (K, V) times their bucket's matrix; out of range: qin = LN(x0) as for any token
+    qin, x0, b = t["blk0.qin"].detach(), t["x0"].detach(), O.bucket_ids(lt)
+    assert float(qin[z].abs().max()) > 0
+    for m, a in (("Q", qin), ("K", x0), ("V", x0)):
+        W = om.params[f"sequential/pamrec/num_blocks_0/self_attention/{m}_timeaware_embedding"].double()[b[~z]].reshape(-1, O.D, O.D)
+        assert torch.allclose(t["blk0." + m].detach()[~z], torch.einsum("ni,nij->nj", a[~z], W), rtol=0, atol=1e-14), m
+    # a table row that only out-of-range tokens would select gets the L2 gradient alone
+    lt2 = batch["item_loop_times_history"].copy()
+    lt2[lt2 == 4] = 10.0
+    g2 = om.train_step(dict(batch, item_loop_times_history=lt2), apply=False)["grads"]
+    for m in "QKV":
+        name = f"sequential/pamrec/num_blocks_1/self_attention/{m}_timeaware_embedding"
+        l2 = om.hp["layer_l2"] * om.params[name].double()
+        assert torch.allclose(g2[name][4], l2[4], rtol=1e-12, atol=0), name
+        assert float((g2[name][3] - l2[3]).abs().max()) > 0, name
