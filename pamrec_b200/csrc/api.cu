@@ -41,7 +41,7 @@ struct PamrecHandle_ {
   // Internal side stream: work that is off the critical path of a step (the id sort of the sparse plan, the weight-gradient
   // GEMMs of the head) is forked from the caller's stream with events and joined back before anything consumes it.
   cudaStream_t side = nullptr;
-  cudaEvent_t ev_side[12] = {};
+  cudaEvent_t ev_side[16] = {};
   cudaEvent_t ev_join = nullptr, ev_plan = nullptr, ev_bucket = nullptr;
   int ev_next = 0;
   const void* plan_for = nullptr;   // batch whose sparse plan is in flight / ready on the side stream (local tables)
@@ -90,7 +90,7 @@ struct PamrecHandle_ {
   template <typename F>
   void fork(cudaStream_t main, F fn) {
     cudaEvent_t e = ev_side[ev_next];
-    ev_next = (ev_next + 1) % 12;
+    ev_next = (ev_next + 1) % 16;
     cudaEventRecord(e, main);
     cudaStreamWaitEvent(side, e, 0);
     fn(side);
@@ -976,24 +976,37 @@ int pamrec_backward(PamrecHandle h, const PamrecBatch* b, void* stream) {
     const float* xin = k == 0 ? h->wf("x0") : h->wf("blk0.out");
     float* gout = k == 1 ? g_a : g_b;
     float* gin = k == 1 ? g_b : g_a;
+    // block 1's weight-gradient inputs must outlive block 0's backward, which rewrites d_Q / d_K / d_V and g_a (layout.h)
+    float* dQ = h->wf(k == 1 ? "blk1.d_Q" : "d_Q");
+    float* dK = h->wf(k == 1 ? "blk1.d_K" : "d_K");
+    float* dV = h->wf(k == 1 ? "blk1.d_V" : "d_V");
+    float* dout = k == 1 ? h->wf("blk1.d_out") : gout;
+    // the block's weight gradients (no consumer before the optimiser) run on the side stream, each half as soon as its inputs
+    // exist: the FFN pair after the FFN backward, the projection after the attention backward; joined at the end of the pass
+    EncDwArgs dw{h->wf(p + "qin"), xin, dQ, dK, dV, h->wi("perm"), ctl, h->wf(p + "y"), h->P(o.ln_b_beta), h->P(o.ln_b_gamma),
+                 h->wf(p + "h"), h->wf(p + "dhr"), dout, h->G(o.wq), h->G(o.wk), h->G(o.wv), h->G(o.w1), h->G(o.b1), h->G(o.w2),
+                 h->G(o.b2), N, true};
     launch_ffn_bwd(h->wf(p + "y"), gout, h->P(o.w1), h->P(o.b1), h->P(o.w2), h->P(o.ln_b_beta), h->P(o.ln_b_gamma), h->wf("d_y"),
-                   h->G(o.w1), h->G(o.b1), h->G(o.w2), h->G(o.b2), h->G(o.ln_b_beta), h->G(o.ln_b_gamma), N, st);
+                   h->wf(p + "h"), h->wf(p + "dhr"), k == 1 ? dout : nullptr, h->G(o.ln_b_beta), h->G(o.ln_b_gamma), N, st);
+    h->fork(st, [&](cudaStream_t s2) { launch_enc_dw(dw, s2); });
     // backward: the MMA kernel keeps K, V, Q and dY of a sample in shared memory (141 KB at T = 200: one CTA per SM), measured slower
     // than the FFMA kernel there (8.5 vs 6.4 ms per step on long_b4095_t200) and faster below (T = 100: 230 vs 292 us, T = 50: 152 vs 196 us)
     if (T <= 128)
       launch_attn_bwd_mma(h->wf(p + "Q"), h->wf(p + "K"), h->wf(p + "V"), h->wf("d_y"), h->wf(p + "pv"), h->wf(p + "ml"),
-                          b->mask, h->wf("d_Q"), h->wf("d_K"), h->wf("d_V"), B, T, st);
+                          b->mask, dQ, dK, dV, B, T, st);
     else
       launch_attn_bwd(h->wf(p + "Q"), h->wf(p + "K"), h->wf(p + "V"), h->wf("d_y"), h->wf(p + "pv"), h->wf(p + "ml"),
-                      b->mask, h->wf("d_Q"), h->wf("d_K"), h->wf("d_V"), B, T, st);
-    launch_proj_bwd(xin, h->wf("d_y"), h->wf("d_Q"), h->wf("d_K"), h->wf("d_V"), h->wi("perm"), ctl, h->wi("tile_bucket"),
-                    h->wi("tile_begin"), h->wi("tile_count"), max_tiles, h->P(o.wq), h->P(o.wk), h->P(o.wv), h->P(o.ln_a_beta),
-                    h->P(o.ln_a_gamma), gin, h->G(o.wq), h->G(o.wk), h->G(o.wv), h->G(o.ln_a_beta), h->G(o.ln_a_gamma), st);
+                      b->mask, dQ, dK, dV, B, T, st);
+    dw.ffn = false;
+    h->fork(st, [&](cudaStream_t s2) { launch_enc_dw(dw, s2); });
+    launch_proj_bwd(xin, h->wf("d_y"), dQ, dK, dV, h->wi("perm"), ctl, h->wi("tile_bucket"), h->wi("tile_begin"), h->wi("tile_count"),
+                    max_tiles, h->P(o.wq), h->P(o.wk), h->P(o.wv), h->P(o.ln_a_beta), h->P(o.ln_a_gamma), gin, h->G(o.ln_a_beta),
+                    h->G(o.ln_a_gamma), st);
   }
   // dX0 is in g_a
   launch_embed_bwd_reduce(g_a, h->wf("d_tgt"), h->wf("d_tgt_total"), h->G(L.pos), h->wd("sp_normsq") + 4,
                           h->sharded() ? nullptr : h->wd("sp_normsq"), B, T, st);
-  h->join(st);                    // the head's weight-gradient GEMMs (side stream) are complete from here on
+  h->join(st);                    // the head's and the encoder's weight gradients (side stream) are complete from here on
   if (crc) return fail(h, "nccl: %s", h->comm.err.c_str());
   return check_cuda(h, "backward");
 }

@@ -44,15 +44,28 @@ void launch_attn_fwd(const float* Q, const float* K, const float* V, const float
                      float* ML, int B, int T, cudaStream_t st);
 void launch_ffn_fwd(const float* Y, const float* W1, const float* b1, const float* W2, const float* b2,
                     const float* ln_beta, const float* ln_gamma, float* OUT, float* Hdbg, int n_tok, cudaStream_t st);
+// dOUT_keep (nullable): receives a copy of dOUT for launch_enc_dw, when the buffer dOUT is overwritten before that runs
 void launch_ffn_bwd(const float* Y, const float* dOUT, const float* W1, const float* b1, const float* W2,
-                    const float* ln_beta, const float* ln_gamma, float* dY, float* dW1, float* db1, float* dW2,
-                    float* db2, float* dbeta, float* dgamma, int n_tok, cudaStream_t st);
+                    const float* ln_beta, const float* ln_gamma, float* dY, float* H, float* DHR, float* dOUT_keep,
+                    float* dbeta, float* dgamma, int n_tok, cudaStream_t st);
 void launch_attn_bwd(const float* Q, const float* K, const float* V, const float* dY, const float* PV, const float* ML,
                      const int* mask, float* dQ, float* dK, float* dV, int B, int T, cudaStream_t st);
 void launch_proj_bwd(const float* X, const float* dY, const float* dQ, const float* dK, const float* dV, const int* perm,
                      const int* ctl, const int* tile_bucket, const int* tile_begin, const int* tile_count, int max_tiles,
                      const float* Wq, const float* Wk, const float* Wv, const float* ln_beta, const float* ln_gamma,
-                     float* dX, float* dWq, float* dWk, float* dWv, float* dbeta, float* dgamma, cudaStream_t st);
+                     float* dX, float* dbeta, float* dgamma, cudaStream_t st);
+// weight gradients of one encoder block from what its backward pass saved (kernels_encoder.cu:k_enc_dw); accumulated atomically
+struct EncDwArgs {
+  const float* qin; const float* x; const float* dQ; const float* dK; const float* dV;   // projection: [N, 40] each
+  const int* perm; const int* ctl;                                                       // bucket sort (launch_bucket_plan)
+  const float* y; const float* ln_beta; const float* ln_gamma;                           // f = LN_b(y)
+  const float* h; const float* dhr; const float* dout;                                   // relu(f W1 + b1), dH o relu', dOUT
+  float* dWq; float* dWk; float* dWv;                                                    // [10, 40, 40]
+  float* dW1; float* db1; float* dW2; float* db2;
+  int n_tok;
+  bool ffn;                                                                              // the FFN pair, else the projection
+};
+void launch_enc_dw(const EncDwArgs& a, cudaStream_t st);
 
 // ---- kernels_attn_mma.cu (attention forward + backward on warp-level tensor-core MMAs, 3xTF32; used up to T = 128)
 int init_attn_mma_kernels(int max_T);

@@ -594,18 +594,16 @@ __device__ __forceinline__ void store_frag_rows(float* __restrict__ dst, const f
 }
 
 // ------------------------------------------------------------------------------------------
-// FFN + LN_b backward.  In: dOUT (grad of block output), Y.  Out: dY, and atomically
-// accumulated dW1, db1, dW2, db2, dbeta, dgamma.  Five 3xTF32 tensor-core GEMMs per token tile:
-//   h = relu(f W1 + b1) [recomputed],  dH = dOUT W2^T,  dF = dOUT + (dH o relu') W1^T,
-//   [dW2; db2] = [h 1]^T dOUT,  [dW1; db1] = [f 1]^T (dH o relu')      (weight gradients: warp-private 32-token slices,
-//   merged in shared memory, one global atomic per element and CTA).
-constexpr int kFfnBwdSmem = (4 * kDD + 3 * kTokTile * kTS + 2 * 41 * kD + 4 * kD + 2 * kD + kTokTile) * 4;
+// FFN + LN_b backward, input-gradient chain.  In: dOUT (grad of block output), Y.  Out: dY, the column sums dbeta / dgamma
+// (one global atomic per element and CTA), and for the weight gradients (k_enc_dw, off the critical path) H = relu(f W1 + b1),
+// DHR = dH o relu' and, when DOUT_KEEP is given, a copy of dOUT that outlives the buffer it came in.  Three 3xTF32 tensor-core
+// GEMMs per token tile:   h = relu(f W1 + b1) [recomputed: its sign is relu'],  dH = dOUT W2^T,  dF = dOUT + (dH o relu') W1^T.
+constexpr int kFfnBwdSmem = (4 * kDD + 3 * kTokTile * kTS + 4 * kD + 2 * kD + kTokTile) * 4;
 __global__ void __launch_bounds__(kTokThreads)
 k_ffn_bwd(const float* __restrict__ Y, const float* __restrict__ dOUT, const float* __restrict__ W1,
           const float* __restrict__ b1, const float* __restrict__ W2, const float* __restrict__ ln_beta,
-          const float* __restrict__ ln_gamma, float* __restrict__ dY, float* __restrict__ dW1, float* __restrict__ db1,
-          float* __restrict__ dW2, float* __restrict__ db2, float* __restrict__ dbeta, float* __restrict__ dgamma,
-          int n_tok) {
+          const float* __restrict__ ln_gamma, float* __restrict__ dY, float* __restrict__ H, float* __restrict__ DHR,
+          float* __restrict__ DOUT_KEEP, float* __restrict__ dbeta, float* __restrict__ dgamma, int n_tok) {
   extern __shared__ __align__(16) float sm[];
   uint32_t* W1hi = reinterpret_cast<uint32_t*>(sm);
   uint32_t* W1lo = W1hi + kDD;
@@ -614,9 +612,7 @@ k_ffn_bwd(const float* __restrict__ Y, const float* __restrict__ dOUT, const flo
   float* xs = sm + 4 * kDD;                    // y, then xhat
   float* hs = xs + kTokTile * kTS;             // h = relu(f W1 + b1), later dH o relu'
   float* gs = hs + kTokTile * kTS;             // dOUT
-  float* acc2 = gs + kTokTile * kTS;           // [41][40]: dW2 rows 0..39, db2 row 40
-  float* acc1 = acc2 + 41 * kD;                // [41][40]: dW1, db1
-  float* pr = acc1 + 41 * kD;                  // b1 | - | beta | gamma
+  float* pr = gs + kTokTile * kTS;             // b1 | - | beta | gamma
   float* red = pr + 4 * kD;                    // dbeta | dgamma
   float* rstd_s = red + 2 * kD;                // per-row 1/std
   const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
@@ -627,7 +623,6 @@ k_ffn_bwd(const float* __restrict__ Y, const float* __restrict__ dOUT, const flo
   load_split_mat(W2hi, W2lo, W2, tid);
   if (tid < kD) { pr[tid] = b1[tid]; pr[2 * kD + tid] = ln_beta[tid]; pr[3 * kD + tid] = ln_gamma[tid]; }
   if (tid < 2 * kD) red[tid] = 0.f;
-  for (int i = tid; i < 2 * 41 * kD; i += kTokThreads) acc2[i] = 0.f;
   load_tile44(xs, Y + tok0 * kD, nullptr, cnt, tid);
   load_tile44(gs, dOUT + tok0 * kD, nullptr, cnt, tid);
   __syncthreads();
@@ -636,6 +631,8 @@ k_ffn_bwd(const float* __restrict__ Y, const float* __restrict__ dOUT, const flo
     ln_row44(xs + tid * kTS, pr + 2 * kD, pr + 3 * kD, mean, rstd, kLnWriteXhat);
     rstd_s[tid] = rstd;
   }
+  if (DOUT_KEEP != nullptr)
+    for (int i = tid; i < cnt * 10; i += kTokThreads) st4(DOUT_KEEP + (tok0 + i / 10) * kD + 4 * (i % 10), ld4(gs + (i / 10) * kTS + 4 * (i % 10)));
   __syncthreads();
   const float* xw = xs + kWarpRows * w * kTS;
   float* hw = hs + kWarpRows * w * kTS;
@@ -658,9 +655,12 @@ k_ffn_bwd(const float* __restrict__ Y, const float* __restrict__ dOUT, const flo
 #pragma unroll
     for (int nt = 0; nt < 5; ++nt) {
       const int r = 16 * mt + g, col = 8 * nt + 2 * t;
-      *reinterpret_cast<float2*>(hw + r * kTS + col) = make_float2(fmaxf(c[mt][nt][0], 0.f), fmaxf(c[mt][nt][1], 0.f));
-      *reinterpret_cast<float2*>(hw + (r + 8) * kTS + col) = make_float2(fmaxf(c[mt][nt][2], 0.f), fmaxf(c[mt][nt][3], 0.f));
+#pragma unroll
+      for (int q = 0; q < 4; ++q) c[mt][nt][q] = fmaxf(c[mt][nt][q], 0.f);
+      *reinterpret_cast<float2*>(hw + r * kTS + col) = make_float2(c[mt][nt][0], c[mt][nt][1]);
+      *reinterpret_cast<float2*>(hw + (r + 8) * kTS + col) = make_float2(c[mt][nt][2], c[mt][nt][3]);
     }
+  store_frag_rows(H, c, tok0, nullptr, kWarpRows * w, cnt, lane);
   __syncwarp();
   // ---- dH = dOUT W2^T, masked by relu'
 #pragma unroll
@@ -682,19 +682,7 @@ k_ffn_bwd(const float* __restrict__ Y, const float* __restrict__ dOUT, const flo
       if (!(h1.x > 0.f)) c[mt][nt][2] = 0.f;
       if (!(h1.y > 0.f)) c[mt][nt][3] = 0.f;
     }
-  // ---- [dW2; db2] += [h 1]^T dOUT over this warp's 32 tokens
-  {
-    float cw[3][5][4];
-#pragma unroll
-    for (int mt = 0; mt < 3; ++mt)
-#pragma unroll
-      for (int nt = 0; nt < 5; ++nt)
-#pragma unroll
-        for (int q = 0; q < 4; ++q) cw[mt][nt][q] = 0.f;
-    warp_gemm_tn_48x40(cw, kWarpRows, [&](int r, int i) { return i < kD ? hw[r * kTS + i] : (i == kD ? 1.f : 0.f); },
-                       [&](int r, int n) { return gw[r * kTS + n]; }, lane);
-    tn_flush_smem(cw, acc2, lane);
-  }
+  store_frag_rows(DHR, c, tok0, nullptr, kWarpRows * w, cnt, lane);
   __syncwarp();
   // ---- hs <- dH o relu'
 #pragma unroll
@@ -717,37 +705,20 @@ k_ffn_bwd(const float* __restrict__ Y, const float* __restrict__ dOUT, const flo
       c[mt][nt][0] = g0.x; c[mt][nt][1] = g0.y; c[mt][nt][2] = g1.x; c[mt][nt][3] = g1.y;
     }
   warp_gemm_rows_x40x40<kMT, true>(c, [&](int r, int k) { return hw[r * kTS + k]; }, W1hi, W1lo, lane);
-  // ---- [dW1; db1] += [f 1]^T (dH o relu')
-  {
-    float cw[3][5][4];
-#pragma unroll
-    for (int mt = 0; mt < 3; ++mt)
-#pragma unroll
-      for (int nt = 0; nt < 5; ++nt)
-#pragma unroll
-        for (int q = 0; q < 4; ++q) cw[mt][nt][q] = 0.f;
-    warp_gemm_tn_48x40(cw, kWarpRows, [&](int r, int i) { return i < kD ? f_elem(r, i) : (i == kD ? 1.f : 0.f); },
-                       [&](int r, int n) { return hw[r * kTS + n]; }, lane);
-    tn_flush_smem(cw, acc1, lane);
-  }
   // ---- LN_b backward, dY out
   ln_bwd_frag(c, [&](int r, int col) { return *reinterpret_cast<const float2*>(xw + r * kTS + col); }, rstd_s + kWarpRows * w, gamma, red, lane);
   store_frag_rows(dY, c, tok0, nullptr, kWarpRows * w, cnt, lane);
   __syncthreads();
-  for (int i = tid; i < kDD; i += kTokThreads) { atomicAdd(dW2 + i, acc2[i]); atomicAdd(dW1 + i, acc1[i]); }
-  if (tid < kD) {
-    atomicAdd(db2 + tid, acc2[kDD + tid]); atomicAdd(db1 + tid, acc1[kDD + tid]);
-    atomicAdd(dbeta + tid, red[tid]); atomicAdd(dgamma + tid, red[kD + tid]);
-  }
+  if (tid < kD) { atomicAdd(dbeta + tid, red[tid]); atomicAdd(dgamma + tid, red[kD + tid]); }
 }
 
 void launch_ffn_bwd(const float* Y, const float* dOUT, const float* W1, const float* b1, const float* W2,
-                    const float* ln_beta, const float* ln_gamma, float* dY, float* dW1, float* db1, float* dW2,
-                    float* db2, float* dbeta, float* dgamma, int n_tok, cudaStream_t st) {
+                    const float* ln_beta, const float* ln_gamma, float* dY, float* H, float* DHR, float* dOUT_keep,
+                    float* dbeta, float* dgamma, int n_tok, cudaStream_t st) {
   PAMREC_PROF("ffn_bwd", 1, st);
   if (n_tok == 0) return;
-  k_ffn_bwd<<<(n_tok + kTokTile - 1) / kTokTile, kTokThreads, kFfnBwdSmem, st>>>(Y, dOUT, W1, b1, W2, ln_beta, ln_gamma, dY, dW1,
-                                                                             db1, dW2, db2, dbeta, dgamma, n_tok);
+  k_ffn_bwd<<<(n_tok + kTokTile - 1) / kTokTile, kTokThreads, kFfnBwdSmem, st>>>(Y, dOUT, W1, b1, W2, ln_beta, ln_gamma, dY, H, DHR,
+                                                                             dOUT_keep, dbeta, dgamma, n_tok);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -869,18 +840,18 @@ void launch_attn_bwd(const float* Q, const float* K, const float* V, const float
 }
 
 // ------------------------------------------------------------------------------------------
-// Projection + LN_a backward (bucket-sorted tiles).  In: X (block input), dY (residual path into qin), dQ, dK, dV.
-// Out: dX; atomically accumulated dWq/dWk/dWv[bucket], dbeta, dgamma.  Six 3xTF32 tensor-core GEMMs per tile:
-//   dqin = dY + dQ Wq^T,   dX = dK Wk^T + dV Wv^T + LN_a'(dqin),   dWq = qin^T dQ,  dWk = x^T dK,  dWv = x^T dV.
-constexpr int kProjBwdSmem = (6 * kDD + 2 * kTokTile * kTS + kDD + 2 * kD + 2 * kD + 2 * kTokTile) * 4;
+// Projection + LN_a backward (bucket-sorted tiles), input-gradient chain.  In: X (block input), dY (residual path into qin),
+// dQ, dK, dV.  Out: dX and the column sums dbeta, dgamma.  Three 3xTF32 tensor-core GEMMs per tile:
+//   dqin = dY + dQ Wq^T,   dX = dK Wk^T + dV Wv^T + LN_a'(dqin).
+// The table gradients dWq/dWk/dWv[bucket] are k_enc_dw's.
+constexpr int kProjBwdSmem = (6 * kDD + 2 * kTokTile * kTS + 2 * kD + 2 * kD + 2 * kTokTile) * 4;
 __global__ void __launch_bounds__(kTokThreads)
 k_proj_bwd(const float* __restrict__ X, const float* __restrict__ dY, const float* __restrict__ dQ,
            const float* __restrict__ dK, const float* __restrict__ dV, const int* __restrict__ perm,
            const int* __restrict__ ctl, const int* __restrict__ tile_bucket, const int* __restrict__ tile_begin,
            const int* __restrict__ tile_count, const float* __restrict__ Wq, const float* __restrict__ Wk,
            const float* __restrict__ Wv, const float* __restrict__ ln_beta, const float* __restrict__ ln_gamma,
-           float* __restrict__ dX, float* __restrict__ dWq, float* __restrict__ dWk, float* __restrict__ dWv,
-           float* __restrict__ dbeta, float* __restrict__ dgamma) {
+           float* __restrict__ dX, float* __restrict__ dbeta, float* __restrict__ dgamma) {
   int tile = blockIdx.x;
   if (tile >= ctl[32]) return;
   extern __shared__ __align__(16) float sm[];
@@ -888,8 +859,7 @@ k_proj_bwd(const float* __restrict__ X, const float* __restrict__ dY, const floa
   uint32_t* Wlo = Whi + 3 * kDD;
   float* xs = sm + 6 * kDD;                                 // x (raw)
   float* gs = xs + kTokTile * kTS;                          // dQ, then dK, then dV
-  float* acc = gs + kTokTile * kTS;                         // [40][40] weight-gradient partial sums of this CTA (one matrix at a time)
-  float* lnp = acc + kDD;                                   // beta | gamma
+  float* lnp = gs + kTokTile * kTS;                         // beta | gamma
   float* red = lnp + 2 * kD;                                // dbeta | dgamma
   float* mean_s = red + 2 * kD;
   float* rstd_s = mean_s + kTokTile;
@@ -897,14 +867,13 @@ k_proj_bwd(const float* __restrict__ X, const float* __restrict__ dY, const floa
   const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
   const int g = lane >> 2, t = lane & 3;
   const int k = tile_bucket[tile], begin = tile_begin[tile], cnt = tile_count[tile];
-  // zero matrices (bucket id outside 0..9): dX = LN_a'(dY) only, and no table row receives a gradient
+  // zero matrices (bucket id outside 0..9): dX = LN_a'(dY) only
   const bool zero = k == kZeroBin;
   load_split_mat(Whi, Wlo, zero ? nullptr : Wq + (int64_t)k * kDD, tid);
   load_split_mat(Whi + kDD, Wlo + kDD, zero ? nullptr : Wk + (int64_t)k * kDD, tid);
   load_split_mat(Whi + 2 * kDD, Wlo + 2 * kDD, zero ? nullptr : Wv + (int64_t)k * kDD, tid);
   if (tid < kD) { lnp[tid] = ln_beta[tid]; lnp[kD + tid] = ln_gamma[tid]; }
   if (tid < 2 * kD) red[tid] = 0.f;
-  for (int i = tid; i < kDD; i += kTokThreads) acc[i] = 0.f;
   if (tid < cnt) toks[tid] = perm[begin + tid];
   __syncthreads();
   load_tile44(xs, X, toks, cnt, tid);
@@ -920,7 +889,6 @@ k_proj_bwd(const float* __restrict__ X, const float* __restrict__ dY, const floa
   const float* gw = gs + kWarpRows * w * kTS;
   const float* mw = mean_s + kWarpRows * w;
   const float* rw = rstd_s + kWarpRows * w;
-  const float* beta = lnp;
   const float* gamma = lnp + kD;
   auto xhat = [&](int r, int i) { return (xw[r * kTS + i] - mw[r]) * rw[r]; };
   auto g_elem = [&](int r, int kk) { return gw[r * kTS + kk]; };
@@ -939,24 +907,6 @@ k_proj_bwd(const float* __restrict__ X, const float* __restrict__ dY, const floa
       }
     }
   warp_gemm_rows_x40x40<kMT, true>(dqin, g_elem, Whi, Wlo, lane);
-  {
-    float cw[3][5][4];
-#pragma unroll
-    for (int mt = 0; mt < 3; ++mt)
-#pragma unroll
-      for (int nt = 0; nt < 5; ++nt)
-#pragma unroll
-        for (int q = 0; q < 4; ++q) cw[mt][nt][q] = 0.f;
-    warp_gemm_tn_48x40(cw, kWarpRows, [&](int r, int i) { return i < kD ? fmaf(gamma[i], xhat(r, i), beta[i]) : 0.f; }, g_elem, lane);
-    tn_flush_smem(cw, acc, lane, kD - 1);
-  }
-  float* dWs[3] = {dWq + (int64_t)k * kDD, dWk + (int64_t)k * kDD, dWv + (int64_t)k * kDD};
-  // one global atomic per element and CTA; the accumulator is cleared for the next matrix (barriers: top of the loop below)
-  auto flush_acc = [&](float* dW) {
-    __syncthreads();
-    for (int i = tid; i < kDD; i += kTokThreads) { if (!zero) atomicAdd(dW + i, acc[i]); acc[i] = 0.f; }
-  };
-  flush_acc(dWs[0]);
   // ---- dX = dK Wk^T + dV Wv^T (+ LN backward below)
 #pragma unroll
   for (int mt = 0; mt < kMT; ++mt)
@@ -970,16 +920,6 @@ k_proj_bwd(const float* __restrict__ X, const float* __restrict__ dY, const floa
     load_tile44(gs, m == 1 ? dK : dV, toks, cnt, tid);
     __syncthreads();
     warp_gemm_rows_x40x40<kMT, true>(dx, g_elem, Whi + m * kDD, Wlo + m * kDD, lane);
-    float cw[3][5][4];
-#pragma unroll
-    for (int mt = 0; mt < 3; ++mt)
-#pragma unroll
-      for (int nt = 0; nt < 5; ++nt)
-#pragma unroll
-        for (int q = 0; q < 4; ++q) cw[mt][nt][q] = 0.f;
-    warp_gemm_tn_48x40(cw, kWarpRows, [&](int r, int i) { return i < kD ? xw[r * kTS + i] : 0.f; }, g_elem, lane);
-    tn_flush_smem(cw, acc, lane, kD - 1);
-    flush_acc(dWs[m]);
   }
   // ---- LN_a backward of dqin, added to dX
   ln_bwd_frag(dqin, [&](int r, int col) { return make_float2(xhat(r, col), xhat(r, col + 1)); }, rw, gamma, red, lane);
@@ -997,10 +937,118 @@ k_proj_bwd(const float* __restrict__ X, const float* __restrict__ dY, const floa
 void launch_proj_bwd(const float* X, const float* dY, const float* dQ, const float* dK, const float* dV, const int* perm,
                      const int* ctl, const int* tile_bucket, const int* tile_begin, const int* tile_count, int max_tiles,
                      const float* Wq, const float* Wk, const float* Wv, const float* ln_beta, const float* ln_gamma,
-                     float* dX, float* dWq, float* dWk, float* dWv, float* dbeta, float* dgamma, cudaStream_t st) {
+                     float* dX, float* dbeta, float* dgamma, cudaStream_t st) {
   PAMREC_PROF("proj_bwd", 1, st);
   k_proj_bwd<<<max_tiles, kTokThreads, kProjBwdSmem, st>>>(X, dY, dQ, dK, dV, perm, ctl, tile_bucket, tile_begin, tile_count, Wq,
-                                                        Wk, Wv, ln_beta, ln_gamma, dX, dWq, dWk, dWv, dbeta, dgamma);
+                                                        Wk, Wv, ln_beta, ln_gamma, dX, dbeta, dgamma);
+}
+
+// ------------------------------------------------------------------------------------------
+// Weight gradients of one encoder block.  Nothing reads them before the optimiser, so api.cu runs this kernel on the side
+// stream, beside the rest of the encoder's backward pass, in two launches per block as soon as their inputs exist:
+//   a.ffn:   [dW1; db1] = [f 1]^T (dH o relu'),  [dW2; db2] = [h 1]^T dOUT      over every token (f = LN_b(y) recomputed);
+//   !a.ffn:  dWq[k] = qin^T dQ,  dWk[k] = x^T dK,  dWv[k] = x^T dV      over the tokens of bucket k (the zero bin adds nothing).
+// The products of a launch (two FFN ones, or bucket x {q, k, v}) are laid end to end as one list of token rows, and CTA i takes
+// the i-th of gridDim.x equal ranges of that list: one or a few long runs per CTA whatever the bucket sizes.  Over a run every warp keeps
+// one 3xTF32 accumulator in registers (warp w: rows 16w .. 16w+15 of each 64-row tile; tiles double-buffered with cp.async);
+// at the end of the run the warps' sums meet in shared memory and leave as one global atomic per element.
+constexpr int kDwRun = 256;                                 // least tokens per CTA the grid is sized for
+constexpr int kEncDwSmem = (4 * kTokTile * kTS + 41 * kD + 2 * kD) * 4;
+__device__ __forceinline__ void cp_async16(float* dst, const float* src, bool valid) {   // !valid: 16 zero bytes
+  const unsigned d = (unsigned)__cvta_generic_to_shared(dst);
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;\n" ::"r"(d), "l"(src), "r"(valid ? 16 : 0));
+}
+__global__ void __launch_bounds__(kTokThreads)
+k_enc_dw(const EncDwArgs a) {
+  extern __shared__ __align__(16) float sm[];               // [2 buffers][A | B][kTokTile][kTS] | acc [41][40] | beta | gamma
+  float* acc = sm + 4 * kTokTile * kTS;
+  float* lnp = acc + 41 * kD;
+  __shared__ int s_cnt[kNB];
+  const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+  if (tid < kD) { lnp[tid] = a.ln_beta[tid]; lnp[kD + tid] = a.ln_gamma[tid]; }
+  if (tid < kNB) s_cnt[tid] = a.ctl[tid];
+  __syncthreads();
+  // products s in [s_lo, s_hi): 0, 1 the FFN ones, 2 + 3k + p bucket k of Q (p = 0), K (1), V (2)
+  const int s_lo = a.ffn ? 0 : 2, s_hi = a.ffn ? 2 : 2 + 3 * kNB;
+  int64_t total = 0;
+  if (a.ffn) total = 2 * (int64_t)a.n_tok;
+  else for (int k = 0; k < kNB; ++k) total += 3 * (int64_t)s_cnt[k];
+  const int64_t chunk = (total + gridDim.x - 1) / gridDim.x;
+  const int64_t lo = blockIdx.x * chunk, hi = min(total, lo + chunk);
+  const int lr = tid >> 1, c0 = 5 * (tid & 1);              // this thread copies row lr, float4 chunks c0 .. c0+4, of A and B
+  int64_t v = 0;
+  int bin0 = 0;                                             // first perm index of bucket k
+  for (int s = s_lo; s < s_hi && v < hi; ++s) {
+    const int k = s < 2 ? -1 : (s - 2) / 3, p = s < 2 ? -1 : (s - 2) % 3;
+    const int64_t len = s < 2 ? a.n_tok : s_cnt[k];
+    const int64_t b = max(lo, v) - v, e = min(hi, v + len) - v;
+    v += len;
+    if (b < e) {
+      const bool bias = s < 2;
+      const float* A = s == 0 ? a.y : s == 1 ? a.h : p == 0 ? a.qin : a.x;
+      const float* Bm = s == 0 ? a.dhr : s == 1 ? a.dout : p == 0 ? a.dQ : p == 1 ? a.dK : a.dV;
+      const int* rows = bias ? nullptr : a.perm + bin0;
+      float* dW = s == 0 ? a.dW1 : s == 1 ? a.dW2 : (p == 0 ? a.dWq : p == 1 ? a.dWk : a.dWv) + (int64_t)k * kDD;
+      float* db = s == 0 ? a.db1 : a.db2;
+      for (int i = tid; i < 41 * kD; i += kTokThreads) acc[i] = 0.f;
+      float cw[3][5][4];
+#pragma unroll
+      for (int mt = 0; mt < 3; ++mt)
+#pragma unroll
+        for (int nt = 0; nt < 5; ++nt)
+#pragma unroll
+          for (int q = 0; q < 4; ++q) cw[mt][nt][q] = 0.f;
+      auto row_of = [&](int64_t i) -> int64_t { return i < e ? (rows ? (int64_t)rows[i] : i) : -1; };
+      auto issue = [&](int buf, int64_t r) {                // one cp.async group per tile; rows past the run are zero-filled
+        float* da = sm + 2 * buf * kTokTile * kTS + lr * kTS + 4 * c0;
+        const int64_t o = (r >= 0 ? r : 0) * kD + 4 * c0;
+#pragma unroll
+        for (int j = 0; j < 5; ++j) {
+          cp_async16(da + 4 * j, A + o + 4 * j, r >= 0);
+          cp_async16(da + kTokTile * kTS + 4 * j, Bm + o + 4 * j, r >= 0);
+        }
+        asm volatile("cp.async.commit_group;\n" ::);
+      };
+      issue(0, row_of(b + lr));
+      int64_t nxt = row_of(b + kTokTile + lr);
+      int buf = 0;
+      for (int64_t t0 = b; t0 < e; t0 += kTokTile, buf ^= 1) {
+        if (t0 + kTokTile < e) issue(buf ^ 1, nxt);
+        else asm volatile("cp.async.commit_group;\n" ::);
+        nxt = row_of(t0 + 2 * kTokTile + lr);
+        asm volatile("cp.async.wait_group 1;\n" ::);
+        __syncthreads();
+        float* As = sm + 2 * buf * kTokTile * kTS;
+        if (s == 0) {                                       // f = LN_b(y), row tid
+          if (tid < kTokTile) { float mean, rstd; ln_row44(As + tid * kTS, lnp, lnp + kD, mean, rstd, kLnWriteF); }
+          __syncthreads();
+        }
+        const float* aw = As + kWarpRows * w * kTS;
+        const float* bw = aw + kTokTile * kTS;
+        warp_gemm_tn_48x40(cw, kWarpRows, [&](int r, int i) { return i < kD ? aw[r * kTS + i] : (i == kD && bias ? 1.f : 0.f); },
+                           [&](int r, int n) { return bw[r * kTS + n]; }, lane);
+        __syncthreads();                                    // the buffer is refilled two tiles on
+      }
+      tn_flush_smem(cw, acc, lane, bias ? kD : kD - 1);
+      __syncthreads();
+      for (int i = tid; i < kDD; i += kTokThreads) atomicAdd(dW + i, acc[i]);
+      if (bias && tid < kD) atomicAdd(db + tid, acc[kDD + tid]);
+      __syncthreads();                                      // acc is cleared by the next run
+    }
+    if (p == 2) bin0 += s_cnt[k];
+  }
+}
+
+void launch_enc_dw(const EncDwArgs& a, cudaStream_t st) {
+  PAMREC_PROF("enc_dw", 1, st);
+  if (a.n_tok == 0) return;
+  int dev = 0, n_sm = 0;
+  cudaGetDevice(&dev);
+  cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
+  // about one wave at two CTAs per SM, and runs of at least kDwRun tokens when every token is in a table bucket
+  const int64_t runs = ((a.ffn ? 2 : 3) * (int64_t)a.n_tok + kDwRun - 1) / kDwRun;
+  const int grid = (int)(runs < 2 * n_sm ? runs : 2 * n_sm);
+  k_enc_dw<<<grid, kTokThreads, kEncDwSmem, st>>>(a);
 }
 
 // Dynamic shared memory above 48 KB is an opt-in per kernel AND per device: pamrec_bind calls this on the handle's device, so
@@ -1014,6 +1062,7 @@ int init_encoder_kernels(int max_T) {
   set((const void*)k_ffn_fwd, kFfnFwdSmem);
   set((const void*)k_ffn_bwd, kFfnBwdSmem);
   set((const void*)k_proj_bwd, kProjBwdSmem);
+  set((const void*)k_enc_dw, kEncDwSmem);
   size_t af = 0, ab = 0;
   for (int T = 1; T <= max_T; ++T) { af = af > attn_fwd_smem(T) ? af : attn_fwd_smem(T); ab = ab > attn_bwd_smem(T) ? ab : attn_bwd_smem(T); }
   set((const void*)k_attn_fwd, af);

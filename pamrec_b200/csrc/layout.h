@@ -426,6 +426,11 @@ struct Layout {
     add_ws("d_Q", PAMREC_F32, {B, T, kD});
     add_ws("d_K", PAMREC_F32, {B, T, kD});
     add_ws("d_V", PAMREC_F32, {B, T, kD});
+    // inputs of the blocks' weight gradients (launch_enc_dw, side stream), which may still be reading them while the main stream
+    // runs the next block's backward: block 1 keeps its own dQ, dK, dV and a copy of its output gradient (d_Q, d_K, d_V and
+    // g_a are block 0's by then); h = relu(f W1 + b1) and dH o relu' of both blocks
+    for (const char* n : {"blk1.d_Q", "blk1.d_K", "blk1.d_V", "blk1.d_out"}) add_ws(n, PAMREC_F32, {B, T, kD});
+    for (const char* n : {"blk0.h", "blk0.dhr", "blk1.h", "blk1.dhr"}) add_ws(n, PAMREC_F32, {B, T, kD});
     // batch-norm statistics, optimiser scratch
     add_bn_ws();
     add_optim_ws();
