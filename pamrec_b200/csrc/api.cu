@@ -4,6 +4,7 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
+#include <functional>
 #include <string>
 #include <vector>
 
@@ -550,8 +551,128 @@ static DenseP dense_p(const float* X, int ldx, int M, int groups, int K, int N, 
   p.W = W; p.w_stride = ws; p.bias = bias; p.b_stride = bs; p.Z = Z; p.ldz = ldz;
   return p;
 }
-static void set_in_bn(DenseP& p, const BnSet& s) { p.in_stat = s.stat; p.in_gamma = s.gamma; p.in_beta = s.beta; }
-static void set_in_bn_dw(DenseDwP& p, const BnSet& s) { p.in_stat = s.stat; p.in_gamma = s.gamma; p.in_beta = s.beta; }
+static DenseDwP dw_p(const float* X, int ldx, int M, int groups, int K, int N, const float* dZ, int lddz, float* dW, int ws,
+                     float* db, int bs) {
+  DenseDwP p;
+  memset(&p, 0, sizeof p);
+  p.X = X; p.ldx = ldx; p.M = M; p.n_groups = groups; p.K = K; p.N = N; p.dZ = dZ; p.lddz = lddz;
+  p.dW = dW; p.w_stride = ws; p.db = db; p.b_stride = bs;
+  return p;
+}
+static DenseDxP dx_p(const float* dZ, int lddz, int M, int K, const float* Wbase, float* dX, int lddx, int accumulate) {
+  DenseDxP p;
+  memset(&p, 0, sizeof p);
+  p.dZ = dZ; p.lddz = lddz; p.M = M; p.K = K; p.Wbase = Wbase; p.dX = dX; p.lddx = lddx; p.accumulate = accumulate;
+  return p;
+}
+static void dx_add(DenseDxP& p, int slice, int out_off, int dz_off, int64_t w_off, int N) {
+  if (slice >= p.n_slices) { p.n_slices = slice + 1; p.out_off[slice] = out_off; p.n_contrib[slice] = 0; }
+  int c = p.n_contrib[slice]++;
+  p.dz_off[slice][c] = dz_off; p.w_off[slice][c] = w_off; p.Ncon[slice][c] = N;
+}
+
+// One group-strided BN MLP (layout.h: MlpOff) bound to its buffers.  Layer 0 of member g reads the columns x_col[g].. of x
+// (leading dimension ldx), layer l > 0 the member's own columns of z[l - 1]; layer l writes the member's columns g * n_of(l).. of
+// z[l] (leading dimension width(l): pre-BN values, the output layer's logits).  dz[l], laid out like z[l], holds the gradient with
+// respect to layer l's post-BN-ReLU activation (the output layer's: its logits).  The gradient of x goes to dx (leading dimension
+// ldx), added to what dx holds when dx_acc: the gates add theirs to the experts'.
+struct MlpBind {
+  const MlpOff* m;
+  int M; double count;                 // rows of this rank; rows that the batch norms normalise over (every rank's)
+  const float* x; int ldx; int x_col[8];
+  float* z[3]; float* dz[3];
+  float* dx; int dx_acc;
+};
+using BnSync = std::function<void(const std::vector<int>&)>;
+static void no_sync(const std::vector<int>&) {}
+
+// Forward pass of MLPs that read the same input, layer by layer: one layer of every MLP, then (training) sync(ids) on the batch-norm
+// sets that layer filled, then their statistics: e0, g0, finalize, e1, g1, finalize.
+static void mlp_forward(PamrecHandle h, std::initializer_list<const MlpBind*> ms, bool training, const BnSync& sync, cudaStream_t st) {
+  const MlpBind& first = **ms.begin();
+  for (int l = 0; l < first.m->n_layers(); ++l) {
+    std::vector<int> ids;
+    for (const MlpBind* b : ms) {
+      const MlpOff& m = *b->m;
+      const int K = m.k_of(l), N = m.n_of(l);
+      DenseP p = dense_p(l ? b->z[l - 1] : b->x, l ? m.width(l - 1) : b->ldx, b->M, m.G, K, N, h->P(m.w_of(l)), K * N,
+                         h->P(m.b_of(l)), N, b->z[l], m.width(l));
+      for (int g = 0; g < m.G; ++g) { p.x_off[g] = l ? g * K : b->x_col[g]; p.z_off[g] = g * N; }
+      if (l) { const BnSet& in = h->bn[m.bn_of(l - 1)]; p.in_stat = in.stat; p.in_gamma = in.gamma; p.in_beta = in.beta; }
+      if (l < 2 && training) { p.out_sums = h->bn[m.bn_of(l)].sums; ids.push_back(m.bn_of(l)); }
+      launch_dense_fwd(p, st);
+    }
+    if (ids.empty()) continue;
+    sync(ids);
+    for (int id : ids) launch_bn_finalize(h->bn[id], first.count, st);
+  }
+}
+
+// Backward pass of MLPs whose output gradients dz[top] are complete, layer by layer from the top.  Per MLP the weight gradient (no
+// consumer before the optimiser: side stream) with the parameter gradients of its layer's batch norm (times g_scale), then the input
+// gradient, which also accumulates the gradient sums of the batch norm below.  sync(ids) runs once those sums of the listed sets are
+// complete: first for the top sets of MLPs without an output layer (their gradient comes from a pooling or mixing kernel; summed
+// here by k_bn_bwd_stats), then after every layer but the first.
+static void mlp_backward(PamrecHandle h, std::initializer_list<const MlpBind*> ms, float g_scale, const BnSync& sync, cudaStream_t st) {
+  const BnSet* bn = h->bn;
+  const MlpBind& first = **ms.begin();
+  std::vector<int> ids;
+  for (const MlpBind* b : ms)
+    if (!b->m->out) { launch_bn_bwd_stats(bn[b->m->bn1], b->dz[1], b->z[1], b->M, st); ids.push_back(b->m->bn1); }
+  if (!ids.empty()) sync(ids);
+  for (int l = first.m->n_layers() - 1; l >= 0; --l) {
+    ids.clear();
+    for (const MlpBind* b : ms) {
+      const MlpOff& m = *b->m;
+      const int K = m.k_of(l), N = m.n_of(l);
+      const int ldx = l ? m.width(l - 1) : b->ldx;
+      DenseDwP w = dw_p(l ? b->z[l - 1] : b->x, ldx, b->M, m.G, K, N, b->dz[l], m.width(l), h->G(m.w_of(l)), K * N,
+                        h->G(m.b_of(l)), N);
+      DenseDxP x = dx_p(b->dz[l], m.width(l), b->M, K, h->buf.dense_param, l ? b->dz[l - 1] : b->dx, ldx, l ? 0 : b->dx_acc);
+      for (int g = 0; g < m.G; ++g) {
+        w.x_off[g] = l ? g * K : b->x_col[g]; w.z_off[g] = g * N;
+        // one slice of dX per input column: the first member reading it opens the slice, later ones add to it in member order
+        int s = 0;
+        while (s < x.n_slices && x.out_off[s] != w.x_off[g]) ++s;
+        dx_add(x, s, w.x_off[g], g * N, m.w_of(l) + (int64_t)g * K * N, N);
+      }
+      if (l) {
+        const BnId id = m.bn_of(l - 1);
+        w.in_stat = bn[id].stat; w.in_gamma = bn[id].gamma; w.in_beta = bn[id].beta;
+        x.o = BnGradOut{b->z[l - 1], bn[id].stat, bn[id].gamma, bn[id].beta, bn[id].bsums};
+        ids.push_back(id);
+      }
+      if (l < 2) {
+        const BnId id = m.bn_of(l);
+        w.g = x.g = BnGrad{b->z[l], bn[id].stat, bn[id].gamma, bn[id].beta, bn[id].bsums, b->count};
+        w.g_dgamma = bn[id].dgamma; w.g_dbeta = bn[id].dbeta; w.g_C = bn[id].C; w.g_scale = g_scale;
+      }
+      h->fork(st, [&](cudaStream_t s2) { launch_dense_dw(w, s2); });
+      launch_dense_dx(x, st);
+    }
+    if (!ids.empty()) sync(ids);
+  }
+}
+
+// The stand-alone head's MLPs (pamrec.py:273 attention-pooling score, :26-50 experts and gates, :212-215 and :71 towers on main |
+// target, sub | target, main | target) bound to their buffers.
+struct HeadMlps { MlpBind score, expert, gate, tower; };
+static HeadMlps head_mlps(PamrecHandle h, const PamrecBatch* b) {
+  const Layout& L = h->L;
+  const int B = b->batch, T = h->cfg.max_seq_len;
+  const double Bg = b->global_batch > 0 ? b->global_batch : B * h->cfg.world_size;
+  float* new_long = h->wf("new_long");
+  float* d_new_long = h->wf("d_new_long");
+  const int tin = L.tower.in;
+  HeadMlps m;
+  m.score = {&L.score, B * T, Bg * T, h->wf("blk1.out"), kD, {0}, {h->wf("z1"), h->wf("z2")}, {h->wf("d_a1"), h->wf("d_z2")},
+             h->wf("g_a"), 1};
+  m.expert = {&L.expert, B, Bg, new_long, kD, {0}, {h->wf("ze0"), h->wf("ze1")}, {h->wf("d_e0"), h->wf("d_e1")}, d_new_long, 0};
+  m.gate = {&L.gate, B, Bg, new_long, kD, {0}, {h->wf("zg0"), h->wf("zg1")}, {h->wf("d_g0"), h->wf("d_g1")}, d_new_long, 1};
+  m.tower = {&L.tower, B, Bg, h->wf("u"), 2 * tin, {0, tin, 0}, {h->wf("zt0"), h->wf("zt1"), h->wf("logits")},
+             {h->wf("d_t0"), h->wf("d_t1"), h->wf("d_logits")}, h->wf("d_u"), 0};
+  return m;
+}
 
 static int sib_forward(PamrecHandle h, const PamrecBatch* b, int training, float* pred_out, cudaStream_t st);
 static int sib_backward(PamrecHandle h, const PamrecBatch* b, cudaStream_t st);
@@ -627,14 +748,11 @@ int pamrec_forward(PamrecHandle h, const PamrecBatch* b, int training, float* pr
 // The stand-alone head (kernels_head.cu): a launch per layer.  Training: batch statistics of the listed sets -> (mean, invstd), moving
 // averages; data parallel: the column sums (plus, once, the listwise-group count) are first summed over the ranks by NCCL.
 static int head_forward(PamrecHandle h, const PamrecBatch* b, bool training, float* pred_out, cudaStream_t st) {
-  const Layout& L = h->L;
-  const int B = b->batch, T = h->cfg.max_seq_len, N = B * T;
+  const int B = b->batch, T = h->cfg.max_seq_len;
   const int W = h->cfg.world_size;
-  const int Bg = b->global_batch > 0 ? b->global_batch : B * W;
-  const double cntN = (double)Bg * T, cntB = (double)Bg;
   int crc = 0;
-  auto sync_finalize = [&](std::initializer_list<int> ids, double cnt, bool with_scalars) {
-    if (!training) return;
+  bool with_scalars = true;            // the listwise-group count travels with the first sums
+  auto sync_sums = [&](const std::vector<int>& ids) {
     if (W > 1 && !crc) {
       PAMREC_PROF("allreduce_bn_fwd", 1, st);
       crc |= h->comm.group_start();
@@ -642,99 +760,28 @@ static int head_forward(PamrecHandle h, const PamrecBatch* b, bool training, flo
       if (with_scalars) crc |= h->comm.all_reduce(h->wd("dp.scalars"), 8, COMM_F64, st);
       crc |= h->comm.group_end();
     }
-    for (int id : ids) launch_bn_finalize(h->bn[id], cnt, st);
+    with_scalars = false;
   };
   if (training && W > 1) {
     cudaMemsetAsync(h->wd("dp.scalars"), 0, 8 * sizeof(double), st);
     launch_count_valid_groups(b->plays, B, h->wd("dp.scalars"), st);
   }
-  const float* H = h->wf("blk1.out");
   BnSet* bn = h->bn;
   if (!training) {
     for (int i = 0; i < BN_COUNT; ++i) launch_bn_eval_stat(bn[i], st);
   }
-  // attention pooling score MLP (pamrec.py:273)
-  {
-    DenseP p = dense_p(H, kD, N, 1, kD, 20, h->P(L.score.w0), 0, h->P(L.score.b0), 0, h->wf("z1"), 20);
-    p.out_sums = training ? bn[BN_S0].sums : nullptr;
-    launch_dense_fwd(p, st);
-    sync_finalize({BN_S0}, cntN, true);
-    DenseP q = dense_p(h->wf("z1"), 20, N, 1, 20, 1, h->P(L.score.w1), 0, h->P(L.score.b1), 0, h->wf("z2"), 1);
-    set_in_bn(q, bn[BN_S0]);
-    q.out_sums = training ? bn[BN_S1].sums : nullptr;
-    launch_dense_fwd(q, st);
-    sync_finalize({BN_S1}, cntN, false);
-  }
-  launch_pool_fwd(H, h->wf("z2"), bn[BN_S1], b->mask, h->wf("new_long"), B, T, st);
-  // MMoE (pamrec.py:26-50)
-  {
-    DenseP e0 = dense_p(h->wf("new_long"), kD, B, 5, kD, 100, h->P(L.expert.w0), 4000, h->P(L.expert.b0), 100, h->wf("ze0"), 500);
-    for (int g = 0; g < 5; ++g) { e0.x_off[g] = 0; e0.z_off[g] = g * 100; }
-    e0.out_sums = training ? bn[BN_E0].sums : nullptr;
-    launch_dense_fwd(e0, st);
-    DenseP g0 = dense_p(h->wf("new_long"), kD, B, 2, kD, 64, h->P(L.gate.w0), 2560, h->P(L.gate.b0), 64, h->wf("zg0"), 128);
-    for (int g = 0; g < 2; ++g) { g0.x_off[g] = 0; g0.z_off[g] = g * 64; }
-    g0.out_sums = training ? bn[BN_G0].sums : nullptr;
-    launch_dense_fwd(g0, st);
-    sync_finalize({BN_E0, BN_G0}, cntB, false);
-    DenseP e1 = dense_p(h->wf("ze0"), 500, B, 5, 100, 64, h->P(L.expert.w1), 6400, h->P(L.expert.b1), 64, h->wf("ze1"), 320);
-    for (int g = 0; g < 5; ++g) { e1.x_off[g] = g * 100; e1.z_off[g] = g * 64; }
-    set_in_bn(e1, bn[BN_E0]);
-    e1.out_sums = training ? bn[BN_E1].sums : nullptr;
-    launch_dense_fwd(e1, st);
-    DenseP g1 = dense_p(h->wf("zg0"), 128, B, 2, 64, 5, h->P(L.gate.w1), 320, h->P(L.gate.b1), 5, h->wf("zg1"), 10);
-    for (int g = 0; g < 2; ++g) { g1.x_off[g] = g * 64; g1.z_off[g] = g * 5; }
-    set_in_bn(g1, bn[BN_G0]);
-    g1.out_sums = training ? bn[BN_G1].sums : nullptr;
-    launch_dense_fwd(g1, st);
-    sync_finalize({BN_E1, BN_G1}, cntB, false);
-  }
+  const HeadMlps m = head_mlps(h, b);
+  mlp_forward(h, {&m.score}, training, sync_sums, st);
+  launch_pool_fwd(h->wf("blk1.out"), h->wf("z2"), bn[BN_S1], b->mask, h->wf("new_long"), B, T, st);
+  mlp_forward(h, {&m.expert, &m.gate}, training, sync_sums, st);
   launch_combine_fwd(h->wf("ze1"), h->wf("zg1"), bn[BN_E1], bn[BN_G1], h->wf("tgt"), h->wf("u"), B, st);
-  // towers: logit_fcn(main|tgt), valid_logit_fcn(sub|tgt), xilidu_logit_fcn(main|tgt)   pamrec.py:212-215, 71
-  {
-    DenseP t0 = dense_p(h->wf("u"), 168, B, 3, 84, 100, h->P(L.tower.w0), 8400, h->P(L.tower.b0), 100, h->wf("zt0"), 300);
-    t0.x_off[0] = 0; t0.x_off[1] = 84; t0.x_off[2] = 0;
-    for (int g = 0; g < 3; ++g) t0.z_off[g] = g * 100;
-    t0.out_sums = training ? bn[BN_T0].sums : nullptr;
-    launch_dense_fwd(t0, st);
-    sync_finalize({BN_T0}, cntB, false);
-    DenseP t1 = dense_p(h->wf("zt0"), 300, B, 3, 100, 64, h->P(L.tower.w1), 6400, h->P(L.tower.b1), 64, h->wf("zt1"), 192);
-    for (int g = 0; g < 3; ++g) { t1.x_off[g] = g * 100; t1.z_off[g] = g * 64; }
-    set_in_bn(t1, bn[BN_T0]);
-    t1.out_sums = training ? bn[BN_T1].sums : nullptr;
-    launch_dense_fwd(t1, st);
-    sync_finalize({BN_T1}, cntB, false);
-    DenseP to = dense_p(h->wf("zt1"), 192, B, 3, 64, 1, h->P(L.tower.wout), 64, h->P(L.tower.bout), 1, h->wf("logits"), 3);
-    for (int g = 0; g < 3; ++g) { to.x_off[g] = g * 64; to.z_off[g] = g; }
-    set_in_bn(to, bn[BN_T1]);
-    launch_dense_fwd(to, st);
-  }
+  mlp_forward(h, {&m.tower}, training, sync_sums, st);
   if (pred_out) launch_sigmoid_col0(h->wf("logits"), pred_out, B, st);
   if (crc) return fail(h, "nccl: %s", h->comm.err.c_str());
   return 0;
 }
 
 // ------------------------------------------------------------------------------------------
-static DenseDwP dw_p(const float* X, int ldx, int M, int groups, int K, int N, const float* dZ, int lddz, float* dW, int ws,
-                     float* db, int bs) {
-  DenseDwP p;
-  memset(&p, 0, sizeof p);
-  p.X = X; p.ldx = ldx; p.M = M; p.n_groups = groups; p.K = K; p.N = N; p.dZ = dZ; p.lddz = lddz;
-  p.dW = dW; p.w_stride = ws; p.db = db; p.b_stride = bs;
-  return p;
-}
-static DenseDxP dx_p(const float* dZ, int lddz, int M, int K, const float* Wbase, float* dX, int lddx, int accumulate) {
-  DenseDxP p;
-  memset(&p, 0, sizeof p);
-  p.dZ = dZ; p.lddz = lddz; p.M = M; p.K = K; p.Wbase = Wbase; p.dX = dX; p.lddx = lddx; p.accumulate = accumulate;
-  return p;
-}
-static void dx_add(DenseDxP& p, int slice, int out_off, int dz_off, int64_t w_off, int N) {
-  if (slice >= p.n_slices) { p.n_slices = slice + 1; p.out_off[slice] = out_off; p.n_contrib[slice] = 0; }
-  int c = p.n_contrib[slice]++;
-  p.dz_off[slice][c] = dz_off; p.w_off[slice][c] = w_off; p.Ncon[slice][c] = N;
-}
-
 // per-call values of the cooperative head kernels; slot0 = first mailbox slot of this kernel's barriers
 static HeadDyn head_dyn(PamrecHandle h, const PamrecBatch* b, bool training, int slot0) {
   HeadDyn d;
@@ -805,14 +852,12 @@ static int build_head(PamrecHandle h, cudaStream_t st) {
 // summed over the ranks by NCCL.  Returns non-zero when an NCCL call failed; the caller reports it after joining the side stream.
 static int head_backward(PamrecHandle h, const PamrecBatch* b, cudaStream_t st) {
   const Layout& L = h->L;
-  const int B = b->batch, T = h->cfg.max_seq_len, N = B * T;
+  const int B = b->batch, T = h->cfg.max_seq_len;
   const int W = h->cfg.world_size;
   const int Bg = b->global_batch > 0 ? b->global_batch : B * W;
-  const double cntN = (double)Bg * T, cntB = (double)Bg;
   const float gs = 1.0f / (float)W;    // BN parameter gradients are already global: the dense all-reduce sums W copies
   BnSet* bn = h->bn;
   int crc = 0;
-  const float* Pb = h->buf.dense_param;
   launch_loss(h->wf("logits"), b->labels_satisfied, b->labels_play, b->plays, h->wf("d_logits"), h->wd("loss_acc"), B, Bg,
               W > 1 ? h->wd("dp.scalars") : nullptr, h->cfg.fuzhu_weight, h->cfg.order_weight,
               h->cfg.loss_kind == PAMREC_LOSS_SOFTMAX ? h->cfg.softmax_group : 0, st);
@@ -820,126 +865,21 @@ static int head_backward(PamrecHandle h, const PamrecBatch* b, cudaStream_t st) 
   // gradient buffer also accumulates the two column sums of its layer's BN, the consumers turn dA into dz while loading.
   // Buffers produced by the mixing / pooling kernels get their sums from k_bn_bwd_stats.  Data parallel: sums over ranks.
   cudaMemsetAsync(h->wd("bn.bsums"), 0, (size_t)L.ws[L.ws_index.at("bn.bsums")].numel * sizeof(double), st);
-  auto sync_bsums = [&](std::initializer_list<int> ids) {
+  auto sync_bsums = [&](const std::vector<int>& ids) {
     if (W == 1 || crc) return;
     PAMREC_PROF("allreduce_bn_bwd", 1, st);
     crc |= h->comm.group_start();
     for (int id : ids) crc |= h->comm.all_reduce(bn[id].bsums, 2 * (int64_t)bn[id].C, COMM_F64, st);
     crc |= h->comm.group_end();
   };
-  auto grad_of = [&](int id, const float* Z, double cnt) {
-    BnGrad g; g.Z = Z; g.stat = bn[id].stat; g.gamma = bn[id].gamma; g.beta = bn[id].beta; g.bsums = bn[id].bsums; g.count = cnt;
-    return g;
-  };
-  auto out_of = [&](int id, const float* Z) {
-    BnGradOut o; o.Z = Z; o.stat = bn[id].stat; o.gamma = bn[id].gamma; o.beta = bn[id].beta; o.bsums = bn[id].bsums;
-    return o;
-  };
-  auto dw_bn = [&](DenseDwP& w, int id, const float* Z, double cnt) {
-    w.g = grad_of(id, Z, cnt); w.g_dgamma = bn[id].dgamma; w.g_dbeta = bn[id].dbeta; w.g_C = bn[id].C; w.g_scale = gs;
-  };
-  // ---- towers
-  {
-    DenseDwP w = dw_p(h->wf("zt1"), 192, B, 3, 64, 1, h->wf("d_logits"), 3, h->G(L.tower.wout), 64, h->G(L.tower.bout), 1);
-    for (int g = 0; g < 3; ++g) { w.x_off[g] = g * 64; w.z_off[g] = g; }
-    set_in_bn_dw(w, bn[BN_T1]);
-    h->fork(st, [&](cudaStream_t s2) { launch_dense_dw(w, s2); });
-    DenseDxP x = dx_p(h->wf("d_logits"), 3, B, 64, Pb, h->wf("d_t1"), 192, 0);
-    for (int g = 0; g < 3; ++g) dx_add(x, g, g * 64, g, L.tower.wout + g * 64, 1);
-    x.o = out_of(BN_T1, h->wf("zt1"));
-    launch_dense_dx(x, st);
-    sync_bsums({BN_T1});
-    DenseDwP w1 = dw_p(h->wf("zt0"), 300, B, 3, 100, 64, h->wf("d_t1"), 192, h->G(L.tower.w1), 6400, h->G(L.tower.b1), 64);
-    for (int g = 0; g < 3; ++g) { w1.x_off[g] = g * 100; w1.z_off[g] = g * 64; }
-    set_in_bn_dw(w1, bn[BN_T0]);
-    dw_bn(w1, BN_T1, h->wf("zt1"), cntB);
-    h->fork(st, [&](cudaStream_t s2) { launch_dense_dw(w1, s2); });
-    DenseDxP x1 = dx_p(h->wf("d_t1"), 192, B, 100, Pb, h->wf("d_t0"), 300, 0);
-    for (int g = 0; g < 3; ++g) dx_add(x1, g, g * 100, g * 64, L.tower.w1 + (int64_t)g * 6400, 64);
-    x1.g = grad_of(BN_T1, h->wf("zt1"), cntB);
-    x1.o = out_of(BN_T0, h->wf("zt0"));
-    launch_dense_dx(x1, st);
-    sync_bsums({BN_T0});
-    DenseDwP w0 = dw_p(h->wf("u"), 168, B, 3, 84, 100, h->wf("d_t0"), 300, h->G(L.tower.w0), 8400, h->G(L.tower.b0), 100);
-    w0.x_off[0] = 0; w0.x_off[1] = 84; w0.x_off[2] = 0;
-    for (int g = 0; g < 3; ++g) w0.z_off[g] = g * 100;
-    dw_bn(w0, BN_T0, h->wf("zt0"), cntB);
-    h->fork(st, [&](cudaStream_t s2) { launch_dense_dw(w0, s2); });
-    DenseDxP x0 = dx_p(h->wf("d_t0"), 300, B, 84, Pb, h->wf("d_u"), 168, 0);
-    dx_add(x0, 0, 0, 0, L.tower.w0, 100);
-    dx_add(x0, 0, 0, 200, L.tower.w0 + 2 * 8400, 100);
-    dx_add(x0, 1, 84, 100, L.tower.w0 + 8400, 100);
-    x0.g = grad_of(BN_T0, h->wf("zt0"), cntB);
-    launch_dense_dx(x0, st);
-  }
+  const HeadMlps m = head_mlps(h, b);
+  mlp_backward(h, {&m.tower}, gs, sync_bsums, st);
   launch_combine_bwd(h->wf("ze1"), h->wf("zg1"), bn[BN_E1], bn[BN_G1], h->wf("d_u"), h->wf("d_e1"), h->wf("d_g1"),
                      h->wf("d_tgt"), B, st);
-  // ---- MMoE
-  {
-    launch_bn_bwd_stats(bn[BN_E1], h->wf("d_e1"), h->wf("ze1"), B, st);
-    launch_bn_bwd_stats(bn[BN_G1], h->wf("d_g1"), h->wf("zg1"), B, st);
-    sync_bsums({BN_E1, BN_G1});
-    DenseDwP we = dw_p(h->wf("ze0"), 500, B, 5, 100, 64, h->wf("d_e1"), 320, h->G(L.expert.w1), 6400, h->G(L.expert.b1), 64);
-    for (int g = 0; g < 5; ++g) { we.x_off[g] = g * 100; we.z_off[g] = g * 64; }
-    set_in_bn_dw(we, bn[BN_E0]);
-    dw_bn(we, BN_E1, h->wf("ze1"), cntB);
-    h->fork(st, [&](cudaStream_t s2) { launch_dense_dw(we, s2); });
-    DenseDxP xe = dx_p(h->wf("d_e1"), 320, B, 100, Pb, h->wf("d_e0"), 500, 0);
-    for (int g = 0; g < 5; ++g) dx_add(xe, g, g * 100, g * 64, L.expert.w1 + (int64_t)g * 6400, 64);
-    xe.g = grad_of(BN_E1, h->wf("ze1"), cntB);
-    xe.o = out_of(BN_E0, h->wf("ze0"));
-    launch_dense_dx(xe, st);
-    DenseDwP wg = dw_p(h->wf("zg0"), 128, B, 2, 64, 5, h->wf("d_g1"), 10, h->G(L.gate.w1), 320, h->G(L.gate.b1), 5);
-    for (int g = 0; g < 2; ++g) { wg.x_off[g] = g * 64; wg.z_off[g] = g * 5; }
-    set_in_bn_dw(wg, bn[BN_G0]);
-    dw_bn(wg, BN_G1, h->wf("zg1"), cntB);
-    h->fork(st, [&](cudaStream_t s2) { launch_dense_dw(wg, s2); });
-    DenseDxP xg = dx_p(h->wf("d_g1"), 10, B, 64, Pb, h->wf("d_g0"), 128, 0);
-    for (int g = 0; g < 2; ++g) dx_add(xg, g, g * 64, g * 5, L.gate.w1 + (int64_t)g * 320, 5);
-    xg.g = grad_of(BN_G1, h->wf("zg1"), cntB);
-    xg.o = out_of(BN_G0, h->wf("zg0"));
-    launch_dense_dx(xg, st);
-    sync_bsums({BN_E0, BN_G0});
-    DenseDwP we0 = dw_p(h->wf("new_long"), kD, B, 5, kD, 100, h->wf("d_e0"), 500, h->G(L.expert.w0), 4000, h->G(L.expert.b0), 100);
-    for (int g = 0; g < 5; ++g) { we0.x_off[g] = 0; we0.z_off[g] = g * 100; }
-    dw_bn(we0, BN_E0, h->wf("ze0"), cntB);
-    h->fork(st, [&](cudaStream_t s2) { launch_dense_dw(we0, s2); });
-    DenseDwP wg0 = dw_p(h->wf("new_long"), kD, B, 2, kD, 64, h->wf("d_g0"), 128, h->G(L.gate.w0), 2560, h->G(L.gate.b0), 64);
-    for (int g = 0; g < 2; ++g) { wg0.x_off[g] = 0; wg0.z_off[g] = g * 64; }
-    dw_bn(wg0, BN_G0, h->wf("zg0"), cntB);
-    h->fork(st, [&](cudaStream_t s2) { launch_dense_dw(wg0, s2); });
-    DenseDxP xe0 = dx_p(h->wf("d_e0"), 500, B, kD, Pb, h->wf("d_new_long"), kD, 0);
-    for (int g = 0; g < 5; ++g) dx_add(xe0, 0, 0, g * 100, L.expert.w0 + (int64_t)g * 4000, 100);
-    xe0.g = grad_of(BN_E0, h->wf("ze0"), cntB);
-    launch_dense_dx(xe0, st);
-    DenseDxP xg0 = dx_p(h->wf("d_g0"), 128, B, kD, Pb, h->wf("d_new_long"), kD, 1);
-    for (int g = 0; g < 2; ++g) dx_add(xg0, 0, 0, g * 64, L.gate.w0 + (int64_t)g * 2560, 64);
-    xg0.g = grad_of(BN_G0, h->wf("zg0"), cntB);
-    launch_dense_dx(xg0, st);
-  }
+  mlp_backward(h, {&m.expert, &m.gate}, gs, sync_bsums, st);
   // ---- attention pooling
-  const float* H = h->wf("blk1.out");
-  float* g_a = h->wf("g_a");
-  launch_pool_bwd(H, h->wf("z2"), bn[BN_S1], b->mask, h->wf("d_new_long"), h->wf("d_z2"), g_a, B, T, st);
-  launch_bn_bwd_stats(bn[BN_S1], h->wf("d_z2"), h->wf("z2"), N, st);
-  sync_bsums({BN_S1});
-  DenseDwP w1 = dw_p(h->wf("z1"), 20, N, 1, 20, 1, h->wf("d_z2"), 1, h->G(L.score.w1), 0, h->G(L.score.b1), 0);
-  set_in_bn_dw(w1, bn[BN_S0]);
-  dw_bn(w1, BN_S1, h->wf("z2"), cntN);
-  h->fork(st, [&](cudaStream_t s2) { launch_dense_dw(w1, s2); });
-  DenseDxP x1 = dx_p(h->wf("d_z2"), 1, N, 20, Pb, h->wf("d_a1"), 20, 0);
-  dx_add(x1, 0, 0, 0, L.score.w1, 1);
-  x1.g = grad_of(BN_S1, h->wf("z2"), cntN);
-  x1.o = out_of(BN_S0, h->wf("z1"));
-  launch_dense_dx(x1, st);
-  sync_bsums({BN_S0});
-  DenseDwP w0 = dw_p(H, kD, N, 1, kD, 20, h->wf("d_a1"), 20, h->G(L.score.w0), 0, h->G(L.score.b0), 0);
-  dw_bn(w0, BN_S0, h->wf("z1"), cntN);
-  h->fork(st, [&](cudaStream_t s2) { launch_dense_dw(w0, s2); });
-  DenseDxP x0 = dx_p(h->wf("d_a1"), 20, N, kD, Pb, g_a, kD, 1);
-  dx_add(x0, 0, 0, 0, L.score.w0, 20);
-  x0.g = grad_of(BN_S0, h->wf("z1"), cntN);
-  launch_dense_dx(x0, st);
+  launch_pool_bwd(h->wf("blk1.out"), h->wf("z2"), bn[BN_S1], b->mask, h->wf("d_new_long"), h->wf("d_z2"), h->wf("g_a"), B, T, st);
+  mlp_backward(h, {&m.score}, gs, sync_bsums, st);
   return crc;
 }
 

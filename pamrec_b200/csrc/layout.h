@@ -21,11 +21,26 @@ struct TensorDesc {
 };
 
 struct BlockOff { int64_t ln_a_beta, ln_a_gamma, wq, wk, wv, w1, b1, w2, b2, ln_b_beta, ln_b_gamma; };
-// 2-layer BN MLP, group-strided: offset of group 0; group g lives at off + g * (numel of one member)
-struct MlpOff { int64_t w0, b0, g0, be0, w1, b1, g1, be1, wout, bout; };
 struct BnOff { int C; int64_t gamma, beta, mm, mv; };
 
 enum BnId { BN_S0 = 0, BN_S1, BN_E0, BN_G0, BN_E1, BN_G1, BN_T0, BN_T1, BN_COUNT };
+
+// 2-layer BN MLP of G group members, in -> h0 -> h1 (-> 1 when out), group-strided: offset of group 0; group g lives at
+// off + g * (numel of one member).  Layer l = 0, 1 (, 2 = output) maps k_of(l) to n_of(l) columns per member; the batch norms
+// of layers 0 and 1 are the sets bn0 (G * h0 channels) and bn1 (G * h1).
+struct MlpOff {
+  int64_t w0, b0, g0, be0, w1, b1, g1, be1, wout, bout;
+  int G = 0, in = 0, h0 = 0, h1 = 0;
+  bool out = false;
+  BnId bn0 = BN_COUNT, bn1 = BN_COUNT;
+  int n_layers() const { return out ? 3 : 2; }
+  int k_of(int l) const { return l == 0 ? in : (l == 1 ? h0 : h1); }
+  int n_of(int l) const { return l == 0 ? h0 : (l == 1 ? h1 : 1); }
+  int width(int l) const { return G * n_of(l); }                       // columns of layer l's output over all members
+  int64_t w_of(int l) const { return l == 0 ? w0 : (l == 1 ? w1 : wout); }
+  int64_t b_of(int l) const { return l == 0 ? b0 : (l == 1 ? b1 : bout); }
+  BnId bn_of(int l) const { return l == 0 ? bn0 : bn1; }               // l = 0, 1
+};
 
 // one row-sharded table as seen by the exchange (PAMREC_TABLES_SHARDED)
 struct ShardDim { int64_t vocab = 0, rps = 0, nk = 0, cap_recv = 0; int width = 0; };
@@ -90,10 +105,11 @@ struct Layout {
     return (size_t)ws[it->second].offset;
   }
 
-  // members: TF scope of each group member; sizes in->h0->h1(->1)
+  // members: TF scope of each group member; sizes in->h0->h1(->1); bn0 / bn1: the batch-norm sets it fills (BN_COUNT: none)
   MlpOff add_mlp(const std::vector<std::string>& scopes, const std::vector<int>& flags, int in, int h0, int h1, bool out,
-                 BnOff* bn0, BnOff* bn1, bool live = true) {
+                 BnId bn0, BnId bn1) {
     MlpOff o{};
+    o.G = (int)scopes.size(); o.in = in; o.h0 = h0; o.h1 = h1; o.out = out; o.bn0 = bn0; o.bn1 = bn1;
     auto role = [&](const char* leaf, std::initializer_list<int64_t> shape) {
       int64_t first = -1;
       for (size_t g = 0; g < scopes.size(); ++g) {
@@ -121,9 +137,8 @@ struct Layout {
     for (int g = 0; g < G; ++g) { int64_t x = add_bn(scopes[g] + "/nn_part/batch_normalization/moving_variance", h0); if (!g) mv0 = x; }
     for (int g = 0; g < G; ++g) { int64_t x = add_bn(scopes[g] + "/nn_part/batch_normalization_1/moving_mean", h1); if (!g) mm1 = x; }
     for (int g = 0; g < G; ++g) { int64_t x = add_bn(scopes[g] + "/nn_part/batch_normalization_1/moving_variance", h1); if (!g) mv1 = x; }
-    if (bn0) *bn0 = BnOff{G * h0, o.g0, o.be0, mm0, mv0};
-    if (bn1) *bn1 = BnOff{G * h1, o.g1, o.be1, mm1, mv1};
-    (void)live;
+    if (bn0 != BN_COUNT) bnoff[bn0] = BnOff{G * h0, o.g0, o.be0, mm0, mv0};
+    if (bn1 != BN_COUNT) bnoff[bn1] = BnOff{G * h1, o.g1, o.be1, mm1, mv1};
     return o;
   }
 
@@ -161,7 +176,7 @@ struct Layout {
     att_mat = add_dense(clsr + "long_term/attention_fcn/attention_mat", {E, E}, L2);          // mmoe.py:315-319
     add_dense(clsr + "short_term/attention_fcn/attention_mat", {E, E}, L2);
     att = add_mlp({clsr + "long_term/attention_fcn/att_fcn", clsr + "short_term/attention_fcn/att_fcn"}, {L2, L2}, 4 * E, 80, 40, true,
-                  &bnoff[BN_S0], &bnoff[BN_S1]);                                                 // mmoe.py:327-329
+                  BN_S0, BN_S1);                                                                 // mmoe.py:327-329
     const int x_dim = 3 * E;
     std::vector<std::string> ex;
     if (model_kind == PAMREC_MODEL_MMOE) {
@@ -175,49 +190,49 @@ struct Layout {
     }
     n_expert = (int)ex.size();
     if (n_expert) {
-      expert = add_mlp(ex, std::vector<int>(ex.size(), L2), x_dim, 100, 64, false, &bnoff[BN_E0], &bnoff[BN_E1]);
-      gate = add_mlp({clsr + "gate_main", clsr + "gate_sub"}, {L2, L2}, x_dim, 64, 5, false, &bnoff[BN_G0], &bnoff[BN_G1]);
+      expert = add_mlp(ex, std::vector<int>(ex.size(), L2), x_dim, 100, 64, false, BN_E0, BN_E1);
+      gate = add_mlp({clsr + "gate_main", clsr + "gate_sub"}, {L2, L2}, x_dim, 64, 5, false, BN_G0, BN_G1);
       tower_in = 64 + E;
     } else {
       bnoff[BN_E0] = bnoff[BN_E1] = bnoff[BN_G0] = bnoff[BN_G1] = BnOff{0, 0, 0, 0, 0};
       tower_in = x_dim;                                                                          // sharebottom.py:200-201
     }
-    tower = add_mlp({"sequential/logit_fcn", "sequential/valid_logit_fcn"}, {L2, L2}, tower_in, 100, 64, true, &bnoff[BN_T0], &bnoff[BN_T1]);
+    tower = add_mlp({"sequential/logit_fcn", "sequential/valid_logit_fcn"}, {L2, L2}, tower_in, 100, 64, true, BN_T0, BN_T1);
     // ---- workspace.  Branch 0 = long_term (satisfied-only history), branch 1 = short_term (full history).
     add_ws("sib.ids_item", PAMREC_I32, {2, N});      // lookups of the item table in branch order (keys of the sparse plan)
     add_ws("sib.ids_cate", PAMREC_I32, {2, N});
     add_ws("sib.h", PAMREC_F32, {2, N, E});         // gathered history tokens item | cate
     add_ws("tgt", PAMREC_F32, {B, E});
     add_ws("sib.feat", PAMREC_F32, {N, 8 * E});      // per branch: a = h A | q | a - q | a * q   (mmoe.py:320-326)
-    add_ws("z1", PAMREC_F32, {N, 160});              // att_fcn layer 0 pre-activations (both branches)
-    add_ws("z2", PAMREC_F32, {N, 80});               // layer 1
-    add_ws("sib.score", PAMREC_F32, {N, 2});         // linear output = attention logits
+    add_ws("z1", PAMREC_F32, {N, att.width(0)});     // att_fcn layer 0 pre-activations (both branches)
+    add_ws("z2", PAMREC_F32, {N, att.width(1)});     // layer 1
+    add_ws("sib.score", PAMREC_F32, {N, att.width(2)});   // linear output = attention logits
     add_ws("sib.aw", PAMREC_F32, {2, N});            // softmax weights, kept for the backward pass
     add_ws("x", PAMREC_F32, {B, x_dim});             // long | short | target
-    add_ws("ze0", PAMREC_F32, {B, (int64_t)n_expert * 100});
-    add_ws("zg0", PAMREC_F32, {B, n_expert ? 128 : 0});
-    add_ws("ze1", PAMREC_F32, {B, (int64_t)n_expert * 64});
-    add_ws("zg1", PAMREC_F32, {B, n_expert ? 10 : 0});
+    add_ws("ze0", PAMREC_F32, {B, expert.width(0)});   // no experts nor gates (share-bottom): 0 columns
+    add_ws("zg0", PAMREC_F32, {B, gate.width(0)});
+    add_ws("ze1", PAMREC_F32, {B, expert.width(1)});
+    add_ws("zg1", PAMREC_F32, {B, gate.width(1)});
     add_ws("u", PAMREC_F32, {B, 2 * (64 + E)});   // main | target | sub | target
-    add_ws("zt0", PAMREC_F32, {B, 200});
-    add_ws("zt1", PAMREC_F32, {B, 128});
-    add_ws("logits", PAMREC_F32, {B, 2});            // logit_fcn (satisfied label), valid_logit_fcn (play label)
+    add_ws("zt0", PAMREC_F32, {B, tower.width(0)});
+    add_ws("zt1", PAMREC_F32, {B, tower.width(1)});
+    add_ws("logits", PAMREC_F32, {B, tower.width(2)});   // logit_fcn (satisfied label), valid_logit_fcn (play label)
     add_ws("losses", PAMREC_F32, {8});
     add_ws("loss_acc", PAMREC_F64, {8});
-    add_ws("d_logits", PAMREC_F32, {B, 2});
-    add_ws("d_t1", PAMREC_F32, {B, 128});
-    add_ws("d_t0", PAMREC_F32, {B, 200});
+    add_ws("d_logits", PAMREC_F32, {B, tower.width(2)});
+    add_ws("d_t1", PAMREC_F32, {B, tower.width(1)});
+    add_ws("d_t0", PAMREC_F32, {B, tower.width(0)});
     add_ws("d_u", PAMREC_F32, {B, 2 * (64 + E)});
-    add_ws("d_e1", PAMREC_F32, {B, (int64_t)n_expert * 64});
-    add_ws("d_g1", PAMREC_F32, {B, n_expert ? 10 : 0});
-    add_ws("d_e0", PAMREC_F32, {B, (int64_t)n_expert * 100});
-    add_ws("d_g0", PAMREC_F32, {B, n_expert ? 128 : 0});
+    add_ws("d_e1", PAMREC_F32, {B, expert.width(1)});
+    add_ws("d_g1", PAMREC_F32, {B, gate.width(1)});
+    add_ws("d_e0", PAMREC_F32, {B, expert.width(0)});
+    add_ws("d_g0", PAMREC_F32, {B, gate.width(0)});
     add_ws("d_x", PAMREC_F32, {B, x_dim});
     add_ws("d_tgt", PAMREC_F32, {B, E});            // from the towers' target columns
     add_ws("d_tgt_total", PAMREC_F32, {B, E});
-    add_ws("sib.d_score", PAMREC_F32, {N, 2});
-    add_ws("sib.d_a1", PAMREC_F32, {N, 80});
-    add_ws("sib.d_a0", PAMREC_F32, {N, 160});
+    add_ws("sib.d_score", PAMREC_F32, {N, att.width(2)});
+    add_ws("sib.d_a1", PAMREC_F32, {N, att.width(1)});
+    add_ws("sib.d_a0", PAMREC_F32, {N, att.width(0)});
     add_ws("sib.d_feat", PAMREC_F32, {N, 8 * E});
     add_ws("sib.d_att", PAMREC_F32, {2, N, E});     // gradient of a = h A
     add_ws("sib.dq", PAMREC_F32, {B, 2, E});        // gradient of the query (target) through the feature rows, per branch
@@ -276,7 +291,7 @@ struct Layout {
     }
     for (int i = 0; i < BN_COUNT; ++i) bnoff[i] = BnOff{0, 0, 0, 0, 0};
     tower_in = 2 * E;
-    tower = add_mlp({"sequential/logit_fcn"}, {L2}, tower_in, 100, 64, true, &bnoff[BN_T0], &bnoff[BN_T1]);   // sequential_base_model.py:76-79
+    tower = add_mlp({"sequential/logit_fcn"}, {L2}, tower_in, 100, 64, true, BN_T0, BN_T1);   // sequential_base_model.py:76-79
     // ---- workspace
     add_ws("sib.ids_item", PAMREC_I32, {2, N});      // satisfied-only ids (looked up), then the full-history ids (L2 rows only)
     add_ws("sib.ids_cate", PAMREC_I32, {2, N});
@@ -294,14 +309,14 @@ struct Layout {
       add_ws(p + "out", PAMREC_F32, {N, E});
     }
     add_ws("u", PAMREC_F32, {B, 2 * E});            // final state | target
-    add_ws("zt0", PAMREC_F32, {B, 100});
-    add_ws("zt1", PAMREC_F32, {B, 64});
-    add_ws("logits", PAMREC_F32, {B, 1});
+    add_ws("zt0", PAMREC_F32, {B, tower.width(0)});
+    add_ws("zt1", PAMREC_F32, {B, tower.width(1)});
+    add_ws("logits", PAMREC_F32, {B, tower.width(2)});
     add_ws("losses", PAMREC_F32, {8});
     add_ws("loss_acc", PAMREC_F64, {8});
-    add_ws("d_logits", PAMREC_F32, {B, 1});
-    add_ws("d_t1", PAMREC_F32, {B, 64});
-    add_ws("d_t0", PAMREC_F32, {B, 100});
+    add_ws("d_logits", PAMREC_F32, {B, tower.width(2)});
+    add_ws("d_t1", PAMREC_F32, {B, tower.width(1)});
+    add_ws("d_t0", PAMREC_F32, {B, tower.width(0)});
     add_ws("d_u", PAMREC_F32, {B, 2 * E});
     add_ws("d_tgt_total", PAMREC_F32, {B, E});
     add_ws("sas.g_a", PAMREC_F32, {N, E});          // gradient of a block's output (ping)
@@ -356,21 +371,20 @@ struct Layout {
       o.ln_b_beta = add_dense(p + "ln_1/Variable", {kD}, L2);
       o.ln_b_gamma = add_dense(p + "ln_1/Variable_1", {kD}, L2);
     }
-    score = add_mlp({"sequential/pamrec/new_long/score_1"}, {L2}, kD, 20, 1, false, &bnoff[BN_S0], &bnoff[BN_S1]);
+    score = add_mlp({"sequential/pamrec/new_long/score_1"}, {L2}, kD, 20, 1, false, BN_S0, BN_S1);
     std::vector<std::string> ex;
     for (int j = 0; j < 5; ++j) ex.push_back("sequential/pamrec/expert_" + std::to_string(j));
-    expert = add_mlp(ex, {L2, L2, L2, L2, L2}, kD, 100, 64, false, &bnoff[BN_E0], &bnoff[BN_E1]);
-    gate = add_mlp({"sequential/pamrec/gate_main", "sequential/pamrec/gate_sub"}, {L2, L2}, kD, 64, 5, false,
-                   &bnoff[BN_G0], &bnoff[BN_G1]);
+    expert = add_mlp(ex, {L2, L2, L2, L2, L2}, kD, 100, 64, false, BN_E0, BN_E1);
+    gate = add_mlp({"sequential/pamrec/gate_main", "sequential/pamrec/gate_sub"}, {L2, L2}, kD, 64, 5, false, BN_G0, BN_G1);
     tower = add_mlp({"sequential/logit_fcn", "sequential/valid_logit_fcn", "xilidu_logit_fcn"}, {L2, L2, 0}, 64 + kE, 100, 64,
-                    true, &bnoff[BN_T0], &bnoff[BN_T1]);
+                    true, BN_T0, BN_T1);
     // dead-for-logits branches (pamrec.py:293-311): variables exist, receive only the L2 gradient
     const char* dead[3] = {"new_distill", "long_term", "short_term"};
     const int dq[3] = {40, 20, 20};
     for (int i = 0; i < 3; ++i) {
       std::string p = std::string("sequential/pamrec/") + dead[i] + "/attention_fcn";
       add_dense(p + "/attention_mat", {kD, dq[i]}, L2 | PAMREC_SEG_DEAD);
-      add_mlp({p + "/att_fcn"}, {L2 | PAMREC_SEG_DEAD}, 4 * dq[i], 80, 40, true, nullptr, nullptr, false);
+      add_mlp({p + "/att_fcn"}, {L2 | PAMREC_SEG_DEAD}, 4 * dq[i], 80, 40, true, BN_COUNT, BN_COUNT);
     }
 
     // ---- workspace
@@ -391,35 +405,35 @@ struct Layout {
       for (const char* n : {"qin", "Q", "K", "V", "y", "pv", "out"}) add_ws(p + n, PAMREC_F32, {B, T, kD});
       add_ws(p + "ml", PAMREC_F32, {B, T, 2});   // softmax row maximum and row sum, kept for the backward pass
     }
-    add_ws("z1", PAMREC_F32, {B, T, 20});
+    add_ws("z1", PAMREC_F32, {B, T, score.width(0)});
     add_ws("z2", PAMREC_F32, {B, T});
     add_ws("pool.aw", PAMREC_F32, {B, T});        // attention-pooling weights, kept for the backward pass (kernels_head2.cu)
     add_ws("head.wT", PAMREC_F32, {3 * 6400 + 3 * 8400 + 5 * 6400 + 2 * 320 + 628 * 40});   // transposed head weights of the dX chain
     add_ws("new_long", PAMREC_F32, {B, kD});
-    add_ws("ze0", PAMREC_F32, {B, 500});
-    add_ws("zg0", PAMREC_F32, {B, 128});
-    add_ws("ze1", PAMREC_F32, {B, 320});
-    add_ws("zg1", PAMREC_F32, {B, 10});
-    add_ws("u", PAMREC_F32, {B, 168});
-    add_ws("zt0", PAMREC_F32, {B, 300});
-    add_ws("zt1", PAMREC_F32, {B, 192});
-    add_ws("logits", PAMREC_F32, {B, 3});
+    add_ws("ze0", PAMREC_F32, {B, expert.width(0)});
+    add_ws("zg0", PAMREC_F32, {B, gate.width(0)});
+    add_ws("ze1", PAMREC_F32, {B, expert.width(1)});
+    add_ws("zg1", PAMREC_F32, {B, gate.width(1)});
+    add_ws("u", PAMREC_F32, {B, 2 * tower.in});      // main | target | sub | target
+    add_ws("zt0", PAMREC_F32, {B, tower.width(0)});
+    add_ws("zt1", PAMREC_F32, {B, tower.width(1)});
+    add_ws("logits", PAMREC_F32, {B, tower.width(2)});
     add_ws("losses", PAMREC_F32, {8});
     add_ws("loss_acc", PAMREC_F64, {8});          // [0] data [1] aux [2] order [3] regular
     // gradients
-    add_ws("d_logits", PAMREC_F32, {B, 3});
-    add_ws("d_t1", PAMREC_F32, {B, 192});
-    add_ws("d_t0", PAMREC_F32, {B, 300});
-    add_ws("d_u", PAMREC_F32, {B, 168});
-    add_ws("d_e1", PAMREC_F32, {B, 320});
-    add_ws("d_g1", PAMREC_F32, {B, 10});
-    add_ws("d_e0", PAMREC_F32, {B, 500});
-    add_ws("d_g0", PAMREC_F32, {B, 128});
+    add_ws("d_logits", PAMREC_F32, {B, tower.width(2)});
+    add_ws("d_t1", PAMREC_F32, {B, tower.width(1)});
+    add_ws("d_t0", PAMREC_F32, {B, tower.width(0)});
+    add_ws("d_u", PAMREC_F32, {B, 2 * tower.in});
+    add_ws("d_e1", PAMREC_F32, {B, expert.width(1)});
+    add_ws("d_g1", PAMREC_F32, {B, gate.width(1)});
+    add_ws("d_e0", PAMREC_F32, {B, expert.width(0)});
+    add_ws("d_g0", PAMREC_F32, {B, gate.width(0)});
     add_ws("d_new_long", PAMREC_F32, {B, kD});
     add_ws("d_tgt", PAMREC_F32, {B, kE});
     add_ws("d_tgt_total", PAMREC_F32, {B, kE});
     add_ws("d_z2", PAMREC_F32, {B, T});
-    add_ws("d_a1", PAMREC_F32, {B, T, 20});
+    add_ws("d_a1", PAMREC_F32, {B, T, score.width(0)});
     add_ws("g_a", PAMREC_F32, {B, T, kD});        // ping-pong grads of block outputs / inputs
     add_ws("g_b", PAMREC_F32, {B, T, kD});
     add_ws("d_y", PAMREC_F32, {B, T, kD});
