@@ -201,6 +201,25 @@ int64_t pamrec_shard_rows(PamrecHandle h, int64_t vocab_rows);
 /* sum-all-reduce of a caller buffer over the handle's communicator (dtype PAMREC_F32 / PAMREC_F64 / PAMREC_I32) */
 int pamrec_comm_all_reduce(PamrecHandle h, void* dptr, int64_t count, int dtype, void* stream);
 
+/* Histograms of fp32 device tensors, as tf.summary.histogram builds them (tensorflow/core/lib/histogram/histogram.cc): the 1551
+ * default bucket limits (1e-12 * 1.1^k below 1e20 by repeated double products, their negatives, 0 and +-DBL_MAX), a value x
+ * counted in bucket upper_bound(limits, (double)x), and min / max / num / sum / sum_squares in double.  Segment s is counts[s]
+ * floats at the device pointer ptrs[s] (host array; n <= 512, counts < 2^31).  Non-finite values are counted, not binned.
+ * Outputs (device): stats[s * (5 + 2 * world) + i] = num, sum, sum_squares, non-finite count, compacted length (i = 0..4), then
+ * one min slot per rank (DBL_MAX where the rank had no finite value) and one max slot per rank (-DBL_MAX), zero in the slots of
+ * the other ranks; out[2 * (out_offsets[s] + j) + 0 / 1] = (bucket limit, count) of the j-th entry of segment s, compacted as
+ * Histogram::EncodeToProto(preserve_zero_buckets = false) does: every non-empty bucket, and one entry with the last limit of
+ * every run of empty buckets.  A segment of c elements has at most min(1551, 2c + 1) entries; entries past
+ * out_offsets[s + 1] - out_offsets[s] are dropped while the length still counts them.  reduce != 0 with world_size > 1: collective;
+ * the counts and stats are summed over the ranks before the compaction, so every rank gets the histograms of the union of the
+ * ranks' segments (a rank passes count 0 for a segment it does not hold).  scratch == NULL: *scratch_bytes receives the device
+ * scratch these counts need and nothing is launched.  Launches go to `stream`; the outputs are ready when it reaches them. */
+int pamrec_histograms(PamrecHandle h, const float* const* ptrs, const int64_t* counts, int n, int reduce, const int64_t* out_offsets,
+                      double* stats, double* out, void* scratch, int64_t* scratch_bytes, void* stream);
+/* Host only: the 1551 bucket limits pamrec_histograms uses (limits_out, may be NULL) and the compaction of one host array of 1551
+ * bucket counts into (limit, count) pairs (pairs_out: up to 2 * 1551 doubles, *n_pairs entries; counts may be NULL). */
+int pamrec_histogram_buckets(const int32_t* counts, double* limits_out, double* pairs_out, int* n_pairs);
+
 /* Stand-alone HBM kernels for roofline measurement (same kernels the step uses). */
 int pamrec_bench_gather(PamrecHandle h, const int32_t* item_ids, const int32_t* cate_ids, const int32_t* tgt_items,
                         const int32_t* tgt_cates, int64_t n_rows, int32_t T, float* out, void* stream);

@@ -18,6 +18,7 @@ IPC_HANDLE_BYTES = 64
 GROUP = 5
 DEBUG_SAVE_FFN_HIDDEN = 1
 DEBUG_HEAD_TRACE = 2
+HIST_BUCKETS, HIST_MAX_SEGMENTS = 1551, 512          # pamrec_histograms: default bucket limits, segments per call
 
 
 class PamrecConfig(C.Structure):
@@ -91,6 +92,9 @@ EXPORTS = {
     "pamrec_comm_mailbox_open": (C.c_int, [C.c_void_p, C.c_char_p]),
     "pamrec_shard_rows": (C.c_int64, [C.c_void_p, C.c_int64]),
     "pamrec_comm_all_reduce": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_void_p]),
+    "pamrec_histograms": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                    C.c_void_p, C.POINTER(C.c_int64), C.c_void_p]),
+    "pamrec_histogram_buckets": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_int)]),
     "pamrec_bench_gather": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32,
                                       C.c_void_p, C.c_void_p]),
     "pamrec_bench_table_adam": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p]),

@@ -3,6 +3,7 @@
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
+#include <algorithm>
 #include <cstdlib>
 #include <functional>
 #include <string>
@@ -1131,6 +1132,63 @@ int pamrec_comm_all_reduce(PamrecHandle h, void* dptr, int64_t count, int dtype,
   if (!h) return -1;
   CommType t = dtype == PAMREC_F64 ? COMM_F64 : (dtype == PAMREC_I32 ? COMM_I32 : COMM_F32);
   if (h->comm.all_reduce(dptr, count, t, (cudaStream_t)stream)) return fail(h, "nccl: %s", h->comm.err.c_str());
+  return 0;
+}
+
+int pamrec_histograms(PamrecHandle h, const float* const* ptrs, const int64_t* counts, int n, int reduce, const int64_t* out_offsets,
+                      double* stats, double* out, void* scratch, int64_t* scratch_bytes, void* stream) {
+  if (!h) return -1;
+  if (n < 1 || n > kHistMaxSeg || !counts || !scratch_bytes) return fail(h, "histograms: 1 to %d segments and their counts", kHistMaxSeg);
+  const double* pos = hist_positive_limits();
+  if (!pos) return fail(h, "histograms: the default bucket table does not have %d positive limits", kHistPos);
+  static thread_local HistArgs a;                          // ~20 KB: not on the stack
+  std::copy(pos, pos + kHistPos, a.pos);
+  a.n = n; a.world = h->cfg.world_size; a.rank = h->cfg.rank;
+  int64_t items = 0;
+  for (int s = 0; s < n; ++s) {
+    if (counts[s] < 0 || counts[s] >= ((int64_t)1 << 31)) return fail(h, "histograms: segment %d has %lld elements", s, (long long)counts[s]);
+    a.first_item[s] = (int)items;
+    items += hist_items(counts[s]);
+  }
+  if (items >= ((int64_t)1 << 31)) return fail(h, "histograms: too many elements");
+  a.first_item[n] = (int)items;
+  const size_t bins_bytes = ((size_t)n * kHistBuckets * sizeof(int) + 255) / 256 * 256;
+  const int64_t need = (int64_t)(bins_bytes + (size_t)items * 5 * sizeof(double));
+  if (!scratch) { *scratch_bytes = need; return 0; }
+  if (*scratch_bytes < need) return fail(h, "histograms: scratch of %lld bytes, %lld needed", (long long)*scratch_bytes, (long long)need);
+  if (!ptrs || !out_offsets || !stats || !out) return fail(h, "histograms: null argument");
+  for (int s = 0; s <= n; ++s) {
+    a.out_off[s] = out_offsets[s];
+    if (s < n && (out_offsets[s + 1] < out_offsets[s] || (counts[s] && !ptrs[s]))) return fail(h, "histograms: segment %d", s);
+  }
+  for (int s = 0; s < n; ++s) { a.ptr[s] = ptrs[s]; a.count[s] = counts[s]; }
+  ProfBind _pb(h);
+  cudaStream_t st = (cudaStream_t)stream;
+  int* bins = static_cast<int*>(scratch);
+  double* part = reinterpret_cast<double*>(static_cast<char*>(scratch) + bins_bytes);
+  cudaMemsetAsync(bins, 0, (size_t)n * kHistBuckets * sizeof(int), st);
+  launch_hist_bin(a, (int)items, bins, part, stats, st);
+  if (reduce && a.world > 1) {
+    if (h->comm.all_reduce(bins, (int64_t)n * kHistBuckets, COMM_I32, st) ||
+        h->comm.all_reduce(stats, (int64_t)n * hist_stats_width(a.world), COMM_F64, st))
+      return fail(h, "nccl: %s", h->comm.err.c_str());
+  }
+  launch_hist_compact(a, bins, stats, out, st);
+  return check_cuda(h, "histograms");
+}
+
+int pamrec_histogram_buckets(const int32_t* counts, double* limits_out, double* pairs_out, int* n_pairs) {
+  const double* pos = hist_positive_limits();
+  if (!pos) return -1;
+  if (limits_out)
+    for (int b = 0; b < kHistBuckets; ++b) limits_out[b] = hist_limit(pos, b);
+  if (counts) {
+    if (!pairs_out || !n_pairs) return -1;
+    int k = 0;
+    for (int b = 0; b < kHistBuckets; ++b)
+      if (hist_emits(counts, b)) { pairs_out[2 * k] = hist_limit(pos, b); pairs_out[2 * k + 1] = (double)counts[b]; ++k; }
+    *n_pairs = k;
+  }
   return 0;
 }
 

@@ -1,5 +1,6 @@
 // Launcher declarations shared by the translation units of libpamrec_b200.so.
 #pragma once
+#include <cfloat>
 #include <string>
 #include <vector>
 
@@ -246,5 +247,36 @@ void launch_shard_route(const SparseTable& req, int64_t n, int world, int64_t rp
                         int* inv, cudaStream_t st);
 void launch_serve_rows(const float* shard, const int* ids, int64_t n, int width, float* out, cudaStream_t st);
 void launch_count_valid_groups(const float* plays, int B, double* out, cudaStream_t st);
+
+// ---- kernels_summary.cu (histograms of TensorBoard summaries, tensorflow/core/lib/histogram/histogram.cc)
+constexpr int kHistPos = 774;                      // positive default limits p_k = 1e-12 * 1.1^k below 1e20
+constexpr int kHistBuckets = 2 * kHistPos + 3;     // 1551 sorted limits: -DBL_MAX, -p_773 .. -p_0, 0, p_0 .. p_773, DBL_MAX
+constexpr int kHistZero = kHistPos + 1;            // index of the limit 0.0
+constexpr int kHistChunk = 1 << 16;                // elements binned by one CTA
+constexpr int kHistMaxSeg = 512;                   // segments of one launch
+// per segment, doubles: num, sum, sum_squares, non-finite values, compacted length, then one min and one max slot per rank
+enum { HIST_NUM = 0, HIST_SUM, HIST_SUM_SQUARES, HIST_NONFINITE, HIST_LEN, HIST_SLOTS };
+__host__ __device__ inline int hist_stats_width(int world) { return HIST_SLOTS + 2 * world; }
+__host__ __device__ inline double hist_limit(const double* pos, int b) {
+  if (b == 0) return -DBL_MAX;
+  if (b < kHistZero) return -pos[kHistZero - 1 - b];
+  if (b == kHistZero) return 0.0;
+  if (b < kHistBuckets - 1) return pos[b - kHistZero - 1];
+  return DBL_MAX;
+}
+// EncodeToProto(preserve_zero_buckets = false): a non-empty bucket, or the last bucket of a run of empty ones
+__host__ __device__ inline bool hist_emits(const int* cnt, int b) { return cnt[b] > 0 || b == kHistBuckets - 1 || cnt[b + 1] > 0; }
+struct HistArgs {                                  // passed by value (__grid_constant__, about 20 KB)
+  double pos[kHistPos];
+  const float* ptr[kHistMaxSeg];
+  int64_t count[kHistMaxSeg];
+  int first_item[kHistMaxSeg + 1];                 // work items (CTAs of k_hist_bin) before each segment
+  int64_t out_off[kHistMaxSeg + 1];                // (limit, count) pairs of the output before each segment
+  int n, world, rank;
+};
+const double* hist_positive_limits();              // nullptr if the table does not come out at kHistPos entries
+int64_t hist_items(int64_t count);
+void launch_hist_bin(const HistArgs& a, int total_items, int* bins, double* part, double* stats, cudaStream_t st);
+void launch_hist_compact(const HistArgs& a, const int* bins, double* stats, double* out, cudaStream_t st);
 
 }  // namespace pamrec

@@ -89,6 +89,33 @@ class PendingHost:
         return self._value
 
 
+class PendingHistograms:
+    """Histograms queued by Engine.histograms; ``result()`` waits for their device->host copy."""
+
+    def __init__(self, slot, plan):
+        self._slot, self._plan, self._value = slot, plan, None
+
+    def result(self):
+        if self._value is None:
+            slot, p = self._slot, self._plan
+            slot["event"].synchronize()
+            stats = slot["stats"].numpy().reshape(len(p["names"]), -1)
+            pairs = slot["out"].numpy().reshape(-1, 2)
+            world, out = p["world"], {}
+            for s, name in enumerate(p["names"]):
+                st = stats[s]
+                n, lo = int(st[4]), int(p["offsets"][s])
+                if n > p["offsets"][s + 1] - lo:
+                    raise PamrecError(f"histogram of {name}: {n} compacted entries, room for {p['offsets'][s + 1] - lo}")
+                out[name] = dict(min=float(st[5:5 + world].min()), max=float(st[5 + world:5 + 2 * world].max()), num=float(st[0]),
+                                 sum=float(st[1]), sum_squares=float(st[2]), nonfinite=int(st[3]),
+                                 bucket_limit=pairs[lo:lo + n, 0].copy(), bucket=pairs[lo:lo + n, 1].copy())
+            self._value = out
+            slot["owner"] = None
+            self._slot = None
+        return self._value
+
+
 class Engine:
     def __init__(self, n_users, n_items, n_cates, max_seq_len, max_batch, hp=None, sparse_adam="dense_exact",
                  world_size=1, rank=0, tables=None, model="pamrec", graph=None, emb_dims=EMB_DIMS):
@@ -154,6 +181,7 @@ class Engine:
         self._dev_step = None                        # value of the device-side step counter, when known to equal self.step
         self.frozen = {n: np.zeros(f(n_users, self.emb_dims), np.float32) for n, f in FROZEN.items()
                        if model != "sasrec" or not n.endswith("play_lookup")}
+        self._hist_plans, self._frozen_dev = {}, {}     # Engine.histograms: per name list, and device copies of self.frozen
 
     # ------------------------------------------------------------------ inventory (host only)
     def _query(self, pool):
@@ -288,6 +316,7 @@ class Engine:
                 self.bn(name).copy_(t.to(self.device))
             elif name in self.frozen:
                 self.frozen[name] = np.asarray(val, dtype=np.float32).copy()
+                self._frozen_dev.pop(name, None)
             else:
                 raise KeyError(f"unknown variable {name}")
 
@@ -509,6 +538,74 @@ class Engine:
         slot["event"].record(torch.cuda.current_stream(self.device))
         slot["owner"] = PendingHost(slot, n)
         return slot["owner"]
+
+    def histograms(self, names):
+        """Queue on the engine's stream the histograms of the variables ``names`` (TF names, as get_variables() gives them), binned
+        on the device with TensorFlow's default buckets (pamrec_histograms).  Returns a PendingHistograms: ``result()`` gives
+        {name: dict(min, max, num, sum, sum_squares, bucket_limit, bucket, nonfinite)}, the HistogramProto fields of
+        tf.summary.histogram plus the count of non-finite values.  A table is binned over its vocabulary rows.  With world_size
+        > 1 this is collective (every rank passes the same names): a sharded table is binned shard by shard and the counts summed
+        over the ranks; every other variable is the same on all ranks and binned by rank 0.  Every rank receives the result."""
+        names = tuple(names)
+        p = self._hist_plans.get(names)
+        if p is None:
+            p = self._hist_plans[names] = self._hist_plan(names)
+        ptrs = (C.c_void_p * len(names))(*[self._hist_ptr(n) for n in names])
+        slot = p["slots"][p["next"]]
+        p["next"] ^= 1
+        if slot["owner"] is not None:
+            slot["owner"].result()
+        scratch = C.c_int64(p["scratch"].numel())
+        self._check(self.lib.pamrec_histograms(self.handle, ptrs, p["counts"], len(names), int(self.world > 1), p["offsets"],
+                                               C.c_void_p(p["stats"].data_ptr()), C.c_void_p(p["out"].data_ptr()),
+                                               C.c_void_p(p["scratch"].data_ptr()), C.byref(scratch), self._stream()))
+        slot["stats"].copy_(p["stats"], non_blocking=True)
+        slot["out"].copy_(p["out"], non_blocking=True)
+        slot["event"].record(torch.cuda.current_stream(self.device))
+        slot["owner"] = PendingHistograms(slot, p)
+        return slot["owner"]
+
+    def _hist_plan(self, names):
+        """Segment sizes, output offsets and the device / pinned buffers of one list of names (kept for the engine's lifetime)."""
+        if not 1 <= len(names) <= L.HIST_MAX_SEGMENTS:
+            raise PamrecError(f"histograms of 1 to {L.HIST_MAX_SEGMENTS} variables per call, not {len(names)}")
+        shapes = self.variable_shapes()
+        counts, caps = [], []
+        for name in names:
+            if name not in shapes:
+                raise KeyError(f"unknown variable {name}")
+            total = int(np.prod(shapes[name]))
+            if name in self.tables_by_name and self.tables == "sharded":
+                pre, k = self.tables_by_name[name]
+                mine = len(range(self.rank, self._vocab(pre), self.world)) * self.emb_dims[k]   # this shard's vocabulary rows
+            else:
+                mine = total if self.rank == 0 else 0
+            counts.append(mine)
+            caps.append(min(L.HIST_BUCKETS, 2 * total + 1))
+        offsets = np.concatenate([[0], np.cumsum(caps)]).astype(np.int64)
+        counts_c = (C.c_int64 * len(names))(*counts)
+        offsets_c = (C.c_int64 * (len(names) + 1))(*offsets.tolist())
+        need = C.c_int64(0)
+        self._check(self.lib.pamrec_histograms(self.handle, None, counts_c, len(names), int(self.world > 1), None, None, None, None,
+                                               C.byref(need), None))
+        sw = 5 + 2 * self.world
+        f64 = lambda n, **kw: torch.empty(n, dtype=torch.float64, **kw)
+        return dict(names=names, world=self.world, counts=counts_c, offsets=offsets_c, next=0,
+                    scratch=torch.empty(need.value, dtype=torch.uint8, device=self.device),
+                    stats=f64(len(names) * sw, device=self.device), out=f64(int(offsets[-1]) * 2, device=self.device),
+                    slots=[dict(stats=f64(len(names) * sw).pin_memory(), out=f64(int(offsets[-1]) * 2).pin_memory(),
+                                event=torch.cuda.Event(), owner=None) for _ in range(2)])
+
+    def _hist_ptr(self, name):
+        if name in self.tables_by_name:
+            return self.pool[self.tables_by_name[name][0] + "_w"].data_ptr()
+        if name in self.info[L.POOL_DENSE]:
+            return self.dense(name).data_ptr()
+        if name in self.info[L.POOL_BN]:
+            return self.bn(name).data_ptr()
+        if name not in self._frozen_dev:                         # host-side constants: one device copy until set_variables
+            self._frozen_dev[name] = torch.from_numpy(self.frozen[name]).to(self.device)
+        return self._frozen_dev[name].data_ptr()
 
     def set_debug(self, flags):
         """Test hooks (include/pamrec_b200.h: PAMREC_DEBUG_*)."""

@@ -19,8 +19,9 @@ import torch
 
 from . import checkpoint as CK
 from . import dist as D
+from . import summary as SUM
 from .deeprec_utils import cal_metric, cal_weighted_metric, filter_single_class_users, load_dict
-from .engine import Engine
+from .engine import Engine, PamrecError
 from .prefetch import Prefetcher
 from .sequential_iterator import LocalFeed
 
@@ -195,6 +196,8 @@ class BaseModel:
              float(hp.cross_l2) == 0.0, "L1 / cross regularisation must be 0")
         need(1 <= hp.max_seq_length <= 256, "max_seq_length must be in [1, 256]")
         need(hp.batch_size % 5 == 0, "batch_size must be a multiple of 5 (IT:684-685, PAM:73-75)")
+        need(isinstance(getattr(hp, "summary_step", 1), int) and getattr(hp, "summary_step", 1) >= 1,
+             "summary_step must be an integer >= 1")
 
     def _check_mixing(self, hp, need):
         need(list(hp.expert_layer_sizes) == [100, 64] and list(hp.gate_layer_sizes) == [64, 5] and hp.expert_num == 5,
@@ -300,6 +303,34 @@ class SequentialBaseModel(BaseModel):
         """SBM:557-560 / BM:388-399 -> [pred]."""
         return [self._score(feed_dict)]
 
+    # ------------------------------------------------------------------ summaries (SBM:268-274)
+    _writer = None
+
+    def _pending_step(self, losses):
+        """Wrap a queued step's PendingLosses.  With ``write_tfevents`` every ``summary_step``-th optimiser step (an extension:
+        the reference summarises every step, summary_step = 1, the default) also queues the histograms of every checkpoint
+        variable on the device behind it; the handle's result() then carries the serialized Summary and hands it to the open
+        event file."""
+        eng = self.engine
+        hist = None
+        if self.hparams.write_tfevents and eng.step % getattr(self.hparams, "summary_step", 1) == 0:
+            hist = eng.histograms(eng.variable_shapes())
+        return _PendingStep(losses, self.SCALARS, hist, eng.step, self)
+
+    def _open_summaries(self):
+        """fit / fit_step: a new event file in SUMMARIES_DIR when write_tfevents is set (rank 0 writes; every rank bins)."""
+        if self.hparams.write_tfevents and self.hparams.SUMMARIES_DIR and self.engine.rank == 0:
+            self._writer = SUM.EventFileWriter(self.hparams.SUMMARIES_DIR)
+
+    def _flush_summaries(self):
+        if self._writer is not None:
+            self._writer.flush()
+
+    def _close_summaries(self):
+        if self._writer is not None:
+            w, self._writer = self._writer, None
+            w.close()
+
     # ------------------------------------------------------------------ loops
     def _maybe_save(self, progress, tag):
         if self.hparams.save_model and self.hparams.MODEL_DIR:
@@ -316,6 +347,14 @@ class SequentialBaseModel(BaseModel):
             raise ValueError("Please specify a positive integer of negative numbers for validation.")
         if self.need_sample and self.train_num_ngs < 1:
             self.train_num_ngs = 1
+        self._open_summaries()
+        try:
+            self._fit_epochs(train_file, valid_file, valid_num_ngs, eval_metric)
+        finally:
+            self._close_summaries()
+        return self
+
+    def _fit_epochs(self, train_file, valid_file, valid_num_ngs, eval_metric):
         eval_info = []
         best_metric, self.best_epoch = 0, 0
         for epoch in range(1, self.hparams.epochs + 1):
@@ -323,6 +362,7 @@ class SequentialBaseModel(BaseModel):
             file_iterator = Prefetcher(self.iterator.load_data_from_file(train_file, min_seq_length=self.min_seq_length,
                                                                          batch_num_ngs=self.train_num_ngs))
             self.batch_train(file_iterator, self.sess)
+            self._flush_summaries()
             valid_res = self.run_weighted_eval(valid_file, valid_num_ngs)
             print("eval valid at epoch {0}: {1}".format(epoch, ",".join(str(k) + ":" + str(v) for k, v in valid_res.items())))
             eval_info.append((epoch, valid_res))
@@ -338,12 +378,19 @@ class SequentialBaseModel(BaseModel):
             self._maybe_save(progress, "epoch_" + str(epoch))
         print(eval_info)
         print("best step: {0}".format(self.best_epoch))
-        return self
 
     def fit_step(self, train_file, valid_file, valid_num_ngs, eval_metric="group_auc"):
         """SBM:239-377: step loop, evaluation every ``eval_step`` steps, early stop on steps, checkpoint on improvement."""
         if self.need_sample and self.train_num_ngs < 1:
             self.train_num_ngs = 1
+        self._open_summaries()
+        try:
+            self._fit_steps(train_file, valid_file, valid_num_ngs, eval_metric)
+        finally:
+            self._close_summaries()
+        return self
+
+    def _fit_steps(self, train_file, valid_file, valid_num_ngs, eval_metric):
         eval_info = []
         best_metric, self.best_step = 0, 0
         step = 0
@@ -367,6 +414,7 @@ class SequentialBaseModel(BaseModel):
                 if step % self.hparams.eval_step == 0:
                     self.step_train(step - 1, pending.result())
                     pending = None
+                    self._flush_summaries()
                     valid_res = self.run_weighted_eval(valid_file, valid_num_ngs)
                     print("eval valid at epoch {0} step {1}: {2}".format(
                         epoch, step, ",".join(str(k) + ":" + str(v) for k, v in valid_res.items())))
@@ -387,7 +435,6 @@ class SequentialBaseModel(BaseModel):
                 self.step_train(step - 1, pending.result())
         print(eval_info)
         print("best step: {0}".format(self.best_step))
-        return self
 
     def run_eval(self, filename, num_ngs):
         """SBM:380-413."""
@@ -448,18 +495,36 @@ class SequentialBaseModel(BaseModel):
 
 
 class _PendingStep:
-    def __init__(self, pending):
-        self._pending = pending
+    """A queued train step: ``result()`` gives train()'s tuple (update, extra_update_ops, <one float per loss name>, summary).
+    summary is None unless histograms were queued behind the step; then it is the serialized Summary of the loss scalars and
+    the histograms, also handed to the model's open event file at the optimiser step ``step``."""
+
+    def __init__(self, pending, scalars, hist=None, step=0, model=None):
+        self._pending, self._scalars, self._hist, self._step, self._model = pending, scalars, hist, step, model
+        self._value = None
 
     def result(self):
-        l = self._pending.result()
-        return [None, None, float(l[0]), float(l[1]), float(l[2]), float(l[3]), float(l[4]), None]
+        if self._value is None:
+            l = self._pending.result()
+            values = [float(v) for v in l[:len(self._scalars)]]
+            summary = None
+            if self._hist is not None:
+                hist = self._hist.result()
+                for name, h in hist.items():
+                    if h["nonfinite"]:
+                        raise PamrecError("Nan in summary histogram for: {} (step {})".format(name, self._step))
+                summary = SUM.summary_proto(zip(self._scalars, values), hist.items())
+                if self._model._writer is not None:
+                    self._model._writer.add_summary(summary, self._step)
+            self._value = [None, None] + values + [summary]
+        return self._value
 
 
 class PAMRECModel(SequentialBaseModel):
     """PAM:25: the playback-duration-augmented model.  The graph (embeddings, time-aware 2-block encoder, attention
     pooling, MMoE, three towers, four-term loss, per-tensor clip + Adam) is libpamrec_b200.so."""
     ENGINE_MODEL = "pamrec"
+    SCALARS = ("loss", "data_loss", "regular_loss", "auxiliary_data_loss", "order_loss")     # train()'s tuple, PAM:444-448
 
     def _build_graph(self):
         hp = self.hparams
@@ -512,7 +577,7 @@ class PAMRECModel(SequentialBaseModel):
             db = eng.upload(local, training=True, staged=True, global_batch=n)
         else:
             db = eng.upload(feed_dict, training=True, staged=True)
-        return _PendingStep(eng.train_step_async(db))
+        return self._pending_step(eng.train_step_async(db))
 
     def step_train(self, step, step_result):
         """PAM:455-465."""
@@ -544,12 +609,6 @@ class PAMRECModel(SequentialBaseModel):
 
 
 # ----------------------------------------------------------------------------- sibling multi-task baselines (SURVEY.md section 8(f) N3)
-class _PendingStep7(_PendingStep):
-    def result(self):
-        l = self._pending.result()
-        return [None, None, float(l[0]), float(l[1]), float(l[2]), float(l[3]), None]
-
-
 class _DinMultiTask(PAMRECModel):
     """What MMoEModel_original, PLEModel and ShareBottomModel share (models/sequential/mmoe.py, ple.py, sharebottom.py): the
     input pipeline, DIN attention pooling of the satisfied-only and of the full history against the target (`_attention_fcn`),
@@ -557,6 +616,8 @@ class _DinMultiTask(PAMRECModel):
     that train() returns (no order loss, MM:341-373).  One GPU.  Embedding widths (item / cate / user): 16 / 4 (config/mmoe.yaml)
     or 32 / 8 (the reference's ple.yaml and sharebottom.yaml, and 32 / 8 / 16 in its sasrec.yaml), each with a user width of 16,
     20 or 40; the kernels are compiled for both item / cate pairs."""
+
+    SCALARS = ("loss", "data_loss", "regular_loss", "auxiliary_data_loss")                  # MM:341-373
 
     def _check_supported(self, hp):
         super()._check_supported(hp)
@@ -573,7 +634,7 @@ class _DinMultiTask(PAMRECModel):
             raise ValueError("pamrec_b200: the sibling models run on one GPU")
 
     def train_async(self, sess, feed_dict):
-        return _PendingStep7(self.engine.train_step_async(self.engine.upload(feed_dict, training=True, staged=True)))
+        return self._pending_step(self.engine.train_step_async(self.engine.upload(feed_dict, training=True, staged=True)))
 
     def step_train(self, step, step_result):
         """MM:375-385."""
@@ -606,23 +667,15 @@ class ShareBottomModel(_DinMultiTask):
         pass
 
 
-class _PendingStep5(_PendingStep):
-    def result(self):
-        l = self._pending.result()
-        return [None, None, float(l[0]), float(l[1]), None]
-
-
 class SASRecModel(_DinMultiTask):
     """models/sequential/sasrec.py:16: the satisfied-only history + a position table through two (item + cate)-wide self-attention blocks with
     dense Q / K / V, read out at the last satisfied position, one tower; loss = data + regular.  train() returns the base class's
     5-tuple (update, extra_update_ops, loss, data_loss, summary) (BM:350-372)."""
     ENGINE_MODEL = "sasrec"
+    SCALARS = ("loss", "data_loss")                                                        # BM:350-372
 
     def _check_mixing(self, hp, need):
         pass
-
-    def train_async(self, sess, feed_dict):
-        return _PendingStep5(self.engine.train_step_async(self.engine.upload(feed_dict, training=True, staged=True)))
 
     def step_train(self, step, step_result):
         """SBM:227-236."""
