@@ -22,6 +22,17 @@ struct Xchg {
   int64_t n_send = 0, n_recv = 0;
 };
 
+// One id space (layout.h: IdSpace) bound to the workspace and the caller's tables by pamrec_bind.
+struct IdTables {
+  const IdSpace* d = nullptr;
+  SparseTable req;           // plan of this rank's lookups ("sp.<name>.*")
+  SparseTable own;           // sharded: plan of the rows the other ranks asked this rank for ("so.<name>.*"), on the local shard
+  SparseTable tab[2];        // the parameter tables, each on the plan of its update (own when sharded, else req)
+  const int* sib_ids;        // siblings: the history lookups of a batch, written by the gather ("sib.ids_<name>")
+  int* inv; int* send_ids; int* off; int* recv_ids; float* rows; float* xrows;   // sharded: the exchange ("sh.<name>.*")
+  Xchg x;                    // sharded: the exchange of the current batch
+};
+
 struct PamrecHandle_ {
   PamrecConfig cfg;
   Layout L;
@@ -35,7 +46,7 @@ struct PamrecHandle_ {
   std::vector<int> h_seg_id, h_seg_tab;
   Comm comm;
   int* h_counts = nullptr;      // pinned [2][world][4]: send | recv counts of the current batch (sharded tables)
-  Xchg xc[3];                   // item, cate, user
+  IdTables sp[3];               // L.idsp bound: item, cate, user
   bool xc_users = false;        // the current exchange carried user ids (training)
   bool sharded() const { return cfg.table_mode == PAMREC_TABLES_SHARDED; }
   bool sibling() const { return cfg.model_kind != PAMREC_MODEL_PAMREC; }
@@ -284,6 +295,50 @@ static BnSet make_bn(PamrecHandle h, int id, const char* name) {
   return s;
 }
 
+static void bind_id_spaces(PamrecHandle h) {
+  const PamrecBuffers& u = h->buf;
+  float* const w[4] = {u.item_w, u.cate_w, u.ulong_w, u.ushort_w};
+  float* const m[4] = {u.item_m, u.cate_m, u.ulong_m, u.ushort_m};
+  float* const v[4] = {u.item_v, u.cate_v, u.ulong_v, u.ushort_v};
+  int* nuniq = h->wi("sp.nuniq");
+  double* normsq = h->wd("sp_normsq");
+  for (int t = 0; t < h->L.n_idsp; ++t) {
+    const IdSpace& d = h->L.idsp[t];
+    IdTables& s = h->sp[t];
+    s = IdTables{};
+    s.d = &d;
+    const std::string p = std::string("sp.") + d.name + ".", q = std::string("sh.") + d.name + ".", o = std::string("so.") + d.name + ".";
+    SparseTable& r = s.req;
+    r.width = d.width; r.n_rows = h->sharded() ? d.rows * h->cfg.world_size : d.rows;
+    if (d.slot) {
+      r.keys = h->wi(p + "keys"); r.idx = h->wi(p + "idx"); r.skeys = h->wi(p + "skeys"); r.sidx = h->wi(p + "sidx");
+      r.uidx = h->wi(p + "uidx"); r.slot = h->wi(p + "slot");
+    }
+    r.ukeys = h->wi(p + "ukeys");
+    if (d.accum) r.accum = h->wf(p + "accum");
+    r.nuniq = nuniq + t; r.normsq = normsq + d.tab0;
+    if (h->sibling() && d.accum) s.sib_ids = h->wi(std::string("sib.ids_") + d.name);
+    if (h->sharded()) {
+      SparseTable& a = s.own;
+      a.width = d.width; a.n_rows = d.rows; a.slot = r.slot;
+      a.keys = h->wi(o + "keys"); a.idx = h->wi(o + "idx"); a.skeys = h->wi(o + "skeys"); a.sidx = h->wi(o + "sidx");
+      a.uidx = h->wi(o + "uidx"); a.ukeys = h->wi(o + "ukeys");
+      if (d.accum) a.accum = h->wf(o + "accum");
+      a.nuniq = nuniq + 4 + t;
+      a.normsq = h->wd("sh.scratch");     // the un-deduplicated rows' norm is the requesters' (req.normsq)
+      s.inv = h->wi(q + "inv"); s.send_ids = h->wi(q + "send_ids"); s.off = h->wi(q + "off"); s.recv_ids = h->wi(q + "recv_ids");
+      if (d.accum) { s.rows = h->wf(q + "rows"); s.xrows = h->wf(q + "xrows"); }
+    }
+    for (int k = 0; k < d.n_tab; ++k) {
+      SparseTable& e = s.tab[k];
+      e = h->sharded() ? s.own : s.req;
+      e.w = w[d.tab0 + k]; e.m = m[d.tab0 + k]; e.v = v[d.tab0 + k];
+      e.normsq = normsq + d.tab0 + k;
+      if (d.has0) e.l2_has0 = h->wi("sib.has0") + t;
+    }
+  }
+}
+
 static int build_head(PamrecHandle h, cudaStream_t st);
 static HeadDyn head_dyn(PamrecHandle h, const PamrecBatch* b, bool training, int slot0);
 
@@ -315,14 +370,11 @@ int pamrec_bind(PamrecHandle h, const PamrecBuffers* bufs, void* stream) {
   size_t have = (size_t)h->L.ws[h->L.ws_index["cub_temp"]].numel;
   if (need > have) return fail(h, "cub temp storage: need %zu have %zu", need, have);
   cudaMemsetAsync(h->buf.workspace, 0, h->L.ws_bytes, st);
-  if (h->sharded() || h->sibling()) {
-    cudaMemsetAsync(h->wi("sp.item.slot"), 0xFF, (size_t)h->L.rows_of(h->cfg.n_items) * 4, st);
-    cudaMemsetAsync(h->wi("sp.cate.slot"), 0xFF, (size_t)h->L.rows_of(h->cfg.n_cates) * 4, st);
-    if (h->cfg.model_kind != PAMREC_MODEL_SASREC)
-      cudaMemsetAsync(h->wi("sp.user.slot"), 0xFF, (size_t)h->L.rows_of(h->cfg.n_users) * 4, st);
-  } else {
+  bind_id_spaces(h);
+  for (int t = 0; t < h->L.n_idsp; ++t)
+    if (h->L.idsp[t].slot) cudaMemsetAsync(h->sp[t].req.slot, 0xFF, (size_t)h->L.idsp[t].rows * 4, st);
+  if (!h->sharded() && !h->sibling())
     cudaMemsetAsync(h->wi("sp2.slot"), 0xFF, ((size_t)h->cfg.n_items + h->cfg.n_cates + h->cfg.n_users) * 4, st);
-  }
   if (h->sharded() && !h->h_counts &&
       cudaMallocHost(&h->h_counts, sizeof(int) * (8 * (size_t)h->cfg.world_size + 4)) != cudaSuccess)
     return fail(h, "cudaMallocHost for the exchange counts failed");
@@ -368,15 +420,15 @@ static Sp2 make_sp2(PamrecHandle h, const PamrecBatch* b) {
   s.B = b->batch; s.N = (int64_t)b->batch * c.max_seq_len;
   s.n_items = c.n_items; s.n_cates = c.n_cates; s.n_users = c.n_users;
   s.keys = h->wi("sp2.keys"); s.idx = h->wi("sp2.idx"); s.skeys = h->wi("sp2.skeys"); s.sidx = h->wi("sp2.sidx"); s.uidx = h->wi("sp2.uidx");
-  s.ukeys[0] = h->wi("sp.item.ukeys"); s.ukeys[1] = h->wi("sp.cate.ukeys"); s.ukeys[2] = h->wi("sp.user.ukeys");
   s.nuniq = h->wi("sp.nuniq"); s.meta = h->wi("sp2.meta");
-  s.accum[0] = h->wf("sp.item.accum"); s.accum[1] = h->wf("sp.cate.accum");
-  s.dflag[0] = h->wi("sp2.dflag"); s.dflag[1] = s.dflag[0] + h->L.cub_keys_table;
+  for (int t = 0; t < h->L.n_idsp; ++t) {
+    const IdTables& x = h->sp[t];
+    s.ukeys[t] = x.req.ukeys;
+    if (x.d->accum) s.accum[t] = x.req.accum;
+    for (int k = 0; k < x.d->n_tab; ++k) { s.w[x.d->tab0 + k] = x.tab[k].w; s.m[x.d->tab0 + k] = x.tab[k].m; s.v[x.d->tab0 + k] = x.tab[k].v; }
+  }
+  s.dflag[0] = h->wi("sp2.dflag"); s.dflag[1] = s.dflag[0] + h->L.idsp[0].nk;
   s.l2sq = h->wd("sp2.l2sq"); s.undedup = h->wd("sp_normsq");
-  s.w[0] = h->buf.item_w; s.m[0] = h->buf.item_m; s.v[0] = h->buf.item_v;
-  s.w[1] = h->buf.cate_w; s.m[1] = h->buf.cate_m; s.v[1] = h->buf.cate_v;
-  s.w[2] = h->buf.ulong_w; s.m[2] = h->buf.ulong_m; s.v[2] = h->buf.ulong_v;
-  s.w[3] = h->buf.ushort_w; s.m[3] = h->buf.ushort_m; s.v[3] = h->buf.ushort_v;
   s.dX0 = h->wf("g_a"); s.dT = h->wf("d_tgt_total");
   if (h->replicated()) { s.mode = SP2_DENSE; s.rep_grad = h->rep_grad_in(); }
   else if (c.sparse_adam_mode == PAMREC_ADAM_LAZY) s.mode = SP2_FUSED;
@@ -391,67 +443,55 @@ static AdamP make_adam(PamrecHandle h, float lr_t) {
   return a;
 }
 
-// ------------------------------------------------------------------------------------------
-// Row-sharded tables (PAMREC_TABLES_SHARDED): plan of this rank's lookups, exchange with the owners.
-static const char* const kShardName[3] = {"item", "cate", "user"};
-static const ShardDim& shard_dim(PamrecHandle h, int t) { return t == 0 ? h->L.sh_item : (t == 1 ? h->L.sh_cate : h->L.sh_user); }
+// Sparse update of one id space over the n lookups of plan p, in two halves: the sharded path all-reduces the clip norms between them.
+// Reduce half: duplicate gradient rows summed into p.accum (when g: lookup i < n_hist reads row i of g->hist, the others row
+// i - n_hist of g->tgt, from column g->col on), then the L2 rows of every parameter table.
+struct GradRows { const float* hist; int hist_ld; const float* tgt; int tgt_ld; int col; };
+static int sparse_reduce(PamrecHandle h, const SparseTable& p, int64_t n, int64_t n_hist, const GradRows* g, const SparseTable* tab,
+                         int n_tab, cudaStream_t st) {
+  if (g && launch_sparse_segreduce(p, n, n_hist, g->hist, g->hist_ld, g->col, g->tgt, g->tgt_ld, g->col, p.normsq, st))
+    return fail(h, "no sparse kernels for table width %d", p.width);
+  for (int k = 0; k < n_tab; ++k)
+    if (launch_sparse_l2norm(tab[k], n, h->cfg.embed_l2, h->wd("loss_acc") + 3, st))
+      return fail(h, "no sparse kernels for table width %d", tab[k].width);
+  return 0;
+}
+// Apply half: Adam on every parameter table, then the slot map of their plan back to -1.
+static int sparse_apply(PamrecHandle h, const SparseTable* tab, int n_tab, int64_t n, float lr_t, cudaStream_t st) {
+  const PamrecConfig& c = h->cfg;
+  for (int k = 0; k < n_tab; ++k)
+    if (launch_sparse_adam(tab[k], n, c.sparse_adam_mode, c.embed_l2, lr_t, c.beta1, c.beta2, c.epsilon, c.max_grad_norm, c.is_clip_norm, st))
+      return fail(h, "no sparse kernels for table width %d", tab[k].width);
+  launch_slot_reset(tab[0], n, st);
+  return 0;
+}
 
-// requester side: the "sp.*" arrays describe this rank's own lookups; keys are sharded-table addresses
-static SparseTable req_table(PamrecHandle h, int t) {
-  SparseTable s;
-  memset(&s, 0, sizeof s);
-  const ShardDim& d = shard_dim(h, t);
-  std::string p = std::string("sp.") + kShardName[t] + ".";
-  s.keys = h->wi(p + "keys"); s.idx = h->wi(p + "idx"); s.skeys = h->wi(p + "skeys"); s.sidx = h->wi(p + "sidx");
-  s.uidx = h->wi(p + "uidx"); s.ukeys = h->wi(p + "ukeys");
-  s.width = d.width; s.n_rows = d.rps * h->cfg.world_size;
-  s.accum = d.width ? h->wf(p + "accum") : nullptr;
-  s.nuniq = h->wi("sp.nuniq") + t;
-  s.normsq = h->wd("sp_normsq") + t;
-  return s;
-}
-// owner side: the "so.*" arrays describe the rows other ranks asked this rank for, bound to the local shard
-static SparseTable own_table(PamrecHandle h, int t, bool user_short = false) {
-  SparseTable s;
-  memset(&s, 0, sizeof s);
-  const ShardDim& d = shard_dim(h, t);
-  std::string q = std::string("so.") + kShardName[t] + ".";
-  s.keys = h->wi(q + "keys"); s.idx = h->wi(q + "idx"); s.skeys = h->wi(q + "skeys"); s.sidx = h->wi(q + "sidx");
-  s.uidx = h->wi(q + "uidx"); s.ukeys = h->wi(q + "ukeys");
-  s.slot = h->wi(std::string("sp.") + kShardName[t] + ".slot");
-  s.n_rows = d.rps;
-  s.nuniq = h->wi("sp.nuniq") + 4 + t;
-  double* ns = h->wd("sp_normsq");
-  if (t == 0) { s.width = kI; s.w = h->buf.item_w; s.m = h->buf.item_m; s.v = h->buf.item_v; s.accum = h->wf(q + "accum"); s.normsq = ns; }
-  else if (t == 1) { s.width = kC; s.w = h->buf.cate_w; s.m = h->buf.cate_m; s.v = h->buf.cate_v; s.accum = h->wf(q + "accum"); s.normsq = ns + 1; }
-  else if (!user_short) { s.width = PAMREC_USER_DIM; s.w = h->buf.ulong_w; s.m = h->buf.ulong_m; s.v = h->buf.ulong_v; s.normsq = ns + 2; }
-  else { s.width = PAMREC_USER_DIM; s.w = h->buf.ushort_w; s.m = h->buf.ushort_m; s.v = h->buf.ushort_v; s.normsq = ns + 3; }
-  return s;
-}
+// ------------------------------------------------------------------------------------------
+// Row-sharded tables (PAMREC_TABLES_SHARDED): plan of this rank's lookups ("sp.*": keys are sharded-table addresses), exchange
+// with the owners.
+
+// ids of id space t (0 item, 1 cate, 2 user) that batch b looks up: history (users: the user ids), then targets (users: none)
+static const int* hist_ids(const PamrecBatch* b, int t) { return t == 0 ? b->item_history : (t == 1 ? b->item_cate_history : b->users); }
+static const int* tgt_ids(const PamrecBatch* b, int t) { return t == 0 ? b->items : (t == 1 ? b->cates : nullptr); }
 
 // Forward half of the exchange: unique ids of the batch -> owners; owners' rows -> "sh.<table>.rows", one row per
 // unique id, in the order of the plan's unique list ("sh.<table>.inv" maps every lookup position to its row).
 // ONE host synchronisation: the per-peer counts must reach the host before the variable all-to-alls can be posted.
 static int shard_exchange_fwd(PamrecHandle h, const PamrecBatch* b, bool training, cudaStream_t st) {
   const int W = h->cfg.world_size, B = b->batch, T = h->cfg.max_seq_len;
-  const int64_t N = (int64_t)B * T;
   void* tmp = h->ws<char>("cub_temp");
   const size_t tmp_bytes = (size_t)h->L.ws[h->L.ws_index.at("cub_temp")].numel;
   int* cs = h->wi("sh.counts_send");
   int* cr = h->wi("sh.counts_recv");
   cudaMemsetAsync(cs, 0, sizeof(int) * 4 * W, st);
-  const int nt = training ? 3 : 2;
+  const int nt = training ? 3 : 2;                    // user ids travel when training only: their rows are L2 rows of the update
   h->xc_users = training;
   for (int t = 0; t < nt; ++t) {
-    const ShardDim& d = shard_dim(h, t);
-    SparseTable req = req_table(h, t);
-    const int* hist = t == 0 ? b->item_history : (t == 1 ? b->item_cate_history : b->users);
-    const int* tgt = t == 0 ? b->items : (t == 1 ? b->cates : nullptr);
-    const int64_t n_hist = t < 2 ? N : B, n_tgt = t < 2 ? B : 0;
-    if (launch_sparse_plan(req, hist, tgt, n_hist, n_tgt, W, d.rps, d.rps * W, false, tmp, tmp_bytes, st))
+    const IdTables& s = h->sp[t];
+    const int64_t rps = s.d->rows, n = s.d->lookups(B, T), n_hist = s.d->n_hist(B, T);
+    if (launch_sparse_plan(s.req, hist_ids(b, t), tgt_ids(b, t), n_hist, n - n_hist, W, rps, rps * W, false, tmp, tmp_bytes, st))
       return fail(h, "cub sort failed");
-    std::string p = std::string("sh.") + kShardName[t] + ".";
-    launch_shard_route(req, n_hist + n_tgt, W, d.rps, h->wi(p + "off"), cs, t, h->wi(p + "send_ids"), h->wi(p + "inv"), st);
+    launch_shard_route(s.req, n, W, rps, s.off, cs, t, s.send_ids, s.inv, st);
   }
   {
     PAMREC_PROF("xchg_counts", 1, st);
@@ -464,7 +504,7 @@ static int shard_exchange_fwd(PamrecHandle h, const PamrecBatch* b, bool trainin
     if (h->h_counts[8 * W]) return fail(h, "peer mailbox all-reduce timed out at sync point %d (a rank left the step?)", h->h_counts[8 * W] - 1);
   }
   for (int t = 0; t < 3; ++t) {
-    Xchg& x = h->xc[t];
+    Xchg& x = h->sp[t].x;
     x.soff.assign(W, 0); x.scnt.assign(W, 0); x.roff.assign(W, 0); x.rcnt.assign(W, 0);
     int64_t so = 0, ro = 0;
     for (int p = 0; p < W; ++p) {
@@ -474,16 +514,14 @@ static int shard_exchange_fwd(PamrecHandle h, const PamrecBatch* b, bool trainin
       x.roff[p] = ro; ro += x.rcnt[p];
     }
     x.n_send = so; x.n_recv = ro;
-    if (ro > shard_dim(h, t).cap_recv) return fail(h, "exchange overflow on table %s: %lld rows", kShardName[t], (long long)ro);
+    if (ro > h->sp[t].d->cap_recv) return fail(h, "exchange overflow on table %s: %lld rows", h->sp[t].d->name, (long long)ro);
   }
   {
     PAMREC_PROF("xchg_ids", 1, st);
     int xrc = h->comm.group_start();                  // the group is closed on every path (comm.cu: close_group)
     for (int t = 0; t < nt && !xrc; ++t) {
-      const Xchg& x = h->xc[t];
-      std::string p = std::string("sh.") + kShardName[t] + ".";
-      xrc |= h->comm.all_to_all_v(h->wi(p + "send_ids"), x.soff.data(), x.scnt.data(), h->wi(p + "recv_ids"), x.roff.data(),
-                                  x.rcnt.data(), 1, COMM_I32, st);
+      const IdTables& s = h->sp[t];
+      xrc |= h->comm.all_to_all_v(s.send_ids, s.x.soff.data(), s.x.scnt.data(), s.recv_ids, s.x.roff.data(), s.x.rcnt.data(), 1, COMM_I32, st);
     }
     xrc |= h->comm.group_end();
     if (xrc) return fail(h, "nccl: %s", h->comm.err.c_str());
@@ -493,26 +531,21 @@ static int shard_exchange_fwd(PamrecHandle h, const PamrecBatch* b, bool trainin
     // side stream while the forward and backward passes run (the requester plans above are done with the cub scratch)
     int prc = 0;
     h->fork(st, [&](cudaStream_t s2) {
-      for (int t = 0; t < 3; ++t) {
-        SparseTable own = own_table(h, t);
-        std::string p = std::string("sh.") + kShardName[t] + ".";
-        prc |= launch_sparse_plan(own, h->wi(p + "recv_ids"), nullptr, h->xc[t].n_recv, 0, 1, 0, own.n_rows, true, tmp, tmp_bytes, s2);
-      }
+      for (const IdTables& s : h->sp)
+        prc |= launch_sparse_plan(s.own, s.recv_ids, nullptr, s.x.n_recv, 0, 1, 0, s.own.n_rows, true, tmp, tmp_bytes, s2);
       cudaEventRecord(h->ev_plan, s2);
     });
     if (prc) return fail(h, "cub sort failed");
   }
-  launch_serve_rows(h->buf.item_w, h->wi("sh.item.recv_ids"), h->xc[0].n_recv, kI, h->wf("sh.item.xrows"), st);
-  launch_serve_rows(h->buf.cate_w, h->wi("sh.cate.recv_ids"), h->xc[1].n_recv, kC, h->wf("sh.cate.xrows"), st);
+  for (const IdTables& s : h->sp)
+    if (s.d->accum) launch_serve_rows(s.tab[0].w, s.recv_ids, s.x.n_recv, s.d->width, s.xrows, st);
   {
     PAMREC_PROF("xchg_rows", 1, st);
     int xrc = h->comm.group_start();
-    for (int t = 0; t < 2 && !xrc; ++t) {
-      const Xchg& x = h->xc[t];
-      std::string p = std::string("sh.") + kShardName[t] + ".";
-      xrc |= h->comm.all_to_all_v(h->wf(p + "xrows"), x.roff.data(), x.rcnt.data(), h->wf(p + "rows"), x.soff.data(),
-                                  x.scnt.data(), shard_dim(h, t).width, COMM_F32, st);
-    }
+    for (const IdTables& s : h->sp)
+      if (s.d->accum && !xrc)
+        xrc |= h->comm.all_to_all_v(s.xrows, s.x.roff.data(), s.x.rcnt.data(), s.rows, s.x.soff.data(), s.x.scnt.data(), s.d->width,
+                                    COMM_F32, st);
     xrc |= h->comm.group_end();
     if (xrc) return fail(h, "nccl: %s", h->comm.err.c_str());
   }
@@ -529,9 +562,9 @@ static int embed_forward(PamrecHandle h, const PamrecBatch* b, bool training, fl
   }
   if (int rc = shard_exchange_fwd(h, b, training, st)) return rc;
   const int64_t N = (int64_t)B * T;
-  const int* ii = h->wi("sh.item.inv");
-  const int* ci = h->wi("sh.cate.inv");
-  launch_embed_fwd(ii, ci, ii + N, ci + N, h->wf("sh.item.rows"), h->wf("sh.cate.rows"), h->P(h->L.pos), x0, h->wf("tgt"), B, T, st);
+  const IdTables& si = h->sp[0];
+  const IdTables& sc = h->sp[1];
+  launch_embed_fwd(si.inv, sc.inv, si.inv + N, sc.inv + N, si.rows, sc.rows, h->P(h->L.pos), x0, h->wf("tgt"), B, T, st);
   return 0;
 }
 
@@ -982,7 +1015,6 @@ int pamrec_apply_gradients(PamrecHandle h, const PamrecBatch* b, int64_t step, v
   const Layout& L = h->L;
   const PamrecConfig& c = h->cfg;
   const int B = b->batch, T = c.max_seq_len;
-  const int64_t N = (int64_t)B * T;
   const double b1 = c.beta1, b2 = c.beta2;
   const double tstep = step > 0 ? (double)step : 1.0;
   const float lr_t = (float)((double)c.learning_rate * std::sqrt(1.0 - std::pow(b2, tstep)) / (1.0 - std::pow(b1, tstep)));
@@ -1003,30 +1035,24 @@ int pamrec_apply_gradients(PamrecHandle h, const PamrecBatch* b, int64_t step, v
     Comm& cm = h->comm;
     int crc = 0;
     if (!h->xc_users) return fail(h, "apply_gradients needs pamrec_forward(training=1) on the same batch");   // before any collective
-    for (int t = 0; t < 2; ++t) {
-      SparseTable req = req_table(h, t);
-      const int col = t == 0 ? 0 : kI;
-      launch_sparse_segreduce(req, N + B, N, dX0, kD, col, dT, kE, col, req.normsq, st);
+    for (const IdTables& s : h->sp) {
+      if (!s.d->accum) continue;
+      const GradRows g{dX0, kD, dT, kE, s.d->col};
+      if (int rc = sparse_reduce(h, s.req, s.d->lookups(B, T), s.d->n_hist(B, T), &g, nullptr, 0, st)) return rc;
     }
     {
       PAMREC_PROF("xchg_grads", 1, st);
       crc |= cm.group_start();
-      for (int t = 0; t < 2; ++t) {
-        const Xchg& x = h->xc[t];
-        std::string p = std::string("sh.") + kShardName[t] + ".";
-        crc |= cm.all_to_all_v(req_table(h, t).accum, x.soff.data(), x.scnt.data(), h->wf(p + "xrows"), x.roff.data(), x.rcnt.data(),
-                               shard_dim(h, t).width, COMM_F32, st);
-      }
+      for (const IdTables& s : h->sp)
+        if (s.d->accum)
+          crc |= cm.all_to_all_v(s.req.accum, s.x.soff.data(), s.x.scnt.data(), s.xrows, s.x.roff.data(), s.x.rcnt.data(), s.d->width,
+                                 COMM_F32, st);
       crc |= cm.group_end();
     }
     cudaStreamWaitEvent(st, h->ev_plan, 0);            // owner-side plans (side stream, forked in the forward exchange)
-    for (int t = 0; t < 3; ++t) {
-      SparseTable own = own_table(h, t);
-      const int64_t nr = h->xc[t].n_recv;
-      std::string p = std::string("sh.") + kShardName[t] + ".";
-      if (t < 2) launch_sparse_segreduce(own, nr, nr, h->wf(p + "xrows"), own.width, 0, nullptr, 0, 0, h->wd("sh.scratch"), st);
-      launch_sparse_l2norm(own, nr, c.embed_l2, reg, st);
-      if (t == 2) launch_sparse_l2norm(own_table(h, 2, true), nr, c.embed_l2, reg, st);
+    for (const IdTables& s : h->sp) {
+      const GradRows g{s.xrows, s.d->width, nullptr, 0, 0};
+      if (int rc = sparse_reduce(h, s.own, s.x.n_recv, s.x.n_recv, s.d->accum ? &g : nullptr, s.tab, s.d->n_tab, st)) return rc;
     }
     if (h->use_xr()) {
       peer_allreduce_grads(h, st);
@@ -1039,15 +1065,8 @@ int pamrec_apply_gradients(PamrecHandle h, const PamrecBatch* b, int64_t step, v
       crc |= cm.group_end();
     }
     if (crc) return fail(h, "nccl: %s", cm.err.c_str());
-    for (int t = 0; t < 3; ++t) {
-      SparseTable own = own_table(h, t);
-      const int64_t nr = h->xc[t].n_recv;
-      launch_sparse_adam(own, nr, c.sparse_adam_mode, c.embed_l2, lr_t, c.beta1, c.beta2, c.epsilon, c.max_grad_norm, c.is_clip_norm, st);
-      if (t == 2)
-        launch_sparse_adam(own_table(h, 2, true), nr, c.sparse_adam_mode, c.embed_l2, lr_t, c.beta1, c.beta2, c.epsilon,
-                           c.max_grad_norm, c.is_clip_norm, st);
-      launch_slot_reset(own, nr, st);
-    }
+    for (const IdTables& s : h->sp)
+      if (int rc = sparse_apply(h, s.tab, s.d->n_tab, s.x.n_recv, lr_t, st)) return rc;
   } else {
     // ---- whole tables on this GPU: one-sort plan (side stream, beside the forward pass) -> run walk -> Adam
     if (c.world_size == 1) {

@@ -112,10 +112,6 @@ struct SparseTable {
 void launch_embed_bwd_reduce(const float* dX0, const float* dTgtHead, float* dTgtTotal, float* dPos, double* pos_normsq,
                              double* undedup, int B, int T, cudaStream_t st);
 size_t sparse_temp_bytes(int64_t n_keys);
-// builds keys (history ids then target ids), sorts, finds unique rows, reduces duplicate rows into accum
-int launch_sparse_reduce(const SparseTable& t, const int* hist_ids, const int* tgt_ids, int64_t n_hist, int64_t n_tgt,
-                         const float* hist_grad, int hist_ld, int hist_col, const float* tgt_grad, int tgt_ld, int tgt_col,
-                         void* cub_temp, size_t cub_bytes, cudaStream_t st);
 int launch_sparse_plan(const SparseTable& t, const int* hist_ids, const int* tgt_ids, int64_t n_hist, int64_t n_tgt,
                        int world, int64_t rps, int64_t key_range, bool fill_slot, void* cub_temp, size_t cub_bytes,
                        cudaStream_t st);

@@ -229,15 +229,6 @@ int launch_sparse_segreduce(const SparseTable& t, int64_t n, int64_t n_hist, con
   return 0;
 }
 
-int launch_sparse_reduce(const SparseTable& t, const int* hist_ids, const int* tgt_ids, int64_t n_hist, int64_t n_tgt,
-                         const float* hist_grad, int hist_ld, int hist_col, const float* tgt_grad, int tgt_ld, int tgt_col,
-                         void* cub_temp, size_t cub_bytes, cudaStream_t st) {
-  if (launch_sparse_plan(t, hist_ids, tgt_ids, n_hist, n_tgt, 1, 0, t.n_rows, true, cub_temp, cub_bytes, st)) return -1;
-  if (t.accum != nullptr && hist_grad != nullptr)
-    return launch_sparse_segreduce(t, n_hist + n_tgt, n_hist, hist_grad, hist_ld, hist_col, tgt_grad, tgt_ld, tgt_col, t.normsq, st);
-  return 0;
-}
-
 // L2 rows of the unique ids (sequential_base_model.py:647-664, pamrec.py:173-182)
 template <int W>
 __global__ void __launch_bounds__(256)

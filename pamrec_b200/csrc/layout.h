@@ -42,15 +42,31 @@ struct MlpOff {
   BnId bn_of(int l) const { return l == 0 ? bn0 : bn1; }               // l = 0, 1
 };
 
-// one row-sharded table as seen by the exchange (PAMREC_TABLES_SHARDED)
-struct ShardDim { int64_t vocab = 0, rps = 0, nk = 0, cap_recv = 0; int width = 0; };
+// One id space of the embedding tables (item, category, user): its lookups, the rows this rank holds and the parameter tables
+// it updates.  Workspace: "sp.<name>.*", the plan of this rank's lookups; sharded tables also "sh.<name>.*" (the exchange) and
+// "so.<name>.*" (the owner-side plan of the rows the other ranks asked this rank for).
+struct IdSpace {
+  const char* name = "";
+  int64_t vocab = 0, rows = 0;     // rows of the table; rows held by this rank (Layout::rows_of)
+  int seqs = 0;                    // history sequences looked up per sample, then the target; 0: one lookup per sample (users)
+  int64_t nk = 0;                  // lookups of a batch of Bcap samples
+  int64_t cap_recv = 0;            // sharded: rows the other ranks can ask this rank for, at most min(nk, rows) each
+  int width = 0, col = 0;          // floats per row; first column of the table inside a token or target gradient row
+  int tab0 = 0, n_tab = 1;         // parameter tables tab0 .. tab0 + n_tab - 1 (0 item, 1 cate, 2 user_long, 3 user_short), each
+                                   // with its own sp_normsq slot of the same index
+  bool accum = false;              // the lookups carry gradient rows (item, cate); a user row is an L2 row only
+  bool slot = false;               // per-table plan with a slot map (kernels_optim.cu); else the one-sort plan of kernels_sparse2.cu
+  bool has0 = false;               // row 0 is an L2 row only when sib.has0 says so (SparseTable::l2_has0)
+  int64_t n_hist(int64_t B, int T) const { return seqs ? seqs * B * T : B; }
+  int64_t lookups(int64_t B, int T) const { return seqs ? seqs * B * T + B : B; }
+};
 
 struct Layout {
   int n_users = 0, n_items = 0, n_cates = 0, T = 0, Bcap = 0;
   int world = 1, table_mode = 0;
-  ShardDim sh_item, sh_cate, sh_user;
+  IdSpace idsp[3];                              // item, cate, user (SASRec: no users)
+  int n_idsp = 0;
   int64_t cub_keys = 0;                         // largest key count handed to cub
-  int64_t cub_keys_table = 0;                   // lookups of one table per batch (N + B)
   int64_t rows_of(int64_t vocab) const { return table_mode == PAMREC_TABLES_SHARDED ? (vocab + world - 1) / world : vocab; }
   std::vector<TensorDesc> dense, bn, ws;
   int64_t dense_numel = 0, bn_numel = 0;
@@ -166,6 +182,45 @@ struct Layout {
     add_ws("bn.gbsums", PAMREC_F64, {8, bn_c, 2});   // ... and of the backward sums
   }
 
+  // The id spaces of the model and their sparse-path workspace.  Item and category tables are looked up by `seqs` history
+  // sequences and the target of every sample; the user tables (users) by the user id.
+  void add_id_spaces(int seqs, bool users) {
+    const bool sharded = table_mode == PAMREC_TABLES_SHARDED, sibling = model_kind != PAMREC_MODEL_PAMREC;
+    const int64_t B = Bcap;
+    auto add = [&](const char* name, int64_t vocab, int sq, int width, int col, int tab0, int n_tab) {
+      IdSpace& d = idsp[n_idsp++];
+      d.name = name; d.vocab = vocab; d.rows = rows_of(vocab); d.seqs = sq; d.nk = d.lookups(B, T);
+      d.width = width; d.col = col; d.tab0 = tab0; d.n_tab = n_tab;
+      d.accum = sq > 0; d.slot = sibling || sharded; d.has0 = sibling && sq > 0;
+      const std::string p = std::string("sp.") + name + ".";
+      if (d.slot)
+        for (const char* n : {"keys", "idx", "skeys", "sidx", "uidx"}) add_ws(p + n, PAMREC_I32, {d.nk});
+      add_ws(p + "ukeys", PAMREC_I32, {d.nk});
+      if (d.slot) add_ws(p + "slot", PAMREC_I32, {d.rows});   // table row (of this rank) -> unique index
+      if (d.accum) add_ws(p + "accum", PAMREC_F32, {d.nk, width});
+      if (d.nk > cub_keys) cub_keys = d.nk;
+      if (!sharded) return;
+      // exchange buffers and the owner-side plan
+      d.cap_recv = (int64_t)world * (d.nk < d.rows ? d.nk : d.rows);
+      const std::string q = std::string("sh.") + name + ".", o = std::string("so.") + name + ".";
+      add_ws(q + "inv", PAMREC_I32, {d.nk});
+      add_ws(q + "send_ids", PAMREC_I32, {d.nk});
+      add_ws(q + "off", PAMREC_I32, {128});
+      add_ws(q + "recv_ids", PAMREC_I32, {d.cap_recv});
+      if (d.accum) {
+        add_ws(q + "rows", PAMREC_F32, {d.nk, width});            // rows received from their owners (forward)
+        add_ws(q + "xrows", PAMREC_F32, {d.cap_recv, width});     // owner: rows served (forward) / row gradients received
+        add_ws(o + "accum", PAMREC_F32, {d.cap_recv, width});
+      }
+      for (const char* n : {"keys", "idx", "skeys", "sidx", "uidx", "ukeys"}) add_ws(o + n, PAMREC_I32, {d.cap_recv});
+      if (d.cap_recv > cub_keys) cub_keys = d.cap_recv;
+    };
+    add("item", n_items, seqs, item_dim, 0, 0, 1);
+    add("cate", n_cates, seqs, cate_dim, item_dim, 1, 1);
+    if (users) add("user", n_users, 0, user_dim, 0, 2, 2);
+    add_ws("sp.nuniq", PAMREC_I32, {8});           // 0 item 1 cate 2 user ; 4 5 6 = owner-side plans (sharded tables)
+  }
+
   // MMoEModel_original / PLEModel / ShareBottomModel (oracle/siblings_oracle.py:param_spec has the same inventory, by TF name)
   void build_sibling(const PamrecConfig& c) {
     const int L2 = PAMREC_SEG_L2;
@@ -245,19 +300,8 @@ struct Layout {
     add_bn_ws();
     add_optim_ws();
     // sparse path (kernels_optim.cu, one plan per table): keys = satisfied ids, history ids, target ids
-    const int64_t NK = 2 * N + B;
-    cub_keys_table = NK;
-    for (const char* t : {"item", "cate"}) {
-      std::string p = std::string("sp.") + t + ".";
-      for (const char* n : {"keys", "idx", "skeys", "sidx", "uidx", "ukeys"}) add_ws(p + n, PAMREC_I32, {NK});
-      add_ws(p + "slot", PAMREC_I32, {t[0] == 'i' ? n_items : n_cates});
-      add_ws(p + "accum", PAMREC_F32, {NK, t[0] == 'i' ? item_dim : cate_dim});
-    }
-    for (const char* n : {"keys", "idx", "skeys", "sidx", "uidx", "ukeys"}) add_ws(std::string("sp.user.") + n, PAMREC_I32, {B});
-    add_ws("sp.user.slot", PAMREC_I32, {n_users});
-    add_ws("sp.nuniq", PAMREC_I32, {8});
+    add_id_spaces(2, true);
     add_ws("dp.scalars", PAMREC_F64, {8});
-    cub_keys = NK;
     add_ws("cub_temp", PAMREC_U8, {(int64_t)(16u << 20) + 16 * cub_keys});
     (void)c;
   }
@@ -330,17 +374,8 @@ struct Layout {
     add_ws("sib.has0", PAMREC_I32, {4});
     add_bn_ws();
     add_optim_ws();
-    const int64_t NK = 2 * N + B;
-    cub_keys_table = NK;
-    for (const char* t : {"item", "cate"}) {
-      std::string p = std::string("sp.") + t + ".";
-      for (const char* n : {"keys", "idx", "skeys", "sidx", "uidx", "ukeys"}) add_ws(p + n, PAMREC_I32, {NK});
-      add_ws(p + "slot", PAMREC_I32, {t[0] == 'i' ? n_items : n_cates});
-      add_ws(p + "accum", PAMREC_F32, {NK, t[0] == 'i' ? item_dim : cate_dim});
-    }
-    add_ws("sp.nuniq", PAMREC_I32, {8});
+    add_id_spaces(2, false);                       // SASRec has no user tables (sasrec_param_spec)
     add_ws("dp.scalars", PAMREC_F64, {8});
-    cub_keys = NK;
     add_ws("cub_temp", PAMREC_U8, {(int64_t)(16u << 20) + 16 * cub_keys});
     (void)c;
   }
@@ -451,34 +486,9 @@ struct Layout {
     // sparse path: keys = history ids then target ids.  "sp.*" is the plan of THIS rank's lookups; the slot map
     // (table row -> unique index) always covers the rows this rank owns.
     const int64_t NK = N + B;
-    const bool sharded = table_mode == PAMREC_TABLES_SHARDED;
-    cub_keys_table = NK;
-    for (const char* t : {"item", "cate"}) {
-      std::string p = std::string("sp.") + t + ".";
-      if (sharded) {
-        add_ws(p + "keys", PAMREC_I32, {NK});
-        add_ws(p + "idx", PAMREC_I32, {NK});
-        add_ws(p + "skeys", PAMREC_I32, {NK});
-        add_ws(p + "sidx", PAMREC_I32, {NK});
-        add_ws(p + "uidx", PAMREC_I32, {NK});
-        add_ws(p + "slot", PAMREC_I32, {rows_of(t[0] == 'i' ? n_items : n_cates)});
-      }
-      add_ws(p + "ukeys", PAMREC_I32, {NK});
-      add_ws(p + "accum", PAMREC_F32, {NK, t[0] == 'i' ? kI : kC});
-    }
-    if (sharded) {
-      add_ws("sp.user.keys", PAMREC_I32, {B});
-      add_ws("sp.user.idx", PAMREC_I32, {B});
-      add_ws("sp.user.skeys", PAMREC_I32, {B});
-      add_ws("sp.user.sidx", PAMREC_I32, {B});
-      add_ws("sp.user.uidx", PAMREC_I32, {B});
-      add_ws("sp.user.slot", PAMREC_I32, {rows_of(n_users)});
-    }
-    add_ws("sp.user.ukeys", PAMREC_I32, {B});
-    add_ws("sp.nuniq", PAMREC_I32, {8});           // 0 item 1 cate 2 user ; 4 5 6 = owner-side plans (sharded tables)
+    add_id_spaces(1, true);
     add_ws("dp.scalars", PAMREC_F64, {8});         // [0] listwise groups with a non-zero label sum over all ranks
-    cub_keys = NK;
-    if (!sharded) {
+    if (table_mode != PAMREC_TABLES_SHARDED) {
       // whole tables on this GPU (kernels_sparse2.cu): ONE plan over the lookups of the three id spaces
       const int64_t NKA = 2 * NK + B;
       for (const char* n : {"keys", "idx", "skeys", "sidx", "uidx"}) add_ws(std::string("sp2.") + n, PAMREC_I32, {NKA});
@@ -489,33 +499,7 @@ struct Layout {
       if (table_mode == PAMREC_TABLES_REPLICATED && world > 1)
         add_ws("rep.grad", PAMREC_F32, {(int64_t)n_items * 17 + (int64_t)n_cates * 5 + n_users});
       cub_keys = NKA;
-    }
-    if (table_mode == PAMREC_TABLES_SHARDED) {
-      // exchange buffers ("sh.*") and the owner-side plan of the rows other ranks asked this rank for ("so.*")
-      auto dim = [&](int64_t vocab, int64_t nk, int width) {
-        ShardDim d;
-        d.vocab = vocab; d.rps = rows_of(vocab); d.nk = nk; d.width = width;
-        d.cap_recv = (int64_t)world * (nk < d.rps ? nk : d.rps);   // a rank can ask for at most min(nk, rps) distinct rows
-        return d;
-      };
-      sh_item = dim(n_items, NK, kI); sh_cate = dim(n_cates, NK, kC); sh_user = dim(n_users, B, 0);
-      const ShardDim* dims[3] = {&sh_item, &sh_cate, &sh_user};
-      const char* names[3] = {"item", "cate", "user"};
-      for (int i = 0; i < 3; ++i) {
-        const ShardDim& d = *dims[i];
-        std::string p = std::string("sh.") + names[i] + ".", q = std::string("so.") + names[i] + ".";
-        add_ws(p + "inv", PAMREC_I32, {d.nk});
-        add_ws(p + "send_ids", PAMREC_I32, {d.nk});
-        add_ws(p + "off", PAMREC_I32, {128});
-        add_ws(p + "recv_ids", PAMREC_I32, {d.cap_recv});
-        if (d.width) {
-          add_ws(p + "rows", PAMREC_F32, {d.nk, d.width});          // rows received from their owners (forward)
-          add_ws(p + "xrows", PAMREC_F32, {d.cap_recv, d.width});   // owner: rows served (forward) / row gradients received
-          add_ws(q + "accum", PAMREC_F32, {d.cap_recv, d.width});
-        }
-        for (const char* n : {"keys", "idx", "skeys", "sidx", "uidx", "ukeys"}) add_ws(q + n, PAMREC_I32, {d.cap_recv});
-        if (d.cap_recv > cub_keys) cub_keys = d.cap_recv;
-      }
+    } else {
       add_ws("sh.counts_send", PAMREC_I32, {(int64_t)world * 4});
       add_ws("sh.counts_recv", PAMREC_I32, {(int64_t)world * 4});
       add_ws("sh.scratch", PAMREC_F64, {8});
