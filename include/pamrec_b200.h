@@ -181,6 +181,25 @@ int pamrec_apply_gradients(PamrecHandle h, const PamrecBatch* b, int64_t step, v
 /* forward + backward + apply; losses_out (device, 5 floats): loss, data, regular, auxiliary, order (pamrec.py:444-448) */
 int pamrec_train_step(PamrecHandle h, const PamrecBatch* b, int64_t step, float* losses_out, void* stream);
 
+/* Candidate ranking: every line of `lines` (a scoring batch as pamrec_forward takes it, 1 .. max_batch rows) is scored against every
+ * candidate (cand_items[n_cand], unique item ids in [1, n_items), with their categories cand_cates[n_cand] in [0, n_cates)).  The
+ * score of (line, candidate c) is the pred that pamrec_forward(training = 0) writes for the line with items = c, cates = cate(c);
+ * nothing else of the line changes.  Per line the best top_k (1 .. PAMREC_RANK_MAX_K) candidates go to topk_items / topk_scores
+ * [batch, top_k] in the order score descending, then item id ascending; slots past the last candidate hold id -1, score -inf.
+ * exclude_history != 0 skips the candidates found at a real position (mask > 0) of the line's item_history, except the line's own
+ * item (`items`).  own_rank (nullable, [batch]) = 1 + the number of candidates ordered before the line's own item, -1 when that item
+ * is not a candidate (its score is taken with the candidate's category).  The (line, candidate) rows are scored in chunks of
+ * max_batch rows; the result does not depend on the chunking.  All pointers are device memory; the scratch is the caller's
+ * (pamrec_rank_scratch_bytes; its size does not depend on top_k, which is only checked).  One GPU with whole tables.  The call
+ * overwrites the activation workspace like pamrec_forward(training = 0): never between the forward and the backward pass of a
+ * training step.  It returns once the stream has reached its end: a bad candidate list, or a non-finite score, fails the call
+ * with the candidate or the line named in pamrec_last_error. */
+#define PAMREC_RANK_MAX_K 1024
+int64_t pamrec_rank_scratch_bytes(PamrecHandle h, int32_t top_k);
+int pamrec_rank_candidates(PamrecHandle h, const PamrecBatch* lines, const int32_t* cand_items, const int32_t* cand_cates, int32_t n_cand,
+                           int32_t top_k, int32_t exclude_history, void* scratch, int64_t scratch_bytes, int32_t* topk_items,
+                           float* topk_scores, int32_t* own_rank, void* stream);
+
 /* Multi-GPU plumbing.  The library talks to NCCL directly (dlopen of the libnccl.so.2 that PyTorch ships;
  * `nccl_path` may be NULL to use the loader's search path).  Rank 0 creates the unique id, the host broadcasts
  * the 128 bytes (torch.distributed), every rank calls pamrec_comm_init; afterwards forward / backward /
@@ -233,6 +252,9 @@ int pamrec_bench_table_adam(PamrecHandle h, int64_t step, void* stream);
  * pamrec_head_trace copies the 32 stamps of the last forward (backward = 0) or backward (1) head kernel: [0 .. n-1] barrier
  * releases, [29] n, [30] end of CTA 0, [31] start. */
 #define PAMREC_DEBUG_HEAD_TRACE 2
+/* PAMREC_DEBUG_RANK_EXPAND: pamrec_rank_candidates scores SASRec's candidates through the expansion path (the whole forward pass per
+ * (line, candidate) row) instead of its tower-only path, so that a checker can compare the two. */
+#define PAMREC_DEBUG_RANK_EXPAND 4
 int pamrec_set_debug(PamrecHandle h, int flags);
 int pamrec_head_trace(PamrecHandle h, int backward, uint64_t out[32]);
 /* the same run, per CTA: out[barrier * 256 + cta] = %globaltimer (ns) at which CTA `cta` arrived at barrier `barrier` (16 x 256 words) */

@@ -18,6 +18,8 @@ IPC_HANDLE_BYTES = 64
 GROUP = 5
 DEBUG_SAVE_FFN_HIDDEN = 1
 DEBUG_HEAD_TRACE = 2
+DEBUG_RANK_EXPAND = 4
+RANK_MAX_K = 1024                                    # pamrec_rank_candidates: largest top_k
 HIST_BUCKETS, HIST_MAX_SEGMENTS = 1551, 512          # pamrec_histograms: default bucket limits, segments per call
 
 
@@ -95,6 +97,9 @@ EXPORTS = {
     "pamrec_histograms": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                     C.c_void_p, C.POINTER(C.c_int64), C.c_void_p]),
     "pamrec_histogram_buckets": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_int)]),
+    "pamrec_rank_scratch_bytes": (C.c_int64, [C.c_void_p, C.c_int32]),
+    "pamrec_rank_candidates": (C.c_int, [C.c_void_p, C.POINTER(PamrecBatch), C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,
+                                         C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "pamrec_bench_gather": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32,
                                       C.c_void_p, C.c_void_p]),
     "pamrec_bench_table_adam": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p]),

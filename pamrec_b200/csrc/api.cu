@@ -1134,6 +1134,7 @@ int pamrec_apply_gradients(PamrecHandle h, const PamrecBatch* b, int64_t step, v
 }
 
 #include "api_sibling.inl"
+#include "api_rank.inl"
 
 int pamrec_train_step(PamrecHandle h, const PamrecBatch* b, int64_t step, float* losses_out, void* stream) {
   if (!h) return -1;

@@ -207,6 +207,31 @@ void launch_sas_final_fwd(const float* SEQ, const int* mask, const float* tgt, f
 void launch_sas_final_bwd(const float* dU, const int* mask, float* dSEQ, float* dTgt, int B, int T, int S, cudaStream_t st);
 void launch_sas_pos_bwd(const float* dX0, float* dPos, double* normsq, int B, int T, int S, cudaStream_t st);
 
+// ---- kernels_rank.cu (pamrec_rank_candidates)
+struct RankRows {          // the lines' arrays read by the expansion, and the candidates
+  const int* item_history; const int* cate_history; const float* loop_times; const int* mask; const int* users;
+  const int* sat_item; const int* sat_cate; const int* sat_mask;   // null for PAMRec
+  const int* cand_items; const int* cand_cates;
+};
+struct RankBatch {         // the expanded rows (scratch)
+  int* item_history; int* cate_history; float* loop_times; int* mask; int* users; int* items; int* cates;
+  int* sat_item; int* sat_cate; int* sat_mask;
+};
+struct RankMerge {
+  const float* scores; const int* cand_items; const int* item_history; const int* mask; const int* own_items; const float* own_scores;
+  const int* map; int* count; int* topk_items; float* topk_scores; int* flags;
+  int64_t p0; int64_t l0; int rows, n_cand, n_items, K, T, exclude;
+};
+void launch_rank_map(const int* items, const int* cates, int n, int n_items, int n_cates, int* map, int* flags, cudaStream_t st);
+void launch_rank_begin(const int* items, const int* cates, const int* map, const int* cand_cates, int n_items, int B, int K,
+                       int* own_items, int* own_cates, int* count, int* topk_items, float* topk_scores, cudaStream_t st);
+void launch_rank_expand(const RankRows& a, const RankBatch& d, int64_t p0, int rows, int n_cand, int T, cudaStream_t st);
+void launch_rank_tower_in(const float* U_lines, const int* cand_items, const int* cand_cates, const float* item_w, const float* cate_w,
+                          float* U, int64_t p0, int rows, int n_cand, int item_dim, int cate_dim, cudaStream_t st);
+void launch_rank_merge(const RankMerge& a, int n_lines, cudaStream_t st);
+void launch_rank_finish(const int* own_items, const float* own_scores, const int* map, const int* count, int n_items, int B, int* own_rank,
+                        int* flags, cudaStream_t st);
+
 // ---- kernels_p2p.cu + kernels_head2.cu (data-parallel exchanges through NVLink peer mailboxes)
 constexpr int kP2PMaxDoubles = 2048;     // payload capacity of one mailbox slot (expert + gate layer-0 sums: 1256)
 constexpr int kP2PSlots = 24;            // sync points per step (each has its own slot): 12 forward + 12 backward barriers

@@ -242,6 +242,60 @@ def cal_metric(labels, preds, metrics):
     return res
 
 
+def rank_topk(scores, ids, top_k, keep=None):
+    """Top ``top_k`` of each row of scores [n, c] over the candidate ids [c], in the order of pamrec_rank_candidates: score
+    descending, then id ascending.  keep [n, c] (optional) marks the candidates a row may rank.  Returns (ids [n, top_k] with -1
+    past the last kept candidate, scores [n, top_k] with -inf there)."""
+    scores = np.asarray(scores, np.float32)
+    ids = np.asarray(ids, np.int64)
+    n = scores.shape[0]
+    out_ids = np.full((n, top_k), -1, np.int32)
+    out_sc = np.full((n, top_k), -np.inf, np.float32)
+    for r in range(n):
+        sel = np.arange(ids.size) if keep is None else np.flatnonzero(keep[r])
+        order = sel[np.lexsort((ids[sel], -scores[r, sel].astype(np.float64)))][:top_k]
+        out_ids[r, :order.size] = ids[order]
+        out_sc[r, :order.size] = scores[r, order]
+    return out_ids, out_sc
+
+
+def own_rank(scores, ids, own, keep=None):
+    """Rank of each row's own item among the candidates it may rank: 1 + the candidates ordered before it (score descending, then
+    id ascending); -1 when the own item is not a candidate.  scores [n, c], ids [c], own [n], keep [n, c] as in rank_topk."""
+    scores = np.asarray(scores, np.float32)
+    ids = np.asarray(ids, np.int64)
+    out = np.full(len(own), -1, np.int64)
+    for r, item in enumerate(np.asarray(own, np.int64)):
+        j = np.flatnonzero(ids == item)
+        if j.size == 0:
+            continue
+        s = scores[r]
+        before = (s > s[j[0]]) | ((s == s[j[0]]) & (ids < item))
+        if keep is not None:
+            before &= np.asarray(keep[r], bool)
+        out[r] = 1 + int(before.sum())
+    return out
+
+
+def full_ranking_metrics(ranks, labels, ks=(10,)):
+    """Full-catalogue ranking metrics over the lines with label 1: hit@k (rank <= k), ndcg@k (1 / log2(rank + 1) when rank <= k,
+    else 0) and mrr (1 / rank).  A rank < 1 (the positive is not a candidate) counts as a miss in every metric.  Rounded to 4
+    decimals like cal_metric; an empty set of positives gives 0."""
+    ranks = np.asarray(ranks, np.float64).reshape(-1)
+    pos = np.asarray(labels).reshape(-1) == 1
+    r = ranks[pos]
+    hit_any = r >= 1
+    safe = np.where(hit_any, r, 1.0)
+    mean = lambda v: round(float(np.mean(v)), 4) if v.size else 0.0
+    res = {}
+    for k in ks:
+        inside = hit_any & (r <= k)
+        res["hit@{0}".format(k)] = mean(inside.astype(np.float64))
+        res["ndcg@{0}".format(k)] = mean(np.where(inside, 1.0 / np.log2(safe + 1.0), 0.0))
+    res["mrr"] = mean(np.where(hit_any, 1.0 / safe, 0.0))
+    return res
+
+
 def _user_groups(users, preds, labels):
     """Rows of each user in first-to-last order, users sorted ascending (pandas groupby order)."""
     users = np.asarray(users)

@@ -116,6 +116,22 @@ class PendingHistograms:
         return self._value
 
 
+class PendingRank:
+    """Engine.rank_candidates: ``result()`` waits for the device->host copies and gives (topk_items [B,K] int32, topk_scores [B,K]
+    float32, own_rank [B] int32 or None)."""
+
+    def __init__(self, host, event, want_rank):
+        self._host, self._event, self._want_rank, self._value = host, event, want_rank, None
+
+    def result(self):
+        if self._value is None:
+            self._event.synchronize()
+            items, scores, ranks = (t.numpy().copy() for t in self._host)
+            self._value = (items, scores, ranks if self._want_rank else None)
+            self._host = None
+        return self._value
+
+
 class Engine:
     def __init__(self, n_users, n_items, n_cates, max_seq_len, max_batch, hp=None, sparse_adam="dense_exact",
                  world_size=1, rank=0, tables=None, model="pamrec", graph=None, emb_dims=EMB_DIMS):
@@ -606,6 +622,40 @@ class Engine:
         if name not in self._frozen_dev:                         # host-side constants: one device copy until set_variables
             self._frozen_dev[name] = torch.from_numpy(self.frozen[name]).to(self.device)
         return self._frozen_dev[name].data_ptr()
+
+    def rank_candidates(self, db, cand_items, cand_cates, top_k, exclude_history=False, want_rank=False):
+        """Score every line of the scoring batch ``db`` against every candidate and keep the best ``top_k`` per line
+        (pamrec_rank_candidates: score descending, then item id ascending; slots past the last candidate hold id -1, score -inf).
+        cand_items / cand_cates: unique item ids in [1, n_items) and their categories (device tensors or arrays).  exclude_history
+        skips the candidates at a real position of a line's history, except the line's own item.  want_rank: also the rank of each
+        line's own item among the candidates (-1 when it is not one).  Overwrites the activation workspace like forward(training=False).
+        Returns a PendingRank."""
+        if self.world != 1 or self.tables != "local":
+            raise PamrecError("rank_candidates runs on one GPU with whole tables")
+        if not 1 <= int(top_k) <= L.RANK_MAX_K:
+            raise PamrecError(f"top_k {top_k} outside [1, {L.RANK_MAX_K}]")
+        as_dev = lambda a: torch.as_tensor(np.asarray(a.cpu() if torch.is_tensor(a) else a, np.int32)).to(self.device).contiguous()
+        items, cates = as_dev(cand_items).reshape(-1), as_dev(cand_cates).reshape(-1)
+        if items.numel() != cates.numel():
+            raise PamrecError(f"{items.numel()} candidate items but {cates.numel()} categories")
+        need = int(self.lib.pamrec_rank_scratch_bytes(self.handle, int(top_k)))
+        if need < 0:
+            self._check(-1)
+        if getattr(self, "_rank_scratch", None) is None or self._rank_scratch.numel() < need:
+            self._rank_scratch = torch.empty(need, dtype=torch.uint8, device=self.device)
+        B, K = db.batch, int(top_k)
+        out = (torch.empty((B, K), dtype=torch.int32, device=self.device), torch.empty((B, K), dtype=torch.float32, device=self.device),
+               torch.empty(B, dtype=torch.int32, device=self.device))
+        ptr = lambda t: C.c_void_p(t.data_ptr())
+        self._check(self.lib.pamrec_rank_candidates(self.handle, C.byref(db.struct), ptr(items), ptr(cates), items.numel(), K,
+                                                    int(bool(exclude_history)), ptr(self._rank_scratch), self._rank_scratch.numel(),
+                                                    ptr(out[0]), ptr(out[1]), ptr(out[2]) if want_rank else None, self._stream()))
+        host = tuple(torch.empty(t.shape, dtype=t.dtype).pin_memory() for t in out)
+        for hst, dev in zip(host, out):
+            hst.copy_(dev, non_blocking=True)
+        event = torch.cuda.Event()
+        event.record(torch.cuda.current_stream(self.device))
+        return PendingRank(host, event, want_rank)
 
     def set_debug(self, flags):
         """Test hooks (include/pamrec_b200.h: PAMREC_DEBUG_*)."""

@@ -20,7 +20,7 @@ import torch
 from . import checkpoint as CK
 from . import dist as D
 from . import summary as SUM
-from .deeprec_utils import cal_metric, cal_weighted_metric, filter_single_class_users, load_dict
+from .deeprec_utils import cal_metric, cal_weighted_metric, filter_single_class_users, full_ranking_metrics, load_dict
 from .engine import Engine, PamrecError
 from .prefetch import Prefetcher
 from .sequential_iterator import LocalFeed
@@ -73,6 +73,32 @@ def initial_variables(shapes, hparams, seed):
                 t = torch.randn(shape, generator=g) * std
         out[name] = t.numpy().astype(np.float32)
     return out
+
+
+# ----------------------------------------------------------------------------- candidate ranking
+def candidate_ids(table, candidates, n_items, source="the file"):
+    """Candidate item ids for ranking: every item with a category in ``table`` (item -> category, -1 = unknown; item 0 never)
+    when ``candidates`` is None, else ``candidates`` checked: non-empty integer ids in [1, n_items), no duplicates, each with a
+    known category.  Raises ValueError otherwise."""
+    table = np.asarray(table)
+    if candidates is None:
+        ids = np.flatnonzero(table >= 0)
+        ids = ids[ids >= 1]
+        if ids.size == 0:
+            raise ValueError("no candidates: {} names no item with a category".format(source))
+        return ids
+    ids = np.asarray(candidates).reshape(-1)
+    if ids.size == 0 or not np.issubdtype(ids.dtype, np.integer):
+        raise ValueError("candidates must be a non-empty list of integer vocabulary ids")
+    ids = ids.astype(np.int64)
+    bad = (ids < 1) | (ids >= n_items)
+    if bad.any():
+        raise ValueError("candidate ids must be in [1, {}): {}".format(n_items, ids[bad][:5].tolist()))
+    if np.unique(ids).size != ids.size:
+        raise ValueError("candidates hold duplicate ids")
+    if (table[ids] < 0).any():
+        raise ValueError("candidates without a category in {}: {}".format(source, ids[table[ids] < 0][:5].tolist()))
+    return ids
 
 
 # ----------------------------------------------------------------------------- checkpoints
@@ -492,6 +518,64 @@ class SequentialBaseModel(BaseModel):
             if wt:
                 wt.close()
         return self
+
+    # ------------------------------------------------------------------ candidate ranking (no reference counterpart)
+    def _ranked(self, filename, top_k, exclude_history, candidates, want_rank, **kw):
+        """(feed, topk_items [B,K], topk_scores [B,K], own_rank [B] or None) per scoring batch of ``filename``, every line ranked
+        against the candidates on the device (Engine.rank_candidates)."""
+        eng = self.engine
+        if eng.world > 1 or (torch.distributed.is_available() and torch.distributed.is_initialized()
+                             and torch.distributed.get_world_size() > 1):
+            raise ValueError("candidate ranking runs on one GPU, not under torch.distributed with several ranks")
+        if not 1 <= int(top_k) <= 1024:
+            raise ValueError("top_k must be between 1 and 1024, not {}".format(top_k))
+        table = self.iterator.item_categories([filename])
+        ids = candidate_ids(table, candidates, eng.dims[1], filename)
+        items = torch.as_tensor(ids.astype(np.int32)).to(eng.device)
+        cates = torch.as_tensor(table[ids].astype(np.int32)).to(eng.device)
+
+        def batches():
+            for feed in self.iterator.load_data_from_file(filename, batch_num_ngs=0, **kw):
+                if feed:
+                    db = eng.upload(feed, training=False, staged=True)
+                    yield (feed,) + eng.rank_candidates(db, items, cates, top_k, exclude_history, want_rank).result()
+        return batches()
+
+    def recommend(self, infile_name, outfile_name, top_k=10, exclude_history=True, candidates=None):
+        """The ``top_k`` items this model ranks first for every line of ``infile_name`` (an evaluation file), scored on the device
+        against the candidates: ``candidates=None`` is every item with a known category in the file, else a list of vocabulary
+        ids.  exclude_history skips the items of the line's history (not its own item).  Writes one line per input line:
+        user key, tab, comma-separated item keys, tab, comma-separated float32 scores (best first; fewer when fewer candidates
+        remain).  Returns dict(users [N] user ids, items [N, K] item ids (-1 past the last), scores [N, K] float32)."""
+        user_key = {v: k for k, v in reversed(list(self.iterator.userdict.items()))}
+        item_key = {v: k for k, v in reversed(list(self.iterator.itemdict.items()))}
+        users, items, scores = [], [], []
+        ranked = self._ranked(infile_name, top_k, exclude_history, candidates, False)
+        with open(outfile_name, "w") as wt:
+            for feed, top_items, top_scores, _ in ranked:
+                u = np.asarray(feed["users"]).reshape(-1).astype(np.int64)
+                for r in range(top_items.shape[0]):
+                    n = int((top_items[r] >= 0).sum())
+                    wt.write("{}\t{}\t{}\n".format(user_key.get(int(u[r]), str(int(u[r]))),
+                                                   ",".join(item_key.get(int(i), str(int(i))) for i in top_items[r, :n]),
+                                                   ",".join(str(x) for x in top_scores[r, :n])))
+                users.append(u)
+                items.append(top_items)
+                scores.append(top_scores)
+        cat = lambda parts, shape, dt: np.concatenate(parts) if parts else np.zeros(shape, dt)
+        return dict(users=cat(users, (0,), np.int64), items=cat(items, (0, top_k), np.int32), scores=cat(scores, (0, top_k), np.float32))
+
+    def run_full_ranking_eval(self, filename, ks=(10,), exclude_history=False, candidates=None):
+        """Full-ranking evaluation: every line with label 1 of ``filename`` ranks its own item against all candidates
+        (``candidates`` as in recommend) on the device; hit@k, ndcg@k and mrr averaged over those lines (deeprec_utils
+        full_ranking_metrics; a positive that is not a candidate counts as a miss)."""
+        ks = tuple(int(k) for k in ks)
+        ranks, labels = [], []
+        for feed, _, _, rank in self._ranked(filename, 1, exclude_history, candidates, True, min_seq_length=self.min_seq_length):
+            ranks.append(rank)
+            labels.append(np.asarray(self._labels_users(feed)[0]).reshape(-1))
+        cat = lambda parts: np.concatenate(parts) if parts else np.zeros(0)
+        return full_ranking_metrics(cat(ranks), cat(labels), ks)
 
 
 class _PendingStep:

@@ -539,6 +539,41 @@ class SequentialIterator:
         }
         return res
 
+    def item_categories(self, files):
+        """Item -> category table [n_items] int32 from the target and history columns of ``files`` (the mode of each file follows
+        its basename, as in load_data_from_file): the first occurrence in file order wins (in an evaluation line the target comes
+        before the history); items that never appear get -1, and so does item 0 (padding / unknown)."""
+        table = np.full(len(self.itemdict), -1, np.int32)
+        for infile in files:
+            train = os.path.basename(infile) == "train_data"
+            col = self._tokenize_native(infile, train)
+            if col is None:
+                self.train = train
+                col = self._flatten(self._lines(infile), train)
+            if col is not None:
+                items, cates = col["items"], col["cates"]
+                if not train:
+                    starts = col["offsets"][:-1]
+                    items, cates = np.insert(items, starts, col["tgt_item"]), np.insert(cates, starts, col["tgt_cate"])
+            else:                                                    # ragged history columns: pairs as far as both go
+                h = 1 if train else 6
+                items, cates = [], []
+                for ln in self._lines(infile):
+                    if not ln:
+                        continue
+                    pairs = ([(ln[3], ln[4])] if not train else []) + list(zip(ln[h], ln[h + 1]))
+                    items.extend(p[0] for p in pairs)
+                    cates.extend(p[1] for p in pairs)
+            items = np.asarray(items, np.int64)
+            ok = (items >= 0) & (items < table.size)
+            items, cates = items[ok], np.asarray(cates, np.int64)[ok]
+            uniq, first = np.unique(items, return_index=True)
+            new = table[uniq] < 0
+            table[uniq[new]] = cates[first[new]]
+        if table.size:
+            table[0] = -1
+        return table
+
     def gen_feed_dict(self, data_dict):
         """IT:1143-1181: identity here — the feed mapping is keyed by placeholder name."""
         return {k: data_dict[k] for k in FEED_KEYS}
