@@ -11,22 +11,100 @@ The head masks are recomputed from the stored pre-activations with the kernels' 
 ``fmaf(gamma, (z - mean) * invstd, beta) > 0`` (kernels_head.cu:bn_relu; the sign of an fma equals the sign of the exact value,
 which float64 reproduces because a product of two float32 is exact in float64).  The point-wise FFN's pattern comes from the
 PAMREC_DEBUG_SAVE_FFN_HIDDEN hook (its pre-activation is never stored)."""
+from typing import NamedTuple
+
 import numpy as np
 
 P_ = "sequential/pamrec/"
-SCORE = P_ + "new_long/score_1/nn_part/"
 TOWERS = ("sequential/logit_fcn", "sequential/valid_logit_fcn", "xilidu_logit_fcn")
+CLSR = "sequential/clsr/"
+
+
+class Mlp(NamedTuple):
+    """One batch-norm MLP of a head (layout.h: MlpOff, bound like api.cu:MlpBind): G members in -> h0 -> h1 (-> 1 when out)."""
+    scopes: tuple         # TF scope of each member
+    k: int                # input columns per member
+    h0: int
+    h1: int
+    out: bool             # a linear output layer follows the second batch norm
+    x: str                # workspace buffer of the input, its row width, first input column of each member
+    ldx: int
+    x_col: tuple
+    z: tuple              # per layer: pre-activations (the output layer's logits), all members side by side
+    dz: tuple             # per layer: the gradient buffer of that layer
+    dx: str               # gradient of the input (members reading the same columns add up)
+    bn: tuple             # batch-norm sets of layers 0 and 1 ("bn.<set>.*")
+    tokens: bool          # rows are B * T tokens (else B samples)
+
+    def layers(self):
+        return 3 if self.out else 2
+
+    def k_of(self, l):
+        return (self.k, self.h0, self.h1)[l]
+
+    def n_of(self, l):
+        return (self.h0, self.h1, 1)[l]
+
+    def bn_scope(self, m, l):
+        return self.scopes[m] + "/nn_part/batch_normalization" + ("_1" if l else "")
+
+
+# PAMRec (api.cu:head_mlps): the attention-pooling score, experts and gates on new_long, towers on main | target, sub | target, main | target
+HEAD_MLPS = {
+    "score": Mlp((P_ + "new_long/score_1",), 40, 20, 1, False, "blk1.out", 40, (0,), ("z1", "z2"), ("d_a1", "d_z2"), "g_a",
+                 ("s0", "s1"), True),
+    "expert": Mlp(tuple(f"{P_}expert_{j}" for j in range(5)), 40, 100, 64, False, "new_long", 40, (0,) * 5, ("ze0", "ze1"),
+                  ("d_e0", "d_e1"), "d_new_long", ("e0", "e1"), False),
+    "gate": Mlp((P_ + "gate_main", P_ + "gate_sub"), 40, 64, 5, False, "new_long", 40, (0, 0), ("zg0", "zg1"), ("d_g0", "d_g1"),
+                "d_new_long", ("g0", "g1"), False),
+    "tower": Mlp(TOWERS, 84, 100, 64, True, "u", 168, (0, 84, 0), ("zt0", "zt1", "logits"), ("d_t0", "d_t1", "d_logits"), "d_u",
+                 ("t0", "t1"), False),
+}
+
+
+def expert_scopes(model):
+    if model == "mmoe":
+        return [f"{CLSR}expert_{j}" for j in range(5)]
+    if model == "ple":
+        return [f"{CLSR}share_expert_{j}" for j in range(3)] + [f"{CLSR}main_expert_{j}" for j in range(2)] + [f"{CLSR}sub_expert_{j}" for j in range(2)]
+    return []
+
+
+def sibling_mlps(model, E):
+    """MMoE / PLE / share-bottom at token width E = item + cate (api_sibling.inl:sib_mlps): att_fcn of both DIN branches on their
+    feature rows, experts and gates on x = long | short | target, the towers on main | target, sub | target (share-bottom: x, x)."""
+    towers = ("sequential/logit_fcn", "sequential/valid_logit_fcn")
+    att = tuple(f"{CLSR}{b}/attention_fcn/att_fcn" for b in ("long_term", "short_term"))
+    out = {"att": Mlp(att, 4 * E, 80, 40, True, "sib.feat", 8 * E, (0, 4 * E), ("z1", "z2", "sib.score"),
+                      ("sib.d_a0", "sib.d_a1", "sib.d_score"), "sib.d_feat", ("s0", "s1"), True)}
+    ex = tuple(expert_scopes(model))
+    if ex:
+        out["expert"] = Mlp(ex, 3 * E, 100, 64, False, "x", 3 * E, (0,) * len(ex), ("ze0", "ze1"), ("d_e0", "d_e1"), "d_x", ("e0", "e1"), False)
+        out["gate"] = Mlp((CLSR + "gate_main", CLSR + "gate_sub"), 3 * E, 64, 5, False, "x", 3 * E, (0, 0), ("zg0", "zg1"), ("d_g0", "d_g1"),
+                          "d_x", ("g0", "g1"), False)
+        ti = 64 + E
+        out["tower"] = Mlp(towers, ti, 100, 64, True, "u", 2 * ti, (0, ti), ("zt0", "zt1", "logits"), ("d_t0", "d_t1", "d_logits"), "d_u",
+                           ("t0", "t1"), False)
+    else:
+        out["tower"] = Mlp(towers, 3 * E, 100, 64, True, "x", 3 * E, (0, 0), ("zt0", "zt1", "logits"), ("d_t0", "d_t1", "d_logits"), "d_x",
+                           ("t0", "t1"), False)
+    return out
+
+
+def sas_mlps(E):
+    """SASRec's tower on final state | target (api_sibling.inl:sas_tower)."""
+    return {"tower": Mlp(("sequential/logit_fcn",), 2 * E, 100, 64, True, "u", 2 * E, (0,), ("zt0", "zt1", "logits"),
+                         ("d_t0", "d_t1", "d_logits"), "d_u", ("t0", "t1"), False)}
+
+
+def bn_layers(mlps):
+    """(pre-activation buffer, BN set, columns per member, member BN scopes, rows are tokens) of every batch norm of `mlps`."""
+    return [(m.z[l], m.bn[l], m.n_of(l), [m.bn_scope(i, l) for i in range(len(m.scopes))], m.tokens)
+            for m in mlps.values() for l in (0, 1)]
+
+
 # engine pre-activation buffer, BN set, columns per member, member scopes (oracle key = scope)
-HEAD_BN = [
-    ("ze0", "e0", 100, [f"{P_}expert_{j}/nn_part/batch_normalization" for j in range(5)]),
-    ("ze1", "e1", 64, [f"{P_}expert_{j}/nn_part/batch_normalization_1" for j in range(5)]),
-    ("zg0", "g0", 64, [f"{P_}gate_{g}/nn_part/batch_normalization" for g in ("main", "sub")]),
-    ("zg1", "g1", 5, [f"{P_}gate_{g}/nn_part/batch_normalization_1" for g in ("main", "sub")]),
-    ("zt0", "t0", 100, [s + "/nn_part/batch_normalization" for s in TOWERS]),
-    ("zt1", "t1", 64, [s + "/nn_part/batch_normalization_1" for s in TOWERS]),
-    ("z1", "s0", 20, [SCORE + "batch_normalization"]),
-    ("z2", "s1", 1, [SCORE + "batch_normalization_1"]),
-]
+HEAD_BN = [b[:4] for b in bn_layers(HEAD_MLPS)]
 
 
 def _on(z, stat, gamma, beta):

@@ -8,6 +8,7 @@ import torch
 
 from oracle import pamrec_oracle as O
 from oracle import siblings_oracle as S
+from relu_masks import bn_layers, expert_scopes, sibling_mlps
 
 pytestmark = pytest.mark.gpu
 
@@ -35,14 +36,6 @@ def _close(name, got, ref, rtol=RTOL, report=None):
 def _expect(cond, msg):
     if not cond:
         FAILS.append(str(msg))
-
-
-def expert_scopes(model):
-    if model == "mmoe":
-        return [f"{CLSR}expert_{j}" for j in range(5)]
-    if model == "ple":
-        return [f"{CLSR}share_expert_{j}" for j in range(3)] + [f"{CLSR}main_expert_{j}" for j in range(2)] + [f"{CLSR}sub_expert_{j}" for j in range(2)]
-    return []
 
 
 def _setup(model, nu, ni, nc, T, B, seed):
@@ -80,21 +73,10 @@ def _on(z, stat, gamma, beta):
 
 
 def sibling_relu_masks(eng, model, B, T):
-    ex = expert_scopes(model)
-    att = [f"{CLSR}{b}/attention_fcn/att_fcn" for b in ("long_term", "short_term")]
-    towers = ["sequential/logit_fcn", "sequential/valid_logit_fcn"]
-    gates = [CLSR + "gate_main", CLSR + "gate_sub"]
-    table = [("z1", "s0", 80, [s + "/nn_part/batch_normalization" for s in att], B * T, (B, T)),
-             ("z2", "s1", 40, [s + "/nn_part/batch_normalization_1" for s in att], B * T, (B, T)),
-             ("zt0", "t0", 100, [s + "/nn_part/batch_normalization" for s in towers], B, (B,)),
-             ("zt1", "t1", 64, [s + "/nn_part/batch_normalization_1" for s in towers], B, (B,))]
-    if ex:
-        table += [("ze0", "e0", 100, [s + "/nn_part/batch_normalization" for s in ex], B, (B,)),
-                  ("ze1", "e1", 64, [s + "/nn_part/batch_normalization_1" for s in ex], B, (B,)),
-                  ("zg0", "g0", 64, [s + "/nn_part/batch_normalization" for s in gates], B, (B,)),
-                  ("zg1", "g1", 5, [s + "/nn_part/batch_normalization_1" for s in gates], B, (B,))]
+    """Masks of the last training forward, keyed by BN scope, for every batch norm of the model's MLPs (relu_masks.sibling_mlps)."""
     out = {}
-    for zbuf, bn, width, scopes, rows, lead in table:
+    for zbuf, bn, width, scopes, tokens in bn_layers(sibling_mlps(model, sum(eng.emb_dims[:2]))):
+        rows, lead = (B * T, (B, T)) if tokens else (B, (B,))
         z = eng.ws(zbuf, rows).cpu().numpy().reshape(rows, len(scopes) * width)
         st = eng.ws(f"bn.{bn}.stat").cpu().numpy()
         for m, scope in enumerate(scopes):
