@@ -200,6 +200,24 @@ int pamrec_rank_candidates(PamrecHandle h, const PamrecBatch* lines, const int32
                            int32_t top_k, int32_t exclude_history, void* scratch, int64_t scratch_bytes, int32_t* topk_items,
                            float* topk_scores, int32_t* own_rank, void* stream);
 
+/* Attention weights behind each score.  Runs the scoring forward pass on `b` exactly as pamrec_forward(training = 0) does and
+ * writes, all in device memory:
+ *   pred_out [batch]        the scores, bit-identical to what pamrec_forward(training = 0) writes;
+ *   pool_out [batch][P][T]  the read-out weights over the history (required).  PAMRec (P = 1): the attention-pooling weights a_t
+ *                           (pamrec.py:272-282).  MMoE_original / PLE / ShareBottom (P = 2): slot 0 the branch over the satisfied-
+ *                           only history (satisfied_mask), slot 1 the branch over the full history (mask).  Both are the values the
+ *                           forward pass multiplied with.  SASRec (P = 1): the attention row of encoder block 1 at the position the
+ *                           tower reads (length - 1 of satisfied_mask; row 0 when the line has no satisfied item), equal bit for bit
+ *                           to that row of maps_out;
+ *   maps_out [batch][2][T][T] (nullable) the softmax probabilities of each encoder block, query row by key column, for every query
+ *                           row the forward computes (padded ones included).  PAMRec and SASRec only: a DIN sibling model given a
+ *                           non-null maps_out fails.  Recomputed from the saved queries, keys and softmax row statistics (m, l) as
+ *                           exp(s - m) / l over the live keys.
+ * A masked key weighs exactly 0 when its line has any live key; a line without live keys gets 1 / T everywhere.  One GPU with whole
+ * tables.  The call overwrites the activation workspace like pamrec_forward(training = 0): never between the forward and the
+ * backward pass of a training step. */
+int pamrec_attention(PamrecHandle h, const PamrecBatch* b, float* pred_out, float* pool_out, float* maps_out, void* stream);
+
 /* Multi-GPU plumbing.  The library talks to NCCL directly (dlopen of the libnccl.so.2 that PyTorch ships;
  * `nccl_path` may be NULL to use the loader's search path).  Rank 0 creates the unique id, the host broadcasts
  * the 128 bytes (torch.distributed), every rank calls pamrec_comm_init; afterwards forward / backward /

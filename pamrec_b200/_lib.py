@@ -100,6 +100,7 @@ EXPORTS = {
     "pamrec_rank_scratch_bytes": (C.c_int64, [C.c_void_p, C.c_int32]),
     "pamrec_rank_candidates": (C.c_int, [C.c_void_p, C.POINTER(PamrecBatch), C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,
                                          C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "pamrec_attention": (C.c_int, [C.c_void_p, C.POINTER(PamrecBatch), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "pamrec_bench_gather": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32,
                                       C.c_void_p, C.c_void_p]),
     "pamrec_bench_table_adam": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p]),

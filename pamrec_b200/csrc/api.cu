@@ -713,7 +713,8 @@ static int sib_backward(PamrecHandle h, const PamrecBatch* b, cudaStream_t st);
 static int sib_apply(PamrecHandle h, const PamrecBatch* b, int64_t step, cudaStream_t st);
 static int sas_forward(PamrecHandle h, const PamrecBatch* b, int training, float* pred_out, cudaStream_t st);
 static int sas_backward(PamrecHandle h, const PamrecBatch* b, cudaStream_t st);
-static int head_forward(PamrecHandle h, const PamrecBatch* b, bool training, float* pred_out, cudaStream_t st);
+static int head_forward(PamrecHandle h, const PamrecBatch* b, bool training, float* pred_out, float* aw_out, cudaStream_t st);
+static int pam_forward(PamrecHandle h, const PamrecBatch* b, int training, float* pred_out, bool keep_aw, cudaStream_t st);
 
 int pamrec_forward(PamrecHandle h, const PamrecBatch* b, int training, float* pred_out, void* stream) {
   if (int rc = check_batch(h, b, training != 0)) return rc;
@@ -721,6 +722,11 @@ int pamrec_forward(PamrecHandle h, const PamrecBatch* b, int training, float* pr
   cudaStream_t st = (cudaStream_t)stream;
   if (h->cfg.model_kind == PAMREC_MODEL_SASREC) return sas_forward(h, b, training, pred_out, st);
   if (h->sibling()) return sib_forward(h, b, training, pred_out, st);
+  return pam_forward(h, b, training, pred_out, false, st);
+}
+
+// PAMRec's forward pass; keep_aw (scoring, pamrec_attention): the head also leaves the pooling weights in "pool.aw"
+static int pam_forward(PamrecHandle h, const PamrecBatch* b, int training, float* pred_out, bool keep_aw, cudaStream_t st) {
   const Layout& L = h->L;
   const int B = b->batch, T = h->cfg.max_seq_len, N = B * T;
   float* x0 = h->wf("x0");
@@ -772,8 +778,9 @@ int pamrec_forward(PamrecHandle h, const PamrecBatch* b, int training, float* pr
     // the whole head as ONE persistent cooperative kernel, row-stationary (kernels_head2.cu)
     HeadDyn d = head_dyn(h, b, training != 0, 0);
     d.pred = pred_out;
+    d.keep_aw = keep_aw ? 1 : 0;
     if (launch_head2_fwd(h->head2, d, h->head2_grid, training ? "head_fwd" : "head_score", st)) return check_cuda(h, "cooperative head launch");
-  } else if (int rc = head_forward(h, b, training != 0, pred_out, st)) {
+  } else if (int rc = head_forward(h, b, training != 0, pred_out, keep_aw ? h->wf("pool.aw") : nullptr, st)) {
     return rc;
   }
   return check_cuda(h, "forward");
@@ -781,7 +788,8 @@ int pamrec_forward(PamrecHandle h, const PamrecBatch* b, int training, float* pr
 
 // The stand-alone head (kernels_head.cu): a launch per layer.  Training: batch statistics of the listed sets -> (mean, invstd), moving
 // averages; data parallel: the column sums (plus, once, the listwise-group count) are first summed over the ranks by NCCL.
-static int head_forward(PamrecHandle h, const PamrecBatch* b, bool training, float* pred_out, cudaStream_t st) {
+// aw_out (nullable): the pooling weights are also written there.
+static int head_forward(PamrecHandle h, const PamrecBatch* b, bool training, float* pred_out, float* aw_out, cudaStream_t st) {
   const int B = b->batch, T = h->cfg.max_seq_len;
   const int W = h->cfg.world_size;
   int crc = 0;
@@ -806,7 +814,7 @@ static int head_forward(PamrecHandle h, const PamrecBatch* b, bool training, flo
   }
   const HeadMlps m = head_mlps(h, b);
   mlp_forward(h, {&m.score}, training, sync_sums, st);
-  launch_pool_fwd(h->wf("blk1.out"), h->wf("z2"), bn[BN_S1], b->mask, h->wf("new_long"), B, T, st);
+  launch_pool_fwd(h->wf("blk1.out"), h->wf("z2"), bn[BN_S1], b->mask, h->wf("new_long"), aw_out, B, T, st);
   mlp_forward(h, {&m.expert, &m.gate}, training, sync_sums, st);
   launch_combine_fwd(h->wf("ze1"), h->wf("zg1"), bn[BN_E1], bn[BN_G1], h->wf("tgt"), h->wf("u"), B, st);
   mlp_forward(h, {&m.tower}, training, sync_sums, st);
@@ -1135,6 +1143,7 @@ int pamrec_apply_gradients(PamrecHandle h, const PamrecBatch* b, int64_t step, v
 
 #include "api_sibling.inl"
 #include "api_rank.inl"
+#include "api_attn.inl"
 
 int pamrec_train_step(PamrecHandle h, const PamrecBatch* b, int64_t step, float* losses_out, void* stream) {
   if (!h) return -1;

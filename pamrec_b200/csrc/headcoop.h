@@ -16,6 +16,7 @@ struct HeadDyn {
   unsigned long long* trace;                        // [32] %globaltimer of the kernel start ([31]) and of every barrier release; may be null
   float* pred;                                      // scoring (row-stationary kernels): sigmoid(logit 0) per row, or null
   unsigned long long* trace_cta;                    // debug: [16 barriers][256 CTAs] %globaltimer of every CTA's arrival; may be null
+  int keep_aw;                                      // scoring: also keep the pooling weights in pool.aw (pamrec_attention); 0 elsewhere
 };
 
 }  // namespace pamrec

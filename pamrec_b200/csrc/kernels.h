@@ -82,7 +82,8 @@ void launch_dense_dw(const DenseDwP& p, cudaStream_t st);
 void launch_bn_finalize(const BnSet& s, double count, cudaStream_t st);   // training: sums -> stat, moving update, sums := 0
 void launch_bn_eval_stat(const BnSet& s, cudaStream_t st);                // inference: stat from moving stats
 void launch_bn_bwd_stats(const BnSet& s, const float* dA, const float* Z, int M, cudaStream_t st);
-void launch_pool_fwd(const float* H, const float* Z2, const BnSet& s1, const int* mask, float* new_long, int B, int T,
+// aw_out (nullable): also the pooling weights [B, T] (pamrec_attention)
+void launch_pool_fwd(const float* H, const float* Z2, const BnSet& s1, const int* mask, float* new_long, float* aw_out, int B, int T,
                      cudaStream_t st);
 void launch_pool_bwd(const float* H, const float* Z2, const BnSet& s1, const int* mask, const float* d_new_long, float* dA2,
                      float* dH, int B, int T, cudaStream_t st);
@@ -231,6 +232,18 @@ void launch_rank_tower_in(const float* U_lines, const int* cand_items, const int
 void launch_rank_merge(const RankMerge& a, int n_lines, cudaStream_t st);
 void launch_rank_finish(const int* own_items, const float* own_scores, const int* map, const int* count, int n_items, int B, int* own_rank,
                         int* flags, cudaStream_t st);
+
+// ---- kernels_attn_map.cu (pamrec_attention): the encoder's softmax probabilities, recomputed from the saved queries, keys and row
+// statistics (m, l) of the forward pass: P[q, k] = exp(s_qk - m_q) / l_q over the live keys, 0 on a masked key, 1 / l_q (= 1 / T)
+// everywhere in a sample without live keys.  PAMRec: Q / K [B*T, 40] per block (ld 40), key live when mask != 0; SASRec: the qkv
+// rows (ld 3 S, K at column S), key live when satisfied_mask == 1.  maps (nullable): [B][2][T][T]; pool (SASRec, nullable): block 1's
+// row at the position the tower reads (k_sas_final_fwd), [B][T].  With maps null only that row is computed.
+struct AttnMapArgs {
+  const float* Q[2]; const float* K[2]; const float* ML[2]; int ld;
+  const int* mask; float* maps; float* pool;
+  int B, T;
+};
+void launch_attn_maps(const AttnMapArgs& a, int S, bool sasrec, cudaStream_t st);
 
 // ---- kernels_p2p.cu + kernels_head2.cu (data-parallel exchanges through NVLink peer mailboxes)
 constexpr int kP2PMaxDoubles = 2048;     // payload capacity of one mailbox slot (expert + gate layer-0 sums: 1256)

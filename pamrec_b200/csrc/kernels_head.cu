@@ -153,7 +153,8 @@ __device__ __forceinline__ void pool_weights(const float* __restrict__ Z2, const
 }
 
 __global__ void __launch_bounds__(128) k_pool_fwd(const float* __restrict__ H, const float* __restrict__ Z2, BnSet s1,
-                                                  const int* __restrict__ mask, float* __restrict__ new_long, int B, int T) {
+                                                  const int* __restrict__ mask, float* __restrict__ new_long, float* __restrict__ aw_out,
+                                                  int B, int T) {
   __shared__ float aws[4][PAMREC_MAX_T];
   const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int b = blockIdx.x * 4 + w;
@@ -161,6 +162,7 @@ __global__ void __launch_bounds__(128) k_pool_fwd(const float* __restrict__ H, c
   const int64_t base = (int64_t)b * T;
   float* aw = aws[w];
   pool_weights(Z2, s1, mask, base, T, lane, aw);
+  if (aw_out) for (int t = lane; t < T; t += 32) aw_out[base + t] = aw[t];
   const int tg = lane / 10, c = lane % 10;
   float4 acc = f4_zero();
   if (lane < 30)
@@ -171,10 +173,10 @@ __global__ void __launch_bounds__(128) k_pool_fwd(const float* __restrict__ H, c
     st4(new_long + (int64_t)b * kD + 4 * c, acc);
   }
 }
-void launch_pool_fwd(const float* H, const float* Z2, const BnSet& s1, const int* mask, float* new_long, int B, int T,
+void launch_pool_fwd(const float* H, const float* Z2, const BnSet& s1, const int* mask, float* new_long, float* aw_out, int B, int T,
                      cudaStream_t st) { PAMREC_PROF("pool_fwd", 1, st);
   if (B == 0) return;
-  k_pool_fwd<<<(B + 3) / 4, 128, 0, st>>>(H, Z2, s1, mask, new_long, B, T);
+  k_pool_fwd<<<(B + 3) / 4, 128, 0, st>>>(H, Z2, s1, mask, new_long, aw_out, B, T);
 }
 
 // backward of the pooling: dA2[b,t] = grad wrt s_t (post-ReLU score), dH[b,t,:] = a_t * d_new_long[b,:]

@@ -693,7 +693,7 @@ __global__ void __launch_bounds__(kT2, 1) k_head2_fwd(const __grid_constant__ He
         acc.x += a1.x + a2.x; acc.y += a1.y + a2.y; acc.z += a1.z + a2.z; acc.w += a1.w + a2.w;
         st4(h.new_long + (int64_t)b * kD + 4 * c, acc);
       }
-      if (train) for (int t = lane; t < T; t += 32) h.aw[base + t] = aw[t];   // kept for the backward pass
+      if (train || d.keep_aw) for (int t = lane; t < T; t += 32) h.aw[base + t] = aw[t];   // kept for the backward pass / pamrec_attention
       __syncwarp();
     }
     __syncthreads();

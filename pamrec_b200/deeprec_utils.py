@@ -277,6 +277,20 @@ def own_rank(scores, ids, own, keep=None):
     return out
 
 
+def attention_topk(weights, live, top_k):
+    """The ``top_k`` largest weights of each row of weights [n, T] among its live positions (live [n, T] true), ordered by weight
+    descending, then position ascending.  Returns (positions [n, top_k] int64 with -1 past the last live position, weights
+    [n, top_k] float32 with 0 there)."""
+    w = np.asarray(weights, np.float32)
+    live = np.asarray(live, bool)
+    n, T = w.shape
+    pos = np.broadcast_to(np.arange(T), (n, T))
+    key = np.where(live, -w.astype(np.float64), np.inf)               # dead positions sort last
+    order = np.lexsort((pos, key), axis=-1)[:, :top_k]
+    ok = np.take_along_axis(live, order, -1)
+    return np.where(ok, order, -1).astype(np.int64), np.where(ok, np.take_along_axis(w, order, -1), 0.0).astype(np.float32)
+
+
 def full_ranking_metrics(ranks, labels, ks=(10,)):
     """Full-catalogue ranking metrics over the lines with label 1: hit@k (rank <= k), ndcg@k (1 / log2(rank + 1) when rank <= k,
     else 0) and mrr (1 / rank).  A rank < 1 (the positive is not a candidate) counts as a miss in every metric.  Rounded to 4

@@ -132,6 +132,23 @@ class PendingRank:
         return self._value
 
 
+class PendingAttention:
+    """Engine.attention: ``result()`` waits for the device->host copies and gives dict(pred [B] float32, pool [B, P, T] float32,
+    maps [B, 2, T, T] float32 or None)."""
+
+    def __init__(self, host, event):
+        self._host, self._event, self._value = host, event, None
+
+    def result(self):
+        if self._value is None:
+            self._event.synchronize()
+            pred, pool, maps = self._host
+            # the pinned buffers belong to this result alone: handed out without a further host copy
+            self._value = dict(pred=pred.numpy(), pool=pool.numpy(), maps=None if maps is None else maps.numpy())
+            self._host = None
+        return self._value
+
+
 class Engine:
     def __init__(self, n_users, n_items, n_cates, max_seq_len, max_batch, hp=None, sparse_adam="dense_exact",
                  world_size=1, rank=0, tables=None, model="pamrec", graph=None, emb_dims=EMB_DIMS):
@@ -656,6 +673,31 @@ class Engine:
         event = torch.cuda.Event()
         event.record(torch.cuda.current_stream(self.device))
         return PendingRank(host, event, want_rank)
+
+    def attention(self, db, maps=False):
+        """The attention weights behind each score of the scoring batch ``db`` (pamrec_attention): the forward pass runs as in
+        forward(training=False), whose predictions ``pred`` it also returns bit for bit.  ``pool`` [B, P, T]: the read-out weights
+        over the history (PAMRec: its pooling weights, P = 1; MMoE / PLE / share-bottom: slot 0 the satisfied-only branch, slot 1
+        the full-history branch; SASRec: block 1's attention row at the position its tower reads, P = 1).  maps=True (PAMRec and
+        SASRec): also the softmax probabilities of both encoder blocks, [B, 2, T, T] (query row, key column).  One GPU with whole
+        tables; overwrites the activation workspace like forward(training=False).  Returns a PendingAttention."""
+        if self.world != 1 or self.tables != "local":
+            raise PamrecError("attention runs on one GPU with whole tables")
+        if maps and self.model not in ("pamrec", "sasrec"):
+            raise PamrecError(f"attention maps: {self.model} has no self-attention encoder")
+        B, T = db.batch, self.dims[3]
+        P = 2 if self.model in ("mmoe", "ple", "sharebottom") else 1
+        f32 = lambda *shape: torch.empty(shape, dtype=torch.float32, device=self.device)
+        out = (f32(B), f32(B, P, T), f32(B, 2, T, T) if maps else None)
+        ptr = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
+        self._check(self.lib.pamrec_attention(self.handle, C.byref(db.struct), ptr(out[0]), ptr(out[1]), ptr(out[2]), self._stream()))
+        host = tuple(None if t is None else torch.empty(t.shape, dtype=t.dtype, pin_memory=True) for t in out)
+        for hst, dev in zip(host, out):
+            if dev is not None:
+                hst.copy_(dev, non_blocking=True)
+        event = torch.cuda.Event()
+        event.record(torch.cuda.current_stream(self.device))
+        return PendingAttention(host, event)
 
     def set_debug(self, flags):
         """Test hooks (include/pamrec_b200.h: PAMREC_DEBUG_*)."""

@@ -20,7 +20,7 @@ import torch
 from . import checkpoint as CK
 from . import dist as D
 from . import summary as SUM
-from .deeprec_utils import cal_metric, cal_weighted_metric, filter_single_class_users, full_ranking_metrics, load_dict
+from .deeprec_utils import attention_topk, cal_metric, cal_weighted_metric, filter_single_class_users, full_ranking_metrics, load_dict
 from .engine import Engine, PamrecError
 from .prefetch import Prefetcher
 from .sequential_iterator import LocalFeed
@@ -99,6 +99,14 @@ def candidate_ids(table, candidates, n_items, source="the file"):
     if (table[ids] < 0).any():
         raise ValueError("candidates without a category in {}: {}".format(source, ids[table[ids] < 0][:5].tolist()))
     return ids
+
+
+def attention_line(user, pred, items, weights, item_key):
+    """One line of explain(): user key, tab, the prediction, then per pooling slot a tab and the comma-separated ``item_key:weight``
+    entries of items [P, K] / weights [P, K] (entries with item -1 are left out).  Floats are written as str() of their float32."""
+    cols = [",".join("{}:{}".format(item_key.get(int(i), str(int(i))), np.float32(w)) for i, w in zip(items[s], weights[s]) if i >= 0)
+            for s in range(len(items))]
+    return "\t".join([str(user), str(np.float32(pred))] + cols)
 
 
 # ----------------------------------------------------------------------------- checkpoints
@@ -577,6 +585,61 @@ class SequentialBaseModel(BaseModel):
         cat = lambda parts: np.concatenate(parts) if parts else np.zeros(0)
         return full_ranking_metrics(cat(ranks), cat(labels), ks)
 
+    # ------------------------------------------------------------------ attention weights (no reference counterpart)
+    # per pooling slot: the history columns its weights index (PAMRec: the full history; the DIN siblings: satisfied-only, then
+    # full; SASRec: its satisfied-only input)
+    ATTENTION_SLOTS = (("item_history", "mask"),)
+
+    def explain(self, infile_name, outfile_name, top_k=5, maps=False):
+        """The attention weights behind every score of ``infile_name`` (a scoring file, read as predict reads it), computed on the
+        device by the forward pass that scores the line (Engine.attention).  Writes one line per input line: user key, tab, the
+        prediction, then per pooling slot a tab and up to ``top_k`` comma-separated ``item_key:weight`` entries over the line's real
+        history positions (mask > 0), by weight descending, then position ascending.  maps=True (PAMRec, SASRec) also returns the
+        encoder's attention maps.  Returns dict(users [N], pred [N] float32, pool [N, P, T] float32, positions [N, P, top_k] (indices
+        into the slot's history, -1 past the last), items [N, P, top_k] (-1 there), weights [N, P, top_k] float32 (0 there),
+        maps [N, 2, T, T] float32 or None).  maps=True holds the maps of every line of the file in host memory: N x 2 x T x T x 4
+        bytes (32 GB for 100 000 lines at T = 200, twice that while the batches are joined at the end); for a large file call
+        Engine.attention per batch instead."""
+        eng = self.engine
+        T = eng.dims[3]
+        if eng.world > 1 or (torch.distributed.is_available() and torch.distributed.is_initialized()
+                             and torch.distributed.get_world_size() > 1):
+            raise ValueError("explain runs on one GPU, not under torch.distributed with several ranks")
+        if not isinstance(top_k, (int, np.integer)) or not 1 <= int(top_k) <= T:
+            raise ValueError("top_k must be between 1 and max_seq_length ({}), not {}".format(T, top_k))
+        if maps and eng.model not in ("pamrec", "sasrec"):
+            raise ValueError("attention maps need a self-attention encoder (PAMRec, SASRec), not {}".format(eng.model))
+        top_k = int(top_k)
+        user_key = {v: k for k, v in reversed(list(self.iterator.userdict.items()))}
+        item_key = {v: k for k, v in reversed(list(self.iterator.itemdict.items()))}
+        parts = {k: [] for k in ("users", "pred", "pool", "positions", "items", "weights", "maps")}
+        with open(outfile_name, "w") as wt:
+            for feed in self.iterator.load_data_from_file(infile_name, batch_num_ngs=0):
+                if not feed:
+                    continue
+                got = eng.attention(eng.upload(feed, training=False, staged=True), maps=maps).result()
+                B = got["pred"].shape[0]
+                u = np.asarray(feed["users"]).reshape(-1).astype(np.int64)
+                pos, wts, its = [], [], []
+                for slot, (hist, mask) in enumerate(self.ATTENTION_SLOTS):
+                    h = np.asarray(feed[hist]).reshape(B, T)
+                    p, w = attention_topk(got["pool"][:, slot], np.asarray(feed[mask]).reshape(B, T) > 0, top_k)
+                    pos.append(p)
+                    wts.append(w)
+                    its.append(np.where(p >= 0, np.take_along_axis(h, np.maximum(p, 0), -1), -1))
+                pos, wts, its = np.stack(pos, 1), np.stack(wts, 1), np.stack(its, 1)
+                for r in range(B):
+                    wt.write(attention_line(user_key.get(int(u[r]), str(int(u[r]))), got["pred"][r], its[r], wts[r], item_key) + "\n")
+                for k, v in (("users", u), ("pred", got["pred"]), ("pool", got["pool"]), ("positions", pos), ("items", its),
+                             ("weights", wts), ("maps", got["maps"])):
+                    parts[k].append(v)
+        P = len(self.ATTENTION_SLOTS)
+        empty = dict(users=((0,), np.int64), pred=((0,), np.float32), pool=((0, P, T), np.float32), positions=((0, P, top_k), np.int64),
+                     items=((0, P, top_k), np.int64), weights=((0, P, top_k), np.float32), maps=((0, 2, T, T), np.float32))
+        out = {k: np.concatenate(v) if v else np.zeros(*empty[k]) for k, v in parts.items() if k != "maps"}
+        out["maps"] = (np.concatenate(parts["maps"]) if parts["maps"] else np.zeros(*empty["maps"])) if maps else None
+        return out
+
 
 class _PendingStep:
     """A queued train step: ``result()`` gives train()'s tuple (update, extra_update_ops, <one float per loss name>, summary).
@@ -702,6 +765,7 @@ class _DinMultiTask(PAMRECModel):
     20 or 40; the kernels are compiled for both item / cate pairs."""
 
     SCALARS = ("loss", "data_loss", "regular_loss", "auxiliary_data_loss")                  # MM:341-373
+    ATTENTION_SLOTS = (("satisfied_item_history", "satisfied_mask"), ("item_history", "mask"))
 
     def _check_supported(self, hp):
         super()._check_supported(hp)
@@ -757,6 +821,7 @@ class SASRecModel(_DinMultiTask):
     5-tuple (update, extra_update_ops, loss, data_loss, summary) (BM:350-372)."""
     ENGINE_MODEL = "sasrec"
     SCALARS = ("loss", "data_loss")                                                        # BM:350-372
+    ATTENTION_SLOTS = (("satisfied_item_history", "satisfied_mask"),)
 
     def _check_mixing(self, hp, need):
         pass
